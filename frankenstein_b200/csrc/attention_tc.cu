@@ -1,4 +1,5 @@
-// Attention backward on the 5th-gen tensor cores (tcgen05.mma + TMEM + TMA), head_dim 32, label masks.
+// Attention backward on the 5th-gen tensor cores (tcgen05.mma + TMEM + TMA), head_dim 32, label masks.  The head_dim-64
+// variants of the forward and backward kernels follow the head_dim-32 ones at the end of the file.
 //
 // Same math and mask rule as attention.cu (reference: F.scaled_dot_product_attention backward at
 // models/brainformer.py:168), restructured for Blackwell: every matmul is a tcgen05.mma issued by one thread,
@@ -1389,6 +1390,868 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
   }
 }
 
+// ================================================================================================
+// head_dim 64.  Same work split, label-mask / tile-skip rules, persistent hand-out and softmax as the head_dim-32 kernels
+// above (which stay as they are); [tokens][64] bf16 rows are 128 B, so every tile is TMA-loaded with the 128-byte swizzle.
+//
+// Backward (attn_bwd_tc64_kernel): three score stages (3 x 128 columns) + dV 64 + dK / dQ 64 fill the 512 TMEM columns, so
+// the resident tiles cannot sit in TMEM as at head_dim 32: the score MMAs read both operands from shared memory (SS mode,
+// 4 K steps of 16 + the folded statistics step).  P / dS are still written in place over the consumed score columns and
+// read by the accumulate MMAs from TMEM (TS mode, N = 64, B operand MN-major straight from the streamed tile).  One path
+// only: statistics folded (fk_attn_aug), MN-major accumulate operands.
+// ================================================================================================
+constexpr int kNST64 = 6;                     // streamed stages: tile A 8 KB | tile B 8 KB | statistics rows 2 KB (DKV)
+constexpr int kStage64 = 18432;
+constexpr int kAcc64 = 128 * kNG;             // 384: dV (64 columns), 448: dK / dQ (64 columns)
+
+struct TcSmem64 {
+  static constexpr int resA = 0;                                  // 2 buffers x [128][64] bf16 (16 KB each)
+  static constexpr int resB = 32768;
+  static constexpr int stream = 65536;
+  static constexpr int ids = stream + kNST64 * kStage64;         // [kNG wg][2 buffers][64] int column labels
+  static constexpr int tiles = ids + kNG * 2 * 64 * 4;           // two uint16 visible-tile lists
+  static constexpr int ones = (tiles + 2 * kMaxTiles * 2 + 1023) / 1024 * 1024;   // [2][128][16] bf16, SWIZZLE_32B
+  static constexpr int aug_res = ones + 8192;                    // DQ: 2 buffers x [128][16] statistics rows
+  static constexpr int bars = aug_res + 8192;
+  static constexpr int total = bars + 512;
+};
+static_assert(TcSmem64::total <= 232448, "attn_bwd_tc64_kernel: shared memory");
+
+template <int MODE>
+__global__ void __launch_bounds__(kTcThreads, 1)
+attn_bwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_constant__ CUtensorMap tm_resB,
+                     const __grid_constant__ CUtensorMap tm_stA, const __grid_constant__ CUtensorMap tm_stB,
+                     const __grid_constant__ CUtensorMap tm_aug, const TcParams p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  if ((smem_u32(smem) & 1023u) != 0) __trap();
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + TcSmem64::bars);
+  uint64_t* res_full = bars;               // [2]      resident tiles (+ DQ statistics rows) of item n in buffer n & 1
+  uint64_t* list_ready = bars + 2;         // [1]
+  uint64_t* st_full = bars + 3;            // [kNST64]
+  uint64_t* st_empty = st_full + kNST64;   // [kNST64]
+  uint64_t* sdp_full = st_empty + kNST64;  // [kNG]    S' of stage g written
+  uint64_t* dp_full = sdp_full + kNG;      // [kNG]    dP' of stage g written
+  uint64_t* stage_free = dp_full + kNG;    // [kNG]    the accumulate MMAs reading stage g have retired
+  uint64_t* p_ready = stage_free + kNG;    // [kNG]    P / dS written in place into stage g (4 warps arrive)
+  uint64_t* acc_full = p_ready + kNG;      // [1]
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 1);
+  int* n_tiles_slot = reinterpret_cast<int*>(acc_full + 1) + 1;   // [2]
+  int* item_slot = reinterpret_cast<int*>(acc_full + 1) + 3;      // [2]
+  uint16_t* tile_lists = reinterpret_cast<uint16_t*>(smem + TcSmem64::tiles);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const bool masked = p.row_id != nullptr;
+  const int n_col_tiles = (p.S_col + kCols - 1) / kCols;
+  const int n_row_tiles64 = (p.S_row + 63) / 64;
+  const int n_row_tiles = (p.S_row + kRows - 1) / kRows;
+  const int n_items = n_row_tiles * p.H * p.B;
+
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&tm_resA); tma_prefetch_desc(&tm_resB); tma_prefetch_desc(&tm_stA);
+    tma_prefetch_desc(&tm_stB); tma_prefetch_desc(&tm_aug);
+  }
+  if (warp == 1 && lane == 0) {
+    mbar_init(&res_full[0], 1);
+    mbar_init(&res_full[1], 1);
+    mbar_init(list_ready, 1);
+    for (int i = 0; i < kNST64; ++i) { mbar_init(&st_full[i], 1); mbar_init(&st_empty[i], 1); }
+    for (int i = 0; i < kNG; ++i) {
+      mbar_init(&sdp_full[i], 1);
+      mbar_init(&dp_full[i], 1);
+      mbar_init(&stage_free[i], 1);
+      mbar_init(&p_ready[i], 4);
+    }
+    mbar_init(acc_full, 1);
+    fence_mbar_init();
+  }
+  if (warp == 2) {
+    tmem_alloc(tmem_slot, 512);
+    tmem_relinquish();
+  }
+  if (warp >= 4) {
+    // constant operand tiles of the statistics K step (as in attn_bwd_tc_kernel): row r = 16 bf16, ones in columns 0-2
+    // (picks -lse / c) resp. 3-5 (picks -delta), SWIZZLE_32B pattern.  DKV: A operand (128 key rows); DQ: B operand
+    // (first 64 rows)
+    for (int i = threadIdx.x - 128; i < 2 * 128 * 2; i += kTcThreads - 128) {
+      const int tile = i >> 8, r = (i >> 1) & 127, pc = i & 1;
+      const int c = pc ^ ((r >> 2) & 1);
+      uint4 v = make_uint4(0u, 0u, 0u, 0u);
+      if (c == 0) v = tile == 0 ? make_uint4(0x3F803F80u, 0x00003F80u, 0u, 0u) : make_uint4(0u, 0x3F800000u, 0x3F803F80u, 0u);
+      *reinterpret_cast<uint4*>(smem + TcSmem64::ones + tile * 4096 + r * 32 + pc * 16) = v;
+    }
+    fence_proxy_async();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  int base = 0;
+  uint32_t item_n = 0;
+  int pstage = 0;
+  uint32_t pphase = 0;
+  int pre_cnt = -1;
+  auto build_list = [&](int it, int buf) {       // whole warp (see attn_bwd_tc_kernel)
+    const int rt_ = it % n_row_tiles, b_ = it / (n_row_tiles * p.H);
+    uint16_t* list = tile_lists + buf * kMaxTiles;
+    int row_lo = 0, row_hi = 0;
+    if (masked) {
+      const int i0 = rt_ * 2, i1 = min(rt_ * 2 + 1, n_row_tiles64 - 1);
+      row_lo = min(p.row_min[b_ * n_row_tiles64 + i0], p.row_min[b_ * n_row_tiles64 + i1]);
+      row_hi = max(p.row_max[b_ * n_row_tiles64 + i0], p.row_max[b_ * n_row_tiles64 + i1]);
+    }
+    int cnt = 0;
+    for (int cb = 0; cb < n_col_tiles; cb += 32) {
+      const int t = cb + lane;
+      bool vis = t < n_col_tiles, nm = false;
+      if (vis) {
+        int cmin = 0, cmax = 0;
+        if (masked) { cmin = p.col_min[b_ * n_col_tiles + t]; cmax = p.col_max[b_ * n_col_tiles + t]; }
+        if (MODE == MODE_DKV) {
+          vis = !masked || cmax >= row_lo;
+          nm = masked && (row_hi > cmin);
+        } else {
+          vis = !masked || cmin <= row_hi;
+          nm = (masked && (cmax > row_lo)) || (t * kCols + kCols > p.S_col);
+        }
+      }
+      const unsigned m = __ballot_sync(0xffffffffu, vis);
+      if (vis) list[cnt + __popc(m & ((1u << lane) - 1u))] = static_cast<uint16_t>(t | (nm ? 0x8000 : 0));
+      cnt += __popc(m);
+    }
+    if (lane == 0) n_tiles_slot[buf] = cnt;
+  };
+  if (warp == 2) {
+    int first = 0;
+    if (lane == 0) first = static_cast<int>(atomicAdd(&p.items[0], 1u));
+    first = __shfl_sync(0xffffffffu, first, 0);
+    if (lane == 0) item_slot[0] = first;
+    if (first < n_items) build_list(first, 0);
+  }
+  __syncthreads();
+  for (int item = item_slot[0]; item < n_items; item = item_slot[(item_n + 1) & 1], ++item_n) {
+  const int rt = item % n_row_tiles, h = (item / n_row_tiles) % p.H, b = item / (n_row_tiles * p.H);
+  const int r0 = rt * kRows;
+  const uint16_t* tile_list = tile_lists + (item_n & 1) * kMaxTiles;
+  const int T = n_tiles_slot[item_n & 1];
+
+  if (warp == 2) {
+    int nxt = 0;
+    if (lane == 0) nxt = static_cast<int>(atomicAdd(&p.items[0], 1u));
+    nxt = __shfl_sync(0xffffffffu, nxt, 0);
+    if (lane == 0) item_slot[(item_n + 1) & 1] = nxt;
+    if (nxt < n_items) build_list(nxt, (item_n + 1) & 1);
+    __syncwarp();
+    if (lane == 0) mbar_arrive(list_ready);
+  }
+
+  if (warp == 0) {
+    // ================================ TMA producer ================================
+    const int T_u = __shfl_sync(0xffffffffu, T, 0);
+    auto load_resident = [&](int h_, int r0_, int b_, int buf) {
+      if (elect_one()) {
+        mbar_expect_tx(&res_full[buf], MODE == MODE_DQ ? 32768u + 4096u : 32768u);
+        tma_load_4d(smem + TcSmem64::resA + buf * 16384, &tm_resA, &res_full[buf], 0, h_, r0_, b_);
+        tma_load_4d(smem + TcSmem64::resB + buf * 16384, &tm_resB, &res_full[buf], 0, h_, r0_, b_);
+        if (MODE == MODE_DQ) tma_load_4d(smem + TcSmem64::aug_res + buf * 4096, &tm_aug, &res_full[buf], 0, r0_, h_, b_);
+      }
+      __syncwarp();
+    };
+    auto load_tile = [&](int t, int h_, int b_) {
+      uint8_t* st = smem + TcSmem64::stream + pstage * kStage64;
+      mbar_wait(&st_empty[pstage], pphase ^ 1);
+      if (elect_one()) {
+        mbar_expect_tx(&st_full[pstage], MODE == MODE_DKV ? 16384u + 2048u : 16384u);
+        tma_load_4d(st, &tm_stA, &st_full[pstage], 0, h_, t * kCols, b_);
+        tma_load_4d(st + 8192, &tm_stB, &st_full[pstage], 0, h_, t * kCols, b_);
+        if (MODE == MODE_DKV) tma_load_4d(st + 16384, &tm_aug, &st_full[pstage], 0, t * kCols, h_, b_);   // the queries' statistics rows
+      }
+      __syncwarp();
+      if (++pstage == kNST64) { pstage = 0; pphase ^= 1; }
+    };
+    if (pre_cnt < 0) { load_resident(h, r0, b, item_n & 1); pre_cnt = 0; }
+    for (int j = pre_cnt; j < T_u; ++j) load_tile(__shfl_sync(0xffffffffu, tile_list[j] & 0x7fff, 0), h, b);
+    mbar_wait(list_ready, item_n & 1);
+    const int nxt = __shfl_sync(0xffffffffu, item_slot[(item_n + 1) & 1], 0);
+    pre_cnt = -1;
+    if (nxt < n_items) {
+      const int rt2 = nxt % n_row_tiles, h2 = (nxt / n_row_tiles) % p.H, b2 = nxt / (n_row_tiles * p.H);
+      const uint16_t* list2 = tile_lists + ((item_n + 1) & 1) * kMaxTiles;
+      const int T2 = __shfl_sync(0xffffffffu, n_tiles_slot[(item_n + 1) & 1], 0);
+      load_resident(h2, rt2 * kRows, b2, (item_n + 1) & 1);
+      pre_cnt = 0;
+      const int ahead = T2 < kNST64 / 2 ? T2 : kNST64 / 2;
+      for (int j = 0; j < ahead; ++j, ++pre_cnt) load_tile(__shfl_sync(0xffffffffu, list2[j] & 0x7fff, 0), h2, b2);
+    }
+  } else if (warp == 1) {
+    // ================================ score-MMA issuer (SS mode) ================================
+    constexpr uint32_t idesc_score = umma_idesc_bf16(kRows, kCols);
+    const int T_u = __shfl_sync(0xffffffffu, T, 0);
+    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
+    const uint32_t stream = smem_u32(smem + TcSmem64::stream);
+    const uint32_t buf = item_n & 1;
+    const uint64_t dRA = umma_desc_sw128(smem_u32(smem + TcSmem64::resA) + buf * 16384);
+    const uint64_t dRB = umma_desc_sw128(smem_u32(smem + TcSmem64::resB) + buf * 16384);
+    const uint64_t dOnesS = umma_desc_sw32(smem_u32(smem + TcSmem64::ones));
+    const uint64_t dOnesD = umma_desc_sw32(smem_u32(smem + TcSmem64::ones + 4096));
+    const uint64_t dAugRes = umma_desc_sw32(smem_u32(smem + TcSmem64::aug_res) + buf * 4096);
+    mbar_wait(&res_full[buf], (item_n >> 1) & 1);
+    for (int js = 0; js < T_u; ++js) {
+      const int gt = base + js;
+      const int stage = gt % kNST64, g = gt % kNG, n = gt / kNG;
+      uint64_t dS = umma_desc_sw128(stream + stage * kStage64), dD = umma_desc_sw128(stream + stage * kStage64 + 8192);
+      uint32_t d_s = tmem_u + g * 128, d_dp = tmem_u + g * 128 + 64;
+      // statistics K step: DKV  A = ones (keys), B = the tile's query statistics rows;  DQ  A = resident statistics rows,
+      // B = ones (keys)
+      uint64_t fA_s = dOnesS, fA_d = dOnesD, fB_s = umma_desc_sw32(stream + stage * kStage64 + 16384), fB_d = fB_s;
+      if (MODE == MODE_DQ) { fA_s = fA_d = dAugRes; fB_s = dOnesS; fB_d = dOnesD; }
+      asm volatile("" : "+l"(dS), "+l"(dD), "+r"(d_s), "+r"(d_dp), "+l"(fA_s), "+l"(fA_d), "+l"(fB_s), "+l"(fB_d));
+      mbar_wait(&st_full[stage], (gt / kNST64) & 1);
+      mbar_wait(&stage_free[g], (n & 1) ^ 1);
+      tc_fence_after();
+      if (elect_one()) {
+        // a K step of 16 bf16 = 32 bytes = +2 in the descriptor's (address >> 4) field
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) umma_bf16(d_s, dRA + 2 * kk, dS + 2 * kk, idesc_score, kk > 0 ? 1u : 0u);
+        umma_bf16(d_s, fA_s, fB_s, idesc_score, 1u);
+        umma_commit(&sdp_full[g]);                     // S' complete: the warpgroup starts on the exponentials
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) umma_bf16(d_dp, dRB + 2 * kk, dD + 2 * kk, idesc_score, kk > 0 ? 1u : 0u);
+        umma_bf16(d_dp, fA_d, fB_d, idesc_score, 1u);
+        umma_commit(&dp_full[g]);
+      }
+      __syncwarp();
+    }
+  } else if (warp == 3) {
+    // ================================ accumulate-MMA issuer (TS mode) ================================
+    // B operand straight from the streamed stage: tile [64 tokens][64 dims], 128-byte rows, SWIZZLE_128B = the canonical
+    // MN-major layout (N = 64 dims in one swizzle atom, 8-token groups 1024 B apart); a K step of 16 tokens = 2048 B.
+    // DKV: dV += P^T dO (tile B), dK += dS^T Q (tile A).  DQ: dQ += dS K (tile A).
+    constexpr uint32_t idesc_acc = umma_idesc_bf16(kRows, 64) | (1u << 16);
+    const int T_u = __shfl_sync(0xffffffffu, T, 0);
+    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
+    const uint32_t stream = smem_u32(smem + TcSmem64::stream);
+    for (int ia = 0; ia < T_u; ++ia) {
+      const int gt = base + ia;
+      const int stage = gt % kNST64, g = gt % kNG, n = gt / kNG;
+      uint32_t ta = tmem_u + g * 128;                   // P pairs at +0..31, dS pairs at +64..95 (written in place)
+      uint64_t dMA = umma_desc_sw128(stream + stage * kStage64 + 8192), dMB = umma_desc_sw128(stream + stage * kStage64);
+      asm volatile("" : "+l"(dMA), "+l"(dMB), "+r"(ta));
+      mbar_wait(&p_ready[g], n & 1);
+      tc_fence_after();
+      if (elect_one()) {
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) {
+          if (MODE == MODE_DKV) umma_bf16_ts(tmem_u + kAcc64, ta + kk * 8, dMA + 128 * kk, idesc_acc, (ia > 0 || kk > 0) ? 1u : 0u);
+          umma_bf16_ts(tmem_u + kAcc64 + 64, ta + 64 + kk * 8, dMB + 128 * kk, idesc_acc, (ia > 0 || kk > 0) ? 1u : 0u);
+        }
+        umma_commit(&stage_free[g]);
+        umma_commit(&st_empty[stage]);
+      }
+      __syncwarp();
+    }
+    if (elect_one()) umma_commit(acc_full);
+    __syncwarp();
+  } else if (warp >= 4) {
+    // ================================ compute warpgroups ================================
+    // (the folded-statistics path of attn_bwd_tc_kernel: the score columns of a tile are the same 64 at either head_dim)
+    const int g = (warp - 4) >> 2;
+    const int q4 = warp & 3;
+    const int r = q4 * 32 + lane;
+    const int tid = r;
+    const int row = r0 + r;
+    const bool row_ok = row < p.S_row;
+    int* ids_base = reinterpret_cast<int*>(smem + TcSmem64::ids) + g * 128;
+    const int my_id = masked ? (row_ok ? p.row_id[static_cast<long long>(b) * p.S_row + row]
+                                       : (MODE == MODE_DKV ? 0x7fffffff : -0x7fffffff))
+                             : 0;
+    int pre_i = 0;
+    auto prefetch = [&](int j) {
+      if (j >= T) return;
+      const int c = (tile_list[j] & 0x7fff) * kCols + (tid & 63);
+      const bool ok = c < p.S_col;
+      if ((tile_list[j] & 0x8000) && tid < 64)
+        pre_i = ok ? (masked ? p.col_id[static_cast<long long>(b) * p.S_col + c] : 0) : (MODE == MODE_DKV ? -0x7fffffff : 0x7fffffff);
+    };
+    const int j0 = (g + kNG - base % kNG) % kNG;
+    prefetch(j0);
+    for (int j = j0; j < T; j += kNG) {
+      const int n = (base + j) / kNG;
+      const bool need_mask = (tile_list[j] & 0x8000) != 0;
+      int* s_id = ids_base + (n & 1) * 64;
+      if (need_mask) {
+        named_bar_sync(1 + g, 128);
+        if (tid < 64) s_id[tid] = pre_i;
+        named_bar_sync(1 + g, 128);
+      }
+      prefetch(j + kNG);
+      mbar_wait(&sdp_full[g], n & 1);
+      tc_fence_after();
+      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q4 * 32) << 16) + g * 128;
+      uint32_t sv[2][16], dv[2][16];
+      float pf[16];
+      auto expo = [&](uint32_t (&s16)[16], int i) {
+        if (need_mask) {
+#pragma unroll
+          for (int e = 0; e < 16; ++e) {
+            const int cid = s_id[i * 16 + e];
+            const bool hide = (MODE == MODE_DKV) ? (my_id > cid) : (cid > my_id);
+            if (hide) s16[e] = 0xff800000u;
+          }
+        }
+#pragma unroll
+        for (int e = 0; e < 16; ++e) pf[e] = fast_ex2(__uint_as_float(s16[e]) * p.scale_log2);
+      };
+      tmem_ld16(taddr, sv[0]);
+      tmem_wait1_16(sv[0]);
+      tmem_ld16(taddr + 16, sv[1]);
+      expo(sv[0], 0);
+      mbar_wait(&dp_full[g], n & 1);
+      tc_fence_after();
+      tmem_ld16(taddr + 64, dv[0]);
+#pragma unroll
+      for (int i = 0; i < kSub; ++i) {
+        const int cur = i & 1;
+        if (i < kSub - 1) tmem_wait2_16(dv[cur], sv[cur ^ 1]); else tmem_wait1_16(dv[cur]);
+        if (i < kSub - 1) tmem_ld16(taddr + 64 + (i + 1) * 16, dv[cur ^ 1]);
+        if (i < kSub - 2) tmem_ld16(taddr + (i + 2) * 16, sv[cur]);
+        uint32_t pw[8], dw[8];
+#pragma unroll
+        for (int e2 = 0; e2 < 8; ++e2) {
+          const float s0 = pf[2 * e2] * __uint_as_float(dv[cur][2 * e2]);
+          const float s1 = pf[2 * e2 + 1] * __uint_as_float(dv[cur][2 * e2 + 1]);
+          if (MODE == MODE_DKV) pw[e2] = pack2(pf[2 * e2], pf[2 * e2 + 1]);
+          dw[e2] = pack2(s0, s1);
+        }
+        if (MODE == MODE_DKV) tmem_st8(taddr + i * 8, pw);
+        tmem_st8(taddr + 64 + i * 8, dw);
+        if (i < kSub - 1) expo(sv[cur ^ 1], i + 1);
+      }
+      tmem_wait_st();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&p_ready[g]);
+    }
+    // ---- epilogue: accumulators (64 fp32 columns) -> bf16 -> global; wg0 -> dV, wg1 -> dK / dQ ----
+    mbar_wait(acc_full, item_n & 1);
+    tc_fence_after();
+    const bool writes = (MODE == MODE_DKV) ? (g < 2) : (g == 1);
+    if (writes) {
+      const int which = (MODE == MODE_DKV) ? g : 1;
+      const float sc = (which == 1) ? p.scale : 1.f;
+      __nv_bfloat16* dst = nullptr;
+      const float2* tb = nullptr;
+      if (row_ok) {
+        dst = (which == 0 ? p.out0 + b * p.o0_bs + static_cast<long long>(row) * p.o0_ts
+                          : p.out1 + b * p.o1_bs + static_cast<long long>(row) * p.o1_ts) + h * 64;
+        if (which == 1 && p.rope_table != nullptr) {
+          int ps = p.rope_pos ? p.rope_pos[static_cast<long long>(b) * p.S_row + row] : row + p.rope_offset;
+          ps = min(max(ps, 0), p.rope_len - 1);
+          tb = p.rope_table + static_cast<long long>(ps) * 32;
+        }
+      }
+#pragma unroll
+      for (int half = 0; half < 2; ++half) {
+        uint32_t acc[32];
+        if (T > 0) {
+          tmem_ld32(tmem_base + (static_cast<uint32_t>(q4 * 32) << 16) + kAcc64 + which * 64 + half * 32, acc);
+          tmem_wait1_32(acc);
+        } else {
+#pragma unroll
+          for (int i = 0; i < 32; ++i) acc[i] = 0u;
+        }
+        if (row_ok) {
+#pragma unroll
+          for (int c4 = 0; c4 < 4; ++c4) {
+            uint32_t w[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) {
+              float a0 = __uint_as_float(acc[c4 * 8 + e * 2]) * sc, a1 = __uint_as_float(acc[c4 * 8 + e * 2 + 1]) * sc;
+              if (tb != nullptr) {         // gradient of a rotated operand: rotate back (conjugate)
+                const float2 cs = tb[half * 16 + c4 * 4 + e];
+                const float q0 = a0 * cs.x + a1 * cs.y, q1 = a1 * cs.x - a0 * cs.y;
+                a0 = q0; a1 = q1;
+              }
+              w[e] = pack2(a0, a1);
+            }
+            *reinterpret_cast<uint4*>(dst + half * 32 + c4 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
+          }
+        }
+      }
+    }
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  base += T;
+  }   // item loop
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 512);
+  }
+  if (threadIdx.x == 0) {
+    if (atomicAdd(&p.items[1], 1u) == gridDim.x - 1) {
+      p.items[0] = 0u;
+      p.items[1] = 0u;
+      __threadfence();
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// delta and the statistics rows at head_dim 64 (attn_aug_kernel with 64-wide rows)
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+attn_aug64_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o, const float* __restrict__ lse,
+                  float* __restrict__ delta, __nv_bfloat16* __restrict__ aug, int B, int H, int S, long long o_bs, long long o_ts,
+                  long long do_bs, long long do_ts, float inv_scale_log2) {
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;   // (b, i, h)
+  if (idx >= static_cast<long long>(B) * S * H) return;
+  const int h = static_cast<int>(idx % H);
+  const long long bi = idx / H;
+  const int i = static_cast<int>(bi % S), b = static_cast<int>(bi / S);
+  const uint4* op = reinterpret_cast<const uint4*>(o + b * o_bs + static_cast<long long>(i) * o_ts + h * 64);
+  const uint4* dp = reinterpret_cast<const uint4*>(d_o + b * do_bs + static_cast<long long>(i) * do_ts + h * 64);
+  float acc = 0.f;
+#pragma unroll
+  for (int c = 0; c < 8; ++c) {
+    const uint4 a = op[c], e = dp[c];
+    const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, ew[4] = {e.x, e.y, e.z, e.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j)
+      acc += __uint_as_float(aw[j] << 16) * __uint_as_float(ew[j] << 16) +
+             __uint_as_float(aw[j] & 0xffff0000u) * __uint_as_float(ew[j] & 0xffff0000u);
+  }
+  const long long row = (static_cast<long long>(b) * H + h) * S + i;
+  delta[row] = acc;
+  const float l = lse[row];
+  const float nl = (l < 3.0e38f) ? -l * inv_scale_log2 : -1.0e30f;
+  float v[6];
+  split3(nl, v[0], v[1], v[2]);
+  split3(-acc, v[3], v[4], v[5]);
+  uint4 w;
+  w.x = pack2(v[0], v[1]); w.y = pack2(v[2], v[3]); w.z = pack2(v[4], v[5]); w.w = 0u;
+  uint4* dst = reinterpret_cast<uint4*>(aug + row * 16);
+  dst[0] = w;
+  dst[1] = make_uint4(0u, 0u, 0u, 0u);
+}
+
+// ================================================================================================
+// Forward at head_dim 64 (attn_fwd_tc_kernel with 64-wide heads): Q [128][64] tiles (two per item and buffer, 64 KB),
+// K | V stages of 32 KB (4 stages), score MMAs K = 64 (4 K steps), P V MMAs N = 64.
+// TMEM map: S_g at g*128 (128), P_g at 256 + g*64 (64), O_g at 384 + g*64 (64) = 512 columns.
+// ================================================================================================
+constexpr int kNSTF64 = 4;
+
+struct FwdSmem64 {
+  static constexpr int q = 0;                            // 2 buffers x 2 groups x [128][64] bf16
+  static constexpr int stream = 65536;                   // kNSTF64 x 32 KB: K tile (16 KB) | V tile (16 KB)
+  static constexpr int ids = stream + kNSTF64 * 32768;   // [2 wg][2 buffers][128] int
+  static constexpr int tiles = ids + 2 * 2 * 128 * 4;
+  static constexpr int bars = tiles + 2 * kMaxTiles * 2;
+  static constexpr int total = bars + 256;
+};
+static_assert(FwdSmem64::total <= 232448, "attn_fwd_tc64_kernel: shared memory");
+
+__global__ void __launch_bounds__(kFwdThreads, 1)
+attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
+                     const __grid_constant__ CUtensorMap tm_v, const FwdParams p) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  if ((smem_u32(smem) & 1023u) != 0) __trap();
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FwdSmem64::bars);
+  uint64_t* q_full = bars;                  // [2]
+  uint64_t* list_ready = bars + 2;          // [1]
+  uint64_t* st_full = bars + 3;             // [kNSTF64]
+  uint64_t* st_empty = st_full + kNSTF64;   // [kNSTF64]  two arrivals: the P V MMAs of both warpgroups
+  uint64_t* s_full = st_empty + kNSTF64;    // [2]
+  uint64_t* s_free = s_full + 2;            // [2]
+  uint64_t* p_ready = s_free + 2;           // [2]
+  uint64_t* p_free = p_ready + 2;           // [2]
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(p_free + 2);
+  int* n_tiles_slot = reinterpret_cast<int*>(p_free + 2) + 1;   // [2]
+  int* item_slot = reinterpret_cast<int*>(p_free + 2) + 3;      // [2]
+  uint16_t* tile_lists = reinterpret_cast<uint16_t*>(smem + FwdSmem64::tiles);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const bool masked = p.qid != nullptr;
+  const int n_k_tiles = (p.Sk + kFwdTileK - 1) / kFwdTileK;
+  const int nq64 = (p.Sq + 63) / 64, nk64 = (p.Sk + 63) / 64;
+  const int n_q_tiles = (p.Sq + 255) / 256;
+  const int n_items = n_q_tiles * p.H * p.B;
+
+  if (warp == 0 && lane == 0) { tma_prefetch_desc(&tm_q); tma_prefetch_desc(&tm_k); tma_prefetch_desc(&tm_v); }
+  if (warp == 1 && lane == 0) {
+    mbar_init(&q_full[0], 1);
+    mbar_init(&q_full[1], 1);
+    mbar_init(list_ready, 1);
+    for (int i = 0; i < kNSTF64; ++i) { mbar_init(&st_full[i], 1); mbar_init(&st_empty[i], 2); }
+    for (int i = 0; i < 2; ++i) {
+      mbar_init(&s_full[i], 1);
+      mbar_init(&s_free[i], 4);
+      mbar_init(&p_ready[i], 4);
+      mbar_init(&p_free[i], 1);
+    }
+    fence_mbar_init();
+  }
+  if (warp == 2) {
+    tmem_alloc(tmem_slot, 512);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem_base = *tmem_slot;
+
+  auto build_list = [&](int it, int buf) {       // whole warp (see attn_fwd_tc_kernel)
+    const int qt_ = it % n_q_tiles, b_ = it / (n_q_tiles * p.H);
+    uint16_t* list = tile_lists + buf * kMaxTiles;
+    int wq_lo[2] = {0, 0}, wq_hi[2] = {0, 0};
+    if (masked) {
+#pragma unroll
+      for (int g = 0; g < 2; ++g) {
+        const int i0 = min(qt_ * 4 + g * 2, nq64 - 1), i1 = min(qt_ * 4 + g * 2 + 1, nq64 - 1);
+        wq_lo[g] = min(p.qmin[b_ * nq64 + i0], p.qmin[b_ * nq64 + i1]);
+        wq_hi[g] = max(p.qmax[b_ * nq64 + i0], p.qmax[b_ * nq64 + i1]);
+      }
+    }
+    const int cta_hi = max(wq_hi[0], wq_hi[1]);
+    int cnt = 0;
+    for (int cb = 0; cb < n_k_tiles; cb += 32) {
+      const int t = cb + lane;
+      bool vis = t < n_k_tiles;
+      int flags = 0;
+      if (vis) {
+        int kmn = 0, kmx = 0;
+        if (masked) {
+          const int i0 = min(t * 2, nk64 - 1), i1 = min(t * 2 + 1, nk64 - 1);
+          kmn = min(p.kmin[b_ * nk64 + i0], p.kmin[b_ * nk64 + i1]);
+          kmx = max(p.kmax[b_ * nk64 + i0], p.kmax[b_ * nk64 + i1]);
+          vis = kmn <= cta_hi;
+        }
+        const bool tail = t * kFwdTileK + kFwdTileK > p.Sk;
+        if ((masked && kmx > wq_lo[0]) || tail) flags |= 0x4000;
+        if ((masked && kmx > wq_lo[1]) || tail) flags |= 0x8000;
+      }
+      const unsigned m = __ballot_sync(0xffffffffu, vis);
+      if (vis) list[cnt + __popc(m & ((1u << lane) - 1u))] = static_cast<uint16_t>(t | flags);
+      cnt += __popc(m);
+    }
+    if (lane == 0) n_tiles_slot[buf] = cnt;
+  };
+
+  int base = 0;
+  uint32_t item_n = 0;
+  int pstage = 0;
+  uint32_t pphase = 0;
+  int pre_cnt = -1;
+  if (warp == 2) {
+    int first = 0;
+    if (lane == 0) first = static_cast<int>(atomicAdd(&p.items[0], 1u));
+    first = __shfl_sync(0xffffffffu, first, 0);
+    if (lane == 0) item_slot[0] = first;
+    if (first < n_items) build_list(first, 0);
+  }
+  __syncthreads();
+  for (int item = item_slot[0]; item < n_items; item = item_slot[(item_n + 1) & 1], ++item_n) {
+  const int qt = item % n_q_tiles, h = (item / n_q_tiles) % p.H, b = item / (n_q_tiles * p.H);
+  const int q0 = qt * 256;
+  const uint16_t* tile_list = tile_lists + (item_n & 1) * kMaxTiles;
+  const int T = n_tiles_slot[item_n & 1];
+
+  if (warp == 2) {
+    int nxt = 0;
+    if (lane == 0) nxt = static_cast<int>(atomicAdd(&p.items[0], 1u));
+    nxt = __shfl_sync(0xffffffffu, nxt, 0);
+    if (lane == 0) item_slot[(item_n + 1) & 1] = nxt;
+    if (nxt < n_items) build_list(nxt, (item_n + 1) & 1);
+    __syncwarp();
+    if (lane == 0) mbar_arrive(list_ready);
+  }
+
+  if (warp == 0) {
+    // ================================ TMA producer ================================
+    const int T_u = __shfl_sync(0xffffffffu, T, 0);
+    auto load_q = [&](int h_, int q0_, int b_, int buf) {
+      if (elect_one()) {
+        mbar_expect_tx(&q_full[buf], 32768);
+        tma_load_4d(smem + FwdSmem64::q + buf * 32768, &tm_q, &q_full[buf], 0, h_, q0_, b_);
+        tma_load_4d(smem + FwdSmem64::q + buf * 32768 + 16384, &tm_q, &q_full[buf], 0, h_, q0_ + 128, b_);
+      }
+      __syncwarp();
+    };
+    auto load_tile = [&](int t, int h_, int b_) {
+      uint8_t* st = smem + FwdSmem64::stream + pstage * 32768;
+      mbar_wait(&st_empty[pstage], pphase ^ 1);
+      if (elect_one()) {
+        mbar_expect_tx(&st_full[pstage], 32768);
+        tma_load_4d(st, &tm_k, &st_full[pstage], 0, h_, t * kFwdTileK, b_);
+        tma_load_4d(st + 16384, &tm_v, &st_full[pstage], 0, h_, t * kFwdTileK, b_);      // V tile [128 keys][64 dims]
+      }
+      __syncwarp();
+      if (++pstage == kNSTF64) { pstage = 0; pphase ^= 1; }
+    };
+    if (pre_cnt < 0) { load_q(h, q0, b, item_n & 1); pre_cnt = 0; }
+    for (int j = pre_cnt; j < T_u; ++j) load_tile(__shfl_sync(0xffffffffu, tile_list[j] & 0x3fff, 0), h, b);
+    mbar_wait(list_ready, item_n & 1);
+    const int nxt = __shfl_sync(0xffffffffu, item_slot[(item_n + 1) & 1], 0);
+    pre_cnt = -1;
+    if (nxt < n_items) {
+      const int qt2 = nxt % n_q_tiles, h2 = (nxt / n_q_tiles) % p.H, b2 = nxt / (n_q_tiles * p.H);
+      const uint16_t* list2 = tile_lists + ((item_n + 1) & 1) * kMaxTiles;
+      const int T2 = __shfl_sync(0xffffffffu, n_tiles_slot[(item_n + 1) & 1], 0);
+      load_q(h2, qt2 * 256, b2, (item_n + 1) & 1);
+      pre_cnt = 0;
+      const int ahead = T2 < kNSTF64 / 2 ? T2 : kNSTF64 / 2;
+      for (int j = 0; j < ahead; ++j, ++pre_cnt) load_tile(__shfl_sync(0xffffffffu, list2[j] & 0x3fff, 0), h2, b2);
+    }
+  } else if (warp == 1) {
+    // ================================ score-MMA issuer ================================
+    constexpr uint32_t idesc = umma_idesc_bf16(128, kFwdTileK);
+    const int T_u = __shfl_sync(0xffffffffu, T, 0);
+    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
+    const uint64_t dQ[2] = {umma_desc_sw128(smem_u32(smem + FwdSmem64::q + (item_n & 1) * 32768)),
+                            umma_desc_sw128(smem_u32(smem + FwdSmem64::q + (item_n & 1) * 32768 + 16384))};
+    const uint32_t stream = smem_u32(smem + FwdSmem64::stream);
+    mbar_wait(&q_full[item_n & 1], (item_n >> 1) & 1);
+    tc_fence_after();
+    for (int j = 0; j < T_u; ++j) {
+      const int gj = base + j;
+      const int stage = gj % kNSTF64;
+      mbar_wait(&st_full[stage], (gj / kNSTF64) & 1);
+      const uint64_t dK = umma_desc_sw128(stream + stage * 32768);
+#pragma unroll
+      for (int g = 0; g < 2; ++g) {
+        mbar_wait(&s_free[g], (gj & 1) ^ 1);
+        tc_fence_after();
+        if (elect_one()) {
+#pragma unroll
+          for (int kk = 0; kk < 4; ++kk) umma_bf16(tmem_u + g * 128, dQ[g] + 2 * kk, dK + 2 * kk, idesc, kk > 0 ? 1u : 0u);
+          umma_commit(&s_full[g]);
+        }
+        __syncwarp();
+      }
+    }
+  } else if (warp == 3) {
+    // ================================ P V MMA issuer ================================
+    constexpr uint32_t idesc = umma_idesc_bf16(128, 64);
+    const int T_u = __shfl_sync(0xffffffffu, T, 0);
+    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
+    const uint32_t stream = smem_u32(smem + FwdSmem64::stream);
+    for (int j = 0; j < T_u; ++j) {
+      const int gj = base + j;
+      const int stage = gj % kNSTF64;
+      // V tile [128 keys][64 dims] (128-byte rows, SWIZZLE_128B) read MN-major: N = 64 dims in one swizzle atom, K = keys,
+      // a K step of 16 keys = 2048 B
+      const uint64_t dV = umma_desc_sw128(stream + stage * 32768 + 16384);
+#pragma unroll
+      for (int g = 0; g < 2; ++g) {
+        mbar_wait(&p_ready[g], gj & 1);
+        tc_fence_after();
+        const uint32_t pa = tmem_u + 256 + g * 64, oa = tmem_u + 384 + g * 64;
+        if (elect_one()) {
+#pragma unroll
+          for (int kk = 0; kk < 8; ++kk)
+            umma_bf16_ts(oa, pa + kk * 8, dV + 128 * kk, idesc | (1u << 16), (j > 0 || kk > 0) ? 1u : 0u);
+          umma_commit(&p_free[g]);
+          umma_commit(&st_empty[stage]);
+        }
+        __syncwarp();
+      }
+    }
+  } else if (warp >= 4) {
+    // ================================ softmax warpgroups (as attn_fwd_tc_kernel) ================================
+    const int g = (warp - 4) >> 2;
+    const int q4 = warp & 3;
+    const int r = q4 * 32 + lane;
+    const int tid = (warp - 4 - g * 4) * 32 + lane;
+    const int row = q0 + g * 128 + r;
+    const bool row_ok = row < p.Sq;
+    const int my_id = masked ? (row_ok ? p.qid[static_cast<long long>(b) * p.Sq + row] : -0x7fffffff) : 0;
+    int* ids_base = reinterpret_cast<int*>(smem + FwdSmem64::ids) + g * 256;
+    const uint32_t lane_base = static_cast<uint32_t>(q4 * 32) << 16;
+    const uint32_t s_addr = tmem_base + lane_base + g * 128;
+    const uint32_t p_addr = tmem_base + lane_base + 256 + g * 64;
+    const uint32_t o_addr = tmem_base + lane_base + 384 + g * 64;
+    float m_run = -INFINITY, l_run = 0.f, alpha_pend = 1.f;
+    int pre_i = 0;
+    const uint16_t my_flag = (g == 0) ? 0x4000 : 0x8000;
+    auto prefetch = [&](int j) {
+      if (j >= T || !(tile_list[j] & my_flag)) return;
+      const int c = (tile_list[j] & 0x3fff) * kFwdTileK + tid;
+      pre_i = (c < p.Sk) ? (masked ? p.kid[static_cast<long long>(b) * p.Sk + c] : 0) : 0x7fffffff;
+    };
+    prefetch(0);
+    for (int j = 0; j < T; ++j) {
+      const int gj = base + j;
+      const bool need_mask = (tile_list[j] & my_flag) != 0;
+      int* s_id = ids_base;
+      if (need_mask) {
+        named_bar_sync(1 + g, 128);
+        s_id[tid] = pre_i;
+        named_bar_sync(1 + g, 128);
+      }
+      prefetch(j + 1);
+      mbar_wait(&s_full[g], gj & 1);
+      tc_fence_after();
+      uint32_t sv[2][32];
+      auto mask_chunk = [&](uint32_t (&v)[32], int c) {
+        if (need_mask) {
+#pragma unroll
+          for (int i = 0; i < 32; ++i)
+            if (s_id[c * 32 + i] > my_id) v[i] = 0xff800000u;
+        }
+      };
+      // O_g *= alpha_pend (rare, warp-uniform), 64 columns in two halves
+      auto apply_pending = [&]() {
+        if (__any_sync(0xffffffffu, alpha_pend != 1.f)) {
+#pragma unroll
+          for (int hf = 0; hf < 2; ++hf) {
+            uint32_t ov[32];
+            tmem_ld32(o_addr + hf * 32, ov);
+            tmem_wait1_32(ov);
+#pragma unroll
+            for (int i = 0; i < 32; ++i) ov[i] = __float_as_uint(__uint_as_float(ov[i]) * alpha_pend);
+            tmem_st32(o_addr + hf * 32, ov);
+          }
+          alpha_pend = 1.f;
+        }
+      };
+      float rs = 0.f;
+      bool released = false, redo = false;
+      auto release_scores = [&]() {
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&s_free[g]);
+        released = true;
+      };
+      auto exp_sweep = [&](float m_use, bool optimistic) {
+        rs = 0.f;
+        if (optimistic) tmem_ld32(s_addr, sv[0]);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const int cur = c & 1;
+          tmem_wait1_32(sv[cur]);
+          if (c < 3) tmem_ld32(s_addr + (c + 1) * 32, sv[cur ^ 1]);
+          mask_chunk(sv[cur], c);
+          if (c == 3 && !optimistic) release_scores();
+          uint32_t pw[16];
+#pragma unroll
+          for (int i = 0; i < 16; ++i) {
+            const float p0 = fast_ex2(fmaf(__uint_as_float(sv[cur][2 * i]), p.scale_log2, -m_use));
+            const float p1 = fast_ex2(fmaf(__uint_as_float(sv[cur][2 * i + 1]), p.scale_log2, -m_use));
+            rs += p0 + p1;
+            pw[i] = pack2(p0, p1);
+          }
+          if (c == 0 && optimistic) {
+            mbar_wait(&p_free[g], (gj & 1) ^ 1);
+            tc_fence_after();
+            apply_pending();
+          }
+          tmem_st16(p_addr + c * 16, pw);
+        }
+      };
+      const bool two_pass = __any_sync(0xffffffffu, m_run == -INFINITY);
+      if (!two_pass) {
+        exp_sweep(m_run, true);
+        redo = __any_sync(0xffffffffu, !(rs <= kStaleSum));
+        if (!redo) {
+          release_scores();
+          l_run += rs;
+        }
+      }
+      if (two_pass || redo) {
+        float mx1 = -INFINITY;
+        tmem_ld32(s_addr, sv[0]);
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const int cur = c & 1;
+          tmem_wait1_32(sv[cur]);
+          tmem_ld32(s_addr + ((c + 1) & 3) * 32, sv[cur ^ 1]);
+          mask_chunk(sv[cur], c);
+#pragma unroll
+          for (int i = 0; i < 32; i += 2) mx1 = fmaxf(mx1, fmaxf(__uint_as_float(sv[cur][i]), __uint_as_float(sv[cur][i + 1])));
+        }
+        const float m_tile = mx1 * p.scale_log2;
+        const bool raise = m_tile > m_run + (redo ? 0.f : kRescaleSlack) || m_run == -INFINITY;
+        const float m_new = raise ? fmaxf(m_run, m_tile) : m_run;
+        const float m_use = (m_new == -INFINITY) ? 0.f : m_new;
+        const float alpha = (raise && m_run != -INFINITY) ? fast_ex2(m_run - m_use) : 1.f;
+        if (two_pass) {
+          mbar_wait(&p_free[g], (gj & 1) ^ 1);
+          tc_fence_after();
+          apply_pending();
+        }
+        l_run *= alpha;
+        alpha_pend = alpha;
+        apply_pending();
+        m_run = m_new;
+        redo = false;
+        exp_sweep(m_use, false);
+        l_run += rs;
+      }
+      if (!released) release_scores();
+      tmem_wait_st();
+      tc_fence_before();
+      __syncwarp();
+      if (lane == 0) mbar_arrive(&p_ready[g]);
+    }
+    // ---- epilogue: O / l -> bf16 (64 columns in two halves), LSE ----
+    if (T > 0) {
+      mbar_wait(&p_free[g], ((base + T) & 1) ^ 1);
+      tc_fence_after();
+    }
+    const float inv = (l_run > 0.f) ? alpha_pend / l_run : 0.f;
+    __nv_bfloat16* dst = row_ok ? p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * 64 : nullptr;
+#pragma unroll
+    for (int hf = 0; hf < 2; ++hf) {
+      uint32_t ov[32];
+      if (T > 0) {
+        tmem_ld32(o_addr + hf * 32, ov);
+        tmem_wait1_32(ov);
+      } else {
+#pragma unroll
+        for (int i = 0; i < 32; ++i) ov[i] = 0u;
+      }
+      if (row_ok) {
+#pragma unroll
+        for (int c4 = 0; c4 < 4; ++c4) {
+          uint32_t w[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e)
+            w[e] = pack2(__uint_as_float(ov[c4 * 8 + e * 2]) * inv, __uint_as_float(ov[c4 * 8 + e * 2 + 1]) * inv);
+          *reinterpret_cast<uint4*>(dst + hf * 32 + c4 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
+        }
+      }
+    }
+    if (row_ok && p.lse != nullptr)
+      p.lse[(static_cast<long long>(b) * p.H + h) * p.Sq + row] = (l_run > 0.f) ? m_run + log2f(l_run) : INFINITY;
+  }
+
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  base += T;
+  }   // item loop
+
+  tc_fence_before();
+  __syncthreads();
+  if (warp == 2) {
+    tc_fence_after();
+    tmem_dealloc(tmem_base, 512);
+  }
+  if (threadIdx.x == 0) {
+    if (atomicAdd(&p.items[1], 1u) == gridDim.x - 1) {
+      p.items[0] = 0u;
+      p.items[1] = 0u;
+      __threadfence();
+    }
+  }
+}
+
 }  // namespace fk
 
 using namespace fk;
@@ -1409,6 +2272,81 @@ FK_API int fk_attn_transpose(const void* x, long long bs, long long ts, int B, i
 }
 
 static int bwd_sm_count() { return fk_sm_count(); }
+
+// head_dim 64 backward (attn_bwd_tc64_kernel): one path -- statistics folded (aug required), MN-major accumulate operands
+// (no transposed copies), no stall-accounting build.  Arguments already checked by the caller as far as they are shared.
+static int attn_backward_tc64(const void* q, const void* k, const void* v, const void* d_o, const void* qt, const void* kt,
+                              const void* dot, const void* aug, void* dq, void* dk, void* dv, int B, int H, int S,
+                              long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs, long long v_ts,
+                              long long do_bs, long long do_ts, long long dq_bs, long long dq_ts, long long dk_bs,
+                              long long dk_ts, long long dv_bs, long long dv_ts, const int* qid, const int* kid,
+                              const int* qmin, const int* qmax, const int* kmin, const int* kmax, float scale,
+                              const float* lse, const float* delta, const float* rope_table, int rope_len,
+                              const int* rope_pos, int rope_offset, int parts, unsigned int* counters,
+                              const long long* g_attn_prof, cudaStream_t stream) {
+  FK_REQUIRE(qt == nullptr && kt == nullptr && dot == nullptr, "fk_attn_backward_tc: head_dim 64 takes no transposed operands");
+  FK_REQUIRE(aug != nullptr && (reinterpret_cast<uintptr_t>(aug) & 31) == 0,
+             "fk_attn_backward_tc: head_dim 64 needs the statistics rows of fk_attn_aug (32-byte aligned)");
+  FK_REQUIRE(g_attn_prof == nullptr, "fk_attn_backward_tc_profile: no stall-accounting build at head_dim 64");
+  FK_REQUIRE(!(parts & 2) || (dk && dv), "fk_attn_backward_tc: dK/dV needs dk, dv");
+  FK_REQUIRE(!(parts & 4) || dq, "fk_attn_backward_tc: dQ needs dq");
+  FK_REQUIRE(dq_ts % 8 == 0 && dq_bs % 8 == 0 && dk_ts % 8 == 0 && dk_bs % 8 == 0 && dv_ts % 8 == 0 && dv_bs % 8 == 0,
+             "fk_attn_backward_tc: gradient strides must keep 16-byte alignment");
+  static bool attr_set_dev[FK_MAX_DEVICES];
+  bool& attr_set = attr_set_dev[fk_device_ordinal()];
+  if (!attr_set) {
+    if (cudaFuncSetAttribute(attn_bwd_tc64_kernel<MODE_DKV>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem64::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_bwd_tc64_kernel<MODE_DQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem64::total) != cudaSuccess) {
+      fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
+      return FK_ERR_CUDA;
+    }
+    attr_set = true;
+  }
+  CUtensorMap mQ128, mDO128, mK128, mV128, mQ64, mDO64, mK64, mV64, mAug64, mAug128;
+  int rc = 0;
+  rc |= make_tmap_heads_sw128(&mQ128, q, B, S, H, q_bs, q_ts, kRows);
+  rc |= make_tmap_heads_sw128(&mDO128, d_o, B, S, H, do_bs, do_ts, kRows);
+  rc |= make_tmap_heads_sw128(&mK128, k, B, S, H, k_bs, k_ts, kRows);
+  rc |= make_tmap_heads_sw128(&mV128, v, B, S, H, v_bs, v_ts, kRows);
+  rc |= make_tmap_heads_sw128(&mQ64, q, B, S, H, q_bs, q_ts, kCols);
+  rc |= make_tmap_heads_sw128(&mDO64, d_o, B, S, H, do_bs, do_ts, kCols);
+  rc |= make_tmap_heads_sw128(&mK64, k, B, S, H, k_bs, k_ts, kCols);
+  rc |= make_tmap_heads_sw128(&mV64, v, B, S, H, v_bs, v_ts, kCols);
+  rc |= make_tmap_aug_sw32(&mAug64, aug, B, S, H, kCols);
+  rc |= make_tmap_aug_sw32(&mAug128, aug, B, S, H, kRows);
+  if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
+  const long long n_items = static_cast<long long>((S + kRows - 1) / kRows) * H * B;
+  FK_REQUIRE(n_items < (1ll << 31), "fk_attn_backward_tc: too many work items");
+  const dim3 grid(static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count()), 1, 1);
+  TcParams p = {};
+  p.lse = lse; p.delta = delta;
+  p.B = B; p.H = H; p.S_row = S; p.S_col = S; p.Sq = S; p.scale = scale; p.scale_log2 = scale * 1.4426950408889634f;
+  p.mn_major = 1;
+  p.fold = 1;
+  p.rope_table = reinterpret_cast<const float2*>(rope_table); p.rope_pos = rope_pos; p.rope_len = rope_len; p.rope_offset = rope_offset;
+  int n = 0;
+  if (parts & 2) {
+    TcParams pk = p;
+    pk.row_id = kid; pk.col_id = qid; pk.row_min = kmin; pk.row_max = kmax; pk.col_min = qmin; pk.col_max = qmax;
+    pk.out0 = static_cast<__nv_bfloat16*>(dv); pk.o0_bs = dv_bs; pk.o0_ts = dv_ts;
+    pk.out1 = static_cast<__nv_bfloat16*>(dk); pk.o1_bs = dk_bs; pk.o1_ts = dk_ts;
+    pk.items = counters;
+    attn_bwd_tc64_kernel<MODE_DKV><<<grid, kTcThreads, TcSmem64::total, stream>>>(mK128, mV128, mQ64, mDO64, mAug64, pk);
+    FK_CHECK_LAUNCH();
+    ++n;
+  }
+  if (parts & 4) {
+    TcParams pq = p;
+    pq.row_id = qid; pq.col_id = kid; pq.row_min = qmin; pq.row_max = qmax; pq.col_min = kmin; pq.col_max = kmax;
+    pq.out1 = static_cast<__nv_bfloat16*>(dq); pq.o1_bs = dq_bs; pq.o1_ts = dq_ts;
+    pq.items = counters + 2;
+    attn_bwd_tc64_kernel<MODE_DQ><<<grid, kTcThreads, TcSmem64::total, stream>>>(mQ128, mDO128, mK64, mV64, mAug128, pq);
+    FK_CHECK_LAUNCH();
+    ++n;
+  }
+  fk_count_launch(n);
+  return FK_OK;
+}
 
 // parts: 2 = dK/dV (needs qt, dot), 4 = dQ (needs kt).  delta must already hold rowsum(dO * O) (fk_attn_backward parts=1).
 FK_API int fk_attn_backward_tc(const void* q, const void* k, const void* v, const void* d_o, const void* qt, const void* kt,
@@ -1437,7 +2375,7 @@ FK_API int fk_attn_backward_tc_profile(const void* q, const void* k, const void*
                                const int* rope_pos, int rope_offset, int parts, unsigned int* counters, long long* g_attn_prof,
                                int g_attn_prof_mode, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(head_dim == 32, "fk_attn_backward_tc: only head_dim 32 is built");
+  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_attn_backward_tc: head_dim must be 32 or 64");
   FK_REQUIRE(counters != nullptr, "fk_attn_backward_tc: counters (4 zero-initialised uint32, one set per launch in flight) is null");
   FK_REQUIRE(rope_table == nullptr || rope_len > 0, "fk_attn_backward_tc: rope_len must be positive with a rope table");
   FK_REQUIRE(q && k && v && d_o && lse && delta && B > 0 && H > 0 && S > 0, "fk_attn_backward_tc: bad argument");
@@ -1446,6 +2384,10 @@ FK_API int fk_attn_backward_tc_profile(const void* q, const void* k, const void*
   FK_REQUIRE(qid == nullptr || (qmin && qmax && kmin && kmax), "fk_attn_backward_tc: label ranges missing");
   FK_REQUIRE((S + kCols - 1) / kCols <= kMaxTiles, "fk_attn_backward_tc: sequence too long");
   FK_REQUIRE(Sp >= S && Sp % 8 == 0, "fk_attn_backward_tc: Sp must be >= S and a multiple of 8");
+  if (head_dim == 64)
+    return attn_backward_tc64(q, k, v, d_o, qt, kt, dot, aug, dq, dk, dv, B, H, S, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, do_bs,
+                              do_ts, dq_bs, dq_ts, dk_bs, dk_ts, dv_bs, dv_ts, qid, kid, qmin, qmax, kmin, kmax, scale, lse,
+                              delta, rope_table, rope_len, rope_pos, rope_offset, parts, counters, g_attn_prof, stream);
   static bool attr_set_dev[FK_MAX_DEVICES];
   bool& attr_set = attr_set_dev[fk_device_ordinal()];
   if (!attr_set) {
@@ -1543,16 +2485,19 @@ FK_API int fk_attn_backward_tc_profile(const void* q, const void* k, const void*
   return FK_OK;
 }
 
-// delta = rowsum(dO * O) and the statistics rows the folded backward takes (see attn_aug_kernel): o / d_o bf16 [B, S, H, 32]
-// with strides in elements, lse fp32 [B, H, S] (log2 domain, from the forward), delta fp32 [B, H, S], aug bf16 [B, H, S, 16].
+// delta = rowsum(dO * O) and the statistics rows the folded backward takes (see attn_aug_kernel): o / d_o bf16
+// [B, S, H, head_dim] (32 or 64) with strides in elements, lse fp32 [B, H, S] (log2 domain, from the forward), delta fp32
+// [B, H, S], aug bf16 [B, H, S, 16].
 FK_API int fk_attn_aug(const void* o, const void* d_o, const float* lse, float* delta, void* aug, int B, int H, int S,
-                       long long o_bs, long long o_ts, long long do_bs, long long do_ts, float scale, void* stream_) {
+                       int head_dim, long long o_bs, long long o_ts, long long do_bs, long long do_ts, float scale, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_attn_aug: head_dim must be 32 or 64");
   FK_REQUIRE(o && d_o && lse && delta && aug && B > 0 && H > 0 && S > 0 && scale > 0.f, "fk_attn_aug: bad argument");
   FK_REQUIRE(o_ts % 8 == 0 && do_ts % 8 == 0 && o_bs % 8 == 0 && do_bs % 8 == 0, "fk_attn_aug: strides must keep 16-byte alignment");
   FK_REQUIRE((reinterpret_cast<uintptr_t>(aug) & 31) == 0, "fk_attn_aug: aug must be 32-byte aligned");
   const long long n = static_cast<long long>(B) * S * H;
-  attn_aug_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(
+  auto kern = head_dim == 64 ? attn_aug64_kernel : attn_aug_kernel;
+  kern<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(
       static_cast<const __nv_bfloat16*>(o), static_cast<const __nv_bfloat16*>(d_o), lse, delta, static_cast<__nv_bfloat16*>(aug), B, H, S,
       o_bs, o_ts, do_bs, do_ts, 1.f / (scale * 1.4426950408889634f));
   FK_CHECK_LAUNCH();
@@ -1567,7 +2512,7 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
                               const int* qmax, const int* kmin, const int* kmax, float scale, unsigned int* counters,
                               void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(head_dim == 32, "fk_attn_forward_tc: only head_dim 32 is built");
+  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_attn_forward_tc: head_dim must be 32 or 64");
   FK_REQUIRE(counters != nullptr, "fk_attn_forward_tc: counters (2 zero-initialised uint32, one pair per launch in flight) is null");
   FK_REQUIRE(q && k && v && out && B > 0 && H > 0 && S > 0, "fk_attn_forward_tc: bad argument");
   FK_REQUIRE((qid == nullptr) == (kid == nullptr), "fk_attn_forward_tc: qid and kid go together");
@@ -1577,7 +2522,8 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   static bool attr_set_dev[FK_MAX_DEVICES];
   bool& attr_set = attr_set_dev[fk_device_ordinal()];
   if (!attr_set) {
-    if (cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess) {
+    if (cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
       fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
       return FK_ERR_CUDA;
     }
@@ -1585,9 +2531,10 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   }
   CUtensorMap mQ, mK, mV;
   int rc = 0;
-  rc |= make_tmap_heads_sw64(&mQ, q, B, S, H, q_bs, q_ts, 128);
-  rc |= make_tmap_heads_sw64(&mK, k, B, S, H, k_bs, k_ts, kFwdTileK);
-  rc |= make_tmap_heads_sw64(&mV, v, B, S, H, v_bs, v_ts, kFwdTileK);
+  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : make_tmap_heads_sw64;
+  rc |= make_map(&mQ, q, B, S, H, q_bs, q_ts, 128);
+  rc |= make_map(&mK, k, B, S, H, k_bs, k_ts, kFwdTileK);
+  rc |= make_map(&mV, v, B, S, H, v_bs, v_ts, kFwdTileK);
   if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
   FwdParams p = {};
   p.qid = qid; p.kid = kid; p.qmin = qmin; p.qmax = qmax; p.kmin = kmin; p.kmax = kmax;
@@ -1597,7 +2544,9 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   // persistent CTAs: one per SM (or per work item when there are fewer), looping over (256-query block, head, trial) items
   const long long n_items = static_cast<long long>((S + 255) / 256) * H * B;
   FK_REQUIRE(n_items < (1ll << 31), "fk_attn_forward_tc: too many work items");
-  attn_fwd_tc_kernel<<<static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count()), kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
+  const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
+  if (head_dim == 64) attn_fwd_tc64_kernel<<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
+  else attn_fwd_tc_kernel<<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;

@@ -37,7 +37,9 @@ constexpr int kASlabBytes = 128 * 128;     // 128 rows x 64 bf16
 constexpr int kBSlabBytes = 256 * 128;     // 256 rows x 64 bf16
 constexpr int kGemmSmemLimit = 232448 - 1024;
 
-enum { EPI_STORE = 0, EPI_ROPE = 1, EPI_SWIGLU = 2, EPI_SWIGLU_BWD = 3 };
+enum { EPI_STORE = 0, EPI_ROPE = 1, EPI_SWIGLU = 2, EPI_SWIGLU_BWD = 3, EPI_ROPE64 = 4 };
+// (cos, sin) pairs one epilogue thread holds for its row: one head of 32 columns, or of 64 columns (EPI_ROPE64)
+template <int EPI> constexpr int rope_pairs() { return EPI == EPI_ROPE64 ? 32 : 16; }
 
 struct GemmParams {
   __nv_bfloat16* C;          // [M, N] (EPI_SWIGLU: the fused projection h13; EPI_SWIGLU_BWD: unused)
@@ -47,7 +49,7 @@ struct GemmParams {
   const __nv_bfloat16* aux;  // EPI_SWIGLU_BWD: h13 [M, 2N]
   long long ld_aux;
   const float* bias;         // [N] or null (EPI_STORE)
-  const float2* rope_table;  // EPI_ROPE: [rope_len][16] (cos, sin)
+  const float2* rope_table;  // EPI_ROPE: [rope_len][16] (cos, sin); EPI_ROPE64: [rope_len][32]
   const int* rope_pos;       // [M] or null: position of row m = rope_pos ? rope_pos[m] : (m % rope_S) + rope_offset
   int rope_len, rope_offset, rope_cols, rope_S;
   long long M;
@@ -210,10 +212,10 @@ __device__ __forceinline__ void warp_load_finish_32x64(uint8_t* stg, int lane, c
 }
 
 // One 128 x 256 accumulator tile of the A-resident kernels: this warp's 32 rows (TMEM lane quarter) x 128 columns (half ch).
-template <int EPI, class Release>
+template <int EPI, int NCS, class Release>
 __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUtensorMap& tm_c, const CUtensorMap& tm_c2, uint8_t* stg,
                                                   int stg_tiles, uint32_t& stg_cnt, int lane, int ch, uint32_t taddr, int n0,
-                                                  long long row0, const float2 (&cs)[16], uint64_t* full_bar, uint32_t full_parity,
+                                                  long long row0, const float2 (&cs)[NCS], uint64_t* full_bar, uint32_t full_parity,
                                                   Release release) {
     const long long row = row0 + lane;
     (void)row;
@@ -223,7 +225,7 @@ __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUt
       release();
       return;
     }
-    if (EPI == EPI_STORE || EPI == EPI_ROPE) {
+    if (EPI == EPI_STORE || EPI == EPI_ROPE || EPI == EPI_ROPE64) {
       mbar_wait(full_bar, full_parity);
       tc_fence_after();
 #pragma unroll
@@ -240,13 +242,14 @@ __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUt
         for (int hc = 0; hc < 2; ++hc) {
           float v[32];
           if (hc == 0) to_f32(r0, v); else to_f32(r1, v);
-          if (EPI == EPI_ROPE) {
+          if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
             if (col + hc * 32 < p.rope_cols) {
+              const int c0 = (EPI == EPI_ROPE64) ? hc * 16 : 0;     // a 64-column head spans both 32-column halves
 #pragma unroll
               for (int i = 0; i < 16; ++i) {
                 const float x0 = v[2 * i], x1 = v[2 * i + 1];
-                v[2 * i] = x0 * cs[i].x - x1 * cs[i].y;
-                v[2 * i + 1] = x0 * cs[i].y + x1 * cs[i].x;
+                v[2 * i] = x0 * cs[c0 + i].x - x1 * cs[c0 + i].y;
+                v[2 * i + 1] = x0 * cs[c0 + i].y + x1 * cs[c0 + i].x;
               }
             }
           } else if (p.bias != nullptr && col + hc * 32 < p.N) {
@@ -535,13 +538,14 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
       const int blk = grp * static_cast<int>(cl) + static_cast<int>(rank);
       const long long row0 = ((p.dbg & 8) ? 0ll : static_cast<long long>(blk) * 128) + q * 32;     // first row of this warp (dbg 8: every block writes rows 0..127 -> L2 only)
       const long long row = row0 + lane;
-      float2 cs[16];
-      if (EPI == EPI_ROPE) {
+      constexpr int kCs = rope_pairs<EPI>();
+      float2 cs[kCs];
+      if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
         int ps = 0;
         if (row < p.M) ps = p.rope_pos ? p.rope_pos[row] : static_cast<int>(row % p.rope_S) + p.rope_offset;
         ps = min(max(ps, 0), p.rope_len - 1);
 #pragma unroll
-        for (int i = 0; i < 16; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * 16 + i);
+        for (int i = 0; i < kCs; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * kCs + i);
       }
       for (int t = 0; t < p.ntile; ++t, ++tc) {
         const uint32_t as = tc & 1;
@@ -687,13 +691,14 @@ gemm_res2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
       const int blk = grp * 2 + static_cast<int>(rank);
       const long long row0 = static_cast<long long>(blk) * 128 + q * 32;
       const long long row = row0 + lane;
-      float2 cs[16];
-      if (EPI == EPI_ROPE) {
+      constexpr int kCs = rope_pairs<EPI>();
+      float2 cs[kCs];
+      if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
         int ps = 0;
         if (row < p.M) ps = p.rope_pos ? p.rope_pos[row] : static_cast<int>(row % p.rope_S) + p.rope_offset;
         ps = min(max(ps, 0), p.rope_len - 1);
 #pragma unroll
-        for (int i = 0; i < 16; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * 16 + i);
+        for (int i = 0; i < kCs; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * kCs + i);
       }
       for (int t = 0; t < p.ntile; ++t, ++tc) {
         const uint32_t as = tc & 1;
@@ -1046,7 +1051,7 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
   FK_REQUIRE(K % 8 == 0 && lda % 8 == 0 && ldb % 8 == 0 && lda > 0 && ldb >= K, "fk_gemm_nt: K and the leading dimensions must be multiples of 8 (16-byte rows)");
   FK_REQUIRE(N % 32 == 0, "fk_gemm_nt: N must be a multiple of 32");
   FK_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0, "fk_gemm_nt: operands must be 16-byte aligned");
-  FK_REQUIRE(epilogue >= EPI_STORE && epilogue <= EPI_SWIGLU_BWD, "fk_gemm_nt: unknown epilogue");
+  FK_REQUIRE(epilogue >= EPI_STORE && epilogue <= EPI_ROPE64, "fk_gemm_nt: unknown epilogue");
   GemmParams p = {};
   p.C = static_cast<__nv_bfloat16*>(C); p.ldc = ldc;
   p.C2 = static_cast<__nv_bfloat16*>(C2); p.ldc2 = ldc2;
@@ -1062,10 +1067,11 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
   }
   p.nslab = (K + 63) / 64;
   p.ntile = (N + 255) / 256;
-  if (epilogue == EPI_STORE || epilogue == EPI_ROPE || epilogue == EPI_SWIGLU)
+  if (epilogue == EPI_STORE || epilogue == EPI_ROPE || epilogue == EPI_ROPE64 || epilogue == EPI_SWIGLU)
     FK_REQUIRE(C && ldc % 8 == 0 && ldc >= N && (reinterpret_cast<uintptr_t>(C) & 15) == 0, "fk_gemm_nt: C must be 16-byte aligned with ldc % 8 == 0");
-  if (epilogue == EPI_ROPE) {
-    FK_REQUIRE(rope_table && rope_len > 0 && rope_cols % 32 == 0 && rope_cols <= N && (rope_pos || rope_S > 0), "fk_gemm_nt: bad rope arguments");
+  if (epilogue == EPI_ROPE || epilogue == EPI_ROPE64) {
+    FK_REQUIRE(rope_table && rope_len > 0 && rope_cols % (epilogue == EPI_ROPE64 ? 64 : 32) == 0 && rope_cols <= N && (rope_pos || rope_S > 0),
+               "fk_gemm_nt: bad rope arguments");
     FK_REQUIRE(rope_pos != nullptr || (rope_offset >= 0 && static_cast<long long>(rope_offset) + (M < rope_S ? M : rope_S) <= rope_len),
                "fk_gemm_nt: token positions fall outside the rope table");
   }
@@ -1118,7 +1124,7 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
       attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
       cfg.attrs = attr;
       cfg.numAttrs = 1;
-      static bool done2[4][FK_MAX_DEVICES];
+      static bool done2[5][FK_MAX_DEVICES];
       int r2 = FK_OK;
       cudaError_t le = cudaSuccess;
       switch (epilogue) {
@@ -1129,6 +1135,10 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
         case EPI_ROPE:
           if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_ROPE>, done2[1][dev], kGemmSmemLimit)) != FK_OK) return r2;
           le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_ROPE>, ta, tb, tc, tc2, p);
+          break;
+        case EPI_ROPE64:
+          if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_ROPE64>, done2[4][dev], kGemmSmemLimit)) != FK_OK) return r2;
+          le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_ROPE64>, ta, tb, tc, tc2, p);
           break;
         case EPI_SWIGLU:
           if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_SWIGLU>, done2[2][dev], kGemmSmemLimit)) != FK_OK) return r2;
@@ -1170,7 +1180,7 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
     const long long n_groups = (n_blocks + cl - 1) / cl;
     const long long max_clusters = G / cl;
     const unsigned grid = static_cast<unsigned>((n_groups < max_clusters ? n_groups : max_clusters) * cl);
-    static bool done[4][FK_MAX_DEVICES];
+    static bool done[5][FK_MAX_DEVICES];
     int r2 = FK_OK;
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid, 1, 1);
@@ -1193,6 +1203,10 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
       case EPI_ROPE:
         if ((r2 = set_smem_attr(gemm_res_kernel<EPI_ROPE>, done[1][dev], kGemmSmemLimit)) != FK_OK) return r2;
         le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_ROPE>, ta, tb, tc, tc2, p);
+        break;
+      case EPI_ROPE64:
+        if ((r2 = set_smem_attr(gemm_res_kernel<EPI_ROPE64>, done[4][dev], kGemmSmemLimit)) != FK_OK) return r2;
+        le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_ROPE64>, ta, tb, tc, tc2, p);
         break;
       case EPI_SWIGLU:
         if ((r2 = set_smem_attr(gemm_res_kernel<EPI_SWIGLU>, done[2][dev], kGemmSmemLimit)) != FK_OK) return r2;

@@ -4,7 +4,7 @@ Functional wrappers (``gemm_nt``, ``gemm_tn``) and the ``torch.autograd.Function
 
 * ``linear``       -- ``nn.Linear`` (models/brainformer.py:171 ``project``, ``to_signals``, ...): y = x W^T (+ b);
 * ``qkv_rope``     -- qw / kw / vw as ONE projection (brainformer.py:141-143) with ``apply_rope`` (:70-91, :156-158) applied
-                      to the q | k columns in the GEMM epilogue;
+                      to the q | k columns in the GEMM epilogue (heads of 32 or 64 columns);
 * ``swiglu_mlp``   -- ``w2(silu(w1 x) * w3 x)`` (brainformer.py:119-124): the w1 | w3 projection forms the gate in its
                       epilogue, the backward's d-gated GEMM applies the SwiGLU derivative in its epilogue.
 
@@ -22,7 +22,8 @@ import torch
 from ._lib import FkError, check, lib, on_tensor_device, ptr, require_cuda, require_device, stream, timed
 
 BF16 = torch.bfloat16
-EPI_STORE, EPI_ROPE, EPI_SWIGLU, EPI_SWIGLU_BWD = 0, 1, 2, 3
+EPI_STORE, EPI_ROPE, EPI_SWIGLU, EPI_SWIGLU_BWD, EPI_ROPE64 = 0, 1, 2, 3, 4
+ROPE_EPILOGUE = {32: EPI_ROPE, 64: EPI_ROPE64}          # head width -> RoPE epilogue of the fused q | k | v projection
 # backward of the SwiGLU MLP: "split" = d-gated GEMM + one streaming derivative pass (default, faster); "fused" = the
 # derivative in the GEMM epilogue (kept for A/B measurements and tested in tests/test_gemm_gpu.py)
 MLP_BWD = os.environ.get("FK_MLP_BWD", "split")
@@ -42,7 +43,7 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
             gated: Optional[torch.Tensor] = None, h13: Optional[torch.Tensor] = None, rope=None, rope_cols: int = 0,
             rope_S: int = 0, name: str = "gemm_nt"):
     """C [M, N] bf16 = a [M, K] @ b [N, K]^T on tcgen05 (fp32 accumulate).  See include/fk_b200.h (fk_gemm_nt) for the
-    epilogues.  Returns C (EPI_STORE / EPI_ROPE), (h13, gated) (EPI_SWIGLU) or dh13 (EPI_SWIGLU_BWD)."""
+    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64), (h13, gated) (EPI_SWIGLU) or dh13 (EPI_SWIGLU_BWD)."""
     require_cuda(a, b)
     require_device()
     if a.dtype != BF16 or b.dtype != BF16:
@@ -56,7 +57,7 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
     dev = a.device
     C = C2 = aux = None
     ldc = ldc2 = ld_aux = 0
-    if epilogue in (EPI_STORE, EPI_ROPE):
+    if epilogue in (EPI_STORE, EPI_ROPE, EPI_ROPE64):
         C = torch.empty(M, N, device=dev, dtype=BF16)
         ldc = N
     elif epilogue == EPI_SWIGLU:
@@ -73,7 +74,7 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
     if bias is not None:
         bias_f = bias.detach().float().contiguous()
     table, pos, rope_len, rope_off = None, None, 0, 0
-    if epilogue == EPI_ROPE:
+    if epilogue in (EPI_ROPE, EPI_ROPE64):
         table, pos, rope_len, rope_off = rope.table, rope.pos, rope.table.shape[0], rope.offset
         if pos is not None:
             pos = pos.reshape(-1)
@@ -172,7 +173,10 @@ class _QKVRopeFn(torch.autograd.Function):
         w = torch.cat([wq.detach(), wk.detach(), wv.detach()], dim=0).to(BF16)
         inner = wq.shape[0]
         if rope is not None:
-            qkv = gemm_nt(x2, w, None, EPI_ROPE, rope=rope, rope_cols=2 * inner, rope_S=S, name="gemm_qkv_rope")
+            epi = ROPE_EPILOGUE.get(inner // n_heads)
+            if epi is None:
+                raise FkError(f"qkv_rope: the RoPE epilogue takes heads of 32 or 64 columns, not {inner // n_heads}")
+            qkv = gemm_nt(x2, w, None, epi, rope=rope, rope_cols=2 * inner, rope_S=S, name="gemm_qkv_rope")
         else:
             qkv = gemm_nt(x2, w, None, EPI_STORE, name="gemm_qkv_rope")
         ctx.save_for_backward(x2, w)
