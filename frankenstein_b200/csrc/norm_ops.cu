@@ -107,13 +107,16 @@ norm_fwd_kernel(const TIn* __restrict__ x, const float* __restrict__ w, const fl
 // and stores the current one, so every warp keeps a full row (5 KB at D = 512) in flight all the time -- with the loads
 // of one row at a time and the residual gradient fetched after the reduction (two dependent DRAM round trips per row)
 // the kernel sat at half of the HBM peak.  One CTA of kNormBwdWarps warps per SM, up to 168 registers per thread.
+// AHEAD = false (D > 512): the next row's registers, the current row and the dw/db accumulators of MAXV = 8 do not fit
+// in 168 registers, so the warp loads its current row at the top of the iteration instead (from L2 when the row is a
+// multiple of 16 bytes: the bulk prefetch below puts it there).
 constexpr int kNormBwdWarps = 12;
 #ifndef FK_NORM_BWD_AHEAD
 #define FK_NORM_BWD_AHEAD 2
 #endif
 constexpr int kNormBwdAhead = FK_NORM_BWD_AHEAD;     // rows per warp in flight (1 in registers, the rest on their way into L2)
 
-template <typename TIn, typename TG, typename TDx, int MAXV>
+template <typename TIn, typename TG, typename TDx, int MAXV, bool AHEAD = true>
 __global__ void __launch_bounds__(kNormBwdWarps * 32, 1)
 norm_bwd_kernel(const TIn* __restrict__ x, const TG* __restrict__ g, const float* __restrict__ w, const float* __restrict__ mean_in,
                 const float* __restrict__ rstd_in, TDx* __restrict__ dx, float* __restrict__ dw_part, float* __restrict__ db_part,
@@ -136,6 +139,13 @@ norm_bwd_kernel(const TIn* __restrict__ x, const TG* __restrict__ g, const float
   long long row = static_cast<long long>(blockIdx.x) * kNormBwdWarps + warp;
   const bool has_res = g_res != nullptr;
   float nx[MAXV][4], ng[MAXV][4], nr[MAXV][4], nmean = 0.f, nrstd = 0.f;
+  auto clear = [&]() {
+#pragma unroll
+    for (int i = 0; i < MAXV; ++i) {
+#pragma unroll
+      for (int j = 0; j < 4; ++j) { nx[i][j] = 0.f; ng[i][j] = 0.f; nr[i][j] = 0.f; }
+    }
+  };
   auto fetch = [&](long long r) {
     nmean = rms ? 0.f : mean_in[r];
     nrstd = rstd_in[r];
@@ -149,11 +159,7 @@ norm_bwd_kernel(const TIn* __restrict__ x, const TG* __restrict__ g, const float
       }
     }
   };
-#pragma unroll
-  for (int i = 0; i < MAXV; ++i) {
-#pragma unroll
-    for (int j = 0; j < 4; ++j) { nx[i][j] = 0.f; ng[i][j] = 0.f; nr[i][j] = 0.f; }
-  }
+  clear();
   // rows further ahead are pulled into L2 by bulk prefetches (one lane, no registers), so that the register loads of the
   // next row find them there: kNormBwdAhead rows per warp on their way from DRAM at any time
   const bool pf_ok = (D * sizeof(TIn)) % 16 == 0 && (D * sizeof(TG)) % 16 == 0;
@@ -164,11 +170,12 @@ norm_bwd_kernel(const TIn* __restrict__ x, const TG* __restrict__ g, const float
     if (has_res)
       asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(g_res + r * D), "r"(static_cast<uint32_t>(D * sizeof(float))) : "memory");
   };
-  if (row < M) fetch(row);
+  if (AHEAD && row < M) fetch(row);
 #pragma unroll
   for (int a = 1; a < kNormBwdAhead; ++a) prefetch_l2(row + a * stride);
   for (; row < M; row += stride) {
     prefetch_l2(row + kNormBwdAhead * stride);
+    if (!AHEAD) { clear(); fetch(row); }      // (cleared here, so that no register carries over from the last row)
     float xh[MAXV][4], gv[MAXV][4], gr[MAXV][4];
     const float mean = nmean, rstd = nrstd;
 #pragma unroll
@@ -176,7 +183,7 @@ norm_bwd_kernel(const TIn* __restrict__ x, const TG* __restrict__ g, const float
 #pragma unroll
       for (int j = 0; j < 4; ++j) { xh[i][j] = nx[i][j]; gv[i][j] = ng[i][j]; gr[i][j] = nr[i][j]; }
     }
-    if (row + stride < M) fetch(row + stride);
+    if (AHEAD && row + stride < M) fetch(row + stride);
     float s1 = 0.f, s2 = 0.f;
 #pragma unroll
     for (int i = 0; i < MAXV; ++i) {
@@ -328,7 +335,20 @@ static int launch_norm_bwd(const void* x, const void* g, const float* w, const f
   if (D <= 128) norm_bwd_kernel<TIn, TG, TDx, 1><<<grid, kNormBwdWarps * 32, smem, stream>>>(xi, gi, w, mean, rstd, dxo, dwp, dbp, M, D, rms, g_res, dx_bf16);
   else if (D <= 256) norm_bwd_kernel<TIn, TG, TDx, 2><<<grid, kNormBwdWarps * 32, smem, stream>>>(xi, gi, w, mean, rstd, dxo, dwp, dbp, M, D, rms, g_res, dx_bf16);
   else if (D <= 512) norm_bwd_kernel<TIn, TG, TDx, 4><<<grid, kNormBwdWarps * 32, smem, stream>>>(xi, gi, w, mean, rstd, dxo, dwp, dbp, M, D, rms, g_res, dx_bf16);
-  else return FK_ERR_UNSUPPORTED;
+  else if (D <= 1024) {
+    // above D = 944 the shared memory exceeds the default 48 KB limit of a launch: opt in once per device
+    static bool done[FK_MAX_DEVICES];
+    const int dev = fk_device_ordinal();
+    if (!done[dev]) {
+      if (cudaFuncSetAttribute(norm_bwd_kernel<TIn, TG, TDx, 8, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                               (kNormBwdWarps + 1) * 1024 * static_cast<int>(sizeof(float))) != cudaSuccess) {
+        fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
+        return FK_ERR_CUDA;
+      }
+      done[dev] = true;
+    }
+    norm_bwd_kernel<TIn, TG, TDx, 8, false><<<grid, kNormBwdWarps * 32, smem, stream>>>(xi, gi, w, mean, rstd, dxo, dwp, dbp, M, D, rms, g_res, dx_bf16);
+  } else return FK_ERR_UNSUPPORTED;
   return FK_OK;
 }
 
@@ -404,7 +424,8 @@ FK_API int fk_norm_backward(const void* x, int x_dtype, const void* g, int g_dty
   if (x_dtype == 0 && g_dtype == 1 && dx_dtype == 0) rc = launch_norm_bwd<float, __nv_bfloat16, float>(x, g, weight, mean, rstd, dx, dw_part, db_part, M, D, rms, grid, stream);
   else if (x_dtype == 0 && g_dtype == 0 && dx_dtype == 0) rc = launch_norm_bwd<float, float, float>(x, g, weight, mean, rstd, dx, dw_part, db_part, M, D, rms, grid, stream);
   else if (x_dtype == 1 && g_dtype == 1 && dx_dtype == 1) rc = launch_norm_bwd<__nv_bfloat16, __nv_bfloat16, __nv_bfloat16>(x, g, weight, mean, rstd, dx, dw_part, db_part, M, D, rms, grid, stream);
-  if (rc != FK_OK) { fk_set_last_error("fk_norm_backward: unsupported dtype combination or D > 512", __FILE__, __LINE__); return rc; }
+  if (rc == FK_ERR_UNSUPPORTED) fk_set_last_error("fk_norm_backward: unsupported dtype combination or D > 1024", __FILE__, __LINE__);
+  if (rc != FK_OK) return rc;
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;
@@ -479,7 +500,8 @@ FK_API int fk_add_norm_backward(const float* x_new, const void* g_y, int g_dtype
   int rc = FK_ERR_UNSUPPORTED;
   if (g_dtype == 1) rc = launch_norm_bwd<float, __nv_bfloat16, float>(x_new, g_y, weight, mean, rstd, dx, dw_part, db_part, M, D, rms, grid, stream, g_res, db16);
   else if (g_dtype == 0) rc = launch_norm_bwd<float, float, float>(x_new, g_y, weight, mean, rstd, dx, dw_part, db_part, M, D, rms, grid, stream, g_res, db16);
-  if (rc != FK_OK) { fk_set_last_error("fk_add_norm_backward: unsupported dtype or D > 512", __FILE__, __LINE__); return rc; }
+  if (rc == FK_ERR_UNSUPPORTED) fk_set_last_error("fk_add_norm_backward: unsupported dtype or D > 1024", __FILE__, __LINE__);
+  if (rc != FK_OK) return rc;
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;

@@ -14,6 +14,7 @@ gradient, makes the transposed copy the NT kernel wants -- a few MB).  Weight gr
 """
 from __future__ import annotations
 
+import math
 import os
 from typing import Optional
 
@@ -41,9 +42,10 @@ def _as2d(x: torch.Tensor) -> torch.Tensor:
 @on_tensor_device
 def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = None, epilogue: int = EPI_STORE, *,
             gated: Optional[torch.Tensor] = None, h13: Optional[torch.Tensor] = None, rope=None, rope_cols: int = 0,
-            rope_S: int = 0, name: str = "gemm_nt"):
+            rope_S: int = 0, lead: Optional[tuple] = None, name: str = "gemm_nt"):
     """C [M, N] bf16 = a [M, K] @ b [N, K]^T on tcgen05 (fp32 accumulate).  See include/fk_b200.h (fk_gemm_nt) for the
-    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64), (h13, gated) (EPI_SWIGLU) or dh13 (EPI_SWIGLU_BWD)."""
+    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64), (h13, gated) (EPI_SWIGLU) or dh13 (EPI_SWIGLU_BWD).
+    lead (EPI_STORE): C is allocated as [*lead, N] (prod(lead) = M), a tensor of its own rather than a view of [M, N]."""
     require_cuda(a, b)
     require_device()
     if a.dtype != BF16 or b.dtype != BF16:
@@ -57,8 +59,10 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
     dev = a.device
     C = C2 = aux = None
     ldc = ldc2 = ld_aux = 0
+    if lead is not None and (epilogue != EPI_STORE or math.prod(lead) != M):
+        raise FkError(f"gemm_nt: output shape {(*lead, N)} does not hold [{M}, {N}]")
     if epilogue in (EPI_STORE, EPI_ROPE, EPI_ROPE64):
-        C = torch.empty(M, N, device=dev, dtype=BF16)
+        C = torch.empty(*(lead if lead is not None else (M,)), N, device=dev, dtype=BF16)
         ldc = N
     elif epilogue == EPI_SWIGLU:
         C = torch.empty(M, N, device=dev, dtype=BF16)
@@ -126,12 +130,14 @@ class _LinearFn(torch.autograd.Function):
     def forward(ctx, x, weight, bias):
         x2 = _as2d(x)
         wb = weight.detach().to(BF16).contiguous()
-        y = gemm_nt(x2, wb, bias, EPI_STORE, name="gemm_linear")
+        # y is allocated in x's leading shape rather than returned as a view: attention_qkv rotates q and k of a fused
+        # q | k | v projection in place, which autograd refuses on a view
+        y = gemm_nt(x2, wb, bias, EPI_STORE, lead=tuple(x.shape[:-1]), name="gemm_linear")
         ctx.save_for_backward(x2, wb)
         ctx.in_shape, ctx.in_dtype, ctx.w_dtype = x.shape, x.dtype, weight.dtype
         ctx.has_bias = bias is not None
         ctx.b_dtype = bias.dtype if bias is not None else None
-        return y.view(*x.shape[:-1], weight.shape[0])
+        return y
 
     @staticmethod
     @on_tensor_device

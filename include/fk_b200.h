@@ -110,7 +110,8 @@ int fk_masked_l1_backward(const void* pred, int dtype, const float* gt, const un
 
 /* ---- transformer blocks (models/brainformer.py, models/simple_mae) ---------------------------- */
 /* nn.LayerNorm (brainformer.py:237-239,287) / RMSNorm (simple_mae:181-192).  dtype codes 0=f32 1=bf16.
- * Supported (x, y): (f32,bf16) (f32,f32) (bf16,bf16).  mean/rstd: [M] fp32 saved for backward (mean unused for rms). */
+ * Supported (x, y): (f32,bf16) (f32,f32) (bf16,bf16).  mean/rstd: [M] fp32 saved for backward (mean unused for rms).
+ * D % 4 == 0 and D <= 1024 (forward and backward, also for fk_add_norm_*). */
 int fk_norm_forward(const void* x, int x_dtype, const float* weight, const float* bias, void* y, int y_dtype,
                     float* mean, float* rstd, long long M, int D, float eps, int rms, void* stream);
 /* dw_part/db_part: [fk_norm_backward_grid(), D] partial sums (caller reduces over dim 0).
