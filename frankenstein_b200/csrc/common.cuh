@@ -174,15 +174,6 @@ __device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* m
       : "memory");
 }
 
-// Same with multicast: the box lands at the same shared-memory offset, and completes transaction bytes on the mbarrier at the
-// same offset, in every CTA of the cluster whose bit is set in cta_mask.
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, uint16_t cta_mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "h"(cta_mask)
-      : "memory");
-}
-
 __device__ __forceinline__ void tma_load_4d(void* smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2, int c3) {
   asm volatile(
       "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
@@ -249,12 +240,6 @@ __device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
                : "memory");
-}
-
-// commit that arrives on the mbarrier at the same offset in every CTA of the cluster whose bit is set in cta_mask
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(cta_mask) : "memory");
 }
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;

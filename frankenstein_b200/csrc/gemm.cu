@@ -4,8 +4,8 @@
 // Replaces (reference call sites, models/brainformer.py): the bias-free Linears qw / kw / vw (:141-143, one fused
 // projection) with apply_rope (:70-91, :156-158) in the epilogue; project (:171); the SwiGLU MLP w1 / w3 (:119-124, one
 // fused projection whose epilogue forms silu(w1 x) * (w3 x)) and w2; and their autograd: dX = dY W (same kernel on a
-// transposed weight copy; the MLP's dgated GEMM applies the SwiGLU backward in its epilogue) and dW = dY^T X (fk_gemm_tn,
-// both operands read MN-major straight from the row-major activations, split over the token dimension).
+// transposed weight copy) and dW = dY^T X (fk_gemm_tn, both operands read MN-major straight from the row-major
+// activations, split over the token dimension).
 //
 // Three kernels, all persistent (one CTA per SM), warp-specialised like vq_search.cu: warp 0 = TMA producer,
 // warp 1 = MMA issuer (whole-warp loop, one elected lane issues), warp 2 = TMEM allocator, warps 4-11 = epilogue.
@@ -22,10 +22,6 @@
 //
 // L2 -> SM traffic bounds these shapes as much as the tensor pipe does (K is only 512..4096): a 128-row resident block or
 // a 256 x 256 streamed tile needs one operand byte per 128 flops, about what the L2 fabric delivers at the bf16 peak.
-#include <cstdio>
-#include <cstdlib>
-#include <type_traits>
-
 #include "common.cuh"
 #include "fk_b200.h"
 #include "tma_host.cuh"
@@ -37,25 +33,22 @@ constexpr int kASlabBytes = 128 * 128;     // 128 rows x 64 bf16
 constexpr int kBSlabBytes = 256 * 128;     // 256 rows x 64 bf16
 constexpr int kGemmSmemLimit = 232448 - 1024;
 
-enum { EPI_STORE = 0, EPI_ROPE = 1, EPI_SWIGLU = 2, EPI_SWIGLU_BWD = 3, EPI_ROPE64 = 4 };
+// (epilogue 3 was a SwiGLU backward in the epilogue, removed; the numbers of the others are part of the C ABI)
+enum { EPI_STORE = 0, EPI_ROPE = 1, EPI_SWIGLU = 2, EPI_ROPE64 = 4 };
 // (cos, sin) pairs one epilogue thread holds for its row: one head of 32 columns, or of 64 columns (EPI_ROPE64)
 template <int EPI> constexpr int rope_pairs() { return EPI == EPI_ROPE64 ? 32 : 16; }
 
 struct GemmParams {
-  __nv_bfloat16* C;          // [M, N] (EPI_SWIGLU: the fused projection h13; EPI_SWIGLU_BWD: unused)
+  __nv_bfloat16* C;          // [M, N] (EPI_SWIGLU: the fused projection h13)
   long long ldc;
-  __nv_bfloat16* C2;         // EPI_SWIGLU: gated [M, N/2]; EPI_SWIGLU_BWD: dh13 [M, 2N]
+  __nv_bfloat16* C2;         // EPI_SWIGLU: gated [M, N/2]
   long long ldc2;
-  const __nv_bfloat16* aux;  // EPI_SWIGLU_BWD: h13 [M, 2N]
-  long long ld_aux;
   const float* bias;         // [N] or null (EPI_STORE)
   const float2* rope_table;  // EPI_ROPE: [rope_len][16] (cos, sin); EPI_ROPE64: [rope_len][32]
   const int* rope_pos;       // [M] or null: position of row m = rope_pos ? rope_pos[m] : (m % rope_S) + rope_offset
   int rope_len, rope_offset, rope_cols, rope_S;
   long long M;
   int N, K, nslab, ntile, nstage;
-  int cl;                    // A-resident kernel: CTAs per cluster (1, 2 or 4) that share every weight tile by TMA multicast
-  int dbg;                   // diagnosis (FK_GEMM_DBG): bit 0 = the epilogue releases its accumulator without reading / storing it
 };
 
 __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
@@ -119,37 +112,13 @@ __device__ __forceinline__ void to_f32(const uint32_t (&r)[32], float (&v)[32]) 
 //  each epilogue warp's instruction stream, not by any pipe)
 __device__ __forceinline__ float sigmoidf_fast(float x) { return __fdividef(1.f, 1.f + __expf(-x)); }
 
-// ---- coalesced epilogue I/O through a per-warp 2 KB staging tile (16 rows x 128 bytes, two passes per 32 rows) ----------
+// ---- coalesced epilogue stores through a per-warp 2 KB staging tile (16 rows x 128 bytes, two passes per 32 rows) -------
 // An accumulator row belongs to one thread (TMEM lane = row), so direct stores are 32 rows x 16 bytes per instruction:
 // 32 half-used sectors -- measured, that store path (not the tensor pipe, not L2 reads) paced the A-resident kernel at
-// ~1.9 TB/s of output.  Through the staging tile every global access is a full 128-byte line (8 lanes per row, 4 rows per
-// instruction).  16-byte pieces are XOR-swizzled with (row & 7): row-wise and line-wise patterns are both conflict free.
-//
-// warp_store_32x64: lane l holds columns 0..63 of row (row0 + l) as 32 packed bf16 pairs.
-__device__ __forceinline__ void warp_store_32x64(uint8_t* stg, int lane, const uint32_t (&w)[32], __nv_bfloat16* dst, long long ld,
-                                                 long long row0, long long M, int dbg) {
-#pragma unroll
-  for (int half = 0; half < 2; ++half) {
-    __syncwarp();                                   // the previous pass's readers are done with the tile
-    if ((lane >> 4) == half) {
-      const int r = lane & 15;
-#pragma unroll
-      for (int pc = 0; pc < 8; ++pc)
-        *reinterpret_cast<uint4*>(stg + r * 128 + ((pc ^ (r & 7)) << 4)) = make_uint4(w[4 * pc], w[4 * pc + 1], w[4 * pc + 2], w[4 * pc + 3]);
-    }
-    __syncwarp();
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int r = j * 4 + (lane >> 3), pc = lane & 7;
-      const uint4 v = *reinterpret_cast<const uint4*>(stg + r * 128 + ((pc ^ (r & 7)) << 4));
-      const long long grow = row0 + half * 16 + r;
-      if (dbg & 2) { if (v.x == 0x12345678u && v.y == 0x9abcdef0u) *reinterpret_cast<uint4*>(dst) = v; continue; }   // diagnosis: no global stores
-      if (grow < M) *reinterpret_cast<uint4*>(dst + grow * ld + pc * 8) = v;
-    }
-  }
-}
-// Same through the TMA store engine (one bulk tensor store of the 16 x 128-byte tile per pass instead of 4 STG.128 per lane):
-// the tile layout above IS the 128-byte TMA swizzle; rows / columns outside the tensor are clipped by the hardware.
+// ~1.9 TB/s of output.  Instead each pass writes 16 rows into the staging tile and the TMA store engine writes the tile
+// out in full 128-byte lines.  16-byte pieces are XOR-swizzled with (row & 7), which IS the 128-byte TMA swizzle and keeps
+// the row-wise writes conflict free; rows / columns outside the tensor are clipped by the hardware.
+// Lane l holds columns 0..63 of row (row0 + l) as 32 packed bf16 pairs.
 // A warp's staging area holds `tiles` (1 or 2) such tiles used round-robin (`cnt` = passes so far): with two, the store of
 // one pass is still reading its tile while the next pass fills the other.
 __device__ __forceinline__ void warp_store_32x64_tma(uint8_t* stg0, int tiles, uint32_t& cnt, int lane, const uint32_t (&w)[32],
@@ -179,52 +148,12 @@ __device__ __forceinline__ void warp_store_32x64_tma(uint8_t* stg0, int tiles, u
     }
   }
 }
-// warp_load_32x64: issue the global loads in the full-line pattern (early), then pass them through the tile so that lane l
-// ends up with columns 0..63 of row (row0 + l).
-__device__ __forceinline__ void warp_load_issue_32x64(const __nv_bfloat16* src, long long ld, long long row0, long long M, int lane,
-                                                      uint4 (&v)[8]) {
-#pragma unroll
-  for (int j = 0; j < 8; ++j) {
-    const long long grow = row0 + j * 4 + (lane >> 3);
-    v[j] = (grow < M) ? *reinterpret_cast<const uint4*>(src + grow * ld + (lane & 7) * 8) : make_uint4(0, 0, 0, 0);
-  }
-}
-__device__ __forceinline__ void warp_load_finish_32x64(uint8_t* stg, int lane, const uint4 (&v)[8], uint32_t (&w)[32]) {
-  if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");      // a TMA store may still be reading the tile
-#pragma unroll
-  for (int half = 0; half < 2; ++half) {
-    __syncwarp();
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int r = j * 4 + (lane >> 3), pc = lane & 7;
-      *reinterpret_cast<uint4*>(stg + r * 128 + ((pc ^ (r & 7)) << 4)) = v[half * 4 + j];
-    }
-    __syncwarp();
-    if ((lane >> 4) == half) {
-      const int r = lane & 15;
-#pragma unroll
-      for (int pc = 0; pc < 8; ++pc) {
-        const uint4 t = *reinterpret_cast<const uint4*>(stg + r * 128 + ((pc ^ (r & 7)) << 4));
-        w[4 * pc] = t.x; w[4 * pc + 1] = t.y; w[4 * pc + 2] = t.z; w[4 * pc + 3] = t.w;
-      }
-    }
-  }
-}
-
 // One 128 x 256 accumulator tile of the A-resident kernels: this warp's 32 rows (TMEM lane quarter) x 128 columns (half ch).
 template <int EPI, int NCS, class Release>
 __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUtensorMap& tm_c, const CUtensorMap& tm_c2, uint8_t* stg,
                                                   int stg_tiles, uint32_t& stg_cnt, int lane, int ch, uint32_t taddr, int n0,
                                                   long long row0, const float2 (&cs)[NCS], uint64_t* full_bar, uint32_t full_parity,
                                                   Release release) {
-    const long long row = row0 + lane;
-    (void)row;
-    if (p.dbg & 1) {
-      mbar_wait(full_bar, full_parity);
-      tc_fence_after();
-      release();
-      return;
-    }
     if (EPI == EPI_STORE || EPI == EPI_ROPE || EPI == EPI_ROPE64) {
       mbar_wait(full_bar, full_parity);
       tc_fence_after();
@@ -262,12 +191,9 @@ __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUt
 #pragma unroll
           for (int i = 0; i < 16; ++i) w[hc * 16 + i] = pack_bf16(v[2 * i], v[2 * i + 1]);
         }
-        if (col < p.N) {
-          if (p.dbg & 4) warp_store_32x64(stg, lane, w, p.C + col, p.ldc, row0, p.M, p.dbg);     // diagnosis: LSU stores (N % 64 == 0)
-          else warp_store_32x64_tma(stg, stg_tiles, stg_cnt, lane, w, &tm_c, col, row0);
-        }
+        if (col < p.N) warp_store_32x64_tma(stg, stg_tiles, stg_cnt, lane, w, &tm_c, col, row0);
       }
-    } else if (EPI == EPI_SWIGLU) {
+    } else {   // EPI_SWIGLU
       // tile columns: [0,128) = w1 block, [128,256) = w3 block of the same 128 hidden units (weights interleaved by the
       // host in blocks of 128).  This warp: hidden units ch*64 .. ch*64+63 of the block.
       mbar_wait(full_bar, full_parity);
@@ -307,64 +233,58 @@ __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUt
         }
         warp_store_32x64_tma(stg, stg_tiles, stg_cnt, lane, wa, &tm_c2, (n0 >> 1) + ch * 64, row0);
       }
-    } else {   // EPI_SWIGLU_BWD: accumulator = d gated [M, N]; this warp: hidden block n0/128 + ch (128 units)
-      const long long o0 = 2ll * (n0 + ch * 128);             // column of h1 of the block inside the interleaved h13 / dh13
-      const bool ok = n0 + ch * 128 < p.N;
-      uint4 g1[8], g3[8];
-      if (ok) {                                                // h1 / h3 of the first 64 units: in flight while the MMAs finish
-        warp_load_issue_32x64(p.aux + o0, p.ld_aux, row0, p.M, lane, g1);
-        warp_load_issue_32x64(p.aux + o0 + 128, p.ld_aux, row0, p.M, lane, g3);
-      }
-      mbar_wait(full_bar, full_parity);
-      tc_fence_after();
-#pragma unroll
-      for (int dc = 0; dc < 2; ++dc) {
-        uint32_t w1[32], w3[32];
-        if (ok) {
-          warp_load_finish_32x64(stg, lane, g1, w1);
-          warp_load_finish_32x64(stg, lane, g3, w3);
-        }
-#pragma unroll
-        for (int hc = 0; hc < 2; ++hc) {
-          uint32_t r[32];
-          tmem_ld32(taddr + ch * 128 + dc * 64 + hc * 32, r);
-          tmem_wait_ld32(r);
-          if (dc == 1 && hc == 1) release();
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            float o1[2], o3[2];
-#pragma unroll
-            for (int hh = 0; hh < 2; ++hh) {
-              const uint32_t x1 = w1[hc * 16 + i], x3 = w3[hc * 16 + i];
-              const float h1 = hh ? bf16_hi(x1) : bf16_lo(x1), h3 = hh ? bf16_hi(x3) : bf16_lo(x3);
-              const float dg = __uint_as_float(r[2 * i + hh]);
-              const float sg = sigmoidf_fast(h1);
-              const float silu = h1 * sg;
-              o1[hh] = dg * h3 * (sg + silu * (1.f - sg));     // d silu(x)/dx = s + x s (1 - s)
-              o3[hh] = dg * silu;
-            }
-            w1[hc * 16 + i] = pack_bf16(o1[0], o1[1]);          // in place: d h1 over h1, d h3 over h3
-            w3[hc * 16 + i] = pack_bf16(o3[0], o3[1]);
-          }
-        }
-        if (ok && dc == 0) {                                   // the second 64 units' h1 / h3
-          warp_load_issue_32x64(p.aux + o0 + 64, p.ld_aux, row0, p.M, lane, g1);
-          warp_load_issue_32x64(p.aux + o0 + 64 + 128, p.ld_aux, row0, p.M, lane, g3);
-        }
-        if (ok) {
-          warp_store_32x64_tma(stg, stg_tiles, stg_cnt, lane, w1, &tm_c2, static_cast<int>(o0) + dc * 64, row0);
-          warp_store_32x64_tma(stg, stg_tiles, stg_cnt, lane, w3, &tm_c2, static_cast<int>(o0) + dc * 64 + 128, row0);
-        }
-      }
     }
 }
 
 // ================================================================================================
-// A-resident kernel (K <= 512)
+// A-resident kernels (K <= 512)
 // ================================================================================================
 constexpr int kBStageBytes = 256 * 64;     // 256 rows x 32 bf16 (64-byte rows, SWIZZLE_64B)
 constexpr int kStageTileBytes = 2048;      // per epilogue warp: 16 rows x 128 bytes
 
+// Epilogue warps (4-11) of both A-resident kernels: row block grp * ctas + rank of every group grp0, grp0 + grp_step, ...
+// below n_groups (blocks beyond M: clipped stores), all N tiles of each, the two TMEM accumulator stages in turn.  Each warp
+// owns stg_tiles staging tiles of the CTA's area Stg.  Lane 0 calls arrive(as) once every TMEM read of accumulator stage
+// `as` by this warp has completed.
+template <int EPI, class Arrive>
+__device__ __forceinline__ void res_epilogue_warp(const GemmParams& p, const CUtensorMap& tm_c, const CUtensorMap& tm_c2, uint8_t* Stg,
+                                                  int stg_tiles, uint32_t tmem_base, uint64_t* tmem_full, int grp0, int n_groups,
+                                                  int grp_step, int ctas, int rank, Arrive arrive) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int e = warp - 4;
+  const int q = warp & 3;          // TMEM lane quarter this warp may read
+  const int ch = e >> 2;           // column half of the 256-column tile
+  uint8_t* stg = Stg + e * stg_tiles * kStageTileBytes;
+  uint32_t tc = 0, stg_cnt = 0;
+  for (int grp = grp0; grp < n_groups; grp += grp_step) {
+    const int blk = grp * ctas + rank;
+    const long long row0 = static_cast<long long>(blk) * 128 + q * 32;     // first row of this warp
+    const long long row = row0 + lane;
+    constexpr int kCs = rope_pairs<EPI>();
+    float2 cs[kCs];
+    if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
+      int ps = 0;
+      if (row < p.M) ps = p.rope_pos ? p.rope_pos[row] : static_cast<int>(row % p.rope_S) + p.rope_offset;
+      ps = min(max(ps, 0), p.rope_len - 1);
+#pragma unroll
+      for (int i = 0; i < kCs; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * kCs + i);
+    }
+    for (int t = 0; t < p.ntile; ++t, ++tc) {
+      const uint32_t as = tc & 1;
+      const int n0 = t * 256;
+      const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * 256;
+      auto release = [&]() {
+        tc_fence_before();
+        __syncwarp();
+        if (lane == 0) arrive(as);
+      };
+      res_epilogue_tile<EPI>(p, tm_c, tm_c2, stg, stg_tiles, stg_cnt, lane, ch, taddr, n0, row0, cs, &tmem_full[as], (tc >> 1) & 1, release);
+    }
+  }
+  if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");      // all bulk stores of this warp have completed
+}
+
+// Single CTA per row block: used when the problem has fewer than 4 row blocks (or the device an odd number of SMs).
 template <int EPI>
 __global__ void __launch_bounds__(kGemmThreads, 1)
 gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
@@ -388,7 +308,7 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
   if (warp == 1 && lane == 0) {
     for (int i = 0; i < 8; ++i) {
       mbar_init(&a_full[i], 1); mbar_init(&a_empty[i], 1);
-      mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], static_cast<uint32_t>(p.cl));   // a stage is free once EVERY CTA of the cluster has consumed it
+      mbar_init(&b_full[i], 1); mbar_init(&b_empty[i], 1);
     }
     for (int i = 0; i < 2; ++i) { mbar_init(&tmem_full[i], 1); mbar_init(&tmem_empty[i], 8); }
     fence_mbar_init();
@@ -399,26 +319,14 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
-  // Cluster of p.cl CTAs on p.cl different row blocks that walk the weight matrix in lock step: every CTA loads 1 / cl of
-  // each weight stage and multicasts it to all of them, so a weight byte crosses the L2 -> SM fabric once per cluster
-  // instead of once per CTA (the A-resident shapes are bound by that fabric: one weight byte per 128 flops at cl = 1).
-  const uint32_t cl = static_cast<uint32_t>(p.cl);
-  const uint32_t rank = cl > 1 ? cluster_ctarank() : 0u;
-  const uint16_t cl_mask = static_cast<uint16_t>((1u << cl) - 1u);
-  if (cl > 1) cluster_sync_all();           // every CTA's barriers exist before a peer multicasts to them
-
   const int n_blocks = static_cast<int>((p.M + 127) / 128);
-  const int n_groups = (n_blocks + static_cast<int>(cl) - 1) / static_cast<int>(cl);     // row-block groups, one block per CTA of a cluster
-  const int n_clusters = static_cast<int>(gridDim.x / cl), cluster_id = static_cast<int>(blockIdx.x / cl);
   const int nkb = (p.K + 31) / 32;          // 32-wide k-slabs of B; A slab of k-slab j = j / 2
 
   if (warp == 0) {
     // ================================ TMA producer ================================
     int stage = 0;
     uint32_t phase = 0, it = 0;
-    const uint32_t b_part = kBStageBytes / cl, b_rows = 256u / cl;       // this CTA's share of a weight stage
-    for (int grp = cluster_id; grp < n_groups; grp += n_clusters, ++it) {
-      const int blk = grp * static_cast<int>(cl) + static_cast<int>(rank);     // (beyond M: zero-filled loads, clipped stores)
+    for (int blk = blockIdx.x; blk < n_blocks; blk += gridDim.x, ++it) {
       for (int t = 0; t < p.ntile; ++t) {
         for (int j = 0; j < nkb; ++j) {
           if (t == 0 && (j & 1) == 0) {
@@ -434,11 +342,7 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
           mbar_wait(&b_empty[stage], phase ^ 1);
           if (elect_one()) {
             mbar_expect_tx(&b_full[stage], kBStageBytes);
-            if (cl > 1)
-              tma_load_2d_mc(Bs + stage * kBStageBytes + rank * b_part, &tm_b, &b_full[stage], j * 32,
-                             t * 256 + static_cast<int>(rank * b_rows), cl_mask);
-            else
-              tma_load_2d(Bs + stage * kBStageBytes, &tm_b, &b_full[stage], j * 32, t * 256);
+            tma_load_2d(Bs + stage * kBStageBytes, &tm_b, &b_full[stage], j * 32, t * 256);
           }
           __syncwarp();
           if (++stage == p.nstage) { stage = 0; phase ^= 1; }
@@ -455,52 +359,7 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     // (the loop body is kept minimal: one issuing warp has to turn a 16 KB stage around in the 256 cycles its two MMAs
     //  take -- every integer division, diagnostic branch or descriptor rebuild in here showed up in the GEMM's time)
     const uint64_t adesc0 = umma_desc_sw128(as_addr), bdesc0 = umma_desc_sw64(bs_addr);
-    if (p.nstage == 4 && (nkb & 3) == 0) {
-      // Fast path (K a multiple of 128, four weight stages): the ring position of every k-slab is a compile-time constant, so
-      // barrier addresses and descriptor offsets are immediates and the first / last tile of a row block (the only ones that
-      // touch the A barriers) get their own copies of the loop.  ~60 dependent instructions per 16 KB stage in the generic
-      // loop below cost more than the 256 cycles the stage's two MMAs take; this loop stays under them.
-      uint32_t ring = 0;                                   // completed passes over the 4-stage ring
-      auto run_tile = [&](auto first_c, auto last_c, uint32_t d_tmem) {
-        constexpr bool kFirst = decltype(first_c)::value, kLast = decltype(last_c)::value;
-        uint64_t adesc = adesc0;
-        for (int j4 = 0; j4 < nkb; j4 += 4, ++ring) {
-          const uint32_t ph = ring & 1;
-#pragma unroll
-          for (int st = 0; st < 4; ++st) {
-            if (kFirst && (st & 1) == 0) mbar_wait(&a_full[(j4 >> 1) + (st >> 1)], it & 1);
-            mbar_wait(&b_full[st], ph);
-            tc_fence_after();
-            if (elect_one()) {
-              const uint64_t ad = adesc + static_cast<uint64_t>((st >> 1) * (kASlabBytes >> 4) + (st & 1) * 4);
-              const uint64_t bd = bdesc0 + static_cast<uint64_t>(st * (kBStageBytes >> 4));
-              umma_bf16(d_tmem, ad, bd, idesc, (j4 | st) != 0);
-              umma_bf16(d_tmem, ad + 2, bd + 2, idesc, 1u);
-              if (cl > 1) umma_commit_mc(&b_empty[st], cl_mask); else umma_commit(&b_empty[st]);
-              if (kLast && (st & 1) == 1) umma_commit(&a_empty[(j4 >> 1) + (st >> 1)]);
-            }
-            __syncwarp();
-          }
-          adesc += static_cast<uint64_t>(2 * (kASlabBytes >> 4));
-        }
-      };
-      for (int grp = cluster_id; grp < n_groups; grp += n_clusters, ++it) {
-        for (int t = 0; t < p.ntile; ++t, ++tc) {
-          const uint32_t as = tc & 1;
-          mbar_wait(&tmem_empty[as], ((tc >> 1) & 1) ^ 1);
-          tc_fence_after();
-          const uint32_t d_tmem = tmem_u + as * 256;
-          const bool ft = t == 0, lt = t == p.ntile - 1;
-          if (ft && lt) run_tile(std::true_type{}, std::true_type{}, d_tmem);
-          else if (ft) run_tile(std::true_type{}, std::false_type{}, d_tmem);
-          else if (lt) run_tile(std::false_type{}, std::true_type{}, d_tmem);
-          else run_tile(std::false_type{}, std::false_type{}, d_tmem);
-          if (elect_one()) umma_commit(&tmem_full[as]);
-          __syncwarp();
-        }
-      }
-    } else
-    for (int grp = cluster_id; grp < n_groups; grp += n_clusters, ++it) {
+    for (int blk = blockIdx.x; blk < n_blocks; blk += gridDim.x, ++it) {
       for (int t = 0; t < p.ntile; ++t, ++tc) {
         const uint32_t as = tc & 1;
         mbar_wait(&tmem_empty[as], ((tc >> 1) & 1) ^ 1);
@@ -516,7 +375,7 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
           if (elect_one()) {
             umma_bf16(d_tmem, adesc, bdesc, idesc, j != 0);
             umma_bf16(d_tmem, adesc + 2, bdesc + 2, idesc, 1u);
-            if (cl > 1) umma_commit_mc(&b_empty[stage], cl_mask); else umma_commit(&b_empty[stage]);
+            umma_commit(&b_empty[stage]);
             if (last_tile && ((j & 1) == 1 || j == nkb - 1)) umma_commit(&a_empty[j >> 1]);
           }
           __syncwarp();
@@ -529,42 +388,12 @@ gemm_res_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     }
   } else if (warp >= 4) {
     // ================================ epilogue ================================
-    const int e = warp - 4;
-    const int q = warp & 3;          // TMEM lane quarter this warp may read
-    const int ch = e >> 2;           // column half of the 256-column tile
-    uint8_t* stg = Stg + e * kStageTileBytes;
-    uint32_t tc = 0, stg_cnt = 0;
-    for (int grp = cluster_id; grp < n_groups; grp += n_clusters) {
-      const int blk = grp * static_cast<int>(cl) + static_cast<int>(rank);
-      const long long row0 = ((p.dbg & 8) ? 0ll : static_cast<long long>(blk) * 128) + q * 32;     // first row of this warp (dbg 8: every block writes rows 0..127 -> L2 only)
-      const long long row = row0 + lane;
-      constexpr int kCs = rope_pairs<EPI>();
-      float2 cs[kCs];
-      if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
-        int ps = 0;
-        if (row < p.M) ps = p.rope_pos ? p.rope_pos[row] : static_cast<int>(row % p.rope_S) + p.rope_offset;
-        ps = min(max(ps, 0), p.rope_len - 1);
-#pragma unroll
-        for (int i = 0; i < kCs; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * kCs + i);
-      }
-      for (int t = 0; t < p.ntile; ++t, ++tc) {
-        const uint32_t as = tc & 1;
-        const int n0 = t * 256;
-        const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * 256;
-        auto release = [&]() {           // every TMEM read of this accumulator stage by this warp has completed
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&tmem_empty[as]);
-        };
-        res_epilogue_tile<EPI>(p, tm_c, tm_c2, stg, 1, stg_cnt, lane, ch, taddr, n0, row0, cs, &tmem_full[as], (tc >> 1) & 1, release);
-      }
-    }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");      // all bulk stores of this warp have completed
+    res_epilogue_warp<EPI>(p, tm_c, tm_c2, Stg, 1, tmem_base, tmem_full, static_cast<int>(blockIdx.x), n_blocks,
+                           static_cast<int>(gridDim.x), 1, 0, [&](uint32_t as) { mbar_arrive(&tmem_empty[as]); });
   }
 
   tc_fence_before();
   __syncthreads();
-  if (cl > 1) cluster_sync_all();           // no CTA leaves while a peer may still multicast into it or signal its barriers
   if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, 512); }
 }
 
@@ -682,40 +511,12 @@ gemm_res2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
     }
   } else if (warp >= 4) {
     // ================================ epilogue (both CTAs, own TMEM) ================================
-    const int e = warp - 4;
-    const int q = warp & 3;
-    const int ch = e >> 2;
-    uint8_t* stg = Stg + e * 2 * kStageTileBytes;
-    uint32_t tc = 0, stg_cnt = 0;
-    for (int grp = pair_id; grp < n_groups; grp += n_pairs) {
-      const int blk = grp * 2 + static_cast<int>(rank);
-      const long long row0 = static_cast<long long>(blk) * 128 + q * 32;
-      const long long row = row0 + lane;
-      constexpr int kCs = rope_pairs<EPI>();
-      float2 cs[kCs];
-      if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
-        int ps = 0;
-        if (row < p.M) ps = p.rope_pos ? p.rope_pos[row] : static_cast<int>(row % p.rope_S) + p.rope_offset;
-        ps = min(max(ps, 0), p.rope_len - 1);
-#pragma unroll
-        for (int i = 0; i < kCs; ++i) cs[i] = __ldg(p.rope_table + static_cast<long long>(ps) * kCs + i);
-      }
-      for (int t = 0; t < p.ntile; ++t, ++tc) {
-        const uint32_t as = tc & 1;
-        const int n0 = t * 256;
-        const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + as * 256;
-        auto release = [&]() {           // this warp has read its part of the accumulator stage: tell the leader's issuer
-          tc_fence_before();
-          __syncwarp();
-          if (lane == 0) {
-            if (leader) mbar_arrive(&tmem_empty[as]);
-            else mbar_arrive_cluster(mapa_shared(smem_u32(&tmem_empty[as]), 0));
-          }
-        };
-        res_epilogue_tile<EPI>(p, tm_c, tm_c2, stg, 2, stg_cnt, lane, ch, taddr, n0, row0, cs, &tmem_full[as], (tc >> 1) & 1, release);
-      }
-    }
-    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
+    // (the epilogue warps of both CTAs free an accumulator stage on the leader's barrier)
+    res_epilogue_warp<EPI>(p, tm_c, tm_c2, Stg, 2, tmem_base, tmem_full, pair_id, n_groups, n_pairs, 2, static_cast<int>(rank),
+                           [&](uint32_t as) {
+                             if (leader) mbar_arrive(&tmem_empty[as]);
+                             else mbar_arrive_cluster(mapa_shared(smem_u32(&tmem_empty[as]), 0));
+                           });
   }
 
   tc_fence_before();
@@ -1040,10 +841,36 @@ static int set_smem_attr(Kern* kern, bool& done, int bytes) {
   return FK_OK;
 }
 
+// One A-resident launch: gemm_res2_kernel<EPI> on clusters of 2 CTAs (pair) or gemm_res_kernel<EPI>.
+template <int EPI>
+static int launch_res(bool pair, unsigned grid, int smem_bytes, cudaStream_t stream, const CUtensorMap& ta, const CUtensorMap& tb,
+                      const CUtensorMap& tc, const CUtensorMap& tc2, const GemmParams& p) {
+  static bool done[2][FK_MAX_DEVICES];      // shared-memory opt-in of gemm_res_kernel<EPI> / gemm_res2_kernel<EPI> per device
+  auto* kern = pair ? gemm_res2_kernel<EPI> : gemm_res_kernel<EPI>;
+  const int rc = set_smem_attr(kern, done[pair][fk_device_ordinal()], kGemmSmemLimit);
+  if (rc != FK_OK) return rc;
+  if (!pair) {
+    kern<<<grid, kGemmThreads, smem_bytes, stream>>>(ta, tb, tc, tc2, p);
+    return FK_OK;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid, 1, 1);
+  cfg.blockDim = dim3(kGemmThreads, 1, 1);
+  cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = 1;
+  const cudaError_t le = cudaLaunchKernelEx(&cfg, kern, ta, tb, tc, tc2, p);
+  if (le != cudaSuccess) { fk_set_last_error(cudaGetErrorString(le), __FILE__, __LINE__); return FK_ERR_CUDA; }
+  return FK_OK;
+}
+
 FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb, void* C, long long ldc, long long M, int N,
-                      int K, const float* bias, int epilogue, void* C2, long long ldc2, const void* aux, long long ld_aux,
-                      const float* rope_table, int rope_len, const int* rope_pos, int rope_offset, int rope_cols, int rope_S,
-                      void* stream_) {
+                      int K, const float* bias, int epilogue, void* C2, long long ldc2, const float* rope_table, int rope_len,
+                      const int* rope_pos, int rope_offset, int rope_cols, int rope_S, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   FK_REQUIRE(A && B && M > 0 && N > 0 && K > 0, "fk_gemm_nt: bad argument");
   FK_REQUIRE(M < (1ll << 31) - 256, "fk_gemm_nt: too many rows");
@@ -1051,24 +878,18 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
   FK_REQUIRE(K % 8 == 0 && lda % 8 == 0 && ldb % 8 == 0 && lda > 0 && ldb >= K, "fk_gemm_nt: K and the leading dimensions must be multiples of 8 (16-byte rows)");
   FK_REQUIRE(N % 32 == 0, "fk_gemm_nt: N must be a multiple of 32");
   FK_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0, "fk_gemm_nt: operands must be 16-byte aligned");
+  FK_REQUIRE(epilogue != 3, "fk_gemm_nt: epilogue 3 (SwiGLU backward) was removed; use epilogue 0 for d gated and fk_swiglu_backward_blocked");
   FK_REQUIRE(epilogue >= EPI_STORE && epilogue <= EPI_ROPE64, "fk_gemm_nt: unknown epilogue");
   GemmParams p = {};
   p.C = static_cast<__nv_bfloat16*>(C); p.ldc = ldc;
   p.C2 = static_cast<__nv_bfloat16*>(C2); p.ldc2 = ldc2;
-  p.aux = static_cast<const __nv_bfloat16*>(aux); p.ld_aux = ld_aux;
   p.bias = bias;
   p.rope_table = reinterpret_cast<const float2*>(rope_table); p.rope_pos = rope_pos; p.rope_len = rope_len;
   p.rope_offset = rope_offset; p.rope_cols = rope_cols; p.rope_S = rope_S;
   p.M = M; p.N = N; p.K = K;
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("FK_GEMM_DBG"); dbg = e ? atoi(e) : 0; }
-    p.dbg = dbg;
-  }
   p.nslab = (K + 63) / 64;
   p.ntile = (N + 255) / 256;
-  if (epilogue == EPI_STORE || epilogue == EPI_ROPE || epilogue == EPI_ROPE64 || epilogue == EPI_SWIGLU)
-    FK_REQUIRE(C && ldc % 8 == 0 && ldc >= N && (reinterpret_cast<uintptr_t>(C) & 15) == 0, "fk_gemm_nt: C must be 16-byte aligned with ldc % 8 == 0");
+  FK_REQUIRE(C && ldc % 8 == 0 && ldc >= N && (reinterpret_cast<uintptr_t>(C) & 15) == 0, "fk_gemm_nt: C must be 16-byte aligned with ldc % 8 == 0");
   if (epilogue == EPI_ROPE || epilogue == EPI_ROPE64) {
     FK_REQUIRE(rope_table && rope_len > 0 && rope_cols % (epilogue == EPI_ROPE64 ? 64 : 32) == 0 && rope_cols <= N && (rope_pos || rope_S > 0),
                "fk_gemm_nt: bad rope arguments");
@@ -1077,147 +898,42 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
   }
   if (epilogue == EPI_SWIGLU)
     FK_REQUIRE(N % 256 == 0 && C2 && ldc2 % 8 == 0 && ldc2 >= N / 2 && bias == nullptr, "fk_gemm_nt: SwiGLU epilogue needs N % 256 == 0 and the gated output");
-  if (epilogue == EPI_SWIGLU_BWD)
-    FK_REQUIRE(N % 128 == 0 && C2 && aux && ldc2 % 8 == 0 && ld_aux % 8 == 0 && ldc2 >= 2 * N && ld_aux >= 2 * N && bias == nullptr,
-               "fk_gemm_nt: SwiGLU-backward epilogue needs N % 128 == 0, h13 and dh13");
   FK_REQUIRE(bias == nullptr || epilogue == EPI_STORE, "fk_gemm_nt: bias goes with the plain epilogue");
 
   CUtensorMap ta, tb;
-  const int dev = fk_device_ordinal();
   const int G = fk_sm_count();
   if (K <= 512) {
-    // CTAs per cluster sharing each weight stage by TMA multicast (FK_GEMM_CLUSTER = 1 / 2 / 4).  Default 1: measured on
-    // B200 at M = 524288 (profiles/r02_gemm_experiments.txt), halving the weight traffic with 2-CTA clusters changes the
-    // A-resident GEMMs by < 2 % -- they are not bound by the L2 -> SM fabric but by the look-ahead of the weight ring (80 KB
-    // next to the 128 KB resident block = 1280 cycles at the full MMA rate) -- and 4-CTA clusters do not all fit at once.
-    static int cl_env = -1;
-    if (cl_env < 0) { const char* e = getenv("FK_GEMM_CLUSTER"); cl_env = e ? atoi(e) : 1; if (cl_env != 1 && cl_env != 2 && cl_env != 4) cl_env = 1; }
-    int cl = cl_env;
-    while (cl > 1 && ((M + 127) / 128 < 2ll * cl || G % cl != 0)) cl >>= 1;
-    p.cl = cl;
-    // CTA pairs (cta_group::2, gemm_res2_kernel; default): FK_GEMM_PAIR = 0 selects the single-CTA kernel below (also used
-    // when the problem has fewer than 4 row blocks or the device an odd number of SMs)
-    static int pair_env = -1;
-    if (pair_env < 0) { const char* e = getenv("FK_GEMM_PAIR"); pair_env = e ? atoi(e) : 1; }
-    if (pair_env && (M + 127) / 128 >= 4 && G % 2 == 0) {
-      int rc2 = make_tmap_bf16_2d(&ta, A, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda), 128);
-      rc2 |= make_tmap_bf16_2d_sw64(&tb, B, static_cast<uint64_t>(N), static_cast<uint64_t>(K), static_cast<uint64_t>(ldb), 128);
-      CUtensorMap tc = ta, tc2 = ta;
-      if (C != nullptr) rc2 |= make_tmap_bf16_2d(&tc, C, static_cast<uint64_t>(M), static_cast<uint64_t>(N), static_cast<uint64_t>(ldc), 16);
-      if (C2 != nullptr)
-        rc2 |= make_tmap_bf16_2d(&tc2, C2, static_cast<uint64_t>(M), static_cast<uint64_t>(epilogue == EPI_SWIGLU ? N / 2 : 2 * N),
-                                 static_cast<uint64_t>(ldc2), 16);
-      if (rc2 != FK_OK) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
-      int nstage = (kGemmSmemLimit - 512 - 16 * kStageTileBytes - p.nslab * kASlabBytes) / kB2StageBytes;
-      if (nstage > 16) nstage = 16;
-      p.nstage = nstage;
-      const int smem_bytes = p.nslab * kASlabBytes + nstage * kB2StageBytes + 16 * kStageTileBytes + 512;
-      const long long n_groups = ((M + 127) / 128 + 1) / 2;
-      const long long max_pairs = G / 2;
-      cudaLaunchConfig_t cfg = {};
-      cfg.gridDim = dim3(static_cast<unsigned>((n_groups < max_pairs ? n_groups : max_pairs) * 2), 1, 1);
-      cfg.blockDim = dim3(kGemmThreads, 1, 1);
-      cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
-      cfg.stream = stream;
-      cudaLaunchAttribute attr[1];
-      attr[0].id = cudaLaunchAttributeClusterDimension;
-      attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-      cfg.attrs = attr;
-      cfg.numAttrs = 1;
-      static bool done2[5][FK_MAX_DEVICES];
-      int r2 = FK_OK;
-      cudaError_t le = cudaSuccess;
-      switch (epilogue) {
-        case EPI_STORE:
-          if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_STORE>, done2[0][dev], kGemmSmemLimit)) != FK_OK) return r2;
-          le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_STORE>, ta, tb, tc, tc2, p);
-          break;
-        case EPI_ROPE:
-          if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_ROPE>, done2[1][dev], kGemmSmemLimit)) != FK_OK) return r2;
-          le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_ROPE>, ta, tb, tc, tc2, p);
-          break;
-        case EPI_ROPE64:
-          if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_ROPE64>, done2[4][dev], kGemmSmemLimit)) != FK_OK) return r2;
-          le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_ROPE64>, ta, tb, tc, tc2, p);
-          break;
-        case EPI_SWIGLU:
-          if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_SWIGLU>, done2[2][dev], kGemmSmemLimit)) != FK_OK) return r2;
-          le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_SWIGLU>, ta, tb, tc, tc2, p);
-          break;
-        default:
-          if ((r2 = set_smem_attr(gemm_res2_kernel<EPI_SWIGLU_BWD>, done2[3][dev], kGemmSmemLimit)) != FK_OK) return r2;
-          le = cudaLaunchKernelEx(&cfg, gemm_res2_kernel<EPI_SWIGLU_BWD>, ta, tb, tc, tc2, p);
-          break;
-      }
-      if (le != cudaSuccess) { fk_set_last_error(cudaGetErrorString(le), __FILE__, __LINE__); return FK_ERR_CUDA; }
-      FK_CHECK_LAUNCH();
-      fk_count_launch(1);
-      return FK_OK;
-    }
-    int rc = make_tmap_bf16_2d(&ta, A, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda), 128);
-    rc |= make_tmap_bf16_2d_sw64(&tb, B, static_cast<uint64_t>(N), static_cast<uint64_t>(K), static_cast<uint64_t>(ldb), 256 / cl);
-    if (rc != FK_OK) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
-    // outputs go through the TMA store engine: 16-row x 64-column boxes, 128-byte swizzle
-    CUtensorMap tc = ta, tc2 = ta;
-    if (C != nullptr) rc |= make_tmap_bf16_2d(&tc, C, static_cast<uint64_t>(M), static_cast<uint64_t>(N), static_cast<uint64_t>(ldc), 16);
-    if (C2 != nullptr)
-      rc |= make_tmap_bf16_2d(&tc2, C2, static_cast<uint64_t>(M), static_cast<uint64_t>(epilogue == EPI_SWIGLU ? N / 2 : 2 * N),
-                              static_cast<uint64_t>(ldc2), 16);
-    if (rc != FK_OK) { fk_set_last_error("cuTensorMapEncodeTiled(output) failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
-    int nstage = (kGemmSmemLimit - 512 - 8 * kStageTileBytes - p.nslab * kASlabBytes) / kBStageBytes;
-    if (nstage > 8) nstage = 8;
-    {
-      // FK_GEMM_STAGES = 4 selects the unrolled issue loop (K % 128 == 0) at the price of one stage of look-ahead; measured
-      // slower (0.93 against 0.83 ms for the q|k|v projection): the ring depth matters more than the issue overhead.
-      // Default: every stage that fits (5 at K = 512) with the generic loop.
-      static int st_env = -1;
-      if (st_env < 0) { const char* e = getenv("FK_GEMM_STAGES"); st_env = e ? atoi(e) : 0; }
-      if (st_env == 4 && nstage >= 4 && K % 128 == 0) nstage = 4;
-    }
-    p.nstage = nstage;
-    const int smem_bytes = p.nslab * kASlabBytes + nstage * kBStageBytes + 8 * kStageTileBytes + 512;
+    // CTA pairs (gemm_res2_kernel) hold twice the weight look-ahead of single CTAs (gemm_res_kernel), which are left with
+    // the problems of fewer than 4 row blocks and devices with an odd number of SMs
     const long long n_blocks = (M + 127) / 128;
-    const long long n_groups = (n_blocks + cl - 1) / cl;
-    const long long max_clusters = G / cl;
-    const unsigned grid = static_cast<unsigned>((n_groups < max_clusters ? n_groups : max_clusters) * cl);
-    static bool done[5][FK_MAX_DEVICES];
-    int r2 = FK_OK;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid, 1, 1);
-    cfg.blockDim = dim3(kGemmThreads, 1, 1);
-    cfg.dynamicSmemBytes = static_cast<size_t>(smem_bytes);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = static_cast<unsigned>(cl);
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = cl > 1 ? 1 : 0;
-    cudaError_t le = cudaSuccess;
+    const bool pair = n_blocks >= 4 && G % 2 == 0;
+    int rc = make_tmap_bf16_2d(&ta, A, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda), 128);
+    rc |= make_tmap_bf16_2d_sw64(&tb, B, static_cast<uint64_t>(N), static_cast<uint64_t>(K), static_cast<uint64_t>(ldb), pair ? 128 : 256);
+    // outputs go through the TMA store engine: 16-row x 64-column boxes, 128-byte swizzle
+    CUtensorMap tc, tc2;
+    rc |= make_tmap_bf16_2d(&tc, C, static_cast<uint64_t>(M), static_cast<uint64_t>(N), static_cast<uint64_t>(ldc), 16);
+    tc2 = tc;
+    if (epilogue == EPI_SWIGLU)
+      rc |= make_tmap_bf16_2d(&tc2, C2, static_cast<uint64_t>(M), static_cast<uint64_t>(N / 2), static_cast<uint64_t>(ldc2), 16);
+    if (rc != FK_OK) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
+    // every weight stage that fits next to the resident block and the staging tiles (2 per epilogue warp on pairs)
+    const int stg_bytes = (pair ? 16 : 8) * kStageTileBytes;
+    const int stage_bytes = pair ? kB2StageBytes : kBStageBytes;
+    const int max_stages = pair ? 16 : 8;
+    int nstage = (kGemmSmemLimit - 512 - stg_bytes - p.nslab * kASlabBytes) / stage_bytes;
+    if (nstage > max_stages) nstage = max_stages;
+    p.nstage = nstage;
+    const int smem_bytes = p.nslab * kASlabBytes + nstage * stage_bytes + stg_bytes + 512;
+    const long long n_groups = pair ? (n_blocks + 1) / 2 : n_blocks;     // row blocks per CTA pair / CTA
+    const long long max_groups = pair ? G / 2 : G;
+    const unsigned grid = static_cast<unsigned>((n_groups < max_groups ? n_groups : max_groups) * (pair ? 2 : 1));
     switch (epilogue) {
-      case EPI_STORE:
-        if ((r2 = set_smem_attr(gemm_res_kernel<EPI_STORE>, done[0][dev], kGemmSmemLimit)) != FK_OK) return r2;
-        le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_STORE>, ta, tb, tc, tc2, p);
-        break;
-      case EPI_ROPE:
-        if ((r2 = set_smem_attr(gemm_res_kernel<EPI_ROPE>, done[1][dev], kGemmSmemLimit)) != FK_OK) return r2;
-        le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_ROPE>, ta, tb, tc, tc2, p);
-        break;
-      case EPI_ROPE64:
-        if ((r2 = set_smem_attr(gemm_res_kernel<EPI_ROPE64>, done[4][dev], kGemmSmemLimit)) != FK_OK) return r2;
-        le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_ROPE64>, ta, tb, tc, tc2, p);
-        break;
-      case EPI_SWIGLU:
-        if ((r2 = set_smem_attr(gemm_res_kernel<EPI_SWIGLU>, done[2][dev], kGemmSmemLimit)) != FK_OK) return r2;
-        le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_SWIGLU>, ta, tb, tc, tc2, p);
-        break;
-      default:
-        if ((r2 = set_smem_attr(gemm_res_kernel<EPI_SWIGLU_BWD>, done[3][dev], kGemmSmemLimit)) != FK_OK) return r2;
-        le = cudaLaunchKernelEx(&cfg, gemm_res_kernel<EPI_SWIGLU_BWD>, ta, tb, tc, tc2, p);
-        break;
+      case EPI_STORE: rc = launch_res<EPI_STORE>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
+      case EPI_ROPE: rc = launch_res<EPI_ROPE>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
+      case EPI_SWIGLU: rc = launch_res<EPI_SWIGLU>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
+      default: rc = launch_res<EPI_ROPE64>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
     }
-    if (le != cudaSuccess) { fk_set_last_error(cudaGetErrorString(le), __FILE__, __LINE__); return FK_ERR_CUDA; }
+    if (rc != FK_OK) return rc;
   } else {
     FK_REQUIRE(epilogue == EPI_STORE, "fk_gemm_nt: fused epilogues need K <= 512 (the A-resident kernel)");
     int rc = make_tmap_bf16_2d(&ta, A, static_cast<uint64_t>(M), static_cast<uint64_t>(K), static_cast<uint64_t>(lda), 256);
@@ -1228,7 +944,7 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
     const long long n_units = ((M + 255) / 256) * p.ntile;
     const unsigned grid = static_cast<unsigned>(n_units < G ? n_units : G);
     static bool done[FK_MAX_DEVICES];
-    const int r2 = set_smem_attr(gemm_stream_kernel, done[dev], kGemmSmemLimit);
+    const int r2 = set_smem_attr(gemm_stream_kernel, done[fk_device_ordinal()], kGemmSmemLimit);
     if (r2 != FK_OK) return r2;
     gemm_stream_kernel<<<grid, kGemmThreads, smem_bytes, stream>>>(ta, tb, p);
   }

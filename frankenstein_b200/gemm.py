@@ -6,7 +6,7 @@ Functional wrappers (``gemm_nt``, ``gemm_tn``) and the ``torch.autograd.Function
 * ``qkv_rope``     -- qw / kw / vw as ONE projection (brainformer.py:141-143) with ``apply_rope`` (:70-91, :156-158) applied
                       to the q | k columns in the GEMM epilogue (heads of 32 or 64 columns);
 * ``swiglu_mlp``   -- ``w2(silu(w1 x) * w3 x)`` (brainformer.py:119-124): the w1 | w3 projection forms the gate in its
-                      epilogue, the backward's d-gated GEMM applies the SwiGLU derivative in its epilogue.
+                      epilogue; the backward applies the SwiGLU derivative in one streaming pass after the d-gated GEMM.
 
 Weights stay fp32 ``nn.Parameter``s under their reference names; each call casts them to bf16 (and, for the input
 gradient, makes the transposed copy the NT kernel wants -- a few MB).  Weight gradients come from ``fk_gemm_tn``
@@ -15,7 +15,6 @@ gradient, makes the transposed copy the NT kernel wants -- a few MB).  Weight gr
 from __future__ import annotations
 
 import math
-import os
 from typing import Optional
 
 import torch
@@ -23,11 +22,8 @@ import torch
 from ._lib import FkError, check, lib, on_tensor_device, ptr, require_cuda, require_device, stream, timed
 
 BF16 = torch.bfloat16
-EPI_STORE, EPI_ROPE, EPI_SWIGLU, EPI_SWIGLU_BWD, EPI_ROPE64 = 0, 1, 2, 3, 4
+EPI_STORE, EPI_ROPE, EPI_SWIGLU, EPI_ROPE64 = 0, 1, 2, 4
 ROPE_EPILOGUE = {32: EPI_ROPE, 64: EPI_ROPE64}          # head width -> RoPE epilogue of the fused q | k | v projection
-# backward of the SwiGLU MLP: "split" = d-gated GEMM + one streaming derivative pass (default, faster); "fused" = the
-# derivative in the GEMM epilogue (kept for A/B measurements and tested in tests/test_gemm_gpu.py)
-MLP_BWD = os.environ.get("FK_MLP_BWD", "split")
 
 
 def _as2d(x: torch.Tensor) -> torch.Tensor:
@@ -41,10 +37,9 @@ def _as2d(x: torch.Tensor) -> torch.Tensor:
 
 @on_tensor_device
 def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = None, epilogue: int = EPI_STORE, *,
-            gated: Optional[torch.Tensor] = None, h13: Optional[torch.Tensor] = None, rope=None, rope_cols: int = 0,
-            rope_S: int = 0, lead: Optional[tuple] = None, name: str = "gemm_nt"):
+            rope=None, rope_cols: int = 0, rope_S: int = 0, lead: Optional[tuple] = None, name: str = "gemm_nt"):
     """C [M, N] bf16 = a [M, K] @ b [N, K]^T on tcgen05 (fp32 accumulate).  See include/fk_b200.h (fk_gemm_nt) for the
-    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64), (h13, gated) (EPI_SWIGLU) or dh13 (EPI_SWIGLU_BWD).
+    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64) or (h13, gated) (EPI_SWIGLU).
     lead (EPI_STORE): C is allocated as [*lead, N] (prod(lead) = M), a tensor of its own rather than a view of [M, N]."""
     require_cuda(a, b)
     require_device()
@@ -57,8 +52,8 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
     if a.stride(1) != 1 or b.stride(1) != 1:
         raise FkError("gemm_nt: operands must be row-major")
     dev = a.device
-    C = C2 = aux = None
-    ldc = ldc2 = ld_aux = 0
+    C = C2 = None
+    ldc = ldc2 = 0
     if lead is not None and (epilogue != EPI_STORE or math.prod(lead) != M):
         raise FkError(f"gemm_nt: output shape {(*lead, N)} does not hold [{M}, {N}]")
     if epilogue in (EPI_STORE, EPI_ROPE, EPI_ROPE64):
@@ -68,12 +63,6 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
         C = torch.empty(M, N, device=dev, dtype=BF16)
         C2 = torch.empty(M, N // 2, device=dev, dtype=BF16)
         ldc, ldc2 = N, N // 2
-    elif epilogue == EPI_SWIGLU_BWD:
-        if h13 is None or h13.shape != (M, 2 * N) or h13.dtype != BF16 or not h13.is_contiguous():
-            raise FkError("gemm_nt: the SwiGLU-backward epilogue needs the saved bf16 h13 [M, 2N]")
-        aux, ld_aux = h13, 2 * N
-        C2 = torch.empty(M, 2 * N, device=dev, dtype=BF16)
-        ldc2 = 2 * N
     bias_f = None
     if bias is not None:
         bias_f = bias.detach().float().contiguous()
@@ -86,12 +75,10 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
                 raise FkError("gemm_nt: rope positions must cover every row")
     with timed(name, 2.0 * M * N * K):
         check(lib().fk_gemm_nt(ptr(a), a.stride(0), ptr(b), b.stride(0), ptr(C), ldc, M, N, K, ptr(bias_f), epilogue,
-                               ptr(C2), ldc2, ptr(aux), ld_aux, ptr(table), rope_len, ptr(pos), rope_off, rope_cols, rope_S,
-                               stream()), "fk_gemm_nt")
+                               ptr(C2), ldc2, ptr(table), rope_len, ptr(pos), rope_off, rope_cols, rope_S, stream()),
+              "fk_gemm_nt")
     if epilogue == EPI_SWIGLU:
         return C, C2
-    if epilogue == EPI_SWIGLU_BWD:
-        return C2
     return C
 
 
@@ -246,19 +233,16 @@ class _SwiGLUMLPFn(torch.autograd.Function):
     def backward(ctx, g):
         x2, h13, gated, w13, w2b = ctx.saved_tensors
         g2 = _as2d(g)
-        if MLP_BWD == "fused":
-            dh13 = gemm_nt(g2, w2b.t().contiguous(), None, EPI_SWIGLU_BWD, h13=h13, name="gemm_dgated_swiglu_bwd")
-        else:
-            # d gated on the plain epilogue, then the SwiGLU derivative as one HBM-bound pass over h13 / dh13: the pass is
-            # bound by the 8.6 GB it moves either way, and the streaming kernel keeps more bytes in flight than a GEMM
-            # epilogue can (measured: 1.2 + 1.5 ms against 4.4 ms fused at M = 524288)
-            dg = gemm_nt(g2, w2b.t().contiguous(), None, EPI_STORE, name="gemm_dgated")
-            dh13 = torch.empty_like(h13)
-            M, H = dg.shape
-            with timed("swiglu_bwd", 0.0):
-                check(lib().fk_swiglu_backward_blocked(ptr(h13), ptr(dg), ptr(dh13), M, H, 128, stream()),
-                      "fk_swiglu_backward_blocked")
-            del dg
+        # d gated on the plain epilogue, then the SwiGLU derivative as one HBM-bound pass over h13 / dh13: the pass is
+        # bound by the 8.6 GB it moves either way, and the streaming kernel keeps more bytes in flight than a GEMM
+        # epilogue can (measured: 1.2 + 1.5 ms against 4.4 ms with the derivative in the epilogue at M = 524288)
+        dg = gemm_nt(g2, w2b.t().contiguous(), None, EPI_STORE, name="gemm_dgated")
+        dh13 = torch.empty_like(h13)
+        M, H = dg.shape
+        with timed("swiglu_bwd", 0.0):
+            check(lib().fk_swiglu_backward_blocked(ptr(h13), ptr(dg), ptr(dh13), M, H, 128, stream()),
+                  "fk_swiglu_backward_blocked")
+        del dg
         dw2 = gemm_tn(g2, gated, name="gemm_w2_dw").to(ctx.w_dtype)
         dx = gemm_nt(dh13, w13.t().contiguous(), None, EPI_STORE, name="gemm_w13_dx").view(ctx.in_shape)
         if dx.dtype != ctx.in_dtype and ctx.in_dtype in (torch.float32, torch.float16):
@@ -272,8 +256,8 @@ def mlp_supported(dim: int, hidden: int) -> bool:
 
 
 def swiglu_mlp(x, w1, w3, w2):
-    """w2(silu(w1 x) * (w3 x)) with the gate fused into the w1 | w3 projection (forward) and into the d-gated GEMM
-    (backward)."""
+    """w2(silu(w1 x) * (w3 x)) with the gate fused into the w1 | w3 projection (forward); the backward applies its
+    derivative in one streaming pass after the d-gated GEMM."""
     return _SwiGLUMLPFn.apply(x, w1, w3, w2)
 
 

@@ -241,13 +241,11 @@ int fk_add_norm_backward(const float* x_new, const void* g_y, int g_dtype, const
  *      : (m % rope_S) + rope_offset
  *   2  SwiGLU forward: B = w1 / w3 interleaved in blocks of 128 rows ([w1[0:128]; w3[0:128]; w1[128:256]; ...], N = 2 x
  *      hidden); writes the fused projection C = h13 [M, N] and C2 = gated [M, N/2] = silu(h1) * h3 (brainformer.py:123-124)
- *   3  SwiGLU backward: A = d out, B = w2^T ([hidden, dim]), N = hidden; the accumulator d gated is combined with
- *      aux = h13 [M, 2N] (interleaved as above) into C2 = dh13 [M, 2N]; C is not written.
+ *   3  removed (was the SwiGLU backward; rejected): d gated on epilogue 0, then fk_swiglu_backward_blocked
  *   4  as 1 for heads of 64 columns: rope_table [rope_len][32][2], rope_cols % 64 == 0 */
 int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb, void* C, long long ldc, long long M, int N,
-               int K, const float* bias, int epilogue, void* C2, long long ldc2, const void* aux, long long ld_aux,
-               const float* rope_table, int rope_len, const int* rope_pos, int rope_offset, int rope_cols, int rope_S,
-               void* stream);
+               int K, const float* bias, int epilogue, void* C2, long long ldc2, const float* rope_table, int rope_len,
+               const int* rope_pos, int rope_offset, int rope_cols, int rope_S, void* stream);
 /* out[Na,Nb] (fp32) = A[M,Na]^T x B[M,Nb] (bf16, row-major): the weight gradient dW = dY^T X of an nn.Linear.  The M rows
  * are cut into `splits` = fk_gemm_tn_splits(M, Na, Nb, 0) ranges whose partial sums go to ws (fp32 [splits, Na, Nb]) and
  * are added in a fixed order (bit-reproducible).  Na % 64 == 0, Nb % 64 == 0.  max_ctas <= 0: the SM count. */

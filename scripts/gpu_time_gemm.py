@@ -59,9 +59,6 @@ def main():
     report("w13+swiglu NT res N=4096 K=512", 2.0 * M * 4096 * 512, lambda: gemm.gemm_nt(x512, w13, None, gemm.EPI_SWIGLU),
            lambda: x512 @ w13.t(), M * (512 + 4096 + 2048) * 2)
     h13, gated = gemm.gemm_nt(x512, w13, None, gemm.EPI_SWIGLU)
-    w2t = rnd(2048, 512, s=0.02)
-    report("dgated+swiglu_bwd NT res N=2048 K=512", 2.0 * M * 2048 * 512,
-           lambda: gemm.gemm_nt(x512, w2t, None, gemm.EPI_SWIGLU_BWD, h13=h13), lambda: x512 @ w2t.t(), M * (512 + 8192) * 2)
     # ---- streaming NT ----
     w2 = rnd(512, 2048, s=0.02)
     report("w2    NT stream N=512 K=2048", 2.0 * M * 512 * 2048, lambda: gemm.gemm_nt(gated, w2), lambda: gated @ w2.t(),

@@ -1,6 +1,5 @@
 """The library's own tcgen05 GEMMs (csrc/gemm.cu) against plain PyTorch fp32 matmuls of the same bf16 operands: the NT
-kernels (A-resident for K <= 512, streaming for longer K), their fused epilogues (bias, RoPE, SwiGLU forward / backward)
-and the TN weight-gradient kernel (MN-major operands, split reduction), then the autograd Functions built on them."""
+kernels (A-resident for K <= 512, streaming for longer K), their fused epilogues (bias, RoPE, SwiGLU gate) and the TN weight-gradient kernel (MN-major operands, split reduction), then the autograd Functions built on them."""
 import pytest
 import torch
 import torch.nn.functional as F
@@ -72,7 +71,8 @@ def test_gemm_rope_epilogue(per_sample):
 
 
 @pytest.mark.parametrize("M,D,H", [(300, 64, 128), (1000, 512, 2048), (129, 256, 384)])
-def test_gemm_swiglu_epilogues(M, D, H):
+def test_gemm_swiglu_gate_epilogue(M, D, H):
+    """The w1 | w3 projection with the gate in its epilogue: h13 interleaved in blocks of 128 and gated = silu(h1) * h3."""
     from frankenstein_b200 import gemm
     g = torch.Generator().manual_seed(M)
     x = _rand((M, D), g)
@@ -84,17 +84,55 @@ def test_gemm_swiglu_epilogues(M, D, H):
     close(a.t(), h1_ref, 1e-2, "h1")
     close(b.t(), h3_ref, 1e-2, "h3")
     close(gated, F.silu(h1_ref) * h3_ref, 2e-2, "gated")
-    # backward epilogue: accumulator = d gated = dout @ w2 ; outputs d h1 | d h3 interleaved like h13
-    dout = _rand((M, D), g)
-    w2 = _rand((D, H), g, H ** -0.5)
-    dh13 = gemm.gemm_nt(dout, w2.t().contiguous(), None, gemm.EPI_SWIGLU_BWD, h13=h13)
-    h1 = a.t().float().clone().requires_grad_(True)
-    h3 = b.t().float().clone().requires_grad_(True)
-    dg = dout.float() @ w2.float()
-    (F.silu(h1) * h3 * dg).sum().backward()
-    d1, d3 = gemm._deinterleave(dh13.t().contiguous())
-    close(d1.t(), h1.grad, 2e-2, "d h1")
-    close(d3.t(), h3.grad, 2e-2, "d h3")
+
+
+@pytest.mark.parametrize("M", [300, 4173])          # 3 row blocks: single-CTA kernel; 33 row blocks: CTA pairs
+@pytest.mark.parametrize("epi", ["store", "store_bias", "rope32", "rope64", "swiglu"])
+def test_a_resident_epilogues(epi, M):
+    """Every epilogue on both A-resident kernels (K <= 512), with a partial last row block and, but for SwiGLU, a partial
+    last column tile; RoPE positions are (m % S) + offset."""
+    from frankenstein_b200 import gemm
+    from frankenstein_b200.brainformer import build_complex_rope_cache
+    from frankenstein_b200.ops import RopeSpec
+    g = torch.Generator().manual_seed(M)
+    K, inner, S, off = 256, 128, M // 3, 7
+    x = _rand((M, K), g)
+    if epi == "swiglu":
+        w1, w3 = _rand((256, K), g, K ** -0.5), _rand((256, K), g, K ** -0.5)
+        h13, gated = gemm.gemm_nt(x, gemm._interleave(w1, w3), None, gemm.EPI_SWIGLU)
+        h1, h3 = x.float() @ w1.float().t(), x.float() @ w3.float().t()
+        close(h13, gemm._interleave(h1.t(), h3.t()).t(), 1e-2, "h13")
+        close(gated, F.silu(h1) * h3, 2e-2, "gated")
+        return
+    w = _rand((3 * inner, K), g, K ** -0.5)
+    ref = x.float() @ w.float().t()
+    if epi.startswith("store"):
+        bias = torch.randn(3 * inner, generator=g).cuda() if epi == "store_bias" else None
+        out = gemm.gemm_nt(x, w, bias)
+        if bias is not None:
+            ref = ref + bias
+    else:
+        hd = 32 if epi == "rope32" else 64
+        cache = build_complex_rope_cache(hd, 2048, 10000.0).cuda()
+        out = gemm.gemm_nt(x, w, None, gemm.ROPE_EPILOGUE[hd], rope=RopeSpec(torch.view_as_real(cache).float(), None, off),
+                           rope_cols=2 * inner, rope_S=S)
+        pos = torch.arange(M, device="cuda") % S + off
+        qk = torch.view_as_complex(ref[:, :2 * inner].reshape(M, 2 * inner // hd, hd // 2, 2).contiguous())
+        ref[:, :2 * inner] = torch.view_as_real(qk * cache[pos][:, None, :]).reshape(M, 2 * inner)
+    assert out.shape == (M, 3 * inner)
+    close(out, ref, 1e-2, f"{epi} M={M}")
+
+
+def test_removed_swiglu_backward_epilogue_is_rejected():
+    """Epilogue 3 (the SwiGLU backward, removed) fails on the host, before anything is launched."""
+    from frankenstein_b200._lib import FkError, check, launch_count, lib, ptr, stream
+    a, b = torch.zeros(256, 64, device="cuda", dtype=torch.bfloat16), torch.zeros(256, 64, device="cuda", dtype=torch.bfloat16)
+    c, c2 = torch.empty(256, 256, device="cuda", dtype=torch.bfloat16), torch.empty(256, 512, device="cuda", dtype=torch.bfloat16)
+    n0 = launch_count()
+    with pytest.raises(FkError, match="removed"):
+        check(lib().fk_gemm_nt(ptr(a), 64, ptr(b), 64, ptr(c), 256, 256, 256, 64, None, 3, ptr(c2), 512, None, 0, None, 0,
+                               0, 0, stream()), "fk_gemm_nt")
+    assert launch_count() == n0
 
 
 @pytest.mark.parametrize("M,Na,Nb", [(1000, 512, 512), (4096, 1536, 512), (333, 64, 64), (70000, 4096, 512), (64, 128, 192),
@@ -110,17 +148,17 @@ def test_gemm_tn_matches_fp32_matmul(M, Na, Nb):
     assert torch.equal(out, gemm.gemm_tn(a, b)), "the split reduction must be bit-reproducible"
 
 
-@pytest.mark.parametrize("mlp_bwd", ["split", "fused"])
-def test_linear_qkv_mlp_functions_match_torch(mlp_bwd, monkeypatch):
-    """The autograd Functions (forward + all gradients) against fp32 PyTorch on the same weights; the MLP backward both as
-    d-gated GEMM + streaming SwiGLU derivative (default) and with the derivative in the GEMM epilogue."""
+@pytest.mark.parametrize("head_dim", [32, 64])
+def test_linear_qkv_mlp_functions(head_dim):
+    """The autograd Functions (forward + all gradients) against fp32 PyTorch on the same weights: linear, the SwiGLU MLP
+    (backward: d-gated GEMM, then the streaming SwiGLU derivative) and the fused q | k | v projection with the RoPE
+    epilogue of the given head width."""
     from frankenstein_b200 import gemm
-    monkeypatch.setattr(gemm, "MLP_BWD", mlp_bwd)
     from frankenstein_b200.brainformer import apply_rope, build_complex_rope_cache
     from frankenstein_b200.ops import RopeSpec
     g = torch.Generator().manual_seed(0)
     B, S, D, H, NH = 2, 300, 128, 256, 4
-    inner = NH * 32
+    inner = NH * head_dim
     x = torch.randn(B, S, D, generator=g).cuda()
     wout = torch.randn(B, S, D, generator=g).cuda()
 
@@ -147,14 +185,14 @@ def test_linear_qkv_mlp_functions_match_torch(mlp_bwd, monkeypatch):
         close(a.grad, b.grad, 3e-2, f"mlp {name}")
     # ---- qkv + rope ----
     wq, wk, wv = (params(inner, D, s=D ** -0.5) for _ in range(3))
-    cache = build_complex_rope_cache(32, 512, 10000.0).cuda()
+    cache = build_complex_rope_cache(head_dim, 512, 10000.0).cuda()
     spec = RopeSpec.from_complex(cache, S, last=True)
     wq_out = torch.randn(B, S, 3 * inner, generator=g).cuda()
     xr = x.clone().requires_grad_(True)
     qkv = gemm.qkv_rope(xr, wq, wk, wv, spec, NH)
     ref_p = [t.detach().clone().requires_grad_(True) for t in (x, wq, wk, wv)]
-    q = apply_rope(F.linear(ref_p[0], ref_p[1]).view(B, S, NH, 32), cache).reshape(B, S, inner)
-    k = apply_rope(F.linear(ref_p[0], ref_p[2]).view(B, S, NH, 32), cache).reshape(B, S, inner)
+    q = apply_rope(F.linear(ref_p[0], ref_p[1]).view(B, S, NH, head_dim), cache).reshape(B, S, inner)
+    k = apply_rope(F.linear(ref_p[0], ref_p[2]).view(B, S, NH, head_dim), cache).reshape(B, S, inner)
     ref = torch.cat([q, k, F.linear(ref_p[0], ref_p[3])], dim=-1)
     close(qkv, ref, 2e-2, "qkv rope out")
     # the Function's backward takes the gradient w.r.t. the UNROTATED projection (the attention backward un-rotates dq / dk):
