@@ -178,7 +178,7 @@ attn_fwd_kernel(const AttnParams p) {
     load_tile_async<kTK>(smem_u32(sV[buf]), vg, p.v_ts, tile * kTK, p.Sk);
     if (masked && threadIdx.x < kTK) {
       const int j = tile * kTK + threadIdx.x;
-      sKid[buf][threadIdx.x] = (j < p.Sk) ? p.kid[static_cast<long long>(b) * p.Sk + j] : 0x7fffffff;
+      sKid[buf][threadIdx.x] = (j < p.Sk) ? p.kid[static_cast<long long>(b) * p.Sk + j] : 0;   // (j >= Sk: masked by position)
     }
     cp_async_commit();
   };
@@ -224,9 +224,10 @@ attn_fwd_kernel(const AttnParams p) {
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
           const int col = nt * 8 + t4 * 2 + (e & 1);
-          const int kid = masked ? sKid[buf][col] : ((kt * kTK + col < p.Sk) ? 0 : 0x7fffffff);
+          const int kid = masked ? sKid[buf][col] : 0;
           const int qid = masked ? ((e & 2) ? qid1 : qid0) : 0;
-          if (kid > qid) s[nt][e] = -INFINITY;
+          // keys past Sk are masked by position: no label value may stand for them, a query labelled INT32_MAX sees every key
+          if (kid > qid || kt * kTK + col >= p.Sk) s[nt][e] = -INFINITY;
         }
       }
     }
@@ -554,7 +555,7 @@ __global__ void __launch_bounds__(64)
 attn_label_range_kernel(const int* __restrict__ ids, int B, int S, int* __restrict__ tmin, int* __restrict__ tmax) {
   const int tile = blockIdx.x, b = blockIdx.y, nt = (S + 63) / 64;
   const int i = tile * 64 + threadIdx.x;
-  int lo = 0x7fffffff, hi = -0x7fffffff;
+  int lo = 0x7fffffff, hi = -0x7fffffff - 1;         // INT32_MAX / INT32_MIN: both are valid labels
   if (i < S) lo = hi = ids[static_cast<long long>(b) * S + i];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {

@@ -1214,12 +1214,15 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     auto prefetch = [&](int j) {
       if (j >= T || !(tile_list[j] & my_flag)) return;
       const int c = (tile_list[j] & 0x3fff) * kFwdTileK + tid;
-      pre_i = (c < p.Sk) ? (masked ? p.kid[static_cast<long long>(b) * p.Sk + c] : 0) : 0x7fffffff;
+      pre_i = (masked && c < p.Sk) ? p.kid[static_cast<long long>(b) * p.Sk + c] : 0;   // (c >= Sk: masked by position)
     };
     prefetch(0);
     for (int j = 0; j < T; ++j) {
       const int gj = base + j;                       // key-tile counter across items (barrier parities)
       const bool need_mask = (tile_list[j] & my_flag) != 0;
+      // keys of this tile that exist: < kFwdTileK only in the ragged tail, which always carries the compare flag.  The
+      // columns past Sk are masked by position, not by a sentinel label: every int32 is a valid query label.
+      const int n_valid = p.Sk - (tile_list[j] & 0x3fff) * kFwdTileK;
       int* s_id = ids_base;
       if (need_mask) {
         named_bar_sync(1 + g, 128);                  // the previous masked tile's readers are done with the buffer
@@ -1235,6 +1238,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
 #pragma unroll
           for (int i = 0; i < 32; ++i)
             if (s_id[c * 32 + i] > my_id) v[i] = 0xff800000u;
+          if (n_valid < kFwdTileK) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (c * 32 + i >= n_valid) v[i] = 0xff800000u;
+          }
         }
       };
       // O_g *= alpha_pend (rare, warp-uniform): only legal once the previous tile's P V MMAs have retired
@@ -2082,12 +2090,13 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
     auto prefetch = [&](int j) {
       if (j >= T || !(tile_list[j] & my_flag)) return;
       const int c = (tile_list[j] & 0x3fff) * kFwdTileK + tid;
-      pre_i = (c < p.Sk) ? (masked ? p.kid[static_cast<long long>(b) * p.Sk + c] : 0) : 0x7fffffff;
+      pre_i = (masked && c < p.Sk) ? p.kid[static_cast<long long>(b) * p.Sk + c] : 0;   // (c >= Sk: masked by position)
     };
     prefetch(0);
     for (int j = 0; j < T; ++j) {
       const int gj = base + j;
       const bool need_mask = (tile_list[j] & my_flag) != 0;
+      const int n_valid = p.Sk - (tile_list[j] & 0x3fff) * kFwdTileK;     // < kFwdTileK only in the ragged tail
       int* s_id = ids_base;
       if (need_mask) {
         named_bar_sync(1 + g, 128);
@@ -2103,6 +2112,11 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
 #pragma unroll
           for (int i = 0; i < 32; ++i)
             if (s_id[c * 32 + i] > my_id) v[i] = 0xff800000u;
+          if (n_valid < kFwdTileK) {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (c * 32 + i >= n_valid) v[i] = 0xff800000u;
+          }
         }
       };
       // O_g *= alpha_pend (rare, warp-uniform), 64 columns in two halves

@@ -211,6 +211,8 @@ int fk_attn_backward_tc_profile(const void* q, const void* k, const void* v, con
 /* tcgen05 / TMEM / TMA forward (attention_tc.cu): q / k / v are strided views ([B][S][H][head_dim], head_dim 32 or 64,
  * strides in elements; any other head_dim is rejected before anything is launched);
  * the V tile is read MN-major by the P V MMAs, so no transposed copy is needed; Sq == Sk == S.
+ * Labels: any int32 value is valid in qid and kid, INT32_MIN and INT32_MAX included (a query labelled INT32_MAX sees every
+ * key); the key positions past S of the last tile are masked by position, not by a reserved label.
  * counters: 2 caller-owned uint32, zero on entry, zero again on exit (see fk_attn_backward_tc). */
 int fk_attn_forward_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int S,
                        int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs,
