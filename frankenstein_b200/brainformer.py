@@ -7,7 +7,7 @@ into ``notebooks_trainer/{train_mae,train_brainformer,franky_baseline_gpt2}.ipyn
 fp32 master weights):
 
 * LayerNorm / RMSNorm, SwiGLU gate, RoPE: fused bandwidth-bound kernels (``ops.py`` -> libfk_b200.so);
-* self-attention (head_dim 32 or 64): flash-style kernel with the block-causal / gathered / padding mask
+* self-attention (head_dim 16, 32 or 64): flash-style kernel with the block-causal / gathered / padding mask
   evaluated analytically from integer labels -- the ``[S,S]`` (or ``[B,1,s,s]``) bool masks of the reference
   are never read (``attn_mask`` stays a registered buffer only so checkpoints keep their keys);
 * q/k/v as ONE fused projection (weights stay three ``nn.Linear`` modules for checkpoint compatibility),
@@ -159,12 +159,12 @@ class CausalSelfAttention(nn.Module):
             raise ops.FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
         B, T, _ = x.shape
         spec = rope
-        if isinstance(rope, torch.Tensor) and rope.dim() == 2 and self.head_dim in (32, 64):
+        if isinstance(rope, torch.Tensor) and rope.dim() == 2 and self.head_dim in (16, 32, 64):
             spec = RopeSpec.from_complex(rope, T, last=True)           # reference convention: rope[-T:]
         # unmasked calls with few tokens at head_dim != 32 (the perceiver's self-attention Block) take the few-query kernel
         small_ok = (attn_mask is None and self.head_dim != 32 and ops.small_attention_supported(T, self.head_dim)
                     and (rope is None or (isinstance(rope, torch.Tensor) and rope.dim() == 2)))
-        kernel_ok = (self.head_dim in (32, 64) and not small_ok and (attn_mask is None or isinstance(attn_mask, LabelMask))
+        kernel_ok = (self.head_dim in (16, 32, 64) and not small_ok and (attn_mask is None or isinstance(attn_mask, LabelMask))
                      and (spec is None or isinstance(spec, RopeSpec)))
         inner, dim = self.qw.weight.shape
         if kernel_ok and GEMM_IMPL == "own" and gemm.qkv_supported(dim, inner):
@@ -184,7 +184,7 @@ class CausalSelfAttention(nn.Module):
         else:
             q, k, v = qkv.view(B, T, 3, self.n_heads, self.head_dim).unbind(2)
             if isinstance(rope, RopeSpec):
-                raise ops.FkError("RopeSpec needs the head_dim-32 / 64 kernel path")
+                raise ops.FkError("RopeSpec needs the head_dim-16 / 32 / 64 kernel path")
             if rope is not None:
                 q, k = apply_rope(q, rope), apply_rope(k, rope)
             if isinstance(attn_mask, LabelMask):

@@ -632,6 +632,34 @@ rope64_kernel(__nv_bfloat16* __restrict__ x, long long bs, long long ts, int B, 
   *ptr = make_uint4(w[0], w[1], w[2], w[3]);
 }
 
+// Same at head_dim 16: table [P, 8] float2; one thread = one 16-byte chunk, 2 chunks per head.
+__global__ void __launch_bounds__(256)
+rope16_kernel(__nv_bfloat16* __restrict__ x, long long bs, long long ts, int B, int S, int H, const float2* __restrict__ table,
+              int P, const int* __restrict__ pos, int pos_offset, int inverse) {
+  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+  const long long total = static_cast<long long>(B) * S * H * 2;
+  if (idx >= total) return;
+  const int c = static_cast<int>(idx & 1);
+  const int h = static_cast<int>((idx >> 1) % H);
+  const long long bsidx = (idx >> 1) / H;
+  const int s = static_cast<int>(bsidx % S), b = static_cast<int>(bsidx / S);
+  int ps = pos ? pos[static_cast<long long>(b) * S + s] : s + pos_offset;
+  ps = min(max(ps, 0), P - 1);
+  uint4* ptr = reinterpret_cast<uint4*>(x + b * bs + static_cast<long long>(s) * ts + h * 16 + c * 8);
+  uint4 raw = *ptr;
+  uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
+  const float2* tb = table + static_cast<long long>(ps) * 8 + c * 4;
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
+    const float a = __bfloat162float(v.x), bb = __bfloat162float(v.y);
+    const float2 cs = tb[j];
+    const float sn = inverse ? -cs.y : cs.y;
+    w[j] = pack_bf16(a * cs.x - bb * sn, a * sn + bb * cs.x);
+  }
+  *ptr = make_uint4(w[0], w[1], w[2], w[3]);
+}
+
 }  // namespace fk
 
 using namespace fk;
@@ -722,7 +750,7 @@ FK_API int fk_attn_backward(const void* q, const void* k, const void* v, const v
 FK_API int fk_rope(void* x, long long bs, long long ts, int B, int S, int H, int head_dim, const float* table, int P,
                    const int* pos, int pos_offset, int inverse, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_rope: head_dim must be 32 or 64");
+  FK_REQUIRE(head_dim == 16 || head_dim == 32 || head_dim == 64, "fk_rope: head_dim must be 16, 32 or 64");
   FK_REQUIRE(x && table && B > 0 && S > 0 && H > 0 && P > 0, "fk_rope: bad argument");
   FK_REQUIRE(ts % 8 == 0 && bs % 8 == 0, "fk_rope: strides must keep 16-byte alignment");
   // positions s + pos_offset must lie inside the table (e.g. more tokens than the rope cache holds would make the
@@ -730,7 +758,7 @@ FK_API int fk_rope(void* x, long long bs, long long ts, int B, int S, int H, int
   FK_REQUIRE(pos != nullptr || (pos_offset >= 0 && static_cast<long long>(pos_offset) + S <= P),
              "fk_rope: token positions pos_offset .. pos_offset + S - 1 fall outside the rope table");
   const long long total = static_cast<long long>(B) * S * H * (head_dim / 8);
-  auto kern = head_dim == 64 ? rope64_kernel : rope_kernel;
+  auto kern = head_dim == 64 ? rope64_kernel : head_dim == 16 ? rope16_kernel : rope_kernel;
   kern<<<static_cast<unsigned>((total + 255) / 256), 256, 0, stream>>>(
       static_cast<__nv_bfloat16*>(x), bs, ts, B, S, H, reinterpret_cast<const float2*>(table), P, pos, pos_offset, inverse);
   FK_CHECK_LAUNCH();

@@ -1,5 +1,7 @@
 // Attention backward on the 5th-gen tensor cores (tcgen05.mma + TMEM + TMA), head_dim 32, label masks.  The head_dim-64
-// variants of the forward and backward kernels follow the head_dim-32 ones at the end of the file.
+// variants of the forward and backward kernels follow the head_dim-32 ones at the end of the file.  Head_dim 16 runs the
+// head_dim-32 kernels instantiated with HD = 16 (16-column heads, 32-byte rows and the 32-byte swizzle), on the default
+// path only: folded statistics, MN-major accumulate operands.
 //
 // Same math and mask rule as attention.cu (reference: F.scaled_dot_product_attention backward at
 // models/brainformer.py:168), restructured for Blackwell: every matmul is a tcgen05.mma issued by one thread,
@@ -55,7 +57,7 @@ struct TcParams {
   long long o0_bs, o0_ts, o1_bs, o1_ts;
   int B, H, S_row, S_col, Sq;
   float scale, scale_log2;
-  const float2* rope_table;                            // [rope_len][16] (cos, sin) or null: inverse RoPE fused into the
+  const float2* rope_table;                            // [rope_len][hd/2] (cos, sin) or null: inverse RoPE fused into the
   const int* rope_pos;                                 // store of dK / dQ (position of row = rope_pos ? rope_pos[b][row]
   int rope_len, rope_offset;                           //  : row + rope_offset), replacing two fk_rope passes per layer
   long long* prof;                                     // kProf instantiation: [n_ctas][16] cycle counters
@@ -174,12 +176,33 @@ __device__ __forceinline__ void tmem_wait1_32(uint32_t (&a)[32]) {
                :: "memory");
 }
 
+// Head width HD of the 16 / 32-wide kernels: a [tokens][HD] bf16 row is 2 HD bytes, TMA-loaded with the swizzle of that
+// width (SWIZZLE_32B at 16, SWIZZLE_64B at 32).  A K step of 16 rows of an MN-major tile adds 2 HD in the descriptor's
+// (address >> 4) field.
+template <int HD>
+__device__ __forceinline__ uint64_t umma_desc_rows(uint32_t saddr) {
+  if constexpr (HD == 16) return umma_desc_sw32(saddr);
+  else return umma_desc_sw64(saddr);
+}
+template <int N>
+__device__ __forceinline__ void tmem_ld_wait(uint32_t taddr, uint32_t (&r)[N]) {
+  if constexpr (N == 16) { tmem_ld16(taddr, r); tmem_wait1_16(r); }
+  else { tmem_ld32(taddr, r); tmem_wait1_32(r); }
+}
+template <int N>
+__device__ __forceinline__ void tmem_st_cols(uint32_t taddr, const uint32_t (&r)[N]) {
+  if constexpr (N == 16) tmem_st16(taddr, r);
+  else tmem_st32(taddr, r);
+}
+
 // Work-item hand-out of the persistent kernels: p.items[0] = next item, p.items[1] = CTAs that have finished; the last
 // CTA to finish puts both back to zero, so no host-side reset (and no extra launch) is needed.  The two words belong
 // to the caller (one pair per launch in flight: launches on different streams must be given different pairs), so the
 // library holds no device-side state and is re-entrant per stream.
 
-template <int MODE, int kProf, bool kFold>
+// HD = 16 is instantiated on the default path only (kProf 0, folded statistics, MN-major accumulate operands): the
+// resident tiles take 8 packed TMEM columns each, the score MMAs one K step, the accumulate MMAs N = 16.
+template <int MODE, int kProf, bool kFold, int HD = 32>
 __global__ void __launch_bounds__(kTcThreads, 1)
 attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_constant__ CUtensorMap tm_resB,
                    const __grid_constant__ CUtensorMap tm_stA, const __grid_constant__ CUtensorMap tm_stB,
@@ -344,6 +367,8 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
   }
 
   constexpr uint32_t kStageBytes = (MODE == MODE_DKV) ? 16384u : 12288u;
+  constexpr uint32_t kResBytes = 2u * kRows * HD * 2u;       // resident A | B tiles
+  constexpr uint32_t kTileBytes = 2u * kCols * HD * 2u;      // streamed A | B tiles
 
   if (warp == 0) {
     // ================================ TMA producer ================================
@@ -356,7 +381,7 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
       long long w_se = 0;
       auto load_resident = [&](int h_, int r0_, int b_, int buf) {
         if (elect_one()) {
-          mbar_expect_tx(&res_full[buf], (MODE == MODE_DQ && fold) ? 16384u + 4096u : 16384u);
+          mbar_expect_tx(&res_full[buf], (MODE == MODE_DQ && fold) ? kResBytes + 4096u : kResBytes);
           tma_load_4d(smem + TcSmem::resA + buf * 16384, &tm_resA, &res_full[buf], 0, h_, r0_, b_);
           tma_load_4d(smem + TcSmem::resB + buf * 16384, &tm_resB, &res_full[buf], 0, h_, r0_, b_);
           if (MODE == MODE_DQ && fold) tma_load_4d(smem + TcSmem::aug_res + buf * 4096, &tm_aug, &res_full[buf], 0, r0_, h_, b_);
@@ -367,11 +392,11 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
         uint8_t* st = smem + TcSmem::stream + pstage * 16384;
         wait_acc<kProf>(&st_empty[pstage], pphase ^ 1, w_se);
         if (elect_one()) {
-          mbar_expect_tx(&st_full[pstage], p.mn_major ? ((MODE == MODE_DKV && fold) ? 8192u + 2048u : 8192u) : kStageBytes);
+          mbar_expect_tx(&st_full[pstage], (HD == 16 || p.mn_major) ? ((MODE == MODE_DKV && fold) ? kTileBytes + 2048u : kTileBytes) : kStageBytes);
           tma_load_4d(st, &tm_stA, &st_full[pstage], 0, h_, t * kCols, b_);
           tma_load_4d(st + 4096, &tm_stB, &st_full[pstage], 0, h_, t * kCols, b_);
           if (MODE == MODE_DKV && fold) tma_load_4d(st + 8192, &tm_aug, &st_full[pstage], 0, t * kCols, h_, b_);   // statistics rows of the tile's queries
-          if (!p.mn_major) {
+          if (HD == 32 && !p.mn_major) {
             if (MODE == MODE_DKV) tma_load_2d(st + 8192, &tm_tA, &st_full[pstage], t * kCols, (b_ * p.H + h_) * 32);
             tma_load_2d(st + 12288, &tm_tB, &st_full[pstage], t * kCols, (b_ * p.H + h_) * 32);
           }
@@ -417,7 +442,7 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
         const int stage = gt % kNST, g = gt % kNG, n = gt / kNG;
         // (operands of the MMAs are formed BEFORE the waits: ~50 uniform-datapath instructions that would otherwise sit
         //  on the critical path stage_free -> score MMAs)
-        uint64_t dS = umma_desc_sw64(stream + stage * 16384), dD = umma_desc_sw64(stream + stage * 16384 + 4096);
+        uint64_t dS = umma_desc_rows<HD>(stream + stage * 16384), dD = umma_desc_rows<HD>(stream + stage * 16384 + 4096);
         uint32_t d_s = tmem_u + g * 128, d_dp = tmem_u + g * 128 + 64;
         uint64_t* const bar_full = &sdp_full[g];
         // statistics K step (fold): DKV  A = constant ones tile (keys), B = the tile's query statistics;
@@ -444,13 +469,13 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
           // a K step of 16 bf16 = 32 bytes = +2 in the descriptor's (address >> 4) field
           // TS mode: A = the resident tile in TMEM (K step of 16 elements = 8 packed columns)
           umma_bf16_ts(d_s, tA, dS, idesc_score, 0u);
-          umma_bf16_ts(d_s, tA + 8, dS + 2, idesc_score, 1u);
+          if (HD == 32) umma_bf16_ts(d_s, tA + 8, dS + 2, idesc_score, 1u);
           if (fold) {
             umma_bf16_ts(d_s, MODE == MODE_DKV ? tmem_u + kOnesCol : tmem_u + kAugCol, fB_s, idesc_score, 1u);
             umma_commit(bar_full);                         // S' complete: the warpgroup starts on the exponentials
           }
           umma_bf16_ts(d_dp, tB, dD, idesc_score, 0u);
-          umma_bf16_ts(d_dp, tB + 8, dD + 2, idesc_score, 1u);
+          if (HD == 32) umma_bf16_ts(d_dp, tB + 8, dD + 2, idesc_score, 1u);
           if (fold) {
             umma_bf16_ts(d_dp, MODE == MODE_DKV ? tmem_u + kOnesCol + 8 : tmem_u + kAugCol, fB_d, idesc_score, 1u);
             umma_commit(&dp_full[g]);
@@ -466,7 +491,7 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
   } else if (warp == 3) {
     // ================================ accumulate-MMA issuer ================================
     {
-      constexpr uint32_t idesc_acc = umma_idesc_bf16(kRows, 32);
+      constexpr uint32_t idesc_acc = umma_idesc_bf16(kRows, HD);
       const int T_u = __shfl_sync(0xffffffffu, T, 0);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       const uint32_t stream = smem_u32(smem + TcSmem::stream);
@@ -476,22 +501,23 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
         const int stage = gt % kNST, g = gt % kNG, n = gt / kNG;
         // (operands formed before the wait, see the score issuer)
         uint32_t ta = tmem_u + g * 128;                   // P pairs at +0..31, dS pairs at +64..95 (written in place)
-        uint64_t dMA = umma_desc_sw64(stream + stage * 16384 + 4096), dMB = umma_desc_sw64(stream + stage * 16384);
+        uint64_t dMA = umma_desc_rows<HD>(stream + stage * 16384 + 4096), dMB = umma_desc_rows<HD>(stream + stage * 16384);
         uint64_t* const bar_free = &stage_free[g];
         uint64_t* const bar_empty = &st_empty[stage];
         asm volatile("" : "+l"(dMA), "+l"(dMB), "+r"(ta));      // pin (see the score issuer)
         wait_acc<kProf>(&p_ready[g], n & 1, w_pr);
         if (kFull && trace && lane == 0 && ia < 128) trace[0 * 128 + ia] = clock64();
         tc_fence_after();
-        if (p.mn_major) {
+        if (HD == 16 || p.mn_major) {
           // B operand straight from the score stage: tile [64 tokens][32 dims], 64-byte rows, SWIZZLE_64B = the canonical
-          // MN-major layout (N = 32 dims contiguous, 8-token groups 512 B apart); a K step of 16 tokens = 1024 B.
+          // MN-major layout (N = 32 dims contiguous, 8-token groups 512 B apart); a K step of 16 tokens = 1024 B.  (At
+          // head_dim 16: [64 tokens][16 dims], 32-byte rows, SWIZZLE_32B, 8-token groups 256 B apart, K step 512 B.)
           // DKV: dV += P^T dO (stB), dK += dS^T Q (stA).  DQ: dQ += dS K (stA).
           if (elect_one()) {
 #pragma unroll
             for (int kk = 0; kk < 4; ++kk) {
-              if (MODE == MODE_DKV) umma_bf16_ts(tmem_u + kAccCol, ta + kk * 8, dMA + 64 * kk, idesc_acc | (1u << 16), (ia > 0 || kk > 0) ? 1u : 0u);
-              umma_bf16_ts(tmem_u + kAccCol + 32, ta + 64 + kk * 8, dMB + 64 * kk, idesc_acc | (1u << 16), (ia > 0 || kk > 0) ? 1u : 0u);
+              if (MODE == MODE_DKV) umma_bf16_ts(tmem_u + kAccCol, ta + kk * 8, dMA + 2 * HD * kk, idesc_acc | (1u << 16), (ia > 0 || kk > 0) ? 1u : 0u);
+              umma_bf16_ts(tmem_u + kAccCol + 32, ta + 64 + kk * 8, dMB + 2 * HD * kk, idesc_acc | (1u << 16), (ia > 0 || kk > 0) ? 1u : 0u);
             }
             umma_commit(bar_free);
             umma_commit(bar_empty);
@@ -539,6 +565,18 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
       // ends with a CTA-wide barrier behind acc_full.)
       mbar_wait(&res_full[item_n & 1], (item_n >> 1) & 1);
       const uint32_t lane_addr = tmem_base + (static_cast<uint32_t>(q4 * 32) << 16);
+      if constexpr (HD == 16) {
+        // 32-byte rows, SWIZZLE_32B (the halves swap when bit 2 of r is set): 8 packed columns per tile
+        const int s1 = (r >> 2) & 1;
+#pragma unroll
+        for (int t2 = 0; t2 < 2; ++t2) {
+          const uint8_t* rowp = smem + (t2 ? TcSmem::resB : TcSmem::resA) + (item_n & 1) * 16384 + r * 32;
+          const uint4 w0 = *reinterpret_cast<const uint4*>(rowp + ((0 ^ s1) << 4));
+          const uint4 w1 = *reinterpret_cast<const uint4*>(rowp + ((1 ^ s1) << 4));
+          const uint32_t v8[8] = {w0.x, w0.y, w0.z, w0.w, w1.x, w1.y, w1.z, w1.w};
+          tmem_st8(lane_addr + kResCol + t2 * 16, v8);
+        }
+      } else {
       const int sw = (r >> 1) & 3;
 #pragma unroll
       for (int t2 = 0; t2 < 2; ++t2) {
@@ -550,6 +588,7 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
           v[4 * c] = w.x; v[4 * c + 1] = w.y; v[4 * c + 2] = w.z; v[4 * c + 3] = w.w;
         }
         tmem_st16(lane_addr + kResCol + t2 * 16, v);
+      }
       }
       if (fold && MODE == MODE_DQ) {
         // statistics rows of the resident queries (32-byte rows, SWIZZLE_32B: the halves swap when bit 2 of r is set)
@@ -780,27 +819,26 @@ attn_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_con
     const bool writes = (MODE == MODE_DKV) ? (g < 2) : (g == 1);     // warp-uniform: wg0 -> acc0 (dV), wg1 -> acc1 (dK / dQ)
     if (writes) {
       const int which = (MODE == MODE_DKV) ? g : 1;
-      uint32_t acc[32];
+      uint32_t acc[HD];
       if (T > 0) {                                        // uniform: the whole warp executes the aligned TMEM load
-        tmem_ld32(tmem_base + (static_cast<uint32_t>(q4 * 32) << 16) + kAccCol + which * 32, acc);
-        tmem_wait1_32(acc);
+        tmem_ld_wait<HD>(tmem_base + (static_cast<uint32_t>(q4 * 32) << 16) + kAccCol + which * 32, acc);
       } else {
 #pragma unroll
-        for (int i = 0; i < 32; ++i) acc[i] = 0u;
+        for (int i = 0; i < HD; ++i) acc[i] = 0u;
       }
       if (row_ok) {
         const float sc = (which == 1) ? p.scale : 1.f;
         __nv_bfloat16* dst = (which == 0 ? p.out0 + b * p.o0_bs + static_cast<long long>(row) * p.o0_ts
-                                         : p.out1 + b * p.o1_bs + static_cast<long long>(row) * p.o1_ts) + h * 32;
+                                         : p.out1 + b * p.o1_bs + static_cast<long long>(row) * p.o1_ts) + h * HD;
         // gradient of a rotated operand (dK / dQ): rotate back (conjugate), as fk_rope(inverse = 1) would afterwards
         const float2* tb = nullptr;
         if (which == 1 && p.rope_table != nullptr) {
           int ps = p.rope_pos ? p.rope_pos[static_cast<long long>(b) * p.S_row + row] : row + p.rope_offset;
           ps = min(max(ps, 0), p.rope_len - 1);
-          tb = p.rope_table + static_cast<long long>(ps) * 16;
+          tb = p.rope_table + static_cast<long long>(ps) * (HD / 2);
         }
 #pragma unroll
-        for (int c4 = 0; c4 < 4; ++c4) {
+        for (int c4 = 0; c4 < HD / 8; ++c4) {
           uint32_t w[4];
 #pragma unroll
           for (int e = 0; e < 4; ++e) {
@@ -865,6 +903,7 @@ __device__ __forceinline__ void split3(float x, float& hi, float& mid, float& lo
   lo = __bfloat162float(__float2bfloat16_rn(r1 - mid));
 }
 
+template <int HD>      // 16 or 32 (head_dim 64: attn_aug64_kernel)
 __global__ void __launch_bounds__(256)
 attn_aug_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o, const float* __restrict__ lse,
                 float* __restrict__ delta, __nv_bfloat16* __restrict__ aug, int B, int H, int S, long long o_bs, long long o_ts,
@@ -874,11 +913,11 @@ attn_aug_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __rest
   const int h = static_cast<int>(idx % H);
   const long long bi = idx / H;
   const int i = static_cast<int>(bi % S), b = static_cast<int>(bi / S);
-  const uint4* op = reinterpret_cast<const uint4*>(o + b * o_bs + static_cast<long long>(i) * o_ts + h * 32);
-  const uint4* dp = reinterpret_cast<const uint4*>(d_o + b * do_bs + static_cast<long long>(i) * do_ts + h * 32);
+  const uint4* op = reinterpret_cast<const uint4*>(o + b * o_bs + static_cast<long long>(i) * o_ts + h * HD);
+  const uint4* dp = reinterpret_cast<const uint4*>(d_o + b * do_bs + static_cast<long long>(i) * do_ts + h * HD);
   float acc = 0.f;
 #pragma unroll
-  for (int c = 0; c < 4; ++c) {
+  for (int c = 0; c < HD / 8; ++c) {
     const uint4 a = op[c], e = dp[c];
     const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, ew[4] = {e.x, e.y, e.z, e.w};
 #pragma unroll
@@ -973,6 +1012,9 @@ struct FwdParams {
   unsigned int* items;                                  // caller-owned hand-out counters (see TcParams::items)
 };
 
+// HD = 16: Q / K / V rows of 32 B (SWIZZLE_32B), one score K step, P V MMAs N = 16; O_g uses the first 16 of its 32
+// TMEM columns.
+template <int HD>
 __global__ void __launch_bounds__(kFwdThreads, 1)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                    const __grid_constant__ CUtensorMap tm_v, const FwdParams p) {
@@ -1100,7 +1142,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       const int T_u = __shfl_sync(0xffffffffu, T, 0);
       auto load_q = [&](int h_, int q0_, int b_, int buf) {
         if (elect_one()) {
-          mbar_expect_tx(&q_full[buf], 16384);
+          mbar_expect_tx(&q_full[buf], 2 * 128 * HD * 2);
           tma_load_4d(smem + FwdSmem::q + buf * 16384, &tm_q, &q_full[buf], 0, h_, q0_, b_);
           tma_load_4d(smem + FwdSmem::q + buf * 16384 + 8192, &tm_q, &q_full[buf], 0, h_, q0_ + 128, b_);
         }
@@ -1110,7 +1152,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
         uint8_t* st = smem + FwdSmem::stream + pstage * 16384;
         mbar_wait(&st_empty[pstage], pphase ^ 1);
         if (elect_one()) {
-          mbar_expect_tx(&st_full[pstage], 16384);
+          mbar_expect_tx(&st_full[pstage], 2 * kFwdTileK * HD * 2);
           tma_load_4d(st, &tm_k, &st_full[pstage], 0, h_, t * kFwdTileK, b_);
           tma_load_4d(st + 8192, &tm_v, &st_full[pstage], 0, h_, t * kFwdTileK, b_);      // V tile [128 keys][32 dims]
         }
@@ -1139,8 +1181,8 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       constexpr uint32_t idesc = umma_idesc_bf16(128, kFwdTileK);
       const int T_u = __shfl_sync(0xffffffffu, T, 0);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-      const uint64_t dQ[2] = {umma_desc_sw64(smem_u32(smem + FwdSmem::q + (item_n & 1) * 16384)),
-                              umma_desc_sw64(smem_u32(smem + FwdSmem::q + (item_n & 1) * 16384 + 8192))};
+      const uint64_t dQ[2] = {umma_desc_rows<HD>(smem_u32(smem + FwdSmem::q + (item_n & 1) * 16384)),
+                              umma_desc_rows<HD>(smem_u32(smem + FwdSmem::q + (item_n & 1) * 16384 + 8192))};
       const uint32_t stream = smem_u32(smem + FwdSmem::stream);
       mbar_wait(&q_full[item_n & 1], (item_n >> 1) & 1);
       tc_fence_after();
@@ -1148,14 +1190,14 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
         const int gj = base + j;                     // key-tile counter across items
         const int stage = gj % kNST;
         mbar_wait(&st_full[stage], (gj / kNST) & 1);
-        const uint64_t dK = umma_desc_sw64(stream + stage * 16384);
+        const uint64_t dK = umma_desc_rows<HD>(stream + stage * 16384);
 #pragma unroll
         for (int g = 0; g < 2; ++g) {
           mbar_wait(&s_free[g], (gj & 1) ^ 1);
           tc_fence_after();
           if (elect_one()) {
             umma_bf16(tmem_u + g * 128, dQ[g], dK, idesc, 0u);
-            umma_bf16(tmem_u + g * 128, dQ[g] + 2, dK + 2, idesc, 1u);
+            if (HD == 32) umma_bf16(tmem_u + g * 128, dQ[g] + 2, dK + 2, idesc, 1u);
             umma_commit(&s_full[g]);
           }
           __syncwarp();
@@ -1165,7 +1207,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
   } else if (warp == 3) {
     // ================================ P V MMA issuer ================================
     {
-      constexpr uint32_t idesc = umma_idesc_bf16(128, 32);
+      constexpr uint32_t idesc = umma_idesc_bf16(128, HD);
       const int T_u = __shfl_sync(0xffffffffu, T, 0);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
       const uint32_t stream = smem_u32(smem + FwdSmem::stream);
@@ -1173,8 +1215,8 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
         const int gj = base + j;
         const int stage = gj % kNST;
         // V tile [128 keys][32 dims] (64-byte rows, SWIZZLE_64B) read MN-major: N = dims contiguous, K = keys, a K step of
-        // 16 keys = 1024 B -- no transposed copy of V exists
-        const uint64_t dV = umma_desc_sw64(stream + stage * 16384 + 8192);
+        // 16 keys = 1024 B -- no transposed copy of V exists (head_dim 16: 32-byte rows, SWIZZLE_32B, K step 512 B)
+        const uint64_t dV = umma_desc_rows<HD>(stream + stage * 16384 + 8192);
 #pragma unroll
         for (int g = 0; g < 2; ++g) {
           mbar_wait(&p_ready[g], gj & 1);
@@ -1183,7 +1225,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
           if (elect_one()) {
 #pragma unroll
             for (int kk = 0; kk < 8; ++kk)
-              umma_bf16_ts(oa, pa + kk * 8, dV + 64 * kk, idesc | (1u << 16), (j > 0 || kk > 0) ? 1u : 0u);
+              umma_bf16_ts(oa, pa + kk * 8, dV + 2 * HD * kk, idesc | (1u << 16), (j > 0 || kk > 0) ? 1u : 0u);
             umma_commit(&p_free[g]);
             umma_commit(&st_empty[stage]);
           }
@@ -1248,12 +1290,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       // O_g *= alpha_pend (rare, warp-uniform): only legal once the previous tile's P V MMAs have retired
       auto apply_pending = [&]() {
         if (__any_sync(0xffffffffu, alpha_pend != 1.f)) {
-          uint32_t ov[32];
-          tmem_ld32(o_addr, ov);
-          tmem_wait1_32(ov);
+          uint32_t ov[HD];
+          tmem_ld_wait<HD>(o_addr, ov);
 #pragma unroll
-          for (int i = 0; i < 32; ++i) ov[i] = __float_as_uint(__uint_as_float(ov[i]) * alpha_pend);
-          tmem_st32(o_addr, ov);
+          for (int i = 0; i < HD; ++i) ov[i] = __float_as_uint(__uint_as_float(ov[i]) * alpha_pend);
+          tmem_st_cols<HD>(o_addr, ov);
           alpha_pend = 1.f;
         }
       };
@@ -1351,19 +1392,18 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       mbar_wait(&p_free[g], ((base + T) & 1) ^ 1);     // the last P V MMAs have retired
       tc_fence_after();
     }
-    uint32_t ov[32];
+    uint32_t ov[HD];
     if (T > 0) {
-      tmem_ld32(o_addr, ov);
-      tmem_wait1_32(ov);
+      tmem_ld_wait<HD>(o_addr, ov);
     } else {
 #pragma unroll
-      for (int i = 0; i < 32; ++i) ov[i] = 0u;
+      for (int i = 0; i < HD; ++i) ov[i] = 0u;
     }
     if (row_ok) {
       const float inv = (l_run > 0.f) ? alpha_pend / l_run : 0.f;      // a reference raise after the last tile is still owed to O
-      __nv_bfloat16* dst = p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * 32;
+      __nv_bfloat16* dst = p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * HD;
 #pragma unroll
-      for (int c4 = 0; c4 < 4; ++c4) {
+      for (int c4 = 0; c4 < HD / 8; ++c4) {
         uint32_t w[4];
 #pragma unroll
         for (int e = 0; e < 4; ++e)
@@ -2287,9 +2327,10 @@ FK_API int fk_attn_transpose(const void* x, long long bs, long long ts, int B, i
 
 static int bwd_sm_count() { return fk_sm_count(); }
 
-// head_dim 64 backward (attn_bwd_tc64_kernel): one path -- statistics folded (aug required), MN-major accumulate operands
-// (no transposed copies), no stall-accounting build.  Arguments already checked by the caller as far as they are shared.
-static int attn_backward_tc64(const void* q, const void* k, const void* v, const void* d_o, const void* qt, const void* kt,
+// head_dim 16 (attn_bwd_tc_kernel<.., 16>) and 64 (attn_bwd_tc64_kernel) backward: one path -- statistics folded (aug
+// required), MN-major accumulate operands (no transposed copies), no stall-accounting build.  Arguments already checked by
+// the caller as far as they are shared.
+static int attn_backward_one_path(int head_dim, const void* q, const void* k, const void* v, const void* d_o, const void* qt, const void* kt,
                               const void* dot, const void* aug, void* dq, void* dk, void* dv, int B, int H, int S,
                               long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs, long long v_ts,
                               long long do_bs, long long do_ts, long long dq_bs, long long dq_ts, long long dk_bs,
@@ -2298,10 +2339,10 @@ static int attn_backward_tc64(const void* q, const void* k, const void* v, const
                               const float* lse, const float* delta, const float* rope_table, int rope_len,
                               const int* rope_pos, int rope_offset, int parts, unsigned int* counters,
                               const long long* g_attn_prof, cudaStream_t stream) {
-  FK_REQUIRE(qt == nullptr && kt == nullptr && dot == nullptr, "fk_attn_backward_tc: head_dim 64 takes no transposed operands");
+  FK_REQUIRE(qt == nullptr && kt == nullptr && dot == nullptr, "fk_attn_backward_tc: head_dim 16 / 64 take no transposed operands");
   FK_REQUIRE(aug != nullptr && (reinterpret_cast<uintptr_t>(aug) & 31) == 0,
-             "fk_attn_backward_tc: head_dim 64 needs the statistics rows of fk_attn_aug (32-byte aligned)");
-  FK_REQUIRE(g_attn_prof == nullptr, "fk_attn_backward_tc_profile: no stall-accounting build at head_dim 64");
+             "fk_attn_backward_tc: head_dim 16 / 64 need the statistics rows of fk_attn_aug (32-byte aligned)");
+  FK_REQUIRE(g_attn_prof == nullptr, "fk_attn_backward_tc_profile: no stall-accounting build at head_dim 16 / 64");
   FK_REQUIRE(!(parts & 2) || (dk && dv), "fk_attn_backward_tc: dK/dV needs dk, dv");
   FK_REQUIRE(!(parts & 4) || dq, "fk_attn_backward_tc: dQ needs dq");
   FK_REQUIRE(dq_ts % 8 == 0 && dq_bs % 8 == 0 && dk_ts % 8 == 0 && dk_bs % 8 == 0 && dv_ts % 8 == 0 && dv_bs % 8 == 0,
@@ -2310,7 +2351,9 @@ static int attn_backward_tc64(const void* q, const void* k, const void* v, const
   bool& attr_set = attr_set_dev[fk_device_ordinal()];
   if (!attr_set) {
     if (cudaFuncSetAttribute(attn_bwd_tc64_kernel<MODE_DKV>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem64::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_bwd_tc64_kernel<MODE_DQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem64::total) != cudaSuccess) {
+        cudaFuncSetAttribute(attn_bwd_tc64_kernel<MODE_DQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem64::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_bwd_tc_kernel<MODE_DKV, 0, true, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_bwd_tc_kernel<MODE_DQ, 0, true, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSmem::total) != cudaSuccess) {
       fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
       return FK_ERR_CUDA;
     }
@@ -2318,14 +2361,15 @@ static int attn_backward_tc64(const void* q, const void* k, const void* v, const
   }
   CUtensorMap mQ128, mDO128, mK128, mV128, mQ64, mDO64, mK64, mV64, mAug64, mAug128;
   int rc = 0;
-  rc |= make_tmap_heads_sw128(&mQ128, q, B, S, H, q_bs, q_ts, kRows);
-  rc |= make_tmap_heads_sw128(&mDO128, d_o, B, S, H, do_bs, do_ts, kRows);
-  rc |= make_tmap_heads_sw128(&mK128, k, B, S, H, k_bs, k_ts, kRows);
-  rc |= make_tmap_heads_sw128(&mV128, v, B, S, H, v_bs, v_ts, kRows);
-  rc |= make_tmap_heads_sw128(&mQ64, q, B, S, H, q_bs, q_ts, kCols);
-  rc |= make_tmap_heads_sw128(&mDO64, d_o, B, S, H, do_bs, do_ts, kCols);
-  rc |= make_tmap_heads_sw128(&mK64, k, B, S, H, k_bs, k_ts, kCols);
-  rc |= make_tmap_heads_sw128(&mV64, v, B, S, H, v_bs, v_ts, kCols);
+  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : make_tmap_heads_sw32;
+  rc |= make_map(&mQ128, q, B, S, H, q_bs, q_ts, kRows);
+  rc |= make_map(&mDO128, d_o, B, S, H, do_bs, do_ts, kRows);
+  rc |= make_map(&mK128, k, B, S, H, k_bs, k_ts, kRows);
+  rc |= make_map(&mV128, v, B, S, H, v_bs, v_ts, kRows);
+  rc |= make_map(&mQ64, q, B, S, H, q_bs, q_ts, kCols);
+  rc |= make_map(&mDO64, d_o, B, S, H, do_bs, do_ts, kCols);
+  rc |= make_map(&mK64, k, B, S, H, k_bs, k_ts, kCols);
+  rc |= make_map(&mV64, v, B, S, H, v_bs, v_ts, kCols);
   rc |= make_tmap_aug_sw32(&mAug64, aug, B, S, H, kCols);
   rc |= make_tmap_aug_sw32(&mAug128, aug, B, S, H, kRows);
   if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
@@ -2345,7 +2389,8 @@ static int attn_backward_tc64(const void* q, const void* k, const void* v, const
     pk.out0 = static_cast<__nv_bfloat16*>(dv); pk.o0_bs = dv_bs; pk.o0_ts = dv_ts;
     pk.out1 = static_cast<__nv_bfloat16*>(dk); pk.o1_bs = dk_bs; pk.o1_ts = dk_ts;
     pk.items = counters;
-    attn_bwd_tc64_kernel<MODE_DKV><<<grid, kTcThreads, TcSmem64::total, stream>>>(mK128, mV128, mQ64, mDO64, mAug64, pk);
+    if (head_dim == 64) attn_bwd_tc64_kernel<MODE_DKV><<<grid, kTcThreads, TcSmem64::total, stream>>>(mK128, mV128, mQ64, mDO64, mAug64, pk);
+    else attn_bwd_tc_kernel<MODE_DKV, 0, true, 16><<<grid, kTcThreads, TcSmem::total, stream>>>(mK128, mV128, mQ64, mDO64, mDO64, mQ64, mAug64, pk);
     FK_CHECK_LAUNCH();
     ++n;
   }
@@ -2354,7 +2399,8 @@ static int attn_backward_tc64(const void* q, const void* k, const void* v, const
     pq.row_id = qid; pq.col_id = kid; pq.row_min = qmin; pq.row_max = qmax; pq.col_min = kmin; pq.col_max = kmax;
     pq.out1 = static_cast<__nv_bfloat16*>(dq); pq.o1_bs = dq_bs; pq.o1_ts = dq_ts;
     pq.items = counters + 2;
-    attn_bwd_tc64_kernel<MODE_DQ><<<grid, kTcThreads, TcSmem64::total, stream>>>(mQ128, mDO128, mK64, mV64, mAug128, pq);
+    if (head_dim == 64) attn_bwd_tc64_kernel<MODE_DQ><<<grid, kTcThreads, TcSmem64::total, stream>>>(mQ128, mDO128, mK64, mV64, mAug128, pq);
+    else attn_bwd_tc_kernel<MODE_DQ, 0, true, 16><<<grid, kTcThreads, TcSmem::total, stream>>>(mQ128, mDO128, mK64, mV64, mK64, mK64, mAug128, pq);
     FK_CHECK_LAUNCH();
     ++n;
   }
@@ -2389,7 +2435,7 @@ FK_API int fk_attn_backward_tc_profile(const void* q, const void* k, const void*
                                const int* rope_pos, int rope_offset, int parts, unsigned int* counters, long long* g_attn_prof,
                                int g_attn_prof_mode, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_attn_backward_tc: head_dim must be 32 or 64");
+  FK_REQUIRE(head_dim == 16 || head_dim == 32 || head_dim == 64, "fk_attn_backward_tc: head_dim must be 16, 32 or 64");
   FK_REQUIRE(counters != nullptr, "fk_attn_backward_tc: counters (4 zero-initialised uint32, one set per launch in flight) is null");
   FK_REQUIRE(rope_table == nullptr || rope_len > 0, "fk_attn_backward_tc: rope_len must be positive with a rope table");
   FK_REQUIRE(q && k && v && d_o && lse && delta && B > 0 && H > 0 && S > 0, "fk_attn_backward_tc: bad argument");
@@ -2398,8 +2444,8 @@ FK_API int fk_attn_backward_tc_profile(const void* q, const void* k, const void*
   FK_REQUIRE(qid == nullptr || (qmin && qmax && kmin && kmax), "fk_attn_backward_tc: label ranges missing");
   FK_REQUIRE((S + kCols - 1) / kCols <= kMaxTiles, "fk_attn_backward_tc: sequence too long");
   FK_REQUIRE(Sp >= S && Sp % 8 == 0, "fk_attn_backward_tc: Sp must be >= S and a multiple of 8");
-  if (head_dim == 64)
-    return attn_backward_tc64(q, k, v, d_o, qt, kt, dot, aug, dq, dk, dv, B, H, S, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, do_bs,
+  if (head_dim != 32)
+    return attn_backward_one_path(head_dim, q, k, v, d_o, qt, kt, dot, aug, dq, dk, dv, B, H, S, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, do_bs,
                               do_ts, dq_bs, dq_ts, dk_bs, dk_ts, dv_bs, dv_ts, qid, kid, qmin, qmax, kmin, kmax, scale, lse,
                               delta, rope_table, rope_len, rope_pos, rope_offset, parts, counters, g_attn_prof, stream);
   static bool attr_set_dev[FK_MAX_DEVICES];
@@ -2500,17 +2546,17 @@ FK_API int fk_attn_backward_tc_profile(const void* q, const void* k, const void*
 }
 
 // delta = rowsum(dO * O) and the statistics rows the folded backward takes (see attn_aug_kernel): o / d_o bf16
-// [B, S, H, head_dim] (32 or 64) with strides in elements, lse fp32 [B, H, S] (log2 domain, from the forward), delta fp32
+// [B, S, H, head_dim] (16, 32 or 64) with strides in elements, lse fp32 [B, H, S] (log2 domain, from the forward), delta fp32
 // [B, H, S], aug bf16 [B, H, S, 16].
 FK_API int fk_attn_aug(const void* o, const void* d_o, const float* lse, float* delta, void* aug, int B, int H, int S,
                        int head_dim, long long o_bs, long long o_ts, long long do_bs, long long do_ts, float scale, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_attn_aug: head_dim must be 32 or 64");
+  FK_REQUIRE(head_dim == 16 || head_dim == 32 || head_dim == 64, "fk_attn_aug: head_dim must be 16, 32 or 64");
   FK_REQUIRE(o && d_o && lse && delta && aug && B > 0 && H > 0 && S > 0 && scale > 0.f, "fk_attn_aug: bad argument");
   FK_REQUIRE(o_ts % 8 == 0 && do_ts % 8 == 0 && o_bs % 8 == 0 && do_bs % 8 == 0, "fk_attn_aug: strides must keep 16-byte alignment");
   FK_REQUIRE((reinterpret_cast<uintptr_t>(aug) & 31) == 0, "fk_attn_aug: aug must be 32-byte aligned");
   const long long n = static_cast<long long>(B) * S * H;
-  auto kern = head_dim == 64 ? attn_aug64_kernel : attn_aug_kernel;
+  auto kern = head_dim == 64 ? attn_aug64_kernel : head_dim == 16 ? attn_aug_kernel<16> : attn_aug_kernel<32>;
   kern<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(
       static_cast<const __nv_bfloat16*>(o), static_cast<const __nv_bfloat16*>(d_o), lse, delta, static_cast<__nv_bfloat16*>(aug), B, H, S,
       o_bs, o_ts, do_bs, do_ts, 1.f / (scale * 1.4426950408889634f));
@@ -2526,7 +2572,7 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
                               const int* qmax, const int* kmin, const int* kmax, float scale, unsigned int* counters,
                               void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(head_dim == 32 || head_dim == 64, "fk_attn_forward_tc: head_dim must be 32 or 64");
+  FK_REQUIRE(head_dim == 16 || head_dim == 32 || head_dim == 64, "fk_attn_forward_tc: head_dim must be 16, 32 or 64");
   FK_REQUIRE(counters != nullptr, "fk_attn_forward_tc: counters (2 zero-initialised uint32, one pair per launch in flight) is null");
   FK_REQUIRE(q && k && v && out && B > 0 && H > 0 && S > 0, "fk_attn_forward_tc: bad argument");
   FK_REQUIRE((qid == nullptr) == (kid == nullptr), "fk_attn_forward_tc: qid and kid go together");
@@ -2536,7 +2582,8 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   static bool attr_set_dev[FK_MAX_DEVICES];
   bool& attr_set = attr_set_dev[fk_device_ordinal()];
   if (!attr_set) {
-    if (cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+    if (cudaFuncSetAttribute(attn_fwd_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
         cudaFuncSetAttribute(attn_fwd_tc64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
       fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
       return FK_ERR_CUDA;
@@ -2545,7 +2592,7 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   }
   CUtensorMap mQ, mK, mV;
   int rc = 0;
-  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : make_tmap_heads_sw64;
+  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : head_dim == 16 ? make_tmap_heads_sw32 : make_tmap_heads_sw64;
   rc |= make_map(&mQ, q, B, S, H, q_bs, q_ts, 128);
   rc |= make_map(&mK, k, B, S, H, k_bs, k_ts, kFwdTileK);
   rc |= make_map(&mV, v, B, S, H, v_bs, v_ts, kFwdTileK);
@@ -2560,7 +2607,8 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   FK_REQUIRE(n_items < (1ll << 31), "fk_attn_forward_tc: too many work items");
   const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
   if (head_dim == 64) attn_fwd_tc64_kernel<<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
-  else attn_fwd_tc_kernel<<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
+  else if (head_dim == 16) attn_fwd_tc_kernel<16><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
+  else attn_fwd_tc_kernel<32><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;

@@ -34,9 +34,11 @@ constexpr int kBSlabBytes = 256 * 128;     // 256 rows x 64 bf16
 constexpr int kGemmSmemLimit = 232448 - 1024;
 
 // (epilogue 3 was a SwiGLU backward in the epilogue, removed; the numbers of the others are part of the C ABI)
-enum { EPI_STORE = 0, EPI_ROPE = 1, EPI_SWIGLU = 2, EPI_ROPE64 = 4 };
-// (cos, sin) pairs one epilogue thread holds for its row: one head of 32 columns, or of 64 columns (EPI_ROPE64)
-template <int EPI> constexpr int rope_pairs() { return EPI == EPI_ROPE64 ? 32 : 16; }
+enum { EPI_STORE = 0, EPI_ROPE = 1, EPI_SWIGLU = 2, EPI_ROPE64 = 4, EPI_ROPE16 = 5 };
+// (cos, sin) pairs one epilogue thread holds for its row: one head of 32 columns, of 64 columns (EPI_ROPE64) or of 16
+// columns (EPI_ROPE16)
+template <int EPI> constexpr int rope_pairs() { return EPI == EPI_ROPE64 ? 32 : EPI == EPI_ROPE16 ? 8 : 16; }
+template <int EPI> constexpr bool is_rope() { return EPI == EPI_ROPE || EPI == EPI_ROPE64 || EPI == EPI_ROPE16; }
 
 struct GemmParams {
   __nv_bfloat16* C;          // [M, N] (EPI_SWIGLU: the fused projection h13)
@@ -44,7 +46,7 @@ struct GemmParams {
   __nv_bfloat16* C2;         // EPI_SWIGLU: gated [M, N/2]
   long long ldc2;
   const float* bias;         // [N] or null (EPI_STORE)
-  const float2* rope_table;  // EPI_ROPE: [rope_len][16] (cos, sin); EPI_ROPE64: [rope_len][32]
+  const float2* rope_table;  // EPI_ROPE: [rope_len][16] (cos, sin); EPI_ROPE64: [rope_len][32]; EPI_ROPE16: [rope_len][8]
   const int* rope_pos;       // [M] or null: position of row m = rope_pos ? rope_pos[m] : (m % rope_S) + rope_offset
   int rope_len, rope_offset, rope_cols, rope_S;
   long long M;
@@ -154,7 +156,7 @@ __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUt
                                                   int stg_tiles, uint32_t& stg_cnt, int lane, int ch, uint32_t taddr, int n0,
                                                   long long row0, const float2 (&cs)[NCS], uint64_t* full_bar, uint32_t full_parity,
                                                   Release release) {
-    if (EPI == EPI_STORE || EPI == EPI_ROPE || EPI == EPI_ROPE64) {
+    if (EPI == EPI_STORE || is_rope<EPI>()) {
       mbar_wait(full_bar, full_parity);
       tc_fence_after();
 #pragma unroll
@@ -171,14 +173,15 @@ __device__ __forceinline__ void res_epilogue_tile(const GemmParams& p, const CUt
         for (int hc = 0; hc < 2; ++hc) {
           float v[32];
           if (hc == 0) to_f32(r0, v); else to_f32(r1, v);
-          if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
+          if (is_rope<EPI>()) {
             if (col + hc * 32 < p.rope_cols) {
               const int c0 = (EPI == EPI_ROPE64) ? hc * 16 : 0;     // a 64-column head spans both 32-column halves
 #pragma unroll
               for (int i = 0; i < 16; ++i) {
+                const int ci = (EPI == EPI_ROPE16) ? (i & 7) : c0 + i;   // two 16-column heads per 32-column half
                 const float x0 = v[2 * i], x1 = v[2 * i + 1];
-                v[2 * i] = x0 * cs[c0 + i].x - x1 * cs[c0 + i].y;
-                v[2 * i + 1] = x0 * cs[c0 + i].y + x1 * cs[c0 + i].x;
+                v[2 * i] = x0 * cs[ci].x - x1 * cs[ci].y;
+                v[2 * i + 1] = x0 * cs[ci].y + x1 * cs[ci].x;
               }
             }
           } else if (p.bias != nullptr && col + hc * 32 < p.N) {
@@ -262,7 +265,7 @@ __device__ __forceinline__ void res_epilogue_warp(const GemmParams& p, const CUt
     const long long row = row0 + lane;
     constexpr int kCs = rope_pairs<EPI>();
     float2 cs[kCs];
-    if (EPI == EPI_ROPE || EPI == EPI_ROPE64) {
+    if (is_rope<EPI>()) {
       int ps = 0;
       if (row < p.M) ps = p.rope_pos ? p.rope_pos[row] : static_cast<int>(row % p.rope_S) + p.rope_offset;
       ps = min(max(ps, 0), p.rope_len - 1);
@@ -879,7 +882,7 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
   FK_REQUIRE(N % 32 == 0, "fk_gemm_nt: N must be a multiple of 32");
   FK_REQUIRE((reinterpret_cast<uintptr_t>(A) & 15) == 0 && (reinterpret_cast<uintptr_t>(B) & 15) == 0, "fk_gemm_nt: operands must be 16-byte aligned");
   FK_REQUIRE(epilogue != 3, "fk_gemm_nt: epilogue 3 (SwiGLU backward) was removed; use epilogue 0 for d gated and fk_swiglu_backward_blocked");
-  FK_REQUIRE(epilogue >= EPI_STORE && epilogue <= EPI_ROPE64, "fk_gemm_nt: unknown epilogue");
+  FK_REQUIRE(epilogue >= EPI_STORE && epilogue <= EPI_ROPE16, "fk_gemm_nt: unknown epilogue");
   GemmParams p = {};
   p.C = static_cast<__nv_bfloat16*>(C); p.ldc = ldc;
   p.C2 = static_cast<__nv_bfloat16*>(C2); p.ldc2 = ldc2;
@@ -890,7 +893,7 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
   p.nslab = (K + 63) / 64;
   p.ntile = (N + 255) / 256;
   FK_REQUIRE(C && ldc % 8 == 0 && ldc >= N && (reinterpret_cast<uintptr_t>(C) & 15) == 0, "fk_gemm_nt: C must be 16-byte aligned with ldc % 8 == 0");
-  if (epilogue == EPI_ROPE || epilogue == EPI_ROPE64) {
+  if (epilogue == EPI_ROPE || epilogue == EPI_ROPE64 || epilogue == EPI_ROPE16) {
     FK_REQUIRE(rope_table && rope_len > 0 && rope_cols % (epilogue == EPI_ROPE64 ? 64 : 32) == 0 && rope_cols <= N && (rope_pos || rope_S > 0),
                "fk_gemm_nt: bad rope arguments");
     FK_REQUIRE(rope_pos != nullptr || (rope_offset >= 0 && static_cast<long long>(rope_offset) + (M < rope_S ? M : rope_S) <= rope_len),
@@ -931,7 +934,8 @@ FK_API int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb
       case EPI_STORE: rc = launch_res<EPI_STORE>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
       case EPI_ROPE: rc = launch_res<EPI_ROPE>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
       case EPI_SWIGLU: rc = launch_res<EPI_SWIGLU>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
-      default: rc = launch_res<EPI_ROPE64>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
+      case EPI_ROPE64: rc = launch_res<EPI_ROPE64>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
+      default: rc = launch_res<EPI_ROPE16>(pair, grid, smem_bytes, stream, ta, tb, tc, tc2, p); break;
     }
     if (rc != FK_OK) return rc;
   } else {

@@ -70,6 +70,16 @@ int make_tmap_heads_sw64(CUtensorMap* map, const void* base, int B, int S, int H
   return make_tmap_bf16(map, base, 4, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B);
 }
 
+// bf16 [B][S][H][16] (strided tokens / trials): box = one head's 16 columns (32-byte rows) x box_rows tokens, 32-byte
+// swizzle.  Coordinates: (0, head, token, batch).
+int make_tmap_heads_sw32(CUtensorMap* map, const void* base, int B, int S, int H, long long batch_stride,
+                         long long token_stride, uint32_t box_rows) {
+  const uint64_t dims[4] = {16, static_cast<uint64_t>(H), static_cast<uint64_t>(S), static_cast<uint64_t>(B)};
+  const uint64_t strides[3] = {32, static_cast<uint64_t>(token_stride) * 2, static_cast<uint64_t>(batch_stride) * 2};
+  const uint32_t box[4] = {16, 1, box_rows, 1};
+  return make_tmap_bf16(map, base, 4, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_32B);
+}
+
 // bf16 [B][S][H][64] (strided tokens / trials): box = one head's 64 columns (128-byte rows) x box_rows tokens, 128-byte
 // swizzle.  Coordinates: (0, head, token, batch).
 int make_tmap_heads_sw128(CUtensorMap* map, const void* base, int B, int S, int H, long long batch_stride,

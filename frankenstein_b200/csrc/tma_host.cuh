@@ -32,5 +32,8 @@ int make_tmap_heads_sw64(CUtensorMap* map, const void* base, int B, int S, int H
 // Same for bf16 [B][S][H][64]: box = one head's 64 columns (128-byte rows) x box_rows tokens, 128-byte swizzle.
 int make_tmap_heads_sw128(CUtensorMap* map, const void* base, int B, int S, int H, long long batch_stride,
                           long long token_stride, uint32_t box_rows);
+// Same for bf16 [B][S][H][16]: box = one head's 16 columns (32-byte rows) x box_rows tokens, 32-byte swizzle.
+int make_tmap_heads_sw32(CUtensorMap* map, const void* base, int B, int S, int H, long long batch_stride,
+                         long long token_stride, uint32_t box_rows);
 
 }  // namespace fk

@@ -4,7 +4,7 @@ Functional wrappers (``gemm_nt``, ``gemm_tn``) and the ``torch.autograd.Function
 
 * ``linear``       -- ``nn.Linear`` (models/brainformer.py:171 ``project``, ``to_signals``, ...): y = x W^T (+ b);
 * ``qkv_rope``     -- qw / kw / vw as ONE projection (brainformer.py:141-143) with ``apply_rope`` (:70-91, :156-158) applied
-                      to the q | k columns in the GEMM epilogue (heads of 32 or 64 columns);
+                      to the q | k columns in the GEMM epilogue (heads of 16, 32 or 64 columns);
 * ``swiglu_mlp``   -- ``w2(silu(w1 x) * w3 x)`` (brainformer.py:119-124): the w1 | w3 projection forms the gate in its
                       epilogue; the backward applies the SwiGLU derivative in one streaming pass after the d-gated GEMM.
 
@@ -22,8 +22,10 @@ import torch
 from ._lib import FkError, check, lib, on_tensor_device, ptr, require_cuda, require_device, stream, timed
 
 BF16 = torch.bfloat16
-EPI_STORE, EPI_ROPE, EPI_SWIGLU, EPI_ROPE64 = 0, 1, 2, 4
-ROPE_EPILOGUE = {32: EPI_ROPE, 64: EPI_ROPE64}          # head width -> RoPE epilogue of the fused q | k | v projection
+EPI_STORE, EPI_ROPE, EPI_SWIGLU, EPI_ROPE64, EPI_ROPE16 = 0, 1, 2, 4, 5
+# head width -> RoPE epilogue of the fused q | k | v projection
+ROPE_EPILOGUE = {16: EPI_ROPE16, 32: EPI_ROPE, 64: EPI_ROPE64}
+ROPE_EPILOGUES = tuple(ROPE_EPILOGUE.values())
 
 
 def _as2d(x: torch.Tensor) -> torch.Tensor:
@@ -39,7 +41,7 @@ def _as2d(x: torch.Tensor) -> torch.Tensor:
 def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = None, epilogue: int = EPI_STORE, *,
             rope=None, rope_cols: int = 0, rope_S: int = 0, lead: Optional[tuple] = None, name: str = "gemm_nt"):
     """C [M, N] bf16 = a [M, K] @ b [N, K]^T on tcgen05 (fp32 accumulate).  See include/fk_b200.h (fk_gemm_nt) for the
-    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64) or (h13, gated) (EPI_SWIGLU).
+    epilogues.  Returns C (EPI_STORE / EPI_ROPE / EPI_ROPE64 / EPI_ROPE16) or (h13, gated) (EPI_SWIGLU).
     lead (EPI_STORE): C is allocated as [*lead, N] (prod(lead) = M), a tensor of its own rather than a view of [M, N]."""
     require_cuda(a, b)
     require_device()
@@ -56,7 +58,7 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
     ldc = ldc2 = 0
     if lead is not None and (epilogue != EPI_STORE or math.prod(lead) != M):
         raise FkError(f"gemm_nt: output shape {(*lead, N)} does not hold [{M}, {N}]")
-    if epilogue in (EPI_STORE, EPI_ROPE, EPI_ROPE64):
+    if epilogue == EPI_STORE or epilogue in ROPE_EPILOGUES:
         C = torch.empty(*(lead if lead is not None else (M,)), N, device=dev, dtype=BF16)
         ldc = N
     elif epilogue == EPI_SWIGLU:
@@ -67,7 +69,7 @@ def gemm_nt(a: torch.Tensor, b: torch.Tensor, bias: Optional[torch.Tensor] = Non
     if bias is not None:
         bias_f = bias.detach().float().contiguous()
     table, pos, rope_len, rope_off = None, None, 0, 0
-    if epilogue in (EPI_ROPE, EPI_ROPE64):
+    if epilogue in ROPE_EPILOGUES:
         table, pos, rope_len, rope_off = rope.table, rope.pos, rope.table.shape[0], rope.offset
         if pos is not None:
             pos = pos.reshape(-1)
@@ -168,7 +170,7 @@ class _QKVRopeFn(torch.autograd.Function):
         if rope is not None:
             epi = ROPE_EPILOGUE.get(inner // n_heads)
             if epi is None:
-                raise FkError(f"qkv_rope: the RoPE epilogue takes heads of 32 or 64 columns, not {inner // n_heads}")
+                raise FkError(f"qkv_rope: the RoPE epilogue takes heads of 16, 32 or 64 columns, not {inner // n_heads}")
             qkv = gemm_nt(x2, w, None, epi, rope=rope, rope_cols=2 * inner, rope_S=S, name="gemm_qkv_rope")
         else:
             qkv = gemm_nt(x2, w, None, EPI_STORE, name="gemm_qkv_rope")

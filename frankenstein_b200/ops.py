@@ -289,7 +289,7 @@ class RopeSpec:
 
 @on_tensor_device
 def _rope_inplace(x4, spec: RopeSpec, inverse: bool):
-    """x4: bf16 view [B, S, H, hd], hd 32 or 64 (token stride arbitrary, head stride hd)."""
+    """x4: bf16 view [B, S, H, hd], hd 16, 32 or 64 (token stride arbitrary, head stride hd)."""
     B, S, H, hd = x4.shape
     assert x4.stride(3) == 1 and x4.stride(2) == hd
     check(lib().fk_rope(ptr(x4), x4.stride(0), x4.stride(1), B, S, H, hd, ptr(spec.table), spec.table.shape[0],
@@ -307,7 +307,7 @@ class _AttnQKVFn(torch.autograd.Function):
     @staticmethod
     @on_tensor_device
     def forward(ctx, qkv, n_heads, rope, mask, scale, rope_applied=False):
-        """qkv: bf16 [B, S, 3*H*hd] (hd 32 or 64) fresh output of the fused projection (q|k|v); RoPE is applied in place unless the
+        """qkv: bf16 [B, S, 3*H*hd] (hd 16, 32 or 64) fresh output of the fused projection (q|k|v); RoPE is applied in place unless the
         projection's epilogue already did it (rope_applied: the backward still rotates dq / dk back)."""
         require_cuda(qkv)
         require_device()
@@ -431,19 +431,19 @@ class _AttnQKVFn(torch.autograd.Function):
 
 
 def _check_head_dim(hd: int) -> None:
-    if hd not in (32, 64):
-        raise FkError("the attention kernels are built for head_dim 32 and 64")
-    if hd == 64:
+    if hd not in (16, 32, 64):
+        raise FkError("the attention kernels are built for head_dim 16, 32 and 64")
+    if hd != 32:
         # the cross-check paths (mma.sync kernels, transposed operands, staged statistics) exist at head_dim 32 only
         for name, value, default in (("ATTN_FWD_IMPL", ATTN_FWD_IMPL, "tc"), ("ATTN_BWD_IMPL", ATTN_BWD_IMPL, "tc"),
                                      ("ATTN_BWD_OPERANDS", ATTN_BWD_OPERANDS, "mn"), ("ATTN_BWD_STATS", ATTN_BWD_STATS, "folded")):
             if value != default:
-                raise FkError(f"{name} = {value!r} is a head_dim-32 cross-check; head_dim 64 runs the default path only")
+                raise FkError(f"{name} = {value!r} is a head_dim-32 cross-check; head_dim {hd} runs the default path only")
 
 
 def attention_qkv(qkv, n_heads: int, rope: Optional[RopeSpec] = None, mask: Optional[LabelMask] = None,
                   scale: Optional[float] = None, rope_applied: bool = False):
-    """softmax(q k^T * scale + mask) v over the fused QKV buffer -> [B, S, H*hd] bf16, head_dim hd 32 or 64."""
+    """softmax(q k^T * scale + mask) v over the fused QKV buffer -> [B, S, H*hd] bf16, head_dim hd 16, 32 or 64."""
     hd = qkv.shape[-1] // (3 * n_heads)
     _check_head_dim(hd)
     if scale is None:

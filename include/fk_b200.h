@@ -140,7 +140,7 @@ int fk_swiglu_backward(const void* h13, const void* gy, void* dh13, long long M,
 /* the same derivative on the block-interleaved h13 / dh13 of fk_gemm_nt's SwiGLU epilogue ([w1 block | w3 block] per
  * `block` hidden units); gy [M, H] in hidden-unit order. */
 int fk_swiglu_backward_blocked(const void* h13, const void* gy, void* dh13, long long M, int H, int block, void* stream);
-/* apply_rope (brainformer.py:70-91) in place on bf16 [B,S,H,head_dim] (head_dim 32 or 64, strides in elements); table
+/* apply_rope (brainformer.py:70-91) in place on bf16 [B,S,H,head_dim] (head_dim 16, 32 or 64, strides in elements); table
  * [P,head_dim/2,2] fp32 (cos,sin) = view_as_real(build_complex_rope_cache); pos (nullable) [B,S] int32 else position =
  * s + pos_offset. */
 int fk_rope(void* x, long long bs, long long ts, int B, int S, int H, int head_dim, const float* table, int P,
@@ -163,9 +163,9 @@ int fk_attn_backward(const void* q, const void* k, const void* v, const void* o,
                      long long dk_bs, long long dk_ts, long long dv_bs, long long dv_ts, const int* qid, const int* kid,
                      const int* qmin, const int* qmax, const int* kmin, const int* kmax, float scale, int parts, void* stream);
 
-/* tcgen05 / TMEM / TMA version of the attention backward (attention_tc.cu), head_dim 32 or 64 (q/k/v/d_o/dq/dk/dv:
- * bf16 [B,S,H,head_dim], strides in elements; any other head_dim is rejected before anything is launched).  At head_dim 64
- * there is one path: aug from fk_attn_aug is required, qt = kt = dot = NULL, no stall accounting, gradient strides % 8 == 0.
+/* tcgen05 / TMEM / TMA version of the attention backward (attention_tc.cu), head_dim 16, 32 or 64 (q/k/v/d_o/dq/dk/dv:
+ * bf16 [B,S,H,head_dim], strides in elements; any other head_dim is rejected before anything is launched).  At head_dim 16
+ * and 64 there is one path: aug from fk_attn_aug is required, qt = kt = dot = NULL, no stall accounting, gradient strides % 8 == 0.
  * qt = kt = dot = NULL (default): the
  * contractions over tokens read the Q / dO / K tiles MN-major straight from the strided inputs.  Cross-check mode:
  * fk_attn_transpose makes [B][H][32][Sp] copies (zero padded, Sp % 8 == 0) that serve as K-major operands instead:
@@ -177,7 +177,7 @@ int fk_attn_backward(const void* q, const void* k, const void* v, const void* o,
  * be given different words.  The library itself holds no device-side state: every entry point is re-entrant per stream. */
 int fk_attn_transpose(const void* x, long long bs, long long ts, int B, int S, int H, int head_dim, void* xt, int Sp,
                       void* stream);
-/* fk_attn_aug: o / d_o bf16 [B,S,H,head_dim] (head_dim 32 or 64);
+/* fk_attn_aug: o / d_o bf16 [B,S,H,head_dim] (head_dim 16, 32 or 64);
  * delta [B,H,S] = rowsum(dO * O) and the statistics rows aug (bf16 [B,H,S,16], 32-byte aligned): -lse / c
  * and -delta as three bf16 terms each.  Passed to fk_attn_backward_tc as `aug` (nullable), they enter the score MMAs as one
  * more K step, so S - lse / c and dP - delta leave the tensor core and the compute warps neither stage nor subtract the
@@ -208,7 +208,7 @@ int fk_attn_backward_tc_profile(const void* q, const void* k, const void* v, con
                                 int rope_len, const int* rope_pos, int rope_offset, int parts, unsigned int* counters,
                                 long long* prof, int prof_mode, void* stream);
 
-/* tcgen05 / TMEM / TMA forward (attention_tc.cu): q / k / v are strided views ([B][S][H][head_dim], head_dim 32 or 64,
+/* tcgen05 / TMEM / TMA forward (attention_tc.cu): q / k / v are strided views ([B][S][H][head_dim], head_dim 16, 32 or 64,
  * strides in elements; any other head_dim is rejected before anything is launched);
  * the V tile is read MN-major by the P V MMAs, so no transposed copy is needed; Sq == Sk == S.
  * Labels: any int32 value is valid in qid and kid, INT32_MIN and INT32_MAX included (a query labelled INT32_MAX sees every
@@ -244,7 +244,8 @@ int fk_add_norm_backward(const float* x_new, const void* g_y, int g_dtype, const
  *   2  SwiGLU forward: B = w1 / w3 interleaved in blocks of 128 rows ([w1[0:128]; w3[0:128]; w1[128:256]; ...], N = 2 x
  *      hidden); writes the fused projection C = h13 [M, N] and C2 = gated [M, N/2] = silu(h1) * h3 (brainformer.py:123-124)
  *   3  removed (was the SwiGLU backward; rejected): d gated on epilogue 0, then fk_swiglu_backward_blocked
- *   4  as 1 for heads of 64 columns: rope_table [rope_len][32][2], rope_cols % 64 == 0 */
+ *   4  as 1 for heads of 64 columns: rope_table [rope_len][32][2], rope_cols % 64 == 0
+ *   5  as 1 for heads of 16 columns: rope_table [rope_len][8][2], rope_cols % 32 == 0 */
 int fk_gemm_nt(const void* A, long long lda, const void* B, long long ldb, void* C, long long ldc, long long M, int N,
                int K, const float* bias, int epilogue, void* C2, long long ldc2, const float* rope_table, int rope_len,
                const int* rope_pos, int rope_offset, int rope_cols, int rope_S, void* stream);

@@ -1,14 +1,15 @@
-"""Head_dim 32 against head_dim 64 at the same inner width (512), one JSON line on stdout (and to --out).
+"""Head_dim 16, 32 and 64 at the same inner width (512), one JSON line on stdout (and to --out).
 
-* attention forward + backward, 16 trials x 4096 tokens, block-causal with 256 electrodes, three arms alternated per rep:
+* attention forward + backward, 16 trials x 4096 tokens, block-causal with 256 electrodes, arms alternated per rep:
   (a) 16 x 32 on the head_dim-32 tcgen05 kernels, (b) 8 x 64 on the head_dim-64 tcgen05 kernels, (c) 8 x 64 through
-  library SDPA with the dense [B,1,S,S] bool mask (the only way head_dim 64 ran before).  Per-kernel ms from CUDA events
-  (_lib.TIMER), algorithmic TF/s = the visible-pair flop count of bench.py (forward 2, backward 5 score-shaped matmuls).
-  Each rep runs on a fresh qkv buffer of 201 MB (> the 126 MB L2).
+  library SDPA with the dense [B,1,S,S] bool mask (the only way head_dim 64 ran before), (d) 32 x 16 on the head_dim-16
+  instantiation of the tcgen05 kernels, (e) 32 x 16 through library SDPA with the dense mask.  Per-kernel ms from CUDA
+  events (_lib.TIMER), algorithmic TF/s = the visible-pair flop count of bench.py (forward 2, backward 5 score-shaped
+  matmuls).  Each rep runs on a fresh qkv buffer of 201 MB (> the 126 MB L2).
 * train-step trials/s of the cfg-2 BrainFormer (bench.py ENC_CFG / PER_CFG, 128 trials, bf16 autocast, AdamW + value
-  clip) with 16 x 32 and with 8 x 64 encoder heads.
+  clip) with the encoder heads of each selected tcgen05 arm.
 
-Usage: python scripts/gpu_time_head_dim.py [--reps 7] [--out result.json]
+Usage: python scripts/gpu_time_head_dim.py [--reps 7] [--arms a,b,c,d,e] [--out result.json]
 """
 import argparse
 import json
@@ -41,7 +42,7 @@ def elapsed(fn):
     return a.elapsed_time(b)
 
 
-def attention_arms(reps):
+def attention_arms(reps, selected):
     dev = torch.device("cuda")
     mask = ops.LabelMask.block_causal(B, S, E, dev)
     pairs = float(mask.visible_pairs())
@@ -62,18 +63,23 @@ def attention_arms(reps):
             return t, {k: v[1] for k, v in _lib.TIMER.summary().items()}
         return run
 
-    def sdpa():
-        H, hd = INNER // 64, 64
-        x = (torch.randn(B, S, 3 * INNER, device=dev, generator=g) * 1.2).to(torch.bfloat16).requires_grad_(True)
-        torch.cuda.synchronize()
+    def sdpa(hd):
+        H = INNER // hd
 
-        def body():
-            q, k, v = x.view(B, S, 3, H, hd).unbind(2)
-            o = F.scaled_dot_product_attention(q.transpose(1, 2), k.transpose(1, 2), v.transpose(1, 2), attn_mask=dense)
-            o.transpose(1, 2).reshape(B, S, INNER).backward(w)
-        return elapsed(body), {}
+        def run():
+            x = (torch.randn(B, S, 3 * INNER, device=dev, generator=g) * 1.2).to(torch.bfloat16).requires_grad_(True)
+            torch.cuda.synchronize()
 
-    arms = {"a_16x32_tc": ours(32), "b_8x64_tc": ours(64), "c_8x64_sdpa_dense": sdpa}
+            def body():
+                q, k, v = x.view(B, S, 3, H, hd).unbind(2)
+                o = F.scaled_dot_product_attention(q.transpose(1, 2), k.transpose(1, 2), v.transpose(1, 2), attn_mask=dense)
+                o.transpose(1, 2).reshape(B, S, INNER).backward(w)
+            return elapsed(body), {}
+        return run
+
+    arms = {"a_16x32_tc": ours(32), "b_8x64_tc": ours(64), "c_8x64_sdpa_dense": sdpa(64), "d_32x16_tc": ours(16),
+            "e_32x16_sdpa_dense": sdpa(16)}
+    arms = {k: v for k, v in arms.items() if k[0] in selected}
     for fn in arms.values():          # warm-up of every shape
         fn(); fn()
     times = {k: [] for k in arms}
@@ -101,14 +107,15 @@ def attention_arms(reps):
     return out
 
 
-def train_steps(reps, trials=128):
+def train_steps(reps, selected, trials=128):
     import bench
     from frankenstein_b200.brainformer import BrainFormer, Config, MAEConfig
     dev = torch.device("cuda")
     x, t = bench.synth_batch(trials, 1234)
     x, t = x[..., :256].contiguous().to(dev), t.to(dev)
     models = {}
-    for name, (H, hd) in {"16x32": (16, 32), "8x64": (8, 64)}.items():
+    heads = {"a": ("16x32", 16, 32), "b": ("8x64", 8, 64), "d": ("32x16", 32, 16)}
+    for name, H, hd in (heads[a] for a in "abd" if a in selected):
         enc = dict(bench.ENC_CFG, n_heads=H, n_kv_heads=H, head_dim=hd)
         torch.manual_seed(0)
         m = BrainFormer(Config(encoder=MAEConfig(**enc), **bench.PER_CFG)).to(dev).train()
@@ -140,12 +147,15 @@ def train_steps(reps, trials=128):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--reps", type=int, default=7)
+    ap.add_argument("--arms", default="a,b,c,d,e", help="comma-separated attention arms (train steps: a, b, d among them)")
     ap.add_argument("--out", default=None, help="also write the JSON line to this file")
     args = ap.parse_args()
+    selected = set(args.arms.split(","))
     if not torch.cuda.is_available():
         raise SystemExit("no CUDA device: these are GPU timings")
     rec = {"gpu": gpu_info(), "shape": f"{B} trials x {S} tokens, block-causal E={E}, inner width {INNER}",
-           "attention": attention_arms(args.reps), "train_step_cfg2": train_steps(max(3, args.reps // 2))}
+           "attention": attention_arms(args.reps, selected),
+           "train_step_cfg2": train_steps(max(3, args.reps // 2), selected)}
     line = json.dumps(rec)
     print(line, flush=True)
     if args.out:
