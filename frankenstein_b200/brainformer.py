@@ -411,6 +411,101 @@ class Encoder(nn.Module):
         _, y = run_blocks(self.transformer.h, emb, mask, rope, self.transformer.ln_f, out_dtype, h_delta=h_delta)
         return y
 
+    def stream(self, batch_size: int, out_dtype=torch.float32) -> "EncoderStream":
+        """Online inference: feed the window patch by patch with `EncoderStream.step(x)` and get the outputs of the new
+        tokens only.  The mask is block-causal per time patch, so earlier tokens' outputs never change; each layer keeps the
+        rotated keys and values of the tokens seen so far in a bf16 cache of `block_size` tokens."""
+        return EncoderStream(self, batch_size, out_dtype)
+
+
+class EncoderStream:
+    """Streaming state of an `Encoder` (from `Encoder.stream`): per layer a bf16 k | v cache [B, block_size, 2 * inner],
+    allocated once.  Positions start at 0 when the stream starts; the offline `Encoder.forward` on a partial window uses
+    the last positions of the window instead, a uniform shift that RoPE scores do not see, so the two agree up to bf16
+    rounding."""
+
+    def __init__(self, encoder: Encoder, batch_size: int, out_dtype=torch.float32):
+        cfg = encoder.config
+        if batch_size < 1:
+            raise ops.FkError("EncoderStream: batch_size must be positive")
+        if cfg.head_dim not in (16, 32, 64):
+            raise ops.FkError("EncoderStream: the streaming attention kernel takes head_dim 16, 32 or 64")
+        if len(encoder.transformer.h) == 0:
+            raise ops.FkError("EncoderStream: the encoder has no layers")
+        self.encoder = encoder
+        self.batch_size = batch_size
+        self.out_dtype = out_dtype
+        self.n_heads = cfg.n_heads
+        self.inner = cfg.n_heads * cfg.head_dim
+        dev = encoder.device
+        self.caches = [torch.empty(batch_size, encoder.block_size, 2 * self.inner, device=dev, dtype=BF16)
+                       for _ in encoder.transformer.h]
+        self._length = 0
+
+    @property
+    def length(self) -> int:
+        """tokens cached so far (a multiple of n_electrodes)."""
+        return self._length
+
+    def reset(self) -> None:
+        self._length = 0
+
+    @torch.no_grad()
+    def step(self, x: torch.Tensor) -> torch.Tensor:
+        """x [B, n * patch_size, n_electrodes] (n >= 1 whole patches) -> final-LayerNorm outputs of the n * n_electrodes
+        new tokens, [B, n * n_electrodes, dim] in `out_dtype`.  Raises FkError, leaving the state as it was, on a partial
+        patch, a batch or electrode count that does not match, or a step past the window (block_size tokens)."""
+        enc = self.encoder
+        E, p = enc.n_electrodes, enc.patch_size
+        if x.dim() != 3 or x.shape[0] != self.batch_size or x.shape[2] != E:
+            raise ops.FkError(f"EncoderStream.step: expected [{self.batch_size}, n * {p}, {E}], got {tuple(x.shape)}")
+        B, T, _ = x.shape
+        if T < p or T % p != 0:
+            raise ops.FkError(f"EncoderStream.step: {T} bins is not a positive multiple of patch_size {p}")
+        n_new = (T // p) * E
+        L = self._length
+        if L + n_new > enc.block_size:
+            raise ops.FkError(f"EncoderStream.step: {L} cached + {n_new} new tokens exceed the window of {enc.block_size}")
+        if not x.is_cuda:
+            raise ops.FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
+        w_emb = enc.transformer.emb
+        if GEMM_IMPL == "own" and gemm.patch_embed_supported(T, E, p, w_emb.weight.shape[0]):
+            h_delta = gemm.patch_embed(x.detach(), w_emb.weight, w_emb.bias)
+        else:
+            h_delta = enc.embed(enc.to_patches(x))
+        emb = enc.space_embedding.float().repeat(1, T // p, 1)        # [1, n_new, dim]; added inside the first add+LayerNorm
+        Sk = L + n_new
+        mask = None
+        if T > p:
+            # several patches in one step: block-causal among the new tokens (with one patch every cached key is visible)
+            blk = torch.arange(Sk, device=x.device, dtype=torch.int32) // E
+            mask = LabelMask(blk[L:][None].expand(B, n_new).contiguous(), blk[None].expand(B, Sk).contiguous())
+        rope = RopeSpec(enc.rope_table(), None, L)
+        blocks = enc.transformer.h
+        H, inner = self.n_heads, self.inner
+        l0 = blocks[0].ln_1
+        h, y = ops.add_layer_norm(emb, h_delta, l0.weight, l0.bias, l0.eps)
+        for i, blk_ in enumerate(blocks):
+            at = blk_.attn
+            if GEMM_IMPL == "own" and gemm.qkv_supported(at.qw.weight.shape[1], inner):
+                qkv = gemm.qkv_rope(y, at.qw.weight, at.kw.weight, at.vw.weight, rope, H)
+            else:
+                qkv = _linear_bf16(y, torch.cat([at.qw.weight, at.kw.weight, at.vw.weight], dim=0)).contiguous()
+                q4 = qkv.view(B, n_new, 3, H, -1)
+                ops._rope_inplace(q4[:, :, 0], rope, False)
+                ops._rope_inplace(q4[:, :, 1], rope, False)
+            cache = self.caches[i]
+            cache[:, L:Sk].copy_(qkv[..., inner:])
+            res = ops.attention_kv(qkv[..., :inner], cache[:, :Sk, :inner], cache[:, :Sk, inner:], H, mask)
+            a = _linear_bf16(res, at.project.weight)
+            h, y = ops.add_layer_norm(h, a, blk_.ln_2.weight, blk_.ln_2.bias, blk_.ln_2.eps)
+            m = blk_.mlp(y)
+            nxt = blocks[i + 1].ln_1 if i + 1 < len(blocks) else enc.transformer.ln_f
+            h, y = ops.add_layer_norm(h, m, nxt.weight, nxt.bias, nxt.eps,
+                                      BF16 if i + 1 < len(blocks) else self.out_dtype)
+        self._length = Sk
+        return y
+
 
 class MAE(nn.Module):
     """Masked auto-encoder pre-training  (models/brainformer.py:354-486)."""
@@ -540,3 +635,53 @@ class BrainFormer(nn.Module):
     def inference(self, myo, date_info):
         x = torch.from_numpy(myo)[None].to(self.device).to(self.dtype)
         return self.forward(x, targets=None)[1][0].detach().cpu().numpy().T
+
+    def stream(self, batch_size: int) -> "BrainFormerStream":
+        """Online decoding: `BrainFormerStream.step(x)` takes the next whole patches of the window and returns `pred` as
+        `forward` would for every bin fed so far."""
+        return BrainFormerStream(self, batch_size)
+
+
+class BrainFormerStream:
+    """Streaming state of a `BrainFormer`: an `EncoderStream` plus, per CrossBlock, a bf16 cache of the k | v projection
+    of the context tokens [B, block_size, 2 * inner].  The encoder is block-causal, so the context tokens never change
+    once produced: a step projects only the new ones, then runs the perceiver over the whole cache in place."""
+
+    def __init__(self, model: BrainFormer, batch_size: int):
+        cfg = model.config
+        if not ops.small_attention_supported(model.n_output_tokens, cfg.head_dim):
+            raise ops.FkError("BrainFormerStream: the cross-attention kernel serves <= 64 queries at head_dim 16 / 32 / 64")
+        self.model = model
+        self.encoder_stream = model.encoder.stream(batch_size, out_dtype=BF16)
+        inner = cfg.n_heads * cfg.head_dim
+        block = model.encoder.block_size
+        self.kv = [torch.empty(batch_size, block, 2 * inner, device=model.device, dtype=BF16) for _ in model.perceiver.h]
+
+    @property
+    def length(self) -> int:
+        """context tokens cached so far."""
+        return self.encoder_stream.length
+
+    def reset(self) -> None:
+        self.encoder_stream.reset()
+
+    @torch.no_grad()
+    def step(self, x: torch.Tensor) -> torch.Tensor:
+        """x [B, n * patch_size, n_electrodes] -> pred [B, n_output_tokens, output_dim] fp32 (errors as EncoderStream.step)."""
+        m = self.model
+        L0 = self.encoder_stream.length
+        context = self.encoder_stream.step(x)                     # [B, n_new, dim] bf16
+        L = self.encoder_stream.length
+        for cb, kv in zip(m.perceiver.h, self.kv):
+            ca = cb.cross_attn
+            kv[:, L0:L].copy_(_linear_bf16(context, torch.cat([ca.kw.weight, ca.vw.weight], dim=0)))
+        h = m.learnable_queries.expand(x.shape[0], m.n_output_tokens, -1)
+        for cb, kv in zip(m.perceiver.h, self.kv):
+            ca = cb.cross_attn
+            q = _linear_bf16(cb.ln_1(h), ca.qw.weight)
+            res = ops.small_attention_kv_cached(q, kv[:, :L], ca.n_heads)
+            h = h + _linear_bf16(res, ca.project.weight)
+            h = h + cb.mlp(cb.ln_2(h))
+            h = cb.sa_block(h, attn_mask=m.self_attn_mask, rope=m.rope_cache)
+        pred = m.perceiver.ln_f(h)
+        return _linear_bf16(pred, m.perceiver.to_motion.weight, m.perceiver.to_motion.bias).float()

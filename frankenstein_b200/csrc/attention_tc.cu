@@ -23,6 +23,9 @@
 // read MN-major (K = tokens), the same tile that served the score MMA as a K-major operand (K = head dim).  Tiles are
 // TMA-loaded with the 64-byte swizzle.  The smem data pipe, which bounds an SS-mode version of this kernel, only
 // carries the streamed operands.
+#include <algorithm>
+#include <type_traits>
+
 #include "common.cuh"
 #include "fk_b200.h"
 #include "tma_host.cuh"
@@ -1012,12 +1015,41 @@ struct FwdParams {
   unsigned int* items;                                  // caller-owned hand-out counters (see TcParams::items)
 };
 
+// Key-axis split (kPart instantiations, fk_attn_forward_kv_tc): a work item is (256-query block, key chunk, head, trial);
+// chunk c covers key tiles [c * chunk_tiles, (c + 1) * chunk_tiles).  Instead of O / l the item writes its unnormalised
+// partial O (relative to its reference m) to part_o [B][H][n_chunks][Sq][HD] and (m, l) to part_ml [B][H][n_chunks][Sq][2]
+// (log2 domain; m = -inf, l = 0 for a row that saw no key of the chunk); attn_kv_combine_kernel merges them.  A separate
+// struct keeps the parameter block of the unsplit kernels as it was.
+struct FwdKvParams : FwdParams {
+  float* part_o;
+  float* part_ml;
+  int n_chunks, chunk_tiles;
+};
+template <bool kPart>
+using FwdArgs = std::conditional_t<kPart, FwdKvParams, FwdParams>;
+
+__device__ __forceinline__ long long part_row(const FwdKvParams& p, int b, int h, int chunk, int row) {
+  return ((static_cast<long long>(b) * p.H + h) * p.n_chunks + chunk) * p.Sq + row;
+}
+// N fp32 columns of a partial O row: O * alpha (the reference raise still owed to O after the last tile)
+template <int N>
+__device__ __forceinline__ void store_part_o(float* dst, const uint32_t (&ov)[N], float alpha) {
+#pragma unroll
+  for (int c4 = 0; c4 < N / 4; ++c4)
+    *reinterpret_cast<float4*>(dst + c4 * 4) =
+        make_float4(__uint_as_float(ov[c4 * 4]) * alpha, __uint_as_float(ov[c4 * 4 + 1]) * alpha,
+                    __uint_as_float(ov[c4 * 4 + 2]) * alpha, __uint_as_float(ov[c4 * 4 + 3]) * alpha);
+}
+__device__ __forceinline__ void store_part_ml(float* dst, float m, float l) {
+  *reinterpret_cast<float2*>(dst) = make_float2(l > 0.f ? m : -INFINITY, l);
+}
+
 // HD = 16: Q / K / V rows of 32 B (SWIZZLE_32B), one score K step, P V MMAs N = 16; O_g uses the first 16 of its 32
 // TMEM columns.
-template <int HD>
+template <int HD, bool kPart = false>
 __global__ void __launch_bounds__(kFwdThreads, 1)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
-                   const __grid_constant__ CUtensorMap tm_v, const FwdParams p) {
+                   const __grid_constant__ CUtensorMap tm_v, const FwdArgs<kPart> p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FwdSmem::bars);
@@ -1039,7 +1071,9 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
   const int n_k_tiles = (p.Sk + kFwdTileK - 1) / kFwdTileK;
   const int nq64 = (p.Sq + 63) / 64, nk64 = (p.Sk + 63) / 64;
   const int n_q_tiles = (p.Sq + 255) / 256;
-  const int n_items = n_q_tiles * p.H * p.B;
+  int n_units = n_q_tiles;                        // work units per (head, trial): query blocks (x key chunks when split)
+  if constexpr (kPart) n_units *= p.n_chunks;
+  const int n_items = n_units * p.H * p.B;
 
   if (warp == 0 && lane == 0) { tma_prefetch_desc(&tm_q); tma_prefetch_desc(&tm_k); tma_prefetch_desc(&tm_v); }
   if (warp == 1 && lane == 0) {
@@ -1066,7 +1100,13 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
 
   // key tiles visible to at least one of the item's rows; bits 14 / 15 = warpgroup 0 / 1 must compare labels
   auto build_list = [&](int it, int buf) {       // whole warp
-    const int qt_ = it % n_q_tiles, b_ = it / (n_q_tiles * p.H);
+    const int u_ = it % n_units, b_ = it / (n_units * p.H);
+    const int qt_ = kPart ? u_ % n_q_tiles : u_;
+    int t_lo = 0, t_hi = n_k_tiles;              // key tiles of the item (its chunk when split)
+    if constexpr (kPart) {
+      t_lo = (u_ / n_q_tiles) * p.chunk_tiles;
+      t_hi = min(t_lo + p.chunk_tiles, n_k_tiles);
+    }
     uint16_t* list = tile_lists + buf * kMaxTiles;
     // label ranges of the two warpgroups' rows (two 64-row entries each)
     int wq_lo[2] = {0, 0}, wq_hi[2] = {0, 0};
@@ -1080,9 +1120,9 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     }
     const int cta_hi = max(wq_hi[0], wq_hi[1]);
     int cnt = 0;
-    for (int cb = 0; cb < n_k_tiles; cb += 32) {
+    for (int cb = t_lo; cb < t_hi; cb += 32) {
       const int t = cb + lane;
-      bool vis = t < n_k_tiles;
+      bool vis = t < t_hi;
       int flags = 0;
       if (vis) {
         int kmn = 0, kmx = 0;
@@ -1120,7 +1160,8 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
   }
   __syncthreads();
   for (int item = item_slot[0]; item < n_items; item = item_slot[(item_n + 1) & 1], ++item_n) {
-  const int qt = item % n_q_tiles, h = (item / n_q_tiles) % p.H, b = item / (n_q_tiles * p.H);
+  const int u = item % n_units, h = (item / n_units) % p.H, b = item / (n_units * p.H);
+  const int qt = kPart ? u % n_q_tiles : u;
   const int q0 = qt * 256;
   const uint16_t* tile_list = tile_lists + (item_n & 1) * kMaxTiles;
   const int T = n_tiles_slot[item_n & 1];
@@ -1166,7 +1207,8 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       const int nxt = __shfl_sync(0xffffffffu, item_slot[(item_n + 1) & 1], 0);
       pre_cnt = -1;
       if (nxt < n_items) {
-        const int qt2 = nxt % n_q_tiles, h2 = (nxt / n_q_tiles) % p.H, b2 = nxt / (n_q_tiles * p.H);
+        const int u2 = nxt % n_units, h2 = (nxt / n_units) % p.H, b2 = nxt / (n_units * p.H);
+        const int qt2 = kPart ? u2 % n_q_tiles : u2;
         const uint16_t* list2 = tile_lists + ((item_n + 1) & 1) * kMaxTiles;
         const int T2 = __shfl_sync(0xffffffffu, n_tiles_slot[(item_n + 1) & 1], 0);
         load_q(h2, qt2 * 256, b2, (item_n + 1) & 1);
@@ -1399,7 +1441,13 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
 #pragma unroll
       for (int i = 0; i < HD; ++i) ov[i] = 0u;
     }
-    if (row_ok) {
+    if constexpr (kPart) {
+      if (row_ok) {
+        const long long pr = part_row(p, b, h, u / n_q_tiles, row);
+        store_part_o<HD>(p.part_o + pr * HD, ov, alpha_pend);
+        store_part_ml(p.part_ml + pr * 2, m_run, l_run);
+      }
+    } else if (row_ok) {
       const float inv = (l_run > 0.f) ? alpha_pend / l_run : 0.f;      // a reference raise after the last tile is still owed to O
       __nv_bfloat16* dst = p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * HD;
 #pragma unroll
@@ -1905,9 +1953,10 @@ struct FwdSmem64 {
 };
 static_assert(FwdSmem64::total <= 232448, "attn_fwd_tc64_kernel: shared memory");
 
+template <bool kPart = false>
 __global__ void __launch_bounds__(kFwdThreads, 1)
 attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
-                     const __grid_constant__ CUtensorMap tm_v, const FwdParams p) {
+                     const __grid_constant__ CUtensorMap tm_v, const FwdArgs<kPart> p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FwdSmem64::bars);
@@ -1929,7 +1978,9 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
   const int n_k_tiles = (p.Sk + kFwdTileK - 1) / kFwdTileK;
   const int nq64 = (p.Sq + 63) / 64, nk64 = (p.Sk + 63) / 64;
   const int n_q_tiles = (p.Sq + 255) / 256;
-  const int n_items = n_q_tiles * p.H * p.B;
+  int n_units = n_q_tiles;                        // work units per (head, trial): query blocks (x key chunks when split)
+  if constexpr (kPart) n_units *= p.n_chunks;
+  const int n_items = n_units * p.H * p.B;
 
   if (warp == 0 && lane == 0) { tma_prefetch_desc(&tm_q); tma_prefetch_desc(&tm_k); tma_prefetch_desc(&tm_v); }
   if (warp == 1 && lane == 0) {
@@ -1955,7 +2006,13 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
   const uint32_t tmem_base = *tmem_slot;
 
   auto build_list = [&](int it, int buf) {       // whole warp (see attn_fwd_tc_kernel)
-    const int qt_ = it % n_q_tiles, b_ = it / (n_q_tiles * p.H);
+    const int u_ = it % n_units, b_ = it / (n_units * p.H);
+    const int qt_ = kPart ? u_ % n_q_tiles : u_;
+    int t_lo = 0, t_hi = n_k_tiles;
+    if constexpr (kPart) {
+      t_lo = (u_ / n_q_tiles) * p.chunk_tiles;
+      t_hi = min(t_lo + p.chunk_tiles, n_k_tiles);
+    }
     uint16_t* list = tile_lists + buf * kMaxTiles;
     int wq_lo[2] = {0, 0}, wq_hi[2] = {0, 0};
     if (masked) {
@@ -1968,9 +2025,9 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
     }
     const int cta_hi = max(wq_hi[0], wq_hi[1]);
     int cnt = 0;
-    for (int cb = 0; cb < n_k_tiles; cb += 32) {
+    for (int cb = t_lo; cb < t_hi; cb += 32) {
       const int t = cb + lane;
-      bool vis = t < n_k_tiles;
+      bool vis = t < t_hi;
       int flags = 0;
       if (vis) {
         int kmn = 0, kmx = 0;
@@ -2005,7 +2062,8 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
   }
   __syncthreads();
   for (int item = item_slot[0]; item < n_items; item = item_slot[(item_n + 1) & 1], ++item_n) {
-  const int qt = item % n_q_tiles, h = (item / n_q_tiles) % p.H, b = item / (n_q_tiles * p.H);
+  const int u = item % n_units, h = (item / n_units) % p.H, b = item / (n_units * p.H);
+  const int qt = kPart ? u % n_q_tiles : u;
   const int q0 = qt * 256;
   const uint16_t* tile_list = tile_lists + (item_n & 1) * kMaxTiles;
   const int T = n_tiles_slot[item_n & 1];
@@ -2048,7 +2106,8 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
     const int nxt = __shfl_sync(0xffffffffu, item_slot[(item_n + 1) & 1], 0);
     pre_cnt = -1;
     if (nxt < n_items) {
-      const int qt2 = nxt % n_q_tiles, h2 = (nxt / n_q_tiles) % p.H, b2 = nxt / (n_q_tiles * p.H);
+      const int u2 = nxt % n_units, h2 = (nxt / n_units) % p.H, b2 = nxt / (n_units * p.H);
+      const int qt2 = kPart ? u2 % n_q_tiles : u2;
       const uint16_t* list2 = tile_lists + ((item_n + 1) & 1) * kMaxTiles;
       const int T2 = __shfl_sync(0xffffffffu, n_tiles_slot[(item_n + 1) & 1], 0);
       load_q(h2, qt2 * 256, b2, (item_n + 1) & 1);
@@ -2270,7 +2329,9 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
 #pragma unroll
         for (int i = 0; i < 32; ++i) ov[i] = 0u;
       }
-      if (row_ok) {
+      if constexpr (kPart) {
+        if (row_ok) store_part_o<32>(p.part_o + part_row(p, b, h, u / n_q_tiles, row) * 64 + hf * 32, ov, alpha_pend);
+      } else if (row_ok) {
 #pragma unroll
         for (int c4 = 0; c4 < 4; ++c4) {
           uint32_t w[4];
@@ -2281,8 +2342,11 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
         }
       }
     }
-    if (row_ok && p.lse != nullptr)
+    if constexpr (kPart) {
+      if (row_ok) store_part_ml(p.part_ml + part_row(p, b, h, u / n_q_tiles, row) * 2, m_run, l_run);
+    } else if (row_ok && p.lse != nullptr) {
       p.lse[(static_cast<long long>(b) * p.H + h) * p.Sq + row] = (l_run > 0.f) ? m_run + log2f(l_run) : INFINITY;
+    }
   }
 
   tc_fence_before();
@@ -2304,6 +2368,44 @@ attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_cons
       __threadfence();
     }
   }
+}
+
+// Merge of the key chunks of fk_attn_forward_kv_tc in chunk order (bit-reproducible): one thread per 4 columns of a
+// (trial, head, query) row.  out = sum_c 2^(m_c - M) O_c / sum_c 2^(m_c - M) l_c with M = max_c m_c; a row that saw no
+// key in any chunk gives zeros (lse = +inf, as in the unsplit kernels).
+template <int HD>
+__global__ void __launch_bounds__(256)
+attn_kv_combine_kernel(const float* __restrict__ part_o, const float2* __restrict__ part_ml, __nv_bfloat16* __restrict__ out,
+                       float* __restrict__ lse, int B, int H, int Sq, int n_chunks, long long o_bs, long long o_ts) {
+  constexpr int kG = HD / 4;
+  const long long t = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
+  if (t >= static_cast<long long>(B) * H * Sq * kG) return;
+  const int c4 = static_cast<int>(t % kG);
+  const long long r = t / kG;                       // ((b * H + h) * Sq + row)
+  const int row = static_cast<int>(r % Sq);
+  const long long bh = r / Sq;
+  const int h = static_cast<int>(bh % H), b = static_cast<int>(bh / H);
+  const long long base = bh * n_chunks * Sq + row;  // partial row of chunk c: base + c * Sq
+  float M = -INFINITY;
+  for (int c = 0; c < n_chunks; ++c) M = fmaxf(M, part_ml[base + static_cast<long long>(c) * Sq].x);
+  float L = 0.f, a[4] = {0.f, 0.f, 0.f, 0.f};
+  if (M != -INFINITY) {
+    for (int c = 0; c < n_chunks; ++c) {
+      const long long pr = base + static_cast<long long>(c) * Sq;
+      const float2 ml = part_ml[pr];
+      if (!(ml.y > 0.f)) continue;
+      const float w = exp2f(ml.x - M);
+      const float4 o = *reinterpret_cast<const float4*>(part_o + pr * HD + c4 * 4);
+      L += w * ml.y;
+      a[0] += w * o.x; a[1] += w * o.y; a[2] += w * o.z; a[3] += w * o.w;
+    }
+  }
+  const float inv = L > 0.f ? 1.f / L : 0.f;
+  uint2 wv;
+  wv.x = pack2(a[0] * inv, a[1] * inv);
+  wv.y = pack2(a[2] * inv, a[3] * inv);
+  *reinterpret_cast<uint2*>(out + b * o_bs + static_cast<long long>(row) * o_ts + h * HD + c4 * 4) = wv;
+  if (lse != nullptr && c4 == 0) lse[bh * Sq + row] = L > 0.f ? M + log2f(L) : INFINITY;
 }
 
 }  // namespace fk
@@ -2584,7 +2686,7 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   if (!attr_set) {
     if (cudaFuncSetAttribute(attn_fwd_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
         cudaFuncSetAttribute(attn_fwd_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc64_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
+        cudaFuncSetAttribute(attn_fwd_tc64_kernel<>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
       fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
       return FK_ERR_CUDA;
     }
@@ -2606,10 +2708,97 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   const long long n_items = static_cast<long long>((S + 255) / 256) * H * B;
   FK_REQUIRE(n_items < (1ll << 31), "fk_attn_forward_tc: too many work items");
   const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
-  if (head_dim == 64) attn_fwd_tc64_kernel<<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
+  if (head_dim == 64) attn_fwd_tc64_kernel<><<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
   else if (head_dim == 16) attn_fwd_tc_kernel<16><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
   else attn_fwd_tc_kernel<32><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
   FK_CHECK_LAUNCH();
   fk_count_launch();
+  return FK_OK;
+}
+
+// Split-key forward for queries and keys of different lengths (a streaming step against a key / value cache).
+FK_API int fk_attn_kv_chunks(int B, int H, int Sq, int Sk, int max_ctas) {
+  if (B < 1 || H < 1 || Sq < 1 || Sk < 1) return 1;
+  const long long ctas = max_ctas > 0 ? max_ctas : fk_sm_count();
+  const long long units = static_cast<long long>(B) * H * ((Sq + 255) / 256);
+  const int n_k_tiles = (Sk + kFwdTileK - 1) / kFwdTileK;
+  if (units >= ctas) return 1;
+  const int want = static_cast<int>(std::min<long long>((ctas + units - 1) / units, n_k_tiles));
+  const int per = (n_k_tiles + want - 1) / want;                 // key tiles per chunk; every chunk gets at least one
+  return (n_k_tiles + per - 1) / per;
+}
+
+FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq,
+                                 int Sk, int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts,
+                                 long long v_bs, long long v_ts, long long o_bs, long long o_ts, const int* qid,
+                                 const int* kid, const int* qmin, const int* qmax, const int* kmin, const int* kmax,
+                                 float scale, float* part_o, float* part_ml, int n_chunks, unsigned int* counters,
+                                 void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  FK_REQUIRE(head_dim == 16 || head_dim == 32 || head_dim == 64, "fk_attn_forward_kv_tc: head_dim must be 16, 32 or 64");
+  FK_REQUIRE(counters != nullptr, "fk_attn_forward_kv_tc: counters (2 zero-initialised uint32, one pair per launch in flight) is null");
+  FK_REQUIRE(q && k && v && out && B > 0 && H > 0 && Sq > 0 && Sk > 0, "fk_attn_forward_kv_tc: bad argument");
+  FK_REQUIRE((qid == nullptr) == (kid == nullptr), "fk_attn_forward_kv_tc: qid and kid go together");
+  FK_REQUIRE(qid == nullptr || (qmin && qmax && kmin && kmax), "fk_attn_forward_kv_tc: label ranges missing");
+  FK_REQUIRE((Sk + kFwdTileK - 1) / kFwdTileK <= kMaxTiles && Sk < (1 << 20) && Sq < (1 << 20),
+             "fk_attn_forward_kv_tc: sequence too long");
+  FK_REQUIRE(q_bs % 8 == 0 && q_ts % 8 == 0 && k_bs % 8 == 0 && k_ts % 8 == 0 && v_bs % 8 == 0 && v_ts % 8 == 0 &&
+             o_bs % 8 == 0 && o_ts % 8 == 0 && q_ts >= H * head_dim && k_ts >= H * head_dim && v_ts >= H * head_dim &&
+             o_ts >= H * head_dim, "fk_attn_forward_kv_tc: strides must cover a token's heads and keep 16-byte alignment");
+  const int n_k_tiles = (Sk + kFwdTileK - 1) / kFwdTileK;
+  FK_REQUIRE(n_chunks >= 1 && n_chunks <= n_k_tiles, "fk_attn_forward_kv_tc: n_chunks must be in [1, key tiles of 128]");
+  FK_REQUIRE(n_chunks == 1 || (part_o && part_ml), "fk_attn_forward_kv_tc: part_o / part_ml are needed with more than one chunk");
+  const long long n_units = static_cast<long long>((Sq + 255) / 256) * n_chunks;
+  FK_REQUIRE(n_units * H * B < (1ll << 31), "fk_attn_forward_kv_tc: too many work items");
+  static bool attr_set_dev[FK_MAX_DEVICES];
+  bool& attr_set = attr_set_dev[fk_device_ordinal()];
+  if (!attr_set) {
+    if (cudaFuncSetAttribute(attn_fwd_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc64_kernel<>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
+        cudaFuncSetAttribute(attn_fwd_tc64_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
+      fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
+      return FK_ERR_CUDA;
+    }
+    attr_set = true;
+  }
+  CUtensorMap mQ, mK, mV;
+  int rc = 0;
+  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : head_dim == 16 ? make_tmap_heads_sw32 : make_tmap_heads_sw64;
+  rc |= make_map(&mQ, q, B, Sq, H, q_bs, q_ts, 128);
+  rc |= make_map(&mK, k, B, Sk, H, k_bs, k_ts, kFwdTileK);
+  rc |= make_map(&mV, v, B, Sk, H, v_bs, v_ts, kFwdTileK);
+  if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
+  FwdKvParams p = {};
+  p.qid = qid; p.kid = kid; p.qmin = qmin; p.qmax = qmax; p.kmin = kmin; p.kmax = kmax;
+  p.out = static_cast<__nv_bfloat16*>(out); p.lse = lse; p.o_bs = o_bs; p.o_ts = o_ts;
+  p.B = B; p.H = H; p.Sq = Sq; p.Sk = Sk; p.scale_log2 = scale * 1.4426950408889634f;
+  p.items = counters;
+  p.part_o = part_o; p.part_ml = part_ml; p.n_chunks = n_chunks; p.chunk_tiles = (n_k_tiles + n_chunks - 1) / n_chunks;
+  const long long n_items = n_units * H * B;
+  const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
+  if (n_chunks == 1) {
+    // one chunk: the unsplit kernels write O / l and lse themselves
+    const FwdParams& p1 = p;
+    if (head_dim == 64) attn_fwd_tc64_kernel<><<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p1);
+    else if (head_dim == 16) attn_fwd_tc_kernel<16><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p1);
+    else attn_fwd_tc_kernel<32><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p1);
+    FK_CHECK_LAUNCH();
+    fk_count_launch();
+    return FK_OK;
+  }
+  if (head_dim == 64) attn_fwd_tc64_kernel<true><<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
+  else if (head_dim == 16) attn_fwd_tc_kernel<16, true><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
+  else attn_fwd_tc_kernel<32, true><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
+  FK_CHECK_LAUNCH();
+  const long long n_threads = static_cast<long long>(B) * H * Sq * (head_dim / 4);
+  auto combine = head_dim == 64 ? attn_kv_combine_kernel<64> : head_dim == 16 ? attn_kv_combine_kernel<16> : attn_kv_combine_kernel<32>;
+  combine<<<static_cast<unsigned>((n_threads + 255) / 256), 256, 0, stream>>>(part_o, reinterpret_cast<const float2*>(part_ml),
+                                                                                static_cast<__nv_bfloat16*>(out), lse, B, H, Sq,
+                                                                                n_chunks, o_bs, o_ts);
+  FK_CHECK_LAUNCH();
+  fk_count_launch(2);
   return FK_OK;
 }

@@ -451,6 +451,59 @@ def attention_qkv(qkv, n_heads: int, rope: Optional[RopeSpec] = None, mask: Opti
     return _AttnQKVFn.apply(qkv, n_heads, rope, mask, scale, rope_applied)[0]
 
 
+def _head_view(t: torch.Tensor, H: int, hd: int, what: str) -> torch.Tensor:
+    """[B, S, H*hd] bf16 view -> [B, S, H, hd] view of the same memory (never a copy)."""
+    if t.dim() != 3 or t.shape[-1] != H * hd or t.dtype != torch.bfloat16 or t.stride(2) != 1:
+        raise FkError(f"attention_kv: {what} must be a bf16 [B, S, {H * hd}] view with contiguous columns, "
+                      f"got {tuple(t.shape)} {t.dtype} strides {t.stride()}")
+    if t.stride(0) % 8 != 0 or t.stride(1) % 8 != 0 or t.data_ptr() % 16 != 0:
+        raise FkError(f"attention_kv: {what} strides {t.stride()} must keep 16-byte alignment")
+    return t.as_strided((t.shape[0], t.shape[1], H, hd), (t.stride(0), t.stride(1), hd, 1))
+
+
+@on_tensor_device
+def attention_kv(q, k, v, n_heads: int, mask: Optional[LabelMask] = None, scale: Optional[float] = None):
+    """Inference-only softmax(q k^T * scale + mask) v with queries and keys of different lengths (a streaming step's new
+    tokens against a key / value cache): q [B, Sq, H*hd], k / v [B, Sk, H*hd] bf16 views with any 16-byte aligned batch and
+    token strides (read in place, never copied) -> [B, Sq, H*hd] bf16.  head_dim 16, 32 or 64.  mask: LabelMask(qid [B, Sq],
+    kid [B, Sk]), key j visible to query i iff kid[b, j] <= qid[b, i]; a query that sees no key gives a zero row.
+    The key axis is split into chunks whose partial results are merged in chunk order (bit-reproducible)."""
+    require_cuda(q, k, v)
+    require_device()
+    if torch.is_grad_enabled() and (q.requires_grad or k.requires_grad or v.requires_grad):
+        raise FkError("attention_kv is inference only (no backward): run it under torch.no_grad() or on detached tensors")
+    B, Sq, W = q.shape
+    Sk = k.shape[1]
+    H = n_heads
+    hd = W // H
+    _check_head_dim(hd)
+    if W != H * hd or k.shape != (B, Sk, W) or v.shape != (B, Sk, W):
+        raise FkError(f"attention_kv: q {tuple(q.shape)}, k {tuple(k.shape)}, v {tuple(v.shape)} do not match {H} heads")
+    if Sq < 1 or Sk < 1:
+        raise FkError("attention_kv: empty query or key axis")
+    if mask is not None and (mask.qid.shape != (B, Sq) or mask.kid.shape != (B, Sk)):
+        raise FkError(f"attention_kv: mask labels {tuple(mask.qid.shape)} / {tuple(mask.kid.shape)} do not match "
+                      f"queries ({B}, {Sq}) and keys ({B}, {Sk})")
+    q4, k4, v4 = _head_view(q, H, hd, "q"), _head_view(k, H, hd, "k"), _head_view(v, H, hd, "v")
+    dev = q.device
+    nch = lib().fk_attn_kv_chunks(B, H, Sq, Sk, 0)
+    out = torch.empty(B, Sq, W, device=dev, dtype=torch.bfloat16)
+    part_o = part_ml = None
+    if nch > 1:
+        part_o = torch.empty(B, H, nch, Sq, hd, device=dev, dtype=torch.float32)
+        part_ml = torch.empty(B, H, nch, Sq, 2, device=dev, dtype=torch.float32)
+    m = mask
+    margs = (ptr(m.qid) if m else 0, ptr(m.kid) if m else 0, ptr(m.qmin) if m else 0, ptr(m.qmax) if m else 0,
+             ptr(m.kmin) if m else 0, ptr(m.kmax) if m else 0)
+    scale = float(hd ** -0.5 if scale is None else scale)
+    with timed("attn_fwd_kv", 4.0 * B * H * Sq * Sk * hd):
+        check(lib().fk_attn_forward_kv_tc(ptr(q4), ptr(k4), ptr(v4), ptr(out), None, B, H, Sq, Sk, hd,
+                                          q4.stride(0), q4.stride(1), k4.stride(0), k4.stride(1), v4.stride(0), v4.stride(1),
+                                          out.stride(0), out.stride(1), *margs, scale, ptr(part_o), ptr(part_ml), nch,
+                                          counters(_lib.CTR_ATTN_FWD), stream()), "fk_attn_forward_kv_tc")
+    return out
+
+
 # ------------------------------------------------------------------------------------------------
 # attention with few queries (perceiver resampler: <= 64 queries, head_dim 16 / 32 / 64, no mask)
 # ------------------------------------------------------------------------------------------------
@@ -587,6 +640,40 @@ def small_attention_kv(q, kv, n_heads: int, scale: Optional[float] = None):
     if not (q.is_cuda and kv.is_cuda):
         raise FkError("frankenstein_b200 kernels run on a B200 only (no CPU fallback)")
     return _SmallAttnKVFn.apply(q, kv, n_heads, float(hd ** -0.5 if scale is None else scale), None, 0, 0)
+
+
+@on_tensor_device
+def small_attention_kv_cached(q, kv, n_heads: int, scale: Optional[float] = None):
+    """Inference-only small_attention_kv against a key | value cache: kv [B, S, 2 * H * hd] bf16 is a view with any 16-byte
+    aligned batch / token strides (e.g. the first S tokens of a longer cache), read in place, never copied."""
+    require_cuda(q, kv)
+    require_device()
+    if torch.is_grad_enabled() and (q.requires_grad or kv.requires_grad):
+        raise FkError("small_attention_kv_cached is inference only: run it under torch.no_grad()")
+    q = _rows_ok(q)
+    B, Tq, W = q.shape
+    S = kv.shape[1]
+    H = n_heads
+    hd = W // H
+    if kv.shape != (B, S, 2 * W) or kv.dtype != torch.bfloat16 or kv.stride(2) != 1 or kv.stride(0) % 8 or kv.stride(1) % 8:
+        raise FkError(f"small_attention_kv_cached: q {tuple(q.shape)} and kv {tuple(kv.shape)} (strides {kv.stride()}) "
+                      "do not match or are not 16-byte aligned bf16 rows")
+    if not small_attention_supported(Tq, hd):
+        raise FkError("small_attention serves <= 64 queries at head_dim 16 / 32 / 64")
+    k, v = kv[..., :W], kv[..., W:]
+    dev = q.device
+    nch = lib().fk_small_attn_chunks(S)
+    out = torch.empty(B, Tq, W, device=dev, dtype=torch.bfloat16)
+    lse = torch.empty(B, H, Tq, device=dev, dtype=torch.float32)
+    part_o = torch.empty(B, H, nch, Tq, hd, device=dev, dtype=torch.float32)
+    part_ml = torch.empty(B, H, nch, Tq, 2, device=dev, dtype=torch.float32)
+    scale = float(hd ** -0.5 if scale is None else scale)
+    with timed("small_attn_fwd", 4.0 * B * H * Tq * S * hd):
+        check(lib().fk_small_attn_forward(ptr(q), q.stride(0), q.stride(1), ptr(k), k.stride(0), k.stride(1), ptr(v),
+                                          v.stride(0), v.stride(1), ptr(out), out.stride(0), out.stride(1), ptr(lse), B, H,
+                                          Tq, S, hd, scale, None, 0, 0, 0, ptr(part_o), ptr(part_ml), stream()),
+              "fk_small_attn_forward")
+    return out
 
 
 def small_attention(q, k, v, n_heads: int, scale: Optional[float] = None, rope: Optional[RopeSpec] = None,

@@ -219,6 +219,22 @@ int fk_attn_forward_tc(const void* q, const void* k, const void* v, void* out, f
                        long long v_ts, long long o_bs, long long o_ts, const int* qid, const int* kid, const int* qmin,
                        const int* qmax, const int* kmin, const int* kmax, float scale, unsigned int* counters,
                        void* stream);
+/* The same forward for queries and keys of different lengths (inference against a key / value cache, e.g. one streaming
+ * step of brainformer.Encoder): q [B][Sq][H][head_dim], k / v [B][Sk][H][head_dim] bf16 strided views (all strides % 8 == 0,
+ * token strides >= H * head_dim), head_dim 16, 32 or 64; labels qid [B, Sq], kid [B, Sk] with the ranges of
+ * fk_attn_label_ranges for each side; any other head_dim, Sq < 1, Sk < 1 or bad strides are rejected before anything is
+ * launched (counters untouched).  Work item = (256-query block, key chunk, head, trial): the key axis is cut into n_chunks
+ * chunks of ceil(key tiles / n_chunks) 128-key tiles (1 <= n_chunks <= ceil(Sk / 128); fk_attn_kv_chunks picks enough to
+ * fill max_ctas CTAs, <= 0: all SMs).  n_chunks == 1 runs the unsplit kernel (part_o / part_ml unused).  Otherwise each item
+ * writes unnormalised partials, part_o fp32 [B, H, n_chunks, Sq, head_dim] and part_ml fp32 [B, H, n_chunks, Sq, 2] (running
+ * maximum and sum, log2 domain), and a second launch merges them in chunk order (bit-reproducible).  out bf16; lse
+ * [B, H, Sq] (log2 domain) nullable; a query that sees no key gives a zero row.  counters: as fk_attn_forward_tc. */
+int fk_attn_kv_chunks(int B, int H, int Sq, int Sk, int max_ctas);
+int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq, int Sk,
+                          int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs,
+                          long long v_ts, long long o_bs, long long o_ts, const int* qid, const int* kid, const int* qmin,
+                          const int* qmax, const int* kmin, const int* kmax, float scale, float* part_o, float* part_ml,
+                          int n_chunks, unsigned int* counters, void* stream);
 
 /* Fused residual add + norm on the fp32 residual stream: x_out = x + delta (bf16), y = norm(x_out)
  * (the pair `x = x + branch(...)`; `ln(x)` of models/brainformer.py:243-244).  Backward: dx = norm_backward(g_y) + g_res
