@@ -573,82 +573,29 @@ attn_label_range_kernel(const int* __restrict__ ids, int B, int S, int* __restri
 
 // ------------------------------------------------------------------------------------------------
 // RoPE (brainformer.py:70-91): adjacent pairs rotated by the cached complex exponentials, fp32 math,
-// in place on bf16 [B, S, H, 32] with arbitrary token / batch strides.  inverse = conjugate (backward).
-// table: [P, 16] float2 (cos, sin); position of token (b, s) = pos ? pos[b*S+s] : s + pos_offset.
+// in place on bf16 [B, S, H, HD] (HD = 16, 32 or 64) with arbitrary token / batch strides.  inverse = conjugate (backward).
+// table: [P, HD / 2] float2 (cos, sin); position of token (b, s) = pos ? pos[b*S+s] : s + pos_offset.
 // ------------------------------------------------------------------------------------------------
+template <int HD>
 __global__ void __launch_bounds__(256)
 rope_kernel(__nv_bfloat16* __restrict__ x, long long bs, long long ts, int B, int S, int H, const float2* __restrict__ table,
             int P, const int* __restrict__ pos, int pos_offset, int inverse) {
-  // one thread = 8 consecutive elements (4 pairs) = one 16-byte chunk
+  // one thread = 8 consecutive elements (4 pairs) = one 16-byte chunk, HD / 8 chunks per head
+  constexpr int kChunks = HD / 8;
+  constexpr int kShift = HD == 16 ? 1 : HD == 32 ? 2 : 3;     // log2(kChunks)
   const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const long long total = static_cast<long long>(B) * S * H * 4;
+  const long long total = static_cast<long long>(B) * S * H * kChunks;
   if (idx >= total) return;
-  const int c = static_cast<int>(idx & 3);
-  const int h = static_cast<int>((idx >> 2) % H);
-  const long long bsidx = (idx >> 2) / H;
+  const int c = static_cast<int>(idx & (kChunks - 1));
+  const int h = static_cast<int>((idx >> kShift) % H);
+  const long long bsidx = (idx >> kShift) / H;
   const int s = static_cast<int>(bsidx % S), b = static_cast<int>(bsidx / S);
   int ps = pos ? pos[static_cast<long long>(b) * S + s] : s + pos_offset;
   ps = min(max(ps, 0), P - 1);
-  uint4* ptr = reinterpret_cast<uint4*>(x + b * bs + static_cast<long long>(s) * ts + h * kHD + c * 8);
+  uint4* ptr = reinterpret_cast<uint4*>(x + b * bs + static_cast<long long>(s) * ts + h * HD + c * 8);
   uint4 raw = *ptr;
   uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
-  const float2* tb = table + static_cast<long long>(ps) * 16 + c * 4;
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
-    const float a = __bfloat162float(v.x), bb = __bfloat162float(v.y);
-    const float2 cs = tb[j];
-    const float sn = inverse ? -cs.y : cs.y;
-    w[j] = pack_bf16(a * cs.x - bb * sn, a * sn + bb * cs.x);
-  }
-  *ptr = make_uint4(w[0], w[1], w[2], w[3]);
-}
-
-// Same at head_dim 64: table [P, 32] float2; one thread = one 16-byte chunk, 8 chunks per head.
-__global__ void __launch_bounds__(256)
-rope64_kernel(__nv_bfloat16* __restrict__ x, long long bs, long long ts, int B, int S, int H, const float2* __restrict__ table,
-              int P, const int* __restrict__ pos, int pos_offset, int inverse) {
-  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const long long total = static_cast<long long>(B) * S * H * 8;
-  if (idx >= total) return;
-  const int c = static_cast<int>(idx & 7);
-  const int h = static_cast<int>((idx >> 3) % H);
-  const long long bsidx = (idx >> 3) / H;
-  const int s = static_cast<int>(bsidx % S), b = static_cast<int>(bsidx / S);
-  int ps = pos ? pos[static_cast<long long>(b) * S + s] : s + pos_offset;
-  ps = min(max(ps, 0), P - 1);
-  uint4* ptr = reinterpret_cast<uint4*>(x + b * bs + static_cast<long long>(s) * ts + h * 64 + c * 8);
-  uint4 raw = *ptr;
-  uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
-  const float2* tb = table + static_cast<long long>(ps) * 32 + c * 4;
-#pragma unroll
-  for (int j = 0; j < 4; ++j) {
-    const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
-    const float a = __bfloat162float(v.x), bb = __bfloat162float(v.y);
-    const float2 cs = tb[j];
-    const float sn = inverse ? -cs.y : cs.y;
-    w[j] = pack_bf16(a * cs.x - bb * sn, a * sn + bb * cs.x);
-  }
-  *ptr = make_uint4(w[0], w[1], w[2], w[3]);
-}
-
-// Same at head_dim 16: table [P, 8] float2; one thread = one 16-byte chunk, 2 chunks per head.
-__global__ void __launch_bounds__(256)
-rope16_kernel(__nv_bfloat16* __restrict__ x, long long bs, long long ts, int B, int S, int H, const float2* __restrict__ table,
-              int P, const int* __restrict__ pos, int pos_offset, int inverse) {
-  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-  const long long total = static_cast<long long>(B) * S * H * 2;
-  if (idx >= total) return;
-  const int c = static_cast<int>(idx & 1);
-  const int h = static_cast<int>((idx >> 1) % H);
-  const long long bsidx = (idx >> 1) / H;
-  const int s = static_cast<int>(bsidx % S), b = static_cast<int>(bsidx / S);
-  int ps = pos ? pos[static_cast<long long>(b) * S + s] : s + pos_offset;
-  ps = min(max(ps, 0), P - 1);
-  uint4* ptr = reinterpret_cast<uint4*>(x + b * bs + static_cast<long long>(s) * ts + h * 16 + c * 8);
-  uint4 raw = *ptr;
-  uint32_t w[4] = {raw.x, raw.y, raw.z, raw.w};
-  const float2* tb = table + static_cast<long long>(ps) * 8 + c * 4;
+  const float2* tb = table + static_cast<long long>(ps) * (HD / 2) + c * 4;
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
     const __nv_bfloat162 v = *reinterpret_cast<const __nv_bfloat162*>(&w[j]);
@@ -758,7 +705,7 @@ FK_API int fk_rope(void* x, long long bs, long long ts, int B, int S, int H, int
   FK_REQUIRE(pos != nullptr || (pos_offset >= 0 && static_cast<long long>(pos_offset) + S <= P),
              "fk_rope: token positions pos_offset .. pos_offset + S - 1 fall outside the rope table");
   const long long total = static_cast<long long>(B) * S * H * (head_dim / 8);
-  auto kern = head_dim == 64 ? rope64_kernel : head_dim == 16 ? rope16_kernel : rope_kernel;
+  auto kern = head_dim == 64 ? rope_kernel<64> : head_dim == 16 ? rope_kernel<16> : rope_kernel<32>;
   kern<<<static_cast<unsigned>((total + 255) / 256), 256, 0, stream>>>(
       static_cast<__nv_bfloat16*>(x), bs, ts, B, S, H, reinterpret_cast<const float2*>(table), P, pos, pos_offset, inverse);
   FK_CHECK_LAUNCH();

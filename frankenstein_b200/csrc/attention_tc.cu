@@ -1,7 +1,8 @@
-// Attention backward on the 5th-gen tensor cores (tcgen05.mma + TMEM + TMA), head_dim 32, label masks.  The head_dim-64
-// variants of the forward and backward kernels follow the head_dim-32 ones at the end of the file.  Head_dim 16 runs the
-// head_dim-32 kernels instantiated with HD = 16 (16-column heads, 32-byte rows and the 32-byte swizzle), on the default
-// path only: folded statistics, MN-major accumulate operands.
+// Attention backward on the 5th-gen tensor cores (tcgen05.mma + TMEM + TMA), head_dim 32, label masks.  Head_dim 16 runs
+// the head_dim-32 kernels instantiated with HD = 16 (16-column heads, 32-byte rows and the 32-byte swizzle), on the default
+// path only: folded statistics, MN-major accumulate operands.  The forward and the statistics kernel are instantiated at
+// HD = 64 as well (128-byte rows, the 128-byte swizzle); the head_dim-64 backward is a kernel of its own
+// (attn_bwd_tc64_kernel), after the forward.
 //
 // Same math and mask rule as attention.cu (reference: F.scaled_dot_product_attention backward at
 // models/brainformer.py:168), restructured for Blackwell: every matmul is a tcgen05.mma issued by one thread,
@@ -179,13 +180,14 @@ __device__ __forceinline__ void tmem_wait1_32(uint32_t (&a)[32]) {
                :: "memory");
 }
 
-// Head width HD of the 16 / 32-wide kernels: a [tokens][HD] bf16 row is 2 HD bytes, TMA-loaded with the swizzle of that
-// width (SWIZZLE_32B at 16, SWIZZLE_64B at 32).  A K step of 16 rows of an MN-major tile adds 2 HD in the descriptor's
-// (address >> 4) field.
+// Head width HD of the templated kernels: a [tokens][HD] bf16 row is 2 HD bytes, TMA-loaded with the swizzle of that
+// width (SWIZZLE_32B at 16, SWIZZLE_64B at 32, SWIZZLE_128B at 64).  A K step of 16 rows of an MN-major tile adds 2 HD in
+// the descriptor's (address >> 4) field.
 template <int HD>
 __device__ __forceinline__ uint64_t umma_desc_rows(uint32_t saddr) {
   if constexpr (HD == 16) return umma_desc_sw32(saddr);
-  else return umma_desc_sw64(saddr);
+  else if constexpr (HD == 32) return umma_desc_sw64(saddr);
+  else return umma_desc_sw128(saddr);
 }
 template <int N>
 __device__ __forceinline__ void tmem_ld_wait(uint32_t taddr, uint32_t (&r)[N]) {
@@ -906,7 +908,7 @@ __device__ __forceinline__ void split3(float x, float& hi, float& mid, float& lo
   lo = __bfloat162float(__float2bfloat16_rn(r1 - mid));
 }
 
-template <int HD>      // 16 or 32 (head_dim 64: attn_aug64_kernel)
+template <int HD>      // 16, 32 or 64
 __global__ void __launch_bounds__(256)
 attn_aug_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o, const float* __restrict__ lse,
                 float* __restrict__ delta, __nv_bfloat16* __restrict__ aug, int B, int H, int S, long long o_bs, long long o_ts,
@@ -979,13 +981,14 @@ attn_transpose_kernel(const __nv_bfloat16* __restrict__ x, long long bs, long lo
 
 // ================================================================================================
 // Forward on tcgen05: persistent CTAs; work item = 256 queries of one (head, trial) (two warpgroups, 128 rows each, one
-// thread per row), streaming 128-key tiles (K and V both as [keys][32] SW64 tiles; the P V MMAs read V MN-major).
-// Per tile and warpgroup g:
-//   S_g = Q_g K^T (2 MMAs, N = 128) -> TMEM;  thread: ONE sweep P = 2^(S c - m) against the stale running maximum m,
-//   row sum, bf16 pairs -> operand buffer in TMEM;  O_g += P V (8 TS-mode MMAs, N = 32) accumulating in TMEM.
+// thread per row), streaming 128-key tiles (K and V both as [keys][HD] tiles with the swizzle of their row width; the P V
+// MMAs read V MN-major).  Per tile and warpgroup g:
+//   S_g = Q_g K^T (HD / 16 MMAs, N = 128) -> TMEM;  thread: ONE sweep P = 2^(S c - m) against the stale running maximum m,
+//   row sum, bf16 pairs -> operand buffer in TMEM;  O_g += P V (8 TS-mode MMAs, N = HD) accumulating in TMEM.
 // The reference m is only re-established (row maximum pass, O / l rescaled) for the first visible tile of a row and when
 // the row sum shows that it has gone stale -- O / l is independent of the m that was used.
-// TMEM map: S_g at g*128 (128), P_g at 256 + g*64 (64), O_g at 384 + g*32 (32).
+// TMEM map: S_g at g*128 (128), P_g at 256 + g*64 (64), O_g at 384 + g*32 (32) at head_dim 16 / 32 and at 384 + g*64 (64)
+// at head_dim 64, which fills the 512 columns.
 // ================================================================================================
 constexpr int kFwdTileK = 128;
 constexpr int kFwdThreads = 384;
@@ -994,14 +997,22 @@ constexpr float kRescaleSlack = 8.f;
 // at most 128): the tile is redone with its true maximum
 constexpr float kStaleSum = 256.f;
 
+// Shared memory of the forward at head width HD.  Tile rows are laid out 64 B apart at head_dim 16 and 32 (a 16-wide row
+// fills the first 32 B of its slot) and 128 B apart at 64.  The K | V ring holds 128 KB: 8 stages at 16 / 32, 4 at 64.
+template <int HD>
 struct FwdSmem {
-  static constexpr int q = 0;                           // 2 buffers (item n in buffer n & 1) x 2 groups x 128 x 64 B
-  static constexpr int stream = 32768;                  // kNST x 16 KB: K tile (8 KB) | V tile (8 KB)
-  static constexpr int ids = stream + kNST * 16384;     // [2 wg][2 buffers][128] int
+  static constexpr int row_bytes = HD == 64 ? 128 : 64;
+  static constexpr int q_tile = 128 * row_bytes;        // one warpgroup's Q tile
+  static constexpr int stage = 2 * kFwdTileK * row_bytes;    // K tile | V tile
+  static constexpr int n_stages = 131072 / stage;
+  static constexpr int q = 0;                           // 2 buffers (item n in buffer n & 1) x 2 groups x q_tile
+  static constexpr int stream = 4 * q_tile;             // n_stages x stage
+  static constexpr int ids = stream + n_stages * stage; // [2 wg][2 buffers][128] int
   static constexpr int tiles = ids + 2 * 2 * 128 * 4;
   static constexpr int bars = tiles + 2 * kMaxTiles * 2;     // two lists: the next item's is built while this one runs
   static constexpr int total = bars + 256;
 };
+static_assert(FwdSmem<64>::total <= 232448, "attn_fwd_tc_kernel<64>: shared memory");
 
 
 struct FwdParams {
@@ -1044,27 +1055,33 @@ __device__ __forceinline__ void store_part_ml(float* dst, float m, float l) {
   *reinterpret_cast<float2*>(dst) = make_float2(l > 0.f ? m : -INFINITY, l);
 }
 
-// HD = 16: Q / K / V rows of 32 B (SWIZZLE_32B), one score K step, P V MMAs N = 16; O_g uses the first 16 of its 32
-// TMEM columns.
+// HD = 32: Q / K / V rows of 64 B (SWIZZLE_64B), two score K steps, P V MMAs N = 32.
+// HD = 16: rows of 32 B (SWIZZLE_32B), one score K step, P V MMAs N = 16; O_g uses the first 16 of its 32 TMEM columns.
+// HD = 64: rows of 128 B (SWIZZLE_128B), four score K steps, P V MMAs N = 64; O_g is rescaled and read out in two
+// 32-column halves.
 template <int HD, bool kPart = false>
 __global__ void __launch_bounds__(kFwdThreads, 1)
 attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
                    const __grid_constant__ CUtensorMap tm_v, const FwdArgs<kPart> p) {
+  using Smem = FwdSmem<HD>;
+  constexpr int kStages = Smem::n_stages;
+  constexpr int kOCols = HD == 64 ? 64 : 32;        // TMEM columns of O_g
+  constexpr int kOChunk = HD == 16 ? 16 : 32;       // O_g columns per TMEM load / store: HD / kOChunk chunks
   extern __shared__ __align__(1024) uint8_t smem[];
   if ((smem_u32(smem) & 1023u) != 0) __trap();
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FwdSmem::bars);
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Smem::bars);
   uint64_t* q_full = bars;                  // [2]     Q tiles of item n in buffer n & 1
   uint64_t* list_ready = bars + 2;          // [1]     warp 2 has written the id and the tile list of the next item
-  uint64_t* st_full = bars + 3;             // [kNST]
-  uint64_t* st_empty = st_full + kNST;      // [kNST]  two arrivals: the P V MMAs of both warpgroups
-  uint64_t* s_full = st_empty + kNST;       // [2]     S_g written by the tensor core
+  uint64_t* st_full = bars + 3;             // [kStages]
+  uint64_t* st_empty = st_full + kStages;   // [kStages]  two arrivals: the P V MMAs of both warpgroups
+  uint64_t* s_full = st_empty + kStages;    // [2]     S_g written by the tensor core
   uint64_t* s_free = s_full + 2;            // [2]     S_g read out (4 warps)
   uint64_t* p_ready = s_free + 2;           // [2]     P_g written (4 warps)
   uint64_t* p_free = p_ready + 2;           // [2]     P V MMAs of warpgroup g retired (O_g quiescent, P_g reusable)
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(p_free + 2);
   int* n_tiles_slot = reinterpret_cast<int*>(p_free + 2) + 1;   // [2]
   int* item_slot = reinterpret_cast<int*>(p_free + 2) + 3;      // [2]
-  uint16_t* tile_lists = reinterpret_cast<uint16_t*>(smem + FwdSmem::tiles);
+  uint16_t* tile_lists = reinterpret_cast<uint16_t*>(smem + Smem::tiles);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const bool masked = p.qid != nullptr;
@@ -1080,7 +1097,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     mbar_init(&q_full[0], 1);
     mbar_init(&q_full[1], 1);
     mbar_init(list_ready, 1);
-    for (int i = 0; i < kNST; ++i) { mbar_init(&st_full[i], 1); mbar_init(&st_empty[i], 2); }
+    for (int i = 0; i < kStages; ++i) { mbar_init(&st_full[i], 1); mbar_init(&st_empty[i], 2); }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&s_full[i], 1);
       mbar_init(&s_free[i], 4);
@@ -1184,21 +1201,21 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       auto load_q = [&](int h_, int q0_, int b_, int buf) {
         if (elect_one()) {
           mbar_expect_tx(&q_full[buf], 2 * 128 * HD * 2);
-          tma_load_4d(smem + FwdSmem::q + buf * 16384, &tm_q, &q_full[buf], 0, h_, q0_, b_);
-          tma_load_4d(smem + FwdSmem::q + buf * 16384 + 8192, &tm_q, &q_full[buf], 0, h_, q0_ + 128, b_);
+          tma_load_4d(smem + Smem::q + buf * 2 * Smem::q_tile, &tm_q, &q_full[buf], 0, h_, q0_, b_);
+          tma_load_4d(smem + Smem::q + buf * 2 * Smem::q_tile + Smem::q_tile, &tm_q, &q_full[buf], 0, h_, q0_ + 128, b_);
         }
         __syncwarp();
       };
       auto load_tile = [&](int t, int h_, int b_) {
-        uint8_t* st = smem + FwdSmem::stream + pstage * 16384;
+        uint8_t* st = smem + Smem::stream + pstage * Smem::stage;
         mbar_wait(&st_empty[pstage], pphase ^ 1);
         if (elect_one()) {
           mbar_expect_tx(&st_full[pstage], 2 * kFwdTileK * HD * 2);
           tma_load_4d(st, &tm_k, &st_full[pstage], 0, h_, t * kFwdTileK, b_);
-          tma_load_4d(st + 8192, &tm_v, &st_full[pstage], 0, h_, t * kFwdTileK, b_);      // V tile [128 keys][32 dims]
+          tma_load_4d(st + Smem::stage / 2, &tm_v, &st_full[pstage], 0, h_, t * kFwdTileK, b_);   // V tile [128 keys][HD]
         }
         __syncwarp();
-        if (++pstage == kNST) { pstage = 0; pphase ^= 1; }
+        if (++pstage == kStages) { pstage = 0; pphase ^= 1; }
       };
       if (pre_cnt < 0) { load_q(h, q0, b, item_n & 1); pre_cnt = 0; }
       for (int j = pre_cnt; j < T_u; ++j) load_tile(__shfl_sync(0xffffffffu, tile_list[j] & 0x3fff, 0), h, b);
@@ -1213,7 +1230,7 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
         const int T2 = __shfl_sync(0xffffffffu, n_tiles_slot[(item_n + 1) & 1], 0);
         load_q(h2, qt2 * 256, b2, (item_n + 1) & 1);
         pre_cnt = 0;
-        const int ahead = T2 < kNST / 2 ? T2 : kNST / 2;
+        const int ahead = T2 < kStages / 2 ? T2 : kStages / 2;
         for (int j = 0; j < ahead; ++j, ++pre_cnt) load_tile(__shfl_sync(0xffffffffu, list2[j] & 0x3fff, 0), h2, b2);
       }
     }
@@ -1223,23 +1240,25 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       constexpr uint32_t idesc = umma_idesc_bf16(128, kFwdTileK);
       const int T_u = __shfl_sync(0xffffffffu, T, 0);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-      const uint64_t dQ[2] = {umma_desc_rows<HD>(smem_u32(smem + FwdSmem::q + (item_n & 1) * 16384)),
-                              umma_desc_rows<HD>(smem_u32(smem + FwdSmem::q + (item_n & 1) * 16384 + 8192))};
-      const uint32_t stream = smem_u32(smem + FwdSmem::stream);
+      const uint8_t* q_buf = smem + Smem::q + (item_n & 1) * 2 * Smem::q_tile;
+      const uint64_t dQ[2] = {umma_desc_rows<HD>(smem_u32(q_buf)), umma_desc_rows<HD>(smem_u32(q_buf + Smem::q_tile))};
+      const uint32_t stream = smem_u32(smem + Smem::stream);
       mbar_wait(&q_full[item_n & 1], (item_n >> 1) & 1);
       tc_fence_after();
       for (int j = 0; j < T_u; ++j) {
         const int gj = base + j;                     // key-tile counter across items
-        const int stage = gj % kNST;
-        mbar_wait(&st_full[stage], (gj / kNST) & 1);
-        const uint64_t dK = umma_desc_rows<HD>(stream + stage * 16384);
+        const int stage = gj % kStages;
+        mbar_wait(&st_full[stage], (gj / kStages) & 1);
+        const uint64_t dK = umma_desc_rows<HD>(stream + stage * Smem::stage);
 #pragma unroll
         for (int g = 0; g < 2; ++g) {
           mbar_wait(&s_free[g], (gj & 1) ^ 1);
           tc_fence_after();
           if (elect_one()) {
+            // a K step of 16 dims = 32 B = +2 in the descriptors' (address >> 4) field
             umma_bf16(tmem_u + g * 128, dQ[g], dK, idesc, 0u);
-            if (HD == 32) umma_bf16(tmem_u + g * 128, dQ[g] + 2, dK + 2, idesc, 1u);
+#pragma unroll
+            for (int kk = 1; kk < HD / 16; ++kk) umma_bf16(tmem_u + g * 128, dQ[g] + 2 * kk, dK + 2 * kk, idesc, 1u);
             umma_commit(&s_full[g]);
           }
           __syncwarp();
@@ -1252,18 +1271,19 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       constexpr uint32_t idesc = umma_idesc_bf16(128, HD);
       const int T_u = __shfl_sync(0xffffffffu, T, 0);
       const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-      const uint32_t stream = smem_u32(smem + FwdSmem::stream);
+      const uint32_t stream = smem_u32(smem + Smem::stream);
       for (int j = 0; j < T_u; ++j) {
         const int gj = base + j;
-        const int stage = gj % kNST;
+        const int stage = gj % kStages;
         // V tile [128 keys][32 dims] (64-byte rows, SWIZZLE_64B) read MN-major: N = dims contiguous, K = keys, a K step of
-        // 16 keys = 1024 B -- no transposed copy of V exists (head_dim 16: 32-byte rows, SWIZZLE_32B, K step 512 B)
-        const uint64_t dV = umma_desc_rows<HD>(stream + stage * 16384 + 8192);
+        // 16 keys = 1024 B -- no transposed copy of V exists (head_dim 16: 32-byte rows, SWIZZLE_32B, K step 512 B;
+        // head_dim 64: 128-byte rows, SWIZZLE_128B, N = 64 dims in one swizzle atom, K step 2048 B)
+        const uint64_t dV = umma_desc_rows<HD>(stream + stage * Smem::stage + Smem::stage / 2);
 #pragma unroll
         for (int g = 0; g < 2; ++g) {
           mbar_wait(&p_ready[g], gj & 1);
           tc_fence_after();
-          const uint32_t pa = tmem_u + 256 + g * 64, oa = tmem_u + 384 + g * 32;
+          const uint32_t pa = tmem_u + 256 + g * 64, oa = tmem_u + 384 + g * kOCols;
           if (elect_one()) {
 #pragma unroll
             for (int kk = 0; kk < 8; ++kk)
@@ -1284,11 +1304,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     const int row = q0 + g * 128 + r;
     const bool row_ok = row < p.Sq;
     const int my_id = masked ? (row_ok ? p.qid[static_cast<long long>(b) * p.Sq + row] : -0x7fffffff) : 0;
-    int* ids_base = reinterpret_cast<int*>(smem + FwdSmem::ids) + g * 256;
+    int* ids_base = reinterpret_cast<int*>(smem + Smem::ids) + g * 256;
     const uint32_t lane_base = static_cast<uint32_t>(q4 * 32) << 16;
     const uint32_t s_addr = tmem_base + lane_base + g * 128;
     const uint32_t p_addr = tmem_base + lane_base + 256 + g * 64;
-    const uint32_t o_addr = tmem_base + lane_base + 384 + g * 32;
+    const uint32_t o_addr = tmem_base + lane_base + 384 + g * kOCols;
     float m_run = -INFINITY, l_run = 0.f, alpha_pend = 1.f;
     int pre_i = 0;
     // key labels of a tile are only fetched and staged for tiles that need the per-element compare (warp-group uniform
@@ -1332,11 +1352,14 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       // O_g *= alpha_pend (rare, warp-uniform): only legal once the previous tile's P V MMAs have retired
       auto apply_pending = [&]() {
         if (__any_sync(0xffffffffu, alpha_pend != 1.f)) {
-          uint32_t ov[HD];
-          tmem_ld_wait<HD>(o_addr, ov);
 #pragma unroll
-          for (int i = 0; i < HD; ++i) ov[i] = __float_as_uint(__uint_as_float(ov[i]) * alpha_pend);
-          tmem_st_cols<HD>(o_addr, ov);
+          for (int hf = 0; hf < HD / kOChunk; ++hf) {
+            uint32_t ov[kOChunk];
+            tmem_ld_wait<kOChunk>(o_addr + hf * 32, ov);
+#pragma unroll
+            for (int i = 0; i < kOChunk; ++i) ov[i] = __float_as_uint(__uint_as_float(ov[i]) * alpha_pend);
+            tmem_st_cols<kOChunk>(o_addr + hf * 32, ov);
+          }
           alpha_pend = 1.f;
         }
       };
@@ -1434,32 +1457,43 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       mbar_wait(&p_free[g], ((base + T) & 1) ^ 1);     // the last P V MMAs have retired
       tc_fence_after();
     }
-    uint32_t ov[HD];
-    if (T > 0) {
-      tmem_ld_wait<HD>(o_addr, ov);
-    } else {
+    // 1 / l (a reference raise after the last tile is still owed to O) and the output row.  At head_dim 64, where O is
+    // read out in two chunks, they are formed before the first one: formed between the chunks they cost 8 more bytes of
+    // spill loads (ptxas -v).
+    float inv = 0.f;
+    __nv_bfloat16* dst = nullptr;
+    auto out_row = [=, &inv, &dst]() {
+      inv = (l_run > 0.f) ? alpha_pend / l_run : 0.f;
+      dst = row_ok ? p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * HD : nullptr;
+    };
+    if constexpr (HD == 64) out_row();
 #pragma unroll
-      for (int i = 0; i < HD; ++i) ov[i] = 0u;
+    for (int hf = 0; hf < HD / kOChunk; ++hf) {
+      uint32_t ov[kOChunk];
+      if (T > 0) {
+        tmem_ld_wait<kOChunk>(o_addr + hf * 32, ov);
+      } else {
+#pragma unroll
+        for (int i = 0; i < kOChunk; ++i) ov[i] = 0u;
+      }
+      if constexpr (kPart) {
+        if (row_ok) store_part_o<kOChunk>(p.part_o + part_row(p, b, h, u / n_q_tiles, row) * HD + hf * 32, ov, alpha_pend);
+      } else if (row_ok) {
+        if constexpr (HD != 64) out_row();
+#pragma unroll
+        for (int c4 = 0; c4 < kOChunk / 8; ++c4) {
+          uint32_t w[4];
+#pragma unroll
+          for (int e = 0; e < 4; ++e)
+            w[e] = pack2(__uint_as_float(ov[c4 * 8 + e * 2]) * inv, __uint_as_float(ov[c4 * 8 + e * 2 + 1]) * inv);
+          *reinterpret_cast<uint4*>(dst + hf * 32 + c4 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
+        }
+      }
     }
     if constexpr (kPart) {
-      if (row_ok) {
-        const long long pr = part_row(p, b, h, u / n_q_tiles, row);
-        store_part_o<HD>(p.part_o + pr * HD, ov, alpha_pend);
-        store_part_ml(p.part_ml + pr * 2, m_run, l_run);
-      }
-    } else if (row_ok) {
-      const float inv = (l_run > 0.f) ? alpha_pend / l_run : 0.f;      // a reference raise after the last tile is still owed to O
-      __nv_bfloat16* dst = p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * HD;
-#pragma unroll
-      for (int c4 = 0; c4 < HD / 8; ++c4) {
-        uint32_t w[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e)
-          w[e] = pack2(__uint_as_float(ov[c4 * 8 + e * 2]) * inv, __uint_as_float(ov[c4 * 8 + e * 2 + 1]) * inv);
-        *reinterpret_cast<uint4*>(dst + c4 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
-      }
-      if (p.lse != nullptr)
-        p.lse[(static_cast<long long>(b) * p.H + h) * p.Sq + row] = (l_run > 0.f) ? m_run + log2f(l_run) : INFINITY;
+      if (row_ok) store_part_ml(p.part_ml + part_row(p, b, h, u / n_q_tiles, row) * 2, m_run, l_run);
+    } else if (row_ok && p.lse != nullptr) {
+      p.lse[(static_cast<long long>(b) * p.H + h) * p.Sq + row] = (l_run > 0.f) ? m_run + log2f(l_run) : INFINITY;
     }
   }
 
@@ -1487,10 +1521,11 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
 }
 
 // ================================================================================================
-// head_dim 64.  Same work split, label-mask / tile-skip rules, persistent hand-out and softmax as the head_dim-32 kernels
-// above (which stay as they are); [tokens][64] bf16 rows are 128 B, so every tile is TMA-loaded with the 128-byte swizzle.
+// Backward at head_dim 64 (the forward at 64 is attn_fwd_tc_kernel<64>).  Same work split, label-mask / tile-skip rules,
+// persistent hand-out and softmax as the head_dim-32 backward above; [tokens][64] bf16 rows are 128 B, so every tile is
+// TMA-loaded with the 128-byte swizzle.
 //
-// Backward (attn_bwd_tc64_kernel): three score stages (3 x 128 columns) + dV 64 + dK / dQ 64 fill the 512 TMEM columns, so
+// attn_bwd_tc64_kernel: three score stages (3 x 128 columns) + dV 64 + dK / dQ 64 fill the 512 TMEM columns, so
 // the resident tiles cannot sit in TMEM as at head_dim 32: the score MMAs read both operands from shared memory (SS mode,
 // 4 K steps of 16 + the folded statistics step).  P / dS are still written in place over the consumed score columns and
 // read by the accumulate MMAs from TMEM (TS mode, N = 64, B operand MN-major straight from the streamed tile).  One path
@@ -1898,478 +1933,6 @@ attn_bwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_resA, const __grid_c
   }
 }
 
-// ------------------------------------------------------------------------------------------------
-// delta and the statistics rows at head_dim 64 (attn_aug_kernel with 64-wide rows)
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-attn_aug64_kernel(const __nv_bfloat16* __restrict__ o, const __nv_bfloat16* __restrict__ d_o, const float* __restrict__ lse,
-                  float* __restrict__ delta, __nv_bfloat16* __restrict__ aug, int B, int H, int S, long long o_bs, long long o_ts,
-                  long long do_bs, long long do_ts, float inv_scale_log2) {
-  const long long idx = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;   // (b, i, h)
-  if (idx >= static_cast<long long>(B) * S * H) return;
-  const int h = static_cast<int>(idx % H);
-  const long long bi = idx / H;
-  const int i = static_cast<int>(bi % S), b = static_cast<int>(bi / S);
-  const uint4* op = reinterpret_cast<const uint4*>(o + b * o_bs + static_cast<long long>(i) * o_ts + h * 64);
-  const uint4* dp = reinterpret_cast<const uint4*>(d_o + b * do_bs + static_cast<long long>(i) * do_ts + h * 64);
-  float acc = 0.f;
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const uint4 a = op[c], e = dp[c];
-    const uint32_t aw[4] = {a.x, a.y, a.z, a.w}, ew[4] = {e.x, e.y, e.z, e.w};
-#pragma unroll
-    for (int j = 0; j < 4; ++j)
-      acc += __uint_as_float(aw[j] << 16) * __uint_as_float(ew[j] << 16) +
-             __uint_as_float(aw[j] & 0xffff0000u) * __uint_as_float(ew[j] & 0xffff0000u);
-  }
-  const long long row = (static_cast<long long>(b) * H + h) * S + i;
-  delta[row] = acc;
-  const float l = lse[row];
-  const float nl = (l < 3.0e38f) ? -l * inv_scale_log2 : -1.0e30f;
-  float v[6];
-  split3(nl, v[0], v[1], v[2]);
-  split3(-acc, v[3], v[4], v[5]);
-  uint4 w;
-  w.x = pack2(v[0], v[1]); w.y = pack2(v[2], v[3]); w.z = pack2(v[4], v[5]); w.w = 0u;
-  uint4* dst = reinterpret_cast<uint4*>(aug + row * 16);
-  dst[0] = w;
-  dst[1] = make_uint4(0u, 0u, 0u, 0u);
-}
-
-// ================================================================================================
-// Forward at head_dim 64 (attn_fwd_tc_kernel with 64-wide heads): Q [128][64] tiles (two per item and buffer, 64 KB),
-// K | V stages of 32 KB (4 stages), score MMAs K = 64 (4 K steps), P V MMAs N = 64.
-// TMEM map: S_g at g*128 (128), P_g at 256 + g*64 (64), O_g at 384 + g*64 (64) = 512 columns.
-// ================================================================================================
-constexpr int kNSTF64 = 4;
-
-struct FwdSmem64 {
-  static constexpr int q = 0;                            // 2 buffers x 2 groups x [128][64] bf16
-  static constexpr int stream = 65536;                   // kNSTF64 x 32 KB: K tile (16 KB) | V tile (16 KB)
-  static constexpr int ids = stream + kNSTF64 * 32768;   // [2 wg][2 buffers][128] int
-  static constexpr int tiles = ids + 2 * 2 * 128 * 4;
-  static constexpr int bars = tiles + 2 * kMaxTiles * 2;
-  static constexpr int total = bars + 256;
-};
-static_assert(FwdSmem64::total <= 232448, "attn_fwd_tc64_kernel: shared memory");
-
-template <bool kPart = false>
-__global__ void __launch_bounds__(kFwdThreads, 1)
-attn_fwd_tc64_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_constant__ CUtensorMap tm_k,
-                     const __grid_constant__ CUtensorMap tm_v, const FwdArgs<kPart> p) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  if ((smem_u32(smem) & 1023u) != 0) __trap();
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + FwdSmem64::bars);
-  uint64_t* q_full = bars;                  // [2]
-  uint64_t* list_ready = bars + 2;          // [1]
-  uint64_t* st_full = bars + 3;             // [kNSTF64]
-  uint64_t* st_empty = st_full + kNSTF64;   // [kNSTF64]  two arrivals: the P V MMAs of both warpgroups
-  uint64_t* s_full = st_empty + kNSTF64;    // [2]
-  uint64_t* s_free = s_full + 2;            // [2]
-  uint64_t* p_ready = s_free + 2;           // [2]
-  uint64_t* p_free = p_ready + 2;           // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(p_free + 2);
-  int* n_tiles_slot = reinterpret_cast<int*>(p_free + 2) + 1;   // [2]
-  int* item_slot = reinterpret_cast<int*>(p_free + 2) + 3;      // [2]
-  uint16_t* tile_lists = reinterpret_cast<uint16_t*>(smem + FwdSmem64::tiles);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool masked = p.qid != nullptr;
-  const int n_k_tiles = (p.Sk + kFwdTileK - 1) / kFwdTileK;
-  const int nq64 = (p.Sq + 63) / 64, nk64 = (p.Sk + 63) / 64;
-  const int n_q_tiles = (p.Sq + 255) / 256;
-  int n_units = n_q_tiles;                        // work units per (head, trial): query blocks (x key chunks when split)
-  if constexpr (kPart) n_units *= p.n_chunks;
-  const int n_items = n_units * p.H * p.B;
-
-  if (warp == 0 && lane == 0) { tma_prefetch_desc(&tm_q); tma_prefetch_desc(&tm_k); tma_prefetch_desc(&tm_v); }
-  if (warp == 1 && lane == 0) {
-    mbar_init(&q_full[0], 1);
-    mbar_init(&q_full[1], 1);
-    mbar_init(list_ready, 1);
-    for (int i = 0; i < kNSTF64; ++i) { mbar_init(&st_full[i], 1); mbar_init(&st_empty[i], 2); }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&s_full[i], 1);
-      mbar_init(&s_free[i], 4);
-      mbar_init(&p_ready[i], 4);
-      mbar_init(&p_free[i], 1);
-    }
-    fence_mbar_init();
-  }
-  if (warp == 2) {
-    tmem_alloc(tmem_slot, 512);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  auto build_list = [&](int it, int buf) {       // whole warp (see attn_fwd_tc_kernel)
-    const int u_ = it % n_units, b_ = it / (n_units * p.H);
-    const int qt_ = kPart ? u_ % n_q_tiles : u_;
-    int t_lo = 0, t_hi = n_k_tiles;
-    if constexpr (kPart) {
-      t_lo = (u_ / n_q_tiles) * p.chunk_tiles;
-      t_hi = min(t_lo + p.chunk_tiles, n_k_tiles);
-    }
-    uint16_t* list = tile_lists + buf * kMaxTiles;
-    int wq_lo[2] = {0, 0}, wq_hi[2] = {0, 0};
-    if (masked) {
-#pragma unroll
-      for (int g = 0; g < 2; ++g) {
-        const int i0 = min(qt_ * 4 + g * 2, nq64 - 1), i1 = min(qt_ * 4 + g * 2 + 1, nq64 - 1);
-        wq_lo[g] = min(p.qmin[b_ * nq64 + i0], p.qmin[b_ * nq64 + i1]);
-        wq_hi[g] = max(p.qmax[b_ * nq64 + i0], p.qmax[b_ * nq64 + i1]);
-      }
-    }
-    const int cta_hi = max(wq_hi[0], wq_hi[1]);
-    int cnt = 0;
-    for (int cb = t_lo; cb < t_hi; cb += 32) {
-      const int t = cb + lane;
-      bool vis = t < t_hi;
-      int flags = 0;
-      if (vis) {
-        int kmn = 0, kmx = 0;
-        if (masked) {
-          const int i0 = min(t * 2, nk64 - 1), i1 = min(t * 2 + 1, nk64 - 1);
-          kmn = min(p.kmin[b_ * nk64 + i0], p.kmin[b_ * nk64 + i1]);
-          kmx = max(p.kmax[b_ * nk64 + i0], p.kmax[b_ * nk64 + i1]);
-          vis = kmn <= cta_hi;
-        }
-        const bool tail = t * kFwdTileK + kFwdTileK > p.Sk;
-        if ((masked && kmx > wq_lo[0]) || tail) flags |= 0x4000;
-        if ((masked && kmx > wq_lo[1]) || tail) flags |= 0x8000;
-      }
-      const unsigned m = __ballot_sync(0xffffffffu, vis);
-      if (vis) list[cnt + __popc(m & ((1u << lane) - 1u))] = static_cast<uint16_t>(t | flags);
-      cnt += __popc(m);
-    }
-    if (lane == 0) n_tiles_slot[buf] = cnt;
-  };
-
-  int base = 0;
-  uint32_t item_n = 0;
-  int pstage = 0;
-  uint32_t pphase = 0;
-  int pre_cnt = -1;
-  if (warp == 2) {
-    int first = 0;
-    if (lane == 0) first = static_cast<int>(atomicAdd(&p.items[0], 1u));
-    first = __shfl_sync(0xffffffffu, first, 0);
-    if (lane == 0) item_slot[0] = first;
-    if (first < n_items) build_list(first, 0);
-  }
-  __syncthreads();
-  for (int item = item_slot[0]; item < n_items; item = item_slot[(item_n + 1) & 1], ++item_n) {
-  const int u = item % n_units, h = (item / n_units) % p.H, b = item / (n_units * p.H);
-  const int qt = kPart ? u % n_q_tiles : u;
-  const int q0 = qt * 256;
-  const uint16_t* tile_list = tile_lists + (item_n & 1) * kMaxTiles;
-  const int T = n_tiles_slot[item_n & 1];
-
-  if (warp == 2) {
-    int nxt = 0;
-    if (lane == 0) nxt = static_cast<int>(atomicAdd(&p.items[0], 1u));
-    nxt = __shfl_sync(0xffffffffu, nxt, 0);
-    if (lane == 0) item_slot[(item_n + 1) & 1] = nxt;
-    if (nxt < n_items) build_list(nxt, (item_n + 1) & 1);
-    __syncwarp();
-    if (lane == 0) mbar_arrive(list_ready);
-  }
-
-  if (warp == 0) {
-    // ================================ TMA producer ================================
-    const int T_u = __shfl_sync(0xffffffffu, T, 0);
-    auto load_q = [&](int h_, int q0_, int b_, int buf) {
-      if (elect_one()) {
-        mbar_expect_tx(&q_full[buf], 32768);
-        tma_load_4d(smem + FwdSmem64::q + buf * 32768, &tm_q, &q_full[buf], 0, h_, q0_, b_);
-        tma_load_4d(smem + FwdSmem64::q + buf * 32768 + 16384, &tm_q, &q_full[buf], 0, h_, q0_ + 128, b_);
-      }
-      __syncwarp();
-    };
-    auto load_tile = [&](int t, int h_, int b_) {
-      uint8_t* st = smem + FwdSmem64::stream + pstage * 32768;
-      mbar_wait(&st_empty[pstage], pphase ^ 1);
-      if (elect_one()) {
-        mbar_expect_tx(&st_full[pstage], 32768);
-        tma_load_4d(st, &tm_k, &st_full[pstage], 0, h_, t * kFwdTileK, b_);
-        tma_load_4d(st + 16384, &tm_v, &st_full[pstage], 0, h_, t * kFwdTileK, b_);      // V tile [128 keys][64 dims]
-      }
-      __syncwarp();
-      if (++pstage == kNSTF64) { pstage = 0; pphase ^= 1; }
-    };
-    if (pre_cnt < 0) { load_q(h, q0, b, item_n & 1); pre_cnt = 0; }
-    for (int j = pre_cnt; j < T_u; ++j) load_tile(__shfl_sync(0xffffffffu, tile_list[j] & 0x3fff, 0), h, b);
-    mbar_wait(list_ready, item_n & 1);
-    const int nxt = __shfl_sync(0xffffffffu, item_slot[(item_n + 1) & 1], 0);
-    pre_cnt = -1;
-    if (nxt < n_items) {
-      const int u2 = nxt % n_units, h2 = (nxt / n_units) % p.H, b2 = nxt / (n_units * p.H);
-      const int qt2 = kPart ? u2 % n_q_tiles : u2;
-      const uint16_t* list2 = tile_lists + ((item_n + 1) & 1) * kMaxTiles;
-      const int T2 = __shfl_sync(0xffffffffu, n_tiles_slot[(item_n + 1) & 1], 0);
-      load_q(h2, qt2 * 256, b2, (item_n + 1) & 1);
-      pre_cnt = 0;
-      const int ahead = T2 < kNSTF64 / 2 ? T2 : kNSTF64 / 2;
-      for (int j = 0; j < ahead; ++j, ++pre_cnt) load_tile(__shfl_sync(0xffffffffu, list2[j] & 0x3fff, 0), h2, b2);
-    }
-  } else if (warp == 1) {
-    // ================================ score-MMA issuer ================================
-    constexpr uint32_t idesc = umma_idesc_bf16(128, kFwdTileK);
-    const int T_u = __shfl_sync(0xffffffffu, T, 0);
-    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-    const uint64_t dQ[2] = {umma_desc_sw128(smem_u32(smem + FwdSmem64::q + (item_n & 1) * 32768)),
-                            umma_desc_sw128(smem_u32(smem + FwdSmem64::q + (item_n & 1) * 32768 + 16384))};
-    const uint32_t stream = smem_u32(smem + FwdSmem64::stream);
-    mbar_wait(&q_full[item_n & 1], (item_n >> 1) & 1);
-    tc_fence_after();
-    for (int j = 0; j < T_u; ++j) {
-      const int gj = base + j;
-      const int stage = gj % kNSTF64;
-      mbar_wait(&st_full[stage], (gj / kNSTF64) & 1);
-      const uint64_t dK = umma_desc_sw128(stream + stage * 32768);
-#pragma unroll
-      for (int g = 0; g < 2; ++g) {
-        mbar_wait(&s_free[g], (gj & 1) ^ 1);
-        tc_fence_after();
-        if (elect_one()) {
-#pragma unroll
-          for (int kk = 0; kk < 4; ++kk) umma_bf16(tmem_u + g * 128, dQ[g] + 2 * kk, dK + 2 * kk, idesc, kk > 0 ? 1u : 0u);
-          umma_commit(&s_full[g]);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp == 3) {
-    // ================================ P V MMA issuer ================================
-    constexpr uint32_t idesc = umma_idesc_bf16(128, 64);
-    const int T_u = __shfl_sync(0xffffffffu, T, 0);
-    const uint32_t tmem_u = __shfl_sync(0xffffffffu, tmem_base, 0);
-    const uint32_t stream = smem_u32(smem + FwdSmem64::stream);
-    for (int j = 0; j < T_u; ++j) {
-      const int gj = base + j;
-      const int stage = gj % kNSTF64;
-      // V tile [128 keys][64 dims] (128-byte rows, SWIZZLE_128B) read MN-major: N = 64 dims in one swizzle atom, K = keys,
-      // a K step of 16 keys = 2048 B
-      const uint64_t dV = umma_desc_sw128(stream + stage * 32768 + 16384);
-#pragma unroll
-      for (int g = 0; g < 2; ++g) {
-        mbar_wait(&p_ready[g], gj & 1);
-        tc_fence_after();
-        const uint32_t pa = tmem_u + 256 + g * 64, oa = tmem_u + 384 + g * 64;
-        if (elect_one()) {
-#pragma unroll
-          for (int kk = 0; kk < 8; ++kk)
-            umma_bf16_ts(oa, pa + kk * 8, dV + 128 * kk, idesc | (1u << 16), (j > 0 || kk > 0) ? 1u : 0u);
-          umma_commit(&p_free[g]);
-          umma_commit(&st_empty[stage]);
-        }
-        __syncwarp();
-      }
-    }
-  } else if (warp >= 4) {
-    // ================================ softmax warpgroups (as attn_fwd_tc_kernel) ================================
-    const int g = (warp - 4) >> 2;
-    const int q4 = warp & 3;
-    const int r = q4 * 32 + lane;
-    const int tid = (warp - 4 - g * 4) * 32 + lane;
-    const int row = q0 + g * 128 + r;
-    const bool row_ok = row < p.Sq;
-    const int my_id = masked ? (row_ok ? p.qid[static_cast<long long>(b) * p.Sq + row] : -0x7fffffff) : 0;
-    int* ids_base = reinterpret_cast<int*>(smem + FwdSmem64::ids) + g * 256;
-    const uint32_t lane_base = static_cast<uint32_t>(q4 * 32) << 16;
-    const uint32_t s_addr = tmem_base + lane_base + g * 128;
-    const uint32_t p_addr = tmem_base + lane_base + 256 + g * 64;
-    const uint32_t o_addr = tmem_base + lane_base + 384 + g * 64;
-    float m_run = -INFINITY, l_run = 0.f, alpha_pend = 1.f;
-    int pre_i = 0;
-    const uint16_t my_flag = (g == 0) ? 0x4000 : 0x8000;
-    auto prefetch = [&](int j) {
-      if (j >= T || !(tile_list[j] & my_flag)) return;
-      const int c = (tile_list[j] & 0x3fff) * kFwdTileK + tid;
-      pre_i = (masked && c < p.Sk) ? p.kid[static_cast<long long>(b) * p.Sk + c] : 0;   // (c >= Sk: masked by position)
-    };
-    prefetch(0);
-    for (int j = 0; j < T; ++j) {
-      const int gj = base + j;
-      const bool need_mask = (tile_list[j] & my_flag) != 0;
-      const int n_valid = p.Sk - (tile_list[j] & 0x3fff) * kFwdTileK;     // < kFwdTileK only in the ragged tail
-      int* s_id = ids_base;
-      if (need_mask) {
-        named_bar_sync(1 + g, 128);
-        s_id[tid] = pre_i;
-        named_bar_sync(1 + g, 128);
-      }
-      prefetch(j + 1);
-      mbar_wait(&s_full[g], gj & 1);
-      tc_fence_after();
-      uint32_t sv[2][32];
-      auto mask_chunk = [&](uint32_t (&v)[32], int c) {
-        if (need_mask) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if (s_id[c * 32 + i] > my_id) v[i] = 0xff800000u;
-          if (n_valid < kFwdTileK) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (c * 32 + i >= n_valid) v[i] = 0xff800000u;
-          }
-        }
-      };
-      // O_g *= alpha_pend (rare, warp-uniform), 64 columns in two halves
-      auto apply_pending = [&]() {
-        if (__any_sync(0xffffffffu, alpha_pend != 1.f)) {
-#pragma unroll
-          for (int hf = 0; hf < 2; ++hf) {
-            uint32_t ov[32];
-            tmem_ld32(o_addr + hf * 32, ov);
-            tmem_wait1_32(ov);
-#pragma unroll
-            for (int i = 0; i < 32; ++i) ov[i] = __float_as_uint(__uint_as_float(ov[i]) * alpha_pend);
-            tmem_st32(o_addr + hf * 32, ov);
-          }
-          alpha_pend = 1.f;
-        }
-      };
-      float rs = 0.f;
-      bool released = false, redo = false;
-      auto release_scores = [&]() {
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&s_free[g]);
-        released = true;
-      };
-      auto exp_sweep = [&](float m_use, bool optimistic) {
-        rs = 0.f;
-        if (optimistic) tmem_ld32(s_addr, sv[0]);
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const int cur = c & 1;
-          tmem_wait1_32(sv[cur]);
-          if (c < 3) tmem_ld32(s_addr + (c + 1) * 32, sv[cur ^ 1]);
-          mask_chunk(sv[cur], c);
-          if (c == 3 && !optimistic) release_scores();
-          uint32_t pw[16];
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            const float p0 = fast_ex2(fmaf(__uint_as_float(sv[cur][2 * i]), p.scale_log2, -m_use));
-            const float p1 = fast_ex2(fmaf(__uint_as_float(sv[cur][2 * i + 1]), p.scale_log2, -m_use));
-            rs += p0 + p1;
-            pw[i] = pack2(p0, p1);
-          }
-          if (c == 0 && optimistic) {
-            mbar_wait(&p_free[g], (gj & 1) ^ 1);
-            tc_fence_after();
-            apply_pending();
-          }
-          tmem_st16(p_addr + c * 16, pw);
-        }
-      };
-      const bool two_pass = __any_sync(0xffffffffu, m_run == -INFINITY);
-      if (!two_pass) {
-        exp_sweep(m_run, true);
-        redo = __any_sync(0xffffffffu, !(rs <= kStaleSum));
-        if (!redo) {
-          release_scores();
-          l_run += rs;
-        }
-      }
-      if (two_pass || redo) {
-        float mx1 = -INFINITY;
-        tmem_ld32(s_addr, sv[0]);
-#pragma unroll
-        for (int c = 0; c < 4; ++c) {
-          const int cur = c & 1;
-          tmem_wait1_32(sv[cur]);
-          tmem_ld32(s_addr + ((c + 1) & 3) * 32, sv[cur ^ 1]);
-          mask_chunk(sv[cur], c);
-#pragma unroll
-          for (int i = 0; i < 32; i += 2) mx1 = fmaxf(mx1, fmaxf(__uint_as_float(sv[cur][i]), __uint_as_float(sv[cur][i + 1])));
-        }
-        const float m_tile = mx1 * p.scale_log2;
-        const bool raise = m_tile > m_run + (redo ? 0.f : kRescaleSlack) || m_run == -INFINITY;
-        const float m_new = raise ? fmaxf(m_run, m_tile) : m_run;
-        const float m_use = (m_new == -INFINITY) ? 0.f : m_new;
-        const float alpha = (raise && m_run != -INFINITY) ? fast_ex2(m_run - m_use) : 1.f;
-        if (two_pass) {
-          mbar_wait(&p_free[g], (gj & 1) ^ 1);
-          tc_fence_after();
-          apply_pending();
-        }
-        l_run *= alpha;
-        alpha_pend = alpha;
-        apply_pending();
-        m_run = m_new;
-        redo = false;
-        exp_sweep(m_use, false);
-        l_run += rs;
-      }
-      if (!released) release_scores();
-      tmem_wait_st();
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&p_ready[g]);
-    }
-    // ---- epilogue: O / l -> bf16 (64 columns in two halves), LSE ----
-    if (T > 0) {
-      mbar_wait(&p_free[g], ((base + T) & 1) ^ 1);
-      tc_fence_after();
-    }
-    const float inv = (l_run > 0.f) ? alpha_pend / l_run : 0.f;
-    __nv_bfloat16* dst = row_ok ? p.out + b * p.o_bs + static_cast<long long>(row) * p.o_ts + h * 64 : nullptr;
-#pragma unroll
-    for (int hf = 0; hf < 2; ++hf) {
-      uint32_t ov[32];
-      if (T > 0) {
-        tmem_ld32(o_addr + hf * 32, ov);
-        tmem_wait1_32(ov);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 32; ++i) ov[i] = 0u;
-      }
-      if constexpr (kPart) {
-        if (row_ok) store_part_o<32>(p.part_o + part_row(p, b, h, u / n_q_tiles, row) * 64 + hf * 32, ov, alpha_pend);
-      } else if (row_ok) {
-#pragma unroll
-        for (int c4 = 0; c4 < 4; ++c4) {
-          uint32_t w[4];
-#pragma unroll
-          for (int e = 0; e < 4; ++e)
-            w[e] = pack2(__uint_as_float(ov[c4 * 8 + e * 2]) * inv, __uint_as_float(ov[c4 * 8 + e * 2 + 1]) * inv);
-          *reinterpret_cast<uint4*>(dst + hf * 32 + c4 * 8) = make_uint4(w[0], w[1], w[2], w[3]);
-        }
-      }
-    }
-    if constexpr (kPart) {
-      if (row_ok) store_part_ml(p.part_ml + part_row(p, b, h, u / n_q_tiles, row) * 2, m_run, l_run);
-    } else if (row_ok && p.lse != nullptr) {
-      p.lse[(static_cast<long long>(b) * p.H + h) * p.Sq + row] = (l_run > 0.f) ? m_run + log2f(l_run) : INFINITY;
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  base += T;
-  }   // item loop
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-  if (threadIdx.x == 0) {
-    if (atomicAdd(&p.items[1], 1u) == gridDim.x - 1) {
-      p.items[0] = 0u;
-      p.items[1] = 0u;
-      __threadfence();
-    }
-  }
-}
-
 // Merge of the key chunks of fk_attn_forward_kv_tc in chunk order (bit-reproducible): one thread per 4 columns of a
 // (trial, head, query) row.  out = sum_c 2^(m_c - M) O_c / sum_c 2^(m_c - M) l_c with M = max_c m_c; a row that saw no
 // key in any chunk gives zeros (lse = +inf, as in the unsplit kernels).
@@ -2658,12 +2221,53 @@ FK_API int fk_attn_aug(const void* o, const void* d_o, const float* lse, float* 
   FK_REQUIRE(o_ts % 8 == 0 && do_ts % 8 == 0 && o_bs % 8 == 0 && do_bs % 8 == 0, "fk_attn_aug: strides must keep 16-byte alignment");
   FK_REQUIRE((reinterpret_cast<uintptr_t>(aug) & 31) == 0, "fk_attn_aug: aug must be 32-byte aligned");
   const long long n = static_cast<long long>(B) * S * H;
-  auto kern = head_dim == 64 ? attn_aug64_kernel : head_dim == 16 ? attn_aug_kernel<16> : attn_aug_kernel<32>;
+  auto kern = head_dim == 64 ? attn_aug_kernel<64> : head_dim == 16 ? attn_aug_kernel<16> : attn_aug_kernel<32>;
   kern<<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(
       static_cast<const __nv_bfloat16*>(o), static_cast<const __nv_bfloat16*>(d_o), lse, delta, static_cast<__nv_bfloat16*>(aug), B, H, S,
       o_bs, o_ts, do_bs, do_ts, 1.f / (scale * 1.4426950408889634f));
   FK_CHECK_LAUNCH();
   fk_count_launch();
+  return FK_OK;
+}
+
+// The forward at head_dim 16, 32 or 64 on `grid` persistent CTAs: tensor maps of q / k / v with the swizzle of the head
+// width, then that width's instantiation; the key-split one when p.n_chunks > 1 (the unsplit kernels take the parameter
+// block without the chunk fields).
+static int attn_fwd_launch(int head_dim, const void* q, const void* k, const void* v, long long q_bs, long long q_ts,
+                           long long k_bs, long long k_ts, long long v_bs, long long v_ts, const FwdKvParams& p,
+                           unsigned grid, cudaStream_t stream) {
+  static bool attr_set_dev[FK_MAX_DEVICES];
+  bool& attr_set = attr_set_dev[fk_device_ordinal()];
+  if (!attr_set) {
+    auto set_smem = [](auto kern, int bytes) {
+      return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess;
+    };
+    if (!set_smem(attn_fwd_tc_kernel<16, false>, FwdSmem<16>::total) || !set_smem(attn_fwd_tc_kernel<16, true>, FwdSmem<16>::total) ||
+        !set_smem(attn_fwd_tc_kernel<32, false>, FwdSmem<32>::total) || !set_smem(attn_fwd_tc_kernel<32, true>, FwdSmem<32>::total) ||
+        !set_smem(attn_fwd_tc_kernel<64, false>, FwdSmem<64>::total) || !set_smem(attn_fwd_tc_kernel<64, true>, FwdSmem<64>::total)) {
+      fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
+      return FK_ERR_CUDA;
+    }
+    attr_set = true;
+  }
+  CUtensorMap mQ, mK, mV;
+  int rc = 0;
+  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : head_dim == 16 ? make_tmap_heads_sw32 : make_tmap_heads_sw64;
+  rc |= make_map(&mQ, q, p.B, p.Sq, p.H, q_bs, q_ts, 128);
+  rc |= make_map(&mK, k, p.B, p.Sk, p.H, k_bs, k_ts, kFwdTileK);
+  rc |= make_map(&mV, v, p.B, p.Sk, p.H, v_bs, v_ts, kFwdTileK);
+  if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
+  const FwdParams& p1 = p;
+  if (p.n_chunks > 1) {
+    if (head_dim == 64) attn_fwd_tc_kernel<64, true><<<grid, kFwdThreads, FwdSmem<64>::total, stream>>>(mQ, mK, mV, p);
+    else if (head_dim == 16) attn_fwd_tc_kernel<16, true><<<grid, kFwdThreads, FwdSmem<16>::total, stream>>>(mQ, mK, mV, p);
+    else attn_fwd_tc_kernel<32, true><<<grid, kFwdThreads, FwdSmem<32>::total, stream>>>(mQ, mK, mV, p);
+  } else {
+    if (head_dim == 64) attn_fwd_tc_kernel<64><<<grid, kFwdThreads, FwdSmem<64>::total, stream>>>(mQ, mK, mV, p1);
+    else if (head_dim == 16) attn_fwd_tc_kernel<16><<<grid, kFwdThreads, FwdSmem<16>::total, stream>>>(mQ, mK, mV, p1);
+    else attn_fwd_tc_kernel<32><<<grid, kFwdThreads, FwdSmem<32>::total, stream>>>(mQ, mK, mV, p1);
+  }
+  FK_CHECK_LAUNCH();
   return FK_OK;
 }
 
@@ -2681,37 +2285,18 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   FK_REQUIRE(qid == nullptr || (qmin && qmax && kmin && kmax), "fk_attn_forward_tc: label ranges missing");
   FK_REQUIRE((S + kFwdTileK - 1) / kFwdTileK <= kMaxTiles && S < (1 << 20), "fk_attn_forward_tc: sequence too long");
   FK_REQUIRE(o_ts % 8 == 0 && o_bs % 8 == 0, "fk_attn_forward_tc: output strides must keep 16-byte alignment");
-  static bool attr_set_dev[FK_MAX_DEVICES];
-  bool& attr_set = attr_set_dev[fk_device_ordinal()];
-  if (!attr_set) {
-    if (cudaFuncSetAttribute(attn_fwd_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc64_kernel<>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
-      fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
-      return FK_ERR_CUDA;
-    }
-    attr_set = true;
-  }
-  CUtensorMap mQ, mK, mV;
-  int rc = 0;
-  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : head_dim == 16 ? make_tmap_heads_sw32 : make_tmap_heads_sw64;
-  rc |= make_map(&mQ, q, B, S, H, q_bs, q_ts, 128);
-  rc |= make_map(&mK, k, B, S, H, k_bs, k_ts, kFwdTileK);
-  rc |= make_map(&mV, v, B, S, H, v_bs, v_ts, kFwdTileK);
-  if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
-  FwdParams p = {};
+  FwdKvParams p = {};
   p.qid = qid; p.kid = kid; p.qmin = qmin; p.qmax = qmax; p.kmin = kmin; p.kmax = kmax;
   p.out = static_cast<__nv_bfloat16*>(out); p.lse = lse; p.o_bs = o_bs; p.o_ts = o_ts;
   p.B = B; p.H = H; p.Sq = S; p.Sk = S; p.scale_log2 = scale * 1.4426950408889634f;
   p.items = counters;
+  p.n_chunks = 1;
   // persistent CTAs: one per SM (or per work item when there are fewer), looping over (256-query block, head, trial) items
   const long long n_items = static_cast<long long>((S + 255) / 256) * H * B;
   FK_REQUIRE(n_items < (1ll << 31), "fk_attn_forward_tc: too many work items");
   const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
-  if (head_dim == 64) attn_fwd_tc64_kernel<><<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
-  else if (head_dim == 16) attn_fwd_tc_kernel<16><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
-  else attn_fwd_tc_kernel<32><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
-  FK_CHECK_LAUNCH();
+  const int rc = attn_fwd_launch(head_dim, q, k, v, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, p, grid, stream);
+  if (rc != FK_OK) return rc;
   fk_count_launch();
   return FK_OK;
 }
@@ -2750,27 +2335,6 @@ FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, vo
   FK_REQUIRE(n_chunks == 1 || (part_o && part_ml), "fk_attn_forward_kv_tc: part_o / part_ml are needed with more than one chunk");
   const long long n_units = static_cast<long long>((Sq + 255) / 256) * n_chunks;
   FK_REQUIRE(n_units * H * B < (1ll << 31), "fk_attn_forward_kv_tc: too many work items");
-  static bool attr_set_dev[FK_MAX_DEVICES];
-  bool& attr_set = attr_set_dev[fk_device_ordinal()];
-  if (!attr_set) {
-    if (cudaFuncSetAttribute(attn_fwd_tc_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc64_kernel<>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc_kernel<16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem::total) != cudaSuccess ||
-        cudaFuncSetAttribute(attn_fwd_tc64_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, FwdSmem64::total) != cudaSuccess) {
-      fk_set_last_error("cudaFuncSetAttribute(max dynamic smem) failed", __FILE__, __LINE__);
-      return FK_ERR_CUDA;
-    }
-    attr_set = true;
-  }
-  CUtensorMap mQ, mK, mV;
-  int rc = 0;
-  auto make_map = head_dim == 64 ? make_tmap_heads_sw128 : head_dim == 16 ? make_tmap_heads_sw32 : make_tmap_heads_sw64;
-  rc |= make_map(&mQ, q, B, Sq, H, q_bs, q_ts, 128);
-  rc |= make_map(&mK, k, B, Sk, H, k_bs, k_ts, kFwdTileK);
-  rc |= make_map(&mV, v, B, Sk, H, v_bs, v_ts, kFwdTileK);
-  if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
   FwdKvParams p = {};
   p.qid = qid; p.kid = kid; p.qmin = qmin; p.qmax = qmax; p.kmin = kmin; p.kmax = kmax;
   p.out = static_cast<__nv_bfloat16*>(out); p.lse = lse; p.o_bs = o_bs; p.o_ts = o_ts;
@@ -2779,20 +2343,13 @@ FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, vo
   p.part_o = part_o; p.part_ml = part_ml; p.n_chunks = n_chunks; p.chunk_tiles = (n_k_tiles + n_chunks - 1) / n_chunks;
   const long long n_items = n_units * H * B;
   const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
+  const int rc = attn_fwd_launch(head_dim, q, k, v, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, p, grid, stream);
+  if (rc != FK_OK) return rc;
   if (n_chunks == 1) {
     // one chunk: the unsplit kernels write O / l and lse themselves
-    const FwdParams& p1 = p;
-    if (head_dim == 64) attn_fwd_tc64_kernel<><<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p1);
-    else if (head_dim == 16) attn_fwd_tc_kernel<16><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p1);
-    else attn_fwd_tc_kernel<32><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p1);
-    FK_CHECK_LAUNCH();
     fk_count_launch();
     return FK_OK;
   }
-  if (head_dim == 64) attn_fwd_tc64_kernel<true><<<grid, kFwdThreads, FwdSmem64::total, stream>>>(mQ, mK, mV, p);
-  else if (head_dim == 16) attn_fwd_tc_kernel<16, true><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
-  else attn_fwd_tc_kernel<32, true><<<grid, kFwdThreads, FwdSmem::total, stream>>>(mQ, mK, mV, p);
-  FK_CHECK_LAUNCH();
   const long long n_threads = static_cast<long long>(B) * H * Sq * (head_dim / 4);
   auto combine = head_dim == 64 ? attn_kv_combine_kernel<64> : head_dim == 16 ? attn_kv_combine_kernel<16> : attn_kv_combine_kernel<32>;
   combine<<<static_cast<unsigned>((n_threads + 255) / 256), 256, 0, stream>>>(part_o, reinterpret_cast<const float2*>(part_ml),

@@ -1,5 +1,5 @@
-"""Self-attention at head_dim 64 on the tcgen05 kernels (attention_tc.cu: attn_fwd_tc64_kernel, attn_bwd_tc64_kernel,
-attn_aug64_kernel), the 64-wide RoPE (fk_rope, GEMM epilogue 4) and the models built with head_dim=64, against fp32
+"""Self-attention at head_dim 64 on the tcgen05 kernels (attention_tc.cu: attn_fwd_tc_kernel<64>, attn_bwd_tc64_kernel,
+attn_aug_kernel<64>), the 64-wide RoPE (fk_rope, GEMM epilogue 4) and the models built with head_dim=64, against fp32
 references on the same bf16-rounded inputs and the head-dim-generic oracle (oracle/brainformer_ref.py)."""
 import math
 
