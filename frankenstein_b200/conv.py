@@ -15,6 +15,10 @@ of a trial beyond its last output step mix in the next trial's padding and are s
   one 2-tap GEMM with N = 2*C_out whose output rows are [y[2v] | y[2v+1]].
 
 All SoundStream convolutions have dilation 1 (vq_brain.py:48-63 builds every ResidualUnit with dilation 1).  No CPU path.
+
+Streaming inference (`causal_conv1d_step`, used by SoundStream.stream) builds the same GEMM rows with the last k - 1 input
+rows of the previous step in place of the causal zero padding (`fk_conv_stream_rows`, which also applies the ELU and the
+ResidualUnit add that feed the convolution), so a step's outputs equal the offline ones row for row.
 """
 from __future__ import annotations
 
@@ -61,6 +65,16 @@ def _w_taps_major(weight: torch.Tensor) -> torch.Tensor:
     out = torch.empty(Cout, k * Cin, device=weight.device, dtype=BF16)
     out.view(Cout, k, Cin).copy_(weight.detach().permute(0, 2, 1))
     return out
+
+
+def _w_transpose_pairs(weight: torch.Tensor, bias):
+    """ConvTranspose1d (k = 4, stride 2) weight [Cin, Cout, 4] -> bf16 [2 Cout, 2 Cin] whose GEMM row v = [x[v-1] | x[v]]
+    gives [y[2v] | y[2v+1]], and the bias doubled to match (fp32 [2 Cout], or None)."""
+    wb = weight.detach().to(BF16)
+    wt = [wb[:, :, j].t() for j in range(4)]                            # [Cout, Cin]
+    w2 = torch.cat([torch.cat([wt[2], wt[0]], dim=1), torch.cat([wt[3], wt[1]], dim=1)], dim=0).contiguous()
+    b2 = None if bias is None else torch.cat([bias.detach().float(), bias.detach().float()])
+    return w2, b2
 
 
 def conv_supported(c_in: int, c_out: int, k: int, stride: int, dilation: int = 1, groups: int = 1) -> bool:
@@ -133,10 +147,7 @@ class _CausalConvTransposeFn(torch.autograd.Function):
         buf = _padded(x, rpt, 1, 2)
         M = B * rpt
         A = _rows(buf, M, 2, 1)                                         # row v = [x[v-1] | x[v]]
-        wb = weight.detach().to(BF16)
-        wt = [wb[:, :, j].t() for j in range(4)]                        # [Cout, Cin]
-        w2 = torch.cat([torch.cat([wt[2], wt[0]], dim=1), torch.cat([wt[3], wt[1]], dim=1)], dim=0).contiguous()   # [2 Cout, 2 Cin]
-        b2 = None if bias is None else torch.cat([bias.detach().float(), bias.detach().float()])
+        w2, b2 = _w_transpose_pairs(weight, bias)
         y = gemm.gemm_nt(A, w2, b2, name="convT_fwd")                   # row v = [y[2v] | y[2v+1]]
         ctx.save_for_backward(buf, weight)
         ctx.meta = (B, T, Cin, Cout, rpt, M, bias is not None, x.dtype)
@@ -164,6 +175,39 @@ class _CausalConvTransposeFn(torch.autograd.Function):
             if dx.dtype != x_dtype:
                 dx = dx.to(x_dtype)
         return dx, dw, db
+
+
+def _row_strides(x3: torch.Tensor):
+    """(batch, token) strides in elements of a [B, T, C] operand; with B == 1 the batch stride is never used."""
+    if x3.stride(2) != 1:
+        raise FkError("streamed convolution operands must have contiguous channels")
+    return (x3.stride(0), x3.stride(1)) if x3.shape[0] > 1 else (x3.shape[1] * x3.stride(1), x3.stride(1))
+
+
+def causal_conv1d_step(x: torch.Tensor, r, elu: bool, hist_in, hist_out, w2: torch.Tensor, bias, taps: int, stride: int = 1):
+    """One step of a streamed causal convolution (inference only): x [B, n, Cin] new rows (fp32 or bf16, row-strided), r
+    (None or bf16 [B, n, Cin]) a residual added to x, `elu` the activation applied to x + r, hist_in / hist_out bf16
+    [B, taps - 1, Cin] the last input rows of the previous step / of this one (None when taps == 1), w2 [Cout, taps * Cin]
+    bf16 (`_w_taps_major`, or `_w_transpose_pairs` for the transposed convolution as 2 taps), bias fp32 or None.
+    Returns (y bf16 [B, n / stride, Cout], the bf16 input rows act(x + r) [B, n, Cin] as a view of the GEMM operand).
+
+    The GEMM rows are those of `_CausalConvFn.forward`, with the history in place of the causal zero padding."""
+    B, n, Cin = x.shape
+    h, s = taps - 1, stride
+    if n % s != 0:
+        raise FkError(f"causal_conv1d_step: {n} rows is not a multiple of the stride {s}")
+    if (hist_in is None) != (h == 0) or (h > 0 and (hist_in.shape != (B, h, Cin) or hist_out.shape != (B, h, Cin))):
+        raise FkError(f"causal_conv1d_step: the history must be [{B}, {h}, {Cin}]")
+    rpt = -(-(n + h) // s) * s                                          # rows per trial, a multiple of the stride
+    total = B * rpt + taps
+    buf = torch.empty(total, Cin, device=x.device, dtype=BF16)
+    rs = (0, 0) if r is None else _row_strides(r)
+    check(lib().fk_conv_stream_rows(ptr(x), 0 if x.dtype == torch.float32 else 1, *_row_strides(x), ptr(r), *rs,
+                                    ptr(hist_in), ptr(hist_out), B, n, h, Cin, int(elu), ptr(buf), rpt, total, stream()),
+          "fk_conv_stream_rows")
+    M = B * rpt // s
+    y = gemm.gemm_nt(_rows(buf, M, taps, s), w2, bias, name="conv_stream")
+    return y.view(B, rpt // s, w2.shape[0])[:, :n // s], buf[:B * rpt].view(B, rpt, Cin)[:, h:h + n]
 
 
 def causal_conv1d_cl(x: torch.Tensor, weight: torch.Tensor, bias, stride: int = 1) -> torch.Tensor:

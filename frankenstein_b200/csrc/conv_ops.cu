@@ -6,8 +6,12 @@
 //                           the data (replaces a memset + a generic strided torch copy that ran at 1.5 TB/s)
 //   colsum_partials_kernel  column sums of a bf16 [M, N] matrix (bias gradient = dY^T 1): per-CTA partials [nb, N] in a fixed
 //                           order; the caller reduces them with fk_norm_reduce_partials (deterministic)
+//   stream_rows_kernel      the GEMM input rows of one STREAMED causal convolution (SoundStream.stream): per trial the h
+//                           history rows of the previous step, then act(x + r) for the n new rows (the ELU between layers
+//                           and the ResidualUnit's `x + layers(x)`, rounded as the offline bf16 ops round), then zeros;
+//                           also writes the next step's history (the last h rows of [history | new rows])
 //
-// Both HBM-bound: 16-byte accesses, persistent grids of 148 * k CTAs.
+// All HBM-bound: 16-byte accesses, persistent grids of 148 * k CTAs.
 #include "common.cuh"
 #include "fk_b200.h"
 
@@ -40,6 +44,75 @@ pad_rows_kernel(const void* __restrict__ x_, long long sb, long long st, long lo
       }
     }
     *reinterpret_cast<uint4*>(out + r * (C8 * 8ll) + c) = v;
+  }
+}
+
+__device__ __forceinline__ void load8_f32(const void* base, int f32, long long off, float (&v)[8]) {
+  if (f32) {
+    const float* p = static_cast<const float*>(base) + off;
+    const float4 a = *reinterpret_cast<const float4*>(p), d = *reinterpret_cast<const float4*>(p + 4);
+    v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = d.x; v[5] = d.y; v[6] = d.z; v[7] = d.w;
+  } else {
+    const uint4 q = *reinterpret_cast<const uint4*>(static_cast<const __nv_bfloat16*>(base) + off);
+    const uint32_t w[4] = {q.x, q.y, q.z, q.w};
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      v[2 * j] = __uint_as_float(w[j] << 16);
+      v[2 * j + 1] = __uint_as_float(w[j] & 0xffff0000u);
+    }
+  }
+}
+
+// new row t of trial b: act(x + r) as bf16.  With r the sum is rounded to bf16 first (torch's bf16 add); ELU (alpha 1) is
+// torch's formula, x > 0 ? x : expm1(x) in fp32, so the row equals F.elu of the offline bf16 tensor bit for bit.
+__device__ __forceinline__ uint4 stream_new_row(const void* x, int x_f32, long long x_sb, long long x_st,
+                                                const __nv_bfloat16* r, long long r_sb, long long r_st, int elu, long long b,
+                                                long long t, int c) {
+  float v[8];
+  load8_f32(x, x_f32, b * x_sb + t * x_st + c, v);
+  if (r != nullptr) {
+    float a[8];
+    load8_f32(r, 0, b * r_sb + t * r_st + c, a);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] = __bfloat162float(__float2bfloat16_rn(v[j] + a[j]));
+  }
+  if (elu) {
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] = v[j] > 0.f ? v[j] : expm1f(v[j]);
+  }
+  return make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+}
+
+// one thread = 8 channels of one row; items [0, total_rows * C8) are rows of out, the next B * h * C8 rows of hist_out
+__global__ void __launch_bounds__(256)
+stream_rows_kernel(const void* __restrict__ x, int x_f32, long long x_sb, long long x_st, const __nv_bfloat16* __restrict__ r,
+                   long long r_sb, long long r_st, const __nv_bfloat16* __restrict__ hist_in, __nv_bfloat16* __restrict__ hist_out,
+                   long long B, long long n, int h, int C8, int elu, long long rpt, long long total_rows,
+                   __nv_bfloat16* __restrict__ out) {
+  const long long n_out = total_rows * C8, n_all = n_out + B * h * C8;
+  const long long C = C8 * 8ll;
+  for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_all;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    long long row, b, t;                       // t = row of trial b in [history | new rows]
+    __nv_bfloat16* dst;
+    if (i < n_out) {
+      row = i / C8;
+      b = row / rpt;
+      t = row - b * rpt;
+      dst = out + row * C;
+    } else {
+      row = (i - n_out) / C8;                  // hist_out row (b, j) = row b * h + j takes row n + j of [history | new rows]
+      b = row / h;
+      t = n + (row - b * h);
+      dst = hist_out + row * C;
+    }
+    const int c = static_cast<int>(i % C8) * 8;
+    uint4 v = make_uint4(0u, 0u, 0u, 0u);
+    if (b < B && t < h)
+      v = *reinterpret_cast<const uint4*>(hist_in + (b * h + t) * C + c);
+    else if (b < B && t < h + n)
+      v = stream_new_row(x, x_f32, x_sb, x_st, r, r_sb, r_st, elu, b, t - h, c);
+    *reinterpret_cast<uint4*>(dst + c) = v;
   }
 }
 
@@ -103,6 +176,32 @@ FK_API int fk_pad_rows(const void* x, int x_dtype, long long B, long long T, int
   else
     pad_rows_kernel<false><<<static_cast<unsigned>(blocks), 256, 0, stream>>>(x, stride_b, stride_t, B, T, C / 8, rows_per_trial, left, total_rows,
                                                                             static_cast<__nv_bfloat16*>(out));
+  FK_CHECK_LAUNCH();
+  fk_count_launch();
+  return FK_OK;
+}
+
+FK_API int fk_conv_stream_rows(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r, long long r_sb,
+                               long long r_st, const void* hist_in, void* hist_out, long long B, long long n, int h, int C,
+                               int act, void* out, long long rows_per_trial, long long total_rows, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  FK_REQUIRE(x && out && B > 0 && n > 0 && h >= 0 && C > 0 && C % 8 == 0, "fk_conv_stream_rows: bad argument (n >= 1, C % 8 == 0)");
+  FK_REQUIRE(x_dtype == 0 || x_dtype == 1, "fk_conv_stream_rows: x must be f32 (0) or bf16 (1)");
+  FK_REQUIRE(act == 0 || act == 1, "fk_conv_stream_rows: act must be 0 (none) or 1 (ELU)");
+  FK_REQUIRE(h == 0 || (hist_in && hist_out && hist_in != hist_out), "fk_conv_stream_rows: h > 0 needs two distinct history buffers");
+  FK_REQUIRE(rows_per_trial >= h + n && total_rows >= B * rows_per_trial, "fk_conv_stream_rows: the row layout does not hold history and new rows");
+  FK_REQUIRE(x_sb % 8 == 0 && x_st % 8 == 0 && x_st >= C && (!r || (r_sb % 8 == 0 && r_st % 8 == 0 && r_st >= C)),
+             "fk_conv_stream_rows: row strides must be multiples of 8 elements and >= C");
+  FK_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(r) | reinterpret_cast<uintptr_t>(hist_in) |
+               reinterpret_cast<uintptr_t>(hist_out) | reinterpret_cast<uintptr_t>(out)) & 15) == 0,
+             "fk_conv_stream_rows: 16-byte aligned buffers");
+  const long long items = (total_rows + B * h) * (C / 8);
+  long long blocks = (items + 255) / 256;
+  const long long cap = static_cast<long long>(fk_sm_count()) * 16;
+  if (blocks > cap) blocks = cap;
+  stream_rows_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(
+      x, x_dtype == 0, x_sb, x_st, static_cast<const __nv_bfloat16*>(r), r_sb, r_st, static_cast<const __nv_bfloat16*>(hist_in),
+      static_cast<__nv_bfloat16*>(hist_out), B, n, h, C / 8, act, rows_per_trial, total_rows, static_cast<__nv_bfloat16*>(out));
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;

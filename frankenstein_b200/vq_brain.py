@@ -14,6 +14,9 @@ underneath:
   GEMMs as implicit GEMMs (``conv.py``: ``[B, T, C]`` activations, im2col rows are overlapping views of the padded
   signal) whenever every layer's channel counts are multiples of 64; other widths, and ``FK_CONV=cudnn``, use cuDNN's
   NHWC kernels on a 4-D view (no permute copies either way).
+
+* ``SoundStream.stream`` (no reference counterpart) tokenizes a recording online, 4 bins at a time, on the same implicit
+  GEMMs with a per-layer history of input rows (``TokenizerStream``).
 """
 from __future__ import annotations
 
@@ -25,7 +28,7 @@ import torch.nn.functional as F
 
 from . import _lib, conv, gemm
 from ._lib import DTYPE_CODE, FkError, check, counters, lib, on_tensor_device, ptr, require_cuda, require_device, stream
-from .vector_quantize import VectorQuantize
+from .vector_quantize import VectorQuantize, finish, prepare_codebook, prepare_input, search
 
 
 # "own" (default): the conv stacks run channels-last on the library's tcgen05 GEMMs (conv.py: im2col rows are overlapping
@@ -303,3 +306,197 @@ class SoundStream(nn.Module):
 
     def calculate_perp(self, indices):
         return perplexity(indices, self.codebook_size)
+
+    def stream(self, batch_size: int, reconstruct: bool = False) -> "TokenizerStream":
+        """Online tokenization: feed a recording 4 bins at a time (or any multiple of 4) with `TokenizerStream.step(x)` and
+        get the codes of the new bins only, at a cost that does not grow with the length of the stream.
+
+        Every layer of the stacks is causal -- CausalConv1d pads on the left only and CausalConvTranspose1d trims its
+        trailing samples (models/vq_brain.py:22-45) -- so the output for bin t never changes once bin t has arrived, and
+        each convolution needs only its last k - 1 input rows (1 for the transposed convolution) from earlier steps.  The
+        encoder's receptive field is 44 bins: token t reads bins 4t - 40 ... 4t + 3.
+
+        The stream converts every weight and the codebook once, here: it tokenizes with the model as it is now.  After
+        training or loading new weights, create a new stream."""
+        return TokenizerStream(self, batch_size, reconstruct)
+
+
+# ------------------------------------------------------------------------------------------------
+# streaming inference (SoundStream.stream)
+# ------------------------------------------------------------------------------------------------
+class _PlanEntry:
+    """One convolution of a flattened stack: its input rows are act(x + r), x = the previous entry's output, r = the input
+    rows of entry `res` (a ResidualUnit's `x + layers(x)`) or none; `hist` = taps - 1 input rows carried between steps."""
+    __slots__ = ("conv", "taps", "hist", "stride", "transposed", "elu", "res")
+
+    def __init__(self, conv_, taps, stride, transposed, elu, res):
+        self.conv, self.taps, self.hist, self.stride = conv_, taps, taps - 1, stride
+        self.transposed, self.elu, self.res = transposed, elu, res
+
+
+def _stream_plan(stack: nn.Module):
+    """Flatten an Encoder / Decoder into its convolutions in order ([_PlanEntry]), checking every module against the
+    structure the stream reproduces: FkError for anything else (other module types or subclasses, other activations, an
+    ELU that does not feed a convolution, dilated / grouped / padded convolutions, a ResidualUnit that changes the rate or
+    the width)."""
+    if type(stack) not in (Encoder, Decoder):
+        raise FkError(f"SoundStream.stream: cannot stream a {type(stack).__name__}")
+    plan = []
+    pending = {"elu": False, "res": None}
+
+    def conv_entry(m, taps, stride, transposed):
+        if m.dilation[0] != 1 or m.groups != 1 or m.padding[0] != 0 or m.padding_mode != "zeros":
+            raise FkError(f"SoundStream.stream: {type(m).__name__} with dilation, groups or padding cannot stream")
+        plan.append(_PlanEntry(m, taps, stride, transposed, pending["elu"], pending["res"]))
+        pending["elu"], pending["res"] = False, None
+
+    def walk(seq):
+        if type(seq) is not nn.Sequential:
+            raise FkError(f"SoundStream.stream: expected an nn.Sequential of layers, got {type(seq).__name__}")
+        for m in seq:
+            t = type(m)
+            if t is nn.ELU:
+                if m.alpha != 1.0 or pending["elu"] or not plan:
+                    raise FkError("SoundStream.stream: an ELU (alpha 1) must follow a layer and feed a convolution")
+                pending["elu"] = True
+            elif t is CausalConv1d:
+                k, s = m.kernel_size[0], m.stride[0]
+                if not (s == 1 or (s == 2 and k == 4)):
+                    raise FkError(f"SoundStream.stream: CausalConv1d k = {k}, stride {s} cannot stream")
+                conv_entry(m, k, s, False)
+            elif t is CausalConvTranspose1d:
+                if m.kernel_size[0] != 4 or m.stride[0] != 2 or m.output_padding[0] != 0:
+                    raise FkError("SoundStream.stream: CausalConvTranspose1d must be k = 4, stride 2")
+                conv_entry(m, 2, 1, True)          # two taps of [x[v-1] | x[v]], output rows [y[2v] | y[2v+1]]
+            elif t is _PointwiseConv1d:
+                if m.kernel_size[0] != 1 or m.stride[0] != 1:
+                    raise FkError("SoundStream.stream: a 1 x 1 convolution must have stride 1")
+                conv_entry(m, 1, 1, False)
+            elif t is ResidualUnit:
+                start = len(plan)               # the unit's input = the input rows of its first convolution
+                walk(m.layers)
+                inner = plan[start:]
+                if (not inner or pending["elu"] or pending["res"] is not None
+                        or any(e.stride != 1 or e.transposed for e in inner)
+                        or inner[0].conv.in_channels != inner[-1].conv.out_channels):
+                    raise FkError("SoundStream.stream: a ResidualUnit must keep the rate and width and end in a convolution")
+                pending["res"] = start
+            elif t in (EncoderBlock, DecoderBlock):
+                walk(m.layers)
+            else:
+                raise FkError(f"SoundStream.stream: cannot stream a {t.__name__}")
+
+    walk(stack.layers)
+    if not plan or pending["elu"] or pending["res"] is not None:
+        raise FkError("SoundStream.stream: the stack must end in a convolution")
+    return plan
+
+
+class _StreamLayer:
+    """A plan entry with its weights converted once (bf16 GEMM layout, fp32 bias) and its two history buffers."""
+
+    def __init__(self, e: _PlanEntry, batch_size: int, device):
+        m = e.conv
+        self.e = e
+        if e.transposed:
+            self.w2, self.bias = conv._w_transpose_pairs(m.weight, m.bias)
+        else:
+            self.w2 = conv._w_taps_major(m.weight)
+            self.bias = None if m.bias is None else m.bias.detach().float().clone()
+        self.hist = (torch.zeros(2, batch_size, e.hist, m.in_channels, device=device, dtype=torch.bfloat16)
+                     if e.hist else None)
+
+
+class TokenizerStream:
+    """Streaming state of a `SoundStream` (from `SoundStream.stream`): per convolution of the encoder (and, with
+    `reconstruct`, of the decoder) the last taps - 1 input rows in bf16, two buffers each -- a step reads one and writes
+    the other, and the roles swap only once the whole step has been enqueued, so a rejected step leaves the state as it
+    was.  Weights and codebook are a snapshot taken at creation."""
+
+    def __init__(self, model: SoundStream, batch_size: int, reconstruct: bool = False):
+        if batch_size < 1:
+            raise FkError("TokenizerStream: batch_size must be positive")
+        stacks = [model.encoder] + ([model.decoder] if reconstruct else [])
+        plans = [_stream_plan(s) for s in stacks]
+        dev = next(model.parameters()).device
+        if dev.type != "cuda":
+            raise FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
+        if not all(s._own_ok() for s in stacks):
+            raise FkError("TokenizerStream: a convolution width is outside the library's implicit GEMMs (cuDNN-only widths "
+                          "cannot stream)")
+        vq = model.quantizer
+        if not vq._is_initted():
+            raise FkError("TokenizerStream: the codebook is not initialised (k-means on a stream chunk is meaningless); "
+                          "train the model or load a checkpoint first")
+        self.batch_size, self.reconstruct, self.device = batch_size, bool(reconstruct), dev
+        self.n_electrodes = model.encoder.layers[0].in_channels
+        self.use_cosine = vq.use_cosine_sim
+        with torch.cuda.device(dev):
+            self._layers = [[_StreamLayer(e, batch_size, dev) for e in p] for p in plans]
+            self._embed = vq.codebook.detach().float().clone().contiguous()
+            self._cb, self._c2pad = prepare_codebook(self._embed, self.use_cosine)
+        self._cur = 0
+        self._length = 0
+
+    @property
+    def length(self) -> int:
+        """bins consumed so far."""
+        return self._length
+
+    def reset(self) -> None:
+        """Start a new recording: the histories become the causal zero padding again."""
+        for layers in self._layers:
+            for L in layers:
+                if L.hist is not None:
+                    L.hist.zero_()
+        self._length = 0
+
+    def _run(self, layers, x):
+        inputs = []
+        cur = self._cur
+        for L in layers:
+            e = L.e
+            r = None if e.res is None else inputs[e.res]
+            h_in, h_out = (None, None) if L.hist is None else (L.hist[cur], L.hist[cur ^ 1])
+            y, rows = conv.causal_conv1d_step(x, r, e.elu, h_in, h_out, L.w2, L.bias, e.taps, e.stride)
+            if e.transposed:
+                y = y.reshape(y.shape[0], 2 * y.shape[1], y.shape[2] // 2)
+            inputs.append(rows)
+            x = y
+        return x
+
+    @torch.no_grad()
+    def step(self, x: torch.Tensor):
+        """x [B, 4n, n_electrodes] (fp32 or bf16, n >= 1) -> (indices [B, n] int64, quantized [B, n, D] fp32), plus, with
+        `reconstruct`, the decoder output o [B, 4n, n_electrodes] (bf16) of the new bins.  The quantizer runs with eval
+        semantics whatever the model's mode (no k-means, no EMA update).  Raises FkError, leaving the state as it was, on
+        a bin count that is not a positive multiple of 4, a batch or channel count that does not match the stream, a CPU
+        tensor or a dtype other than fp32 / bf16."""
+        B, E = self.batch_size, self.n_electrodes
+        if not isinstance(x, torch.Tensor) or x.dim() != 3 or x.shape[0] != B or x.shape[2] != E:
+            raise FkError(f"TokenizerStream.step: expected [{B}, 4n, {E}], got "
+                          f"{tuple(x.shape) if isinstance(x, torch.Tensor) else type(x).__name__}")
+        T = x.shape[1]
+        if T < 4 or T % 4 != 0:
+            raise FkError(f"TokenizerStream.step: {T} bins is not a positive multiple of 4")
+        if not x.is_cuda:
+            raise FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
+        if x.device != self.device:
+            raise FkError(f"TokenizerStream.step: the stream lives on {self.device}, x on {x.device}")
+        if x.dtype not in (torch.float32, torch.bfloat16):
+            raise FkError(f"TokenizerStream.step: x must be fp32 or bf16, got {x.dtype}")
+        if x.stride(2) != 1 or x.stride(0) % 8 or x.stride(1) % 8 or x.data_ptr() % 16:
+            x = x.contiguous()
+        n = T // 4
+        with torch.cuda.device(self.device):
+            e = self._run(self._layers[0], x.detach())
+            D = e.shape[2]
+            xn, xb, _ = prepare_input(e.reshape(B * n, D).contiguous(), self.use_cosine)
+            cand_val, cand_idx = search(xb, self._cb, self._c2pad, self._embed.shape[0], self.use_cosine)
+            indices, quantized, _ = finish(xn, self._embed, cand_val, cand_idx, self.use_cosine, False, 0.0)
+            out = (indices.view(B, n), quantized.view(B, n, D))
+            if self.reconstruct:
+                out = out + (self._run(self._layers[1], out[1]),)
+        self._cur ^= 1
+        self._length += T
+        return out

@@ -128,6 +128,16 @@ int fk_norm_backward(const void* x, int x_dtype, const void* g, int g_dtype, con
  * elements (multiples of 8). */
 int fk_pad_rows(const void* x, int x_dtype, long long B, long long T, int C, long long stride_b, long long stride_t,
                 void* out, long long rows_per_trial, long long left, long long total_rows, void* stream);
+/* The GEMM input rows of one streamed causal convolution (SoundStream.stream; models/vq_brain.py:22-63), fk_pad_rows' layout:
+ * out [(total_rows), C] bf16, trial b's rows at out[b * rows_per_trial ...] are hist_in[b] (h rows), then act(x[b] + r[b])
+ * (n rows), then zeros up to the next trial and in the slack rows.  x [B, n, C]: f32 (0) or bf16 (1); r (nullable) bf16
+ * [B, n, C], the ResidualUnit input added to its 1x1 convolution's output; x + r is rounded to bf16, then act: 0 = none,
+ * 1 = ELU (alpha 1, fp32, torch's x > 0 ? x : expm1(x)), then bf16.  Strides in elements (multiples of 8, token strides
+ * >= C), channels contiguous.  hist_in / hist_out: bf16 [B, h, C], distinct buffers (nullable when h == 0); hist_out[b]
+ * = the last h rows of [hist_in[b] | act(x[b] + r[b])], also when n < h. */
+int fk_conv_stream_rows(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r, long long r_sb,
+                        long long r_st, const void* hist_in, void* hist_out, long long B, long long n, int h, int C,
+                        int act, void* out, long long rows_per_trial, long long total_rows, void* stream);
 /* column sums of a bf16 [M, N] matrix (row stride ld): part [fk_colsum_grid(), N] fp32 per-CTA partials in a fixed order;
  * reduce them with fk_norm_reduce_partials(part, NULL, fk_colsum_grid(), N, out, NULL).  Bias gradient of nn.Linear /
  * nn.Conv1d (sum of dY over tokens). */
