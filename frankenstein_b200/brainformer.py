@@ -422,7 +422,12 @@ class EncoderStream:
     """Streaming state of an `Encoder` (from `Encoder.stream`): per layer a bf16 k | v cache [B, block_size, 2 * inner],
     allocated once.  Positions start at 0 when the stream starts; the offline `Encoder.forward` on a partial window uses
     the last positions of the window instead, a uniform shift that RoPE scores do not see, so the two agree up to bf16
-    rounding."""
+    rounding.
+
+    Each batch row is a session of its own: `reset(rows)` restarts only the given rows, and from then on the rows sit at
+    different positions (`lengths`).  A step still advances every row by the same whole patches; each row continues at its
+    own position, and its outputs depend on its own session only.  Until the first per-row reset (and again after
+    `reset()`) every row is at one position and a step runs the lockstep path."""
 
     def __init__(self, encoder: Encoder, batch_size: int, out_dtype=torch.float32):
         cfg = encoder.config
@@ -438,23 +443,64 @@ class EncoderStream:
         self.n_heads = cfg.n_heads
         self.inner = cfg.n_heads * cfg.head_dim
         dev = encoder.device
-        self.caches = [torch.empty(batch_size, encoder.block_size, 2 * self.inner, device=dev, dtype=BF16)
+        # zeroed: a row's partly visible key tile multiplies P = 0 by the V rows past its length (fk_attn_forward_kv_tc)
+        self.caches = [torch.zeros(batch_size, encoder.block_size, 2 * self.inner, device=dev, dtype=BF16)
                        for _ in encoder.transformer.h]
-        self._length = 0
+        self._lengths = [0] * batch_size
+        # per-row sessions: device lengths in two buffers (a step reads one and writes the other, the roles swap once the
+        # step is enqueued) and the key labels of the whole window, shared by every row and built on first use
+        self._ragged = False
+        self._len_dev = torch.zeros(2, batch_size, device=dev, dtype=torch.int32)
+        self._cur = 0
+        self._keys = None
+
+    @property
+    def lengths(self) -> list:
+        """tokens cached so far, per row (host values: reading them does not wait for the device)."""
+        return list(self._lengths)
 
     @property
     def length(self) -> int:
-        """tokens cached so far (a multiple of n_electrodes)."""
-        return self._length
+        """tokens cached so far (a multiple of n_electrodes), while every row is at the same position."""
+        return ops.stream_length(self._lengths, "EncoderStream.length")
 
-    def reset(self) -> None:
-        self._length = 0
+    def reset(self, rows=None) -> None:
+        """Restart every row (rows None) or only the given row indices; FkError, changing nothing, for an index outside
+        the batch or a duplicate."""
+        if rows is None:
+            self._lengths = [0] * self.batch_size
+            self._ragged = False
+            return
+        idx = ops.stream_rows(rows, self.batch_size, "EncoderStream.reset")
+        if not idx:
+            return
+        cur = self._len_dev[self._cur]
+        if not self._ragged:
+            cur.fill_(self._lengths[0])               # the lockstep path keeps the lengths on the host only
+            self._ragged = True
+        cur.index_fill_(0, torch.tensor(idx, dtype=torch.long).to(cur.device), 0)
+        for r in idx:
+            self._lengths[r] = 0
+
+    def _key_labels(self):
+        """block-causal labels of every cache position, [B, block_size], with their tile ranges (built once)."""
+        if self._keys is None:
+            enc = self.encoder
+            kid = torch.arange(enc.block_size, device=self._len_dev.device, dtype=torch.int32) // enc.n_electrodes
+            self._keys = LabelMask(kid[None].expand(self.batch_size, -1).contiguous())
+        return self._keys
 
     @torch.no_grad()
     def step(self, x: torch.Tensor) -> torch.Tensor:
         """x [B, n * patch_size, n_electrodes] (n >= 1 whole patches) -> final-LayerNorm outputs of the n * n_electrodes
         new tokens, [B, n * n_electrodes, dim] in `out_dtype`.  Raises FkError, leaving the state as it was, on a partial
-        patch, a batch or electrode count that does not match, or a step past the window (block_size tokens)."""
+        patch, a batch or electrode count that does not match, or a step that takes any row past the window (block_size
+        tokens)."""
+        return self._step(x)[0]
+
+    def _step(self, x):
+        """step(x) and, for rows at different positions, the flat cache rows b * block_size + position that the new tokens
+        took (int64 [B * n_new]; None on the lockstep path)."""
         enc = self.encoder
         E, p = enc.n_electrodes, enc.patch_size
         if x.dim() != 3 or x.shape[0] != self.batch_size or x.shape[2] != E:
@@ -463,9 +509,10 @@ class EncoderStream:
         if T < p or T % p != 0:
             raise ops.FkError(f"EncoderStream.step: {T} bins is not a positive multiple of patch_size {p}")
         n_new = (T // p) * E
-        L = self._length
-        if L + n_new > enc.block_size:
-            raise ops.FkError(f"EncoderStream.step: {L} cached + {n_new} new tokens exceed the window of {enc.block_size}")
+        over = [b for b, n in enumerate(self._lengths) if n + n_new > enc.block_size]
+        if over:
+            raise ops.FkError(f"EncoderStream.step: {n_new} new tokens take rows {over} (at {[self._lengths[b] for b in over]} "
+                              f"tokens) past the window of {enc.block_size}")
         if not x.is_cuda:
             raise ops.FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
         w_emb = enc.transformer.emb
@@ -474,13 +521,27 @@ class EncoderStream:
         else:
             h_delta = enc.embed(enc.to_patches(x))
         emb = enc.space_embedding.float().repeat(1, T // p, 1)        # [1, n_new, dim]; added inside the first add+LayerNorm
-        Sk = L + n_new
-        mask = None
-        if T > p:
-            # several patches in one step: block-causal among the new tokens (with one patch every cached key is visible)
-            blk = torch.arange(Sk, device=x.device, dtype=torch.int32) // E
-            mask = LabelMask(blk[L:][None].expand(B, n_new).contiguous(), blk[None].expand(B, Sk).contiguous())
-        rope = RopeSpec(enc.rope_table(), None, L)
+        rows = None
+        if not self._ragged:
+            L = self._lengths[0]
+            Sk = L + n_new
+            mask = None
+            if T > p:
+                # several patches in one step: block-causal among the new tokens (with one patch every cached key is visible)
+                blk = torch.arange(Sk, device=x.device, dtype=torch.int32) // E
+                mask = LabelMask(blk[L:][None].expand(B, n_new).contiguous(), blk[None].expand(B, Sk).contiguous())
+            rope = RopeSpec(enc.rope_table(), None, L)
+        else:
+            # rows at different positions: one launch gives each row's query labels, RoPE positions and cache rows.  The
+            # attention runs over the whole window with fixed key labels, so its key chunks do not depend on the other
+            # rows' lengths; cached positions at or past a row's length belong to later time patches and are masked
+            # (whole tiles of them are skipped by the tile ranges).
+            keys = self._key_labels()
+            qid, qmin, qmax, pos, rows = ops.stream_positions(self._len_dev[self._cur], self._len_dev[self._cur ^ 1], n_new, E,
+                                                              enc.block_size)
+            mask = LabelMask.from_ranges(qid, keys.qid, qmin, qmax, keys.qmin, keys.qmax)
+            rope = RopeSpec(enc.rope_table(), pos, 0)
+            Sk = enc.block_size
         blocks = enc.transformer.h
         H, inner = self.n_heads, self.inner
         l0 = blocks[0].ln_1
@@ -495,7 +556,10 @@ class EncoderStream:
                 ops._rope_inplace(q4[:, :, 0], rope, False)
                 ops._rope_inplace(q4[:, :, 1], rope, False)
             cache = self.caches[i]
-            cache[:, L:Sk].copy_(qkv[..., inner:])
+            if rows is None:
+                cache[:, L:Sk].copy_(qkv[..., inner:])
+            else:
+                cache.view(-1, 2 * inner).index_copy_(0, rows, qkv[..., inner:].reshape(-1, 2 * inner))
             res = ops.attention_kv(qkv[..., :inner], cache[:, :Sk, :inner], cache[:, :Sk, inner:], H, mask)
             a = _linear_bf16(res, at.project.weight)
             h, y = ops.add_layer_norm(h, a, blk_.ln_2.weight, blk_.ln_2.bias, blk_.ln_2.eps)
@@ -503,8 +567,10 @@ class EncoderStream:
             nxt = blocks[i + 1].ln_1 if i + 1 < len(blocks) else enc.transformer.ln_f
             h, y = ops.add_layer_norm(h, m, nxt.weight, nxt.bias, nxt.eps,
                                       BF16 if i + 1 < len(blocks) else self.out_dtype)
-        self._length = Sk
-        return y
+        if self._ragged:
+            self._cur ^= 1
+        self._lengths = [n + n_new for n in self._lengths]
+        return y, rows
 
 
 class MAE(nn.Module):
@@ -645,7 +711,9 @@ class BrainFormer(nn.Module):
 class BrainFormerStream:
     """Streaming state of a `BrainFormer`: an `EncoderStream` plus, per CrossBlock, a bf16 cache of the k | v projection
     of the context tokens [B, block_size, 2 * inner].  The encoder is block-causal, so the context tokens never change
-    once produced: a step projects only the new ones, then runs the perceiver over the whole cache in place."""
+    once produced: a step projects only the new ones, then runs the perceiver over the whole cache in place.  Batch rows
+    are sessions of their own as in `EncoderStream`: after `reset(rows)` the perceiver of each row reads that row's own
+    context tokens only."""
 
     def __init__(self, model: BrainFormer, batch_size: int):
         cfg = model.config
@@ -655,31 +723,43 @@ class BrainFormerStream:
         self.encoder_stream = model.encoder.stream(batch_size, out_dtype=BF16)
         inner = cfg.n_heads * cfg.head_dim
         block = model.encoder.block_size
-        self.kv = [torch.empty(batch_size, block, 2 * inner, device=model.device, dtype=BF16) for _ in model.perceiver.h]
+        self.kv = [torch.zeros(batch_size, block, 2 * inner, device=model.device, dtype=BF16) for _ in model.perceiver.h]
+
+    @property
+    def lengths(self) -> list:
+        """context tokens cached so far, per row."""
+        return self.encoder_stream.lengths
 
     @property
     def length(self) -> int:
-        """context tokens cached so far."""
+        """context tokens cached so far, while every row is at the same position."""
         return self.encoder_stream.length
 
-    def reset(self) -> None:
-        self.encoder_stream.reset()
+    def reset(self, rows=None) -> None:
+        """Restart every row (rows None) or only the given row indices (see `EncoderStream.reset`)."""
+        self.encoder_stream.reset(rows)
 
     @torch.no_grad()
     def step(self, x: torch.Tensor) -> torch.Tensor:
         """x [B, n * patch_size, n_electrodes] -> pred [B, n_output_tokens, output_dim] fp32 (errors as EncoderStream.step)."""
         m = self.model
-        L0 = self.encoder_stream.length
-        context = self.encoder_stream.step(x)                     # [B, n_new, dim] bf16
-        L = self.encoder_stream.length
+        es = self.encoder_stream
+        L0 = es.lengths[0]
+        context, rows = es._step(x)                                # [B, n_new, dim] bf16
+        L = max(es.lengths)
+        k_len = None if rows is None else es._len_dev[es._cur]     # the rows' lengths after this step
         for cb, kv in zip(m.perceiver.h, self.kv):
             ca = cb.cross_attn
-            kv[:, L0:L].copy_(_linear_bf16(context, torch.cat([ca.kw.weight, ca.vw.weight], dim=0)))
+            proj = _linear_bf16(context, torch.cat([ca.kw.weight, ca.vw.weight], dim=0))
+            if rows is None:
+                kv[:, L0:L].copy_(proj)
+            else:
+                kv.view(-1, kv.shape[-1]).index_copy_(0, rows, proj.reshape(-1, kv.shape[-1]))
         h = m.learnable_queries.expand(x.shape[0], m.n_output_tokens, -1)
         for cb, kv in zip(m.perceiver.h, self.kv):
             ca = cb.cross_attn
             q = _linear_bf16(cb.ln_1(h), ca.qw.weight)
-            res = ops.small_attention_kv_cached(q, kv[:, :L], ca.n_heads)
+            res = ops.small_attention_kv_cached(q, kv[:, :L], ca.n_heads, k_len=k_len)
             h = h + _linear_bf16(res, ca.project.weight)
             h = h + cb.mlp(cb.ln_2(h))
             h = cb.sa_block(h, attn_mask=m.self_attn_mask, rope=m.rope_cache)

@@ -572,6 +572,32 @@ attn_label_range_kernel(const int* __restrict__ ids, int B, int S, int* __restri
 }
 
 // ------------------------------------------------------------------------------------------------
+// Positions of a streaming step whose trials sit at different positions (fk_stream_positions): thread (i, b) handles new
+// token i of trial b at position p = len_in[b] + i.  qid is nondecreasing in i, so a 64-token tile's range is the labels of
+// its first and last token.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+stream_positions_kernel(const int* __restrict__ len_in, int* __restrict__ len_out, int n_new, int per_label, int cap,
+                        int* __restrict__ qid, int* __restrict__ qmin, int* __restrict__ qmax, int* __restrict__ pos,
+                        long long* __restrict__ rows) {
+  const int b = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_new) return;
+  const int L = len_in[b];
+  const int p = L + i;
+  const long long o = static_cast<long long>(b) * n_new + i;
+  qid[o] = p / per_label;
+  pos[o] = p;
+  rows[o] = static_cast<long long>(b) * cap + p;
+  if ((i & 63) == 0) {
+    const int t = b * ((n_new + 63) >> 6) + (i >> 6);
+    qmin[t] = p / per_label;
+    qmax[t] = (L + min(i + 63, n_new - 1)) / per_label;
+  }
+  if (i == 0) len_out[b] = L + n_new;
+}
+
+// ------------------------------------------------------------------------------------------------
 // RoPE (brainformer.py:70-91): adjacent pairs rotated by the cached complex exponentials, fp32 math,
 // in place on bf16 [B, S, H, HD] (HD = 16, 32 or 64) with arbitrary token / batch strides.  inverse = conjugate (backward).
 // table: [P, HD / 2] float2 (cos, sin); position of token (b, s) = pos ? pos[b*S+s] : s + pos_offset.
@@ -624,6 +650,20 @@ FK_API int fk_attn_label_ranges(const int* ids, int B, int S, int* tmin, int* tm
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   FK_REQUIRE(ids && tmin && tmax && B > 0 && S > 0, "fk_attn_label_ranges: bad argument");
   attn_label_range_kernel<<<dim3((S + 63) / 64, B), 64, 0, stream>>>(ids, B, S, tmin, tmax);
+  FK_CHECK_LAUNCH();
+  fk_count_launch();
+  return FK_OK;
+}
+
+FK_API int fk_stream_positions(const int* len_in, int* len_out, int B, int n_new, int tokens_per_label, int cap, int* qid,
+                               int* qmin, int* qmax, int* pos, long long* rows, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  FK_REQUIRE(len_in && len_out && len_in != len_out && qid && qmin && qmax && pos && rows,
+             "fk_stream_positions: a buffer is missing, or len_out aliases len_in");
+  FK_REQUIRE(B > 0 && B <= 65535 && n_new > 0 && n_new <= cap && tokens_per_label > 0,
+             "fk_stream_positions: bad sizes (B in [1, 65535], n_new in [1, cap], tokens_per_label >= 1)");
+  stream_positions_kernel<<<dim3((n_new + 255) / 256, B), 256, 0, stream>>>(len_in, len_out, n_new, tokens_per_label, cap, qid,
+                                                                             qmin, qmax, pos, rows);
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;

@@ -6,7 +6,9 @@
 // With <= 64 queries the score matrix of one (trial, head) is at most 64 x S: the work (4.3 GFLOP forward at cfg 4) is far
 // below what K and V cost to read (134 MB), so these are bandwidth-bound CUDA-core kernels, split over the key axis:
 //
-//   small_attn_fwd_kernel      one CTA = (256-key chunk, head, trial): thread j owns key j (its K and V rows live in
+//   small_attn_fwd_kernel      (optionally only the first k_len[b] keys of trial b: a cache whose trials hold different
+//                              numbers of tokens; chunks past that write the empty partial)
+//                              one CTA = (256-key chunk, head, trial): thread j owns key j (its K and V rows live in
 //                              registers), scores against every query (Q in shared memory) -> chunk maximum / sum per
 //                              query -> P in shared memory -> thread (query, 4 dims) sums P V over the chunk's keys
 //                              -> partial (m, l, O) of the chunk
@@ -92,7 +94,7 @@ __device__ __forceinline__ void stage_queries(const SaParams& p, int b, int h, f
 // max / sum over the 256 threads of the CTA for each of Tq values held one per (thread, t) in smem column form
 template <int HD>
 __global__ void __launch_bounds__(kSaKeys)
-small_attn_fwd_kernel(const SaParams p, float* __restrict__ part_o, float* __restrict__ part_ml) {
+small_attn_fwd_kernel(const SaParams p, const int* __restrict__ k_len, float* __restrict__ part_o, float* __restrict__ part_ml) {
   extern __shared__ float sm[];
   float* qs = sm;                                   // [max(Tq, kSaKeys)][HD]: queries, later the chunk's V rows
   float* ps = qs + kSaKeys * HD;                    // [Tq][kSaKeys + 1]
@@ -100,7 +102,18 @@ small_attn_fwd_kernel(const SaParams p, float* __restrict__ part_o, float* __res
   float* mrow = red + 8 * kSaMaxQ;                  // [Tq] chunk maximum, then reused for the sum
   const int chunk = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
   const int j = chunk * kSaKeys + threadIdx.x;
-  const bool ok = j < p.S;
+  const int S = k_len == nullptr ? p.S : min(p.S, k_len[b]);     // keys of this trial that take part
+  const long long pbase = ((static_cast<long long>(b) * p.H + h) * p.n_chunks + chunk) * p.Tq;
+  if (chunk * kSaKeys >= S) {
+    // no key of the chunk takes part: the empty partial (m = -inf, l = 0, O = 0), which the combine merges as a no-op
+    for (int o = threadIdx.x; o < p.Tq * HD; o += kSaKeys) part_o[pbase * HD + o] = 0.f;
+    for (int t = threadIdx.x; t < p.Tq; t += kSaKeys) {
+      part_ml[(pbase + t) * 2] = -INFINITY;
+      part_ml[(pbase + t) * 2 + 1] = 0.f;
+    }
+    return;
+  }
+  const bool ok = j < S;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   stage_queries<HD>(p, b, h, qs);
   float kr[HD], vr[HD];
@@ -145,7 +158,6 @@ small_attn_fwd_kernel(const SaParams p, float* __restrict__ part_o, float* __res
   float* vs = qs;
 #pragma unroll
   for (int d = 0; d < HD; ++d) vs[threadIdx.x * HD + d] = ok ? vr[d] : 0.f;
-  const long long pbase = ((static_cast<long long>(b) * p.H + h) * p.n_chunks + chunk) * p.Tq;
   if (threadIdx.x < p.Tq) {
     float l = 0.f;
 #pragma unroll
@@ -318,8 +330,8 @@ static bool sa_common_ok(const void* q, const void* k, const void* v, int B, int
 FK_API int fk_small_attn_chunks(int S) { return S > 0 ? (S + kSaKeys - 1) / kSaKeys : FK_ERR_BAD_ARG; }
 
 template <int HD>
-static int sa_forward(const SaParams& p, float* part_o, float* part_ml, __nv_bfloat16* out, long long o_bs, long long o_ts, float* lse,
-                      cudaStream_t stream) {
+static int sa_forward(const SaParams& p, const int* k_len, float* part_o, float* part_ml, __nv_bfloat16* out, long long o_bs,
+                      long long o_ts, float* lse, cudaStream_t stream) {
   static bool done[FK_MAX_DEVICES];
   const int dev = fk_device_ordinal();
   const int smem = small_attn_smem_fwd<HD>();
@@ -331,7 +343,7 @@ static int sa_forward(const SaParams& p, float* part_o, float* part_ml, __nv_bfl
     done[dev] = true;
   }
   const dim3 grid(static_cast<unsigned>(p.n_chunks), static_cast<unsigned>(p.H), static_cast<unsigned>(p.B));
-  small_attn_fwd_kernel<HD><<<grid, kSaKeys, smem, stream>>>(p, part_o, part_ml);
+  small_attn_fwd_kernel<HD><<<grid, kSaKeys, smem, stream>>>(p, k_len, part_o, part_ml);
   FK_CHECK_LAUNCH();
   const long long n = static_cast<long long>(p.B) * p.H * p.Tq * HD;
   small_attn_combine_kernel<HD><<<static_cast<unsigned>((n + 255) / 256), 256, 0, stream>>>(part_o, part_ml, p.n_chunks, p.Tq, p.H, p.B,
@@ -344,7 +356,8 @@ static int sa_forward(const SaParams& p, float* part_o, float* part_ml, __nv_bfl
 FK_API int fk_small_attn_forward(const void* q, long long q_bs, long long q_ts, const void* k, long long k_bs, long long k_ts,
                                  const void* v, long long v_bs, long long v_ts, void* out, long long o_bs, long long o_ts,
                                  float* lse, int B, int H, int Tq, int S, int head_dim, float scale, const float* rope_table,
-                                 int rope_len, int rope_q0, int rope_k0, float* part_o, float* part_ml, void* stream_) {
+                                 int rope_len, int rope_q0, int rope_k0, float* part_o, float* part_ml, const int* k_len,
+                                 void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   FK_REQUIRE(sa_common_ok(q, k, v, B, H, Tq, S, head_dim, q_ts, k_ts, v_ts) && out && lse && part_o && part_ml && o_ts % 8 == 0,
              "fk_small_attn_forward: bad argument (<= 64 queries, head_dim 16 / 32 / 64, 16-byte aligned rows)");
@@ -357,9 +370,9 @@ FK_API int fk_small_attn_forward(const void* q, long long q_bs, long long q_ts, 
   p.scale_log2 = scale * 1.4426950408889634f;
   p.rope = reinterpret_cast<const float2*>(rope_table); p.rope_q0 = rope_q0; p.rope_k0 = rope_k0;
   __nv_bfloat16* o = static_cast<__nv_bfloat16*>(out);
-  if (head_dim == 16) return sa_forward<16>(p, part_o, part_ml, o, o_bs, o_ts, lse, stream);
-  if (head_dim == 32) return sa_forward<32>(p, part_o, part_ml, o, o_bs, o_ts, lse, stream);
-  return sa_forward<64>(p, part_o, part_ml, o, o_bs, o_ts, lse, stream);
+  if (head_dim == 16) return sa_forward<16>(p, k_len, part_o, part_ml, o, o_bs, o_ts, lse, stream);
+  if (head_dim == 32) return sa_forward<32>(p, k_len, part_o, part_ml, o, o_bs, o_ts, lse, stream);
+  return sa_forward<64>(p, k_len, part_o, part_ml, o, o_bs, o_ts, lse, stream);
 }
 
 template <int HD>

@@ -6,6 +6,7 @@ LayerNorm / RMSNorm, SwiGLU gate, RoPE and masked flash attention, each a thin
 """
 from __future__ import annotations
 
+import operator
 from typing import Optional
 
 import torch
@@ -245,6 +246,13 @@ class LabelMask:
         return lo, hi
 
     @staticmethod
+    def from_ranges(qid, kid, qmin, qmax, kmin, kmax) -> "LabelMask":
+        """labels whose per-tile ranges are already known (fk_stream_positions writes them with the labels)."""
+        m = LabelMask.__new__(LabelMask)
+        m.qid, m.kid, m.qmin, m.qmax, m.kmin, m.kmax, m._pairs = qid, kid, qmin, qmax, kmin, kmax, None
+        return m
+
+    @staticmethod
     def block_causal(B: int, S: int, tokens_per_block: int, device) -> "LabelMask":
         """brainformer.py:93-111 build_advanced_causal_mask: attend iff block(k) <= block(q)."""
         ids = (torch.arange(S, device=device, dtype=torch.int32) // tokens_per_block)[None].expand(B, S)
@@ -269,6 +277,47 @@ class LabelMask:
     def dense(self) -> torch.Tensor:
         """[B, 1, Sq, Sk] bool, True = attend (only for tests / the library-SDPA compatibility path)."""
         return (self.kid[:, None, None, :] <= self.qid[:, None, :, None])
+
+
+def stream_rows(rows, batch_size: int, what: str) -> list:
+    """Row indices of a per-row stream reset as a list of ints: FkError for an index outside [0, batch_size) or a duplicate."""
+    try:
+        idx = [operator.index(r) for r in rows]
+    except TypeError:
+        raise FkError(f"{what}: rows must be a sequence of integer row indices, got {rows!r}") from None
+    bad = [r for r in idx if not 0 <= r < batch_size]
+    if bad:
+        raise FkError(f"{what}: rows {bad} are outside the batch of {batch_size}")
+    if len(set(idx)) != len(idx):
+        raise FkError(f"{what}: rows {idx} name a row twice")
+    return idx
+
+
+def stream_length(lengths, what: str) -> int:
+    """The one length of a stream whose rows are all at the same position; FkError once they differ."""
+    if any(n != lengths[0] for n in lengths):
+        raise FkError(f"{what}: the rows are at different positions ({list(lengths)}); read `lengths` instead")
+    return lengths[0]
+
+
+@on_tensor_device
+def stream_positions(len_in: torch.Tensor, len_out: torch.Tensor, n_new: int, tokens_per_label: int, cap: int):
+    """One launch for the per-row bookkeeping of a streaming step whose rows sit at different positions: row b holds
+    len_in[b] tokens (device int32 [B]) and appends n_new at positions p = len_in[b] + i.  Returns (qid [B, n_new] =
+    p // tokens_per_label, qmin, qmax [B, ceil(n_new / 64)] its tile ranges, pos [B, n_new] = p, rows int64 [B * n_new] =
+    b * cap + p) and writes len_out = len_in + n_new."""
+    require_cuda(len_in, len_out)
+    B = len_in.shape[0]
+    dev = len_in.device
+    qid = torch.empty(B, n_new, device=dev, dtype=torch.int32)
+    nt = (n_new + 63) // 64
+    qmin = torch.empty(B, nt, device=dev, dtype=torch.int32)
+    qmax = torch.empty(B, nt, device=dev, dtype=torch.int32)
+    pos = torch.empty(B, n_new, device=dev, dtype=torch.int32)
+    rows = torch.empty(B * n_new, device=dev, dtype=torch.int64)
+    check(lib().fk_stream_positions(ptr(len_in), ptr(len_out), B, n_new, tokens_per_label, cap, ptr(qid), ptr(qmin),
+                                    ptr(qmax), ptr(pos), ptr(rows), stream()), "fk_stream_positions")
+    return qid, qmin, qmax, pos, rows
 
 
 class RopeSpec:
@@ -547,7 +596,7 @@ class _SmallAttnFn(torch.autograd.Function):
             check(lib().fk_small_attn_forward(ptr(q), q.stride(0), q.stride(1), ptr(k), k.stride(0), k.stride(1), ptr(v),
                                               v.stride(0), v.stride(1), ptr(out), out.stride(0), out.stride(1), ptr(lse), B, H,
                                               Tq, S, hd, scale, ptr(rope_table), rl, rope_q0, rope_k0, ptr(part_o),
-                                              ptr(part_ml), stream()), "fk_small_attn_forward")
+                                              ptr(part_ml), None, stream()), "fk_small_attn_forward")
         ctx.save_for_backward(q, k, v, out, lse)
         ctx.meta = (H, hd, scale, rope_table, rope_q0, rope_k0, nch)
         return out
@@ -605,7 +654,7 @@ class _SmallAttnKVFn(torch.autograd.Function):
             check(lib().fk_small_attn_forward(ptr(q), q.stride(0), q.stride(1), ptr(k), k.stride(0), k.stride(1), ptr(v),
                                               v.stride(0), v.stride(1), ptr(out), out.stride(0), out.stride(1), ptr(lse), B, H,
                                               Tq, S, hd, scale, ptr(rope_table), rl, rope_q0, rope_k0, ptr(part_o),
-                                              ptr(part_ml), stream()), "fk_small_attn_forward")
+                                              ptr(part_ml), None, stream()), "fk_small_attn_forward")
         ctx.save_for_backward(q, kv, out, lse)
         ctx.meta = (H, hd, scale, rope_table, rope_q0, rope_k0, nch)
         return out
@@ -643,11 +692,16 @@ def small_attention_kv(q, kv, n_heads: int, scale: Optional[float] = None):
 
 
 @on_tensor_device
-def small_attention_kv_cached(q, kv, n_heads: int, scale: Optional[float] = None):
+def small_attention_kv_cached(q, kv, n_heads: int, scale: Optional[float] = None, k_len: Optional[torch.Tensor] = None):
     """Inference-only small_attention_kv against a key | value cache: kv [B, S, 2 * H * hd] bf16 is a view with any 16-byte
-    aligned batch / token strides (e.g. the first S tokens of a longer cache), read in place, never copied."""
-    require_cuda(q, kv)
+    aligned batch / token strides (e.g. the first S tokens of a longer cache), read in place, never copied.
+    k_len: optional device int32 [B], the number of keys of each trial (trials of a cache at different lengths): key j of
+    trial b takes part iff j < min(S, k_len[b]); keys past it are never read, and a trial with no key gives a zero row."""
+    require_cuda(q, kv, k_len)
     require_device()
+    if k_len is not None and (k_len.dtype != torch.int32 or k_len.shape != (q.shape[0],) or not k_len.is_contiguous()):
+        raise FkError(f"small_attention_kv_cached: k_len must be a contiguous int32 [{q.shape[0]}] tensor, got "
+                      f"{k_len.dtype} {tuple(k_len.shape)}")
     if torch.is_grad_enabled() and (q.requires_grad or kv.requires_grad):
         raise FkError("small_attention_kv_cached is inference only: run it under torch.no_grad()")
     q = _rows_ok(q)
@@ -671,7 +725,7 @@ def small_attention_kv_cached(q, kv, n_heads: int, scale: Optional[float] = None
     with timed("small_attn_fwd", 4.0 * B * H * Tq * S * hd):
         check(lib().fk_small_attn_forward(ptr(q), q.stride(0), q.stride(1), ptr(k), k.stride(0), k.stride(1), ptr(v),
                                           v.stride(0), v.stride(1), ptr(out), out.stride(0), out.stride(1), ptr(lse), B, H,
-                                          Tq, S, hd, scale, None, 0, 0, 0, ptr(part_o), ptr(part_ml), stream()),
+                                          Tq, S, hd, scale, None, 0, 0, 0, ptr(part_o), ptr(part_ml), ptr(k_len), stream()),
               "fk_small_attn_forward")
     return out
 

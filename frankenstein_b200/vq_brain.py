@@ -26,7 +26,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import _lib, conv, gemm
+from . import _lib, conv, gemm, ops
 from ._lib import DTYPE_CODE, FkError, check, counters, lib, on_tensor_device, ptr, require_cuda, require_device, stream
 from .vector_quantize import VectorQuantize, finish, prepare_codebook, prepare_input, search
 
@@ -436,20 +436,39 @@ class TokenizerStream:
             self._embed = vq.codebook.detach().float().clone().contiguous()
             self._cb, self._c2pad = prepare_codebook(self._embed, self.use_cosine)
         self._cur = 0
-        self._length = 0
+        self._lengths = [0] * batch_size
+
+    @property
+    def lengths(self) -> list:
+        """bins consumed so far, per row (each row is a recording of its own; see `reset`)."""
+        return list(self._lengths)
 
     @property
     def length(self) -> int:
-        """bins consumed so far."""
-        return self._length
+        """bins consumed so far, while every row is at the same position."""
+        return ops.stream_length(self._lengths, "TokenizerStream.length")
 
-    def reset(self) -> None:
-        """Start a new recording: the histories become the causal zero padding again."""
+    def reset(self, rows=None) -> None:
+        """Start a new recording in every row (rows None) or only in the given row indices: their histories become the
+        causal zero padding again, and the other rows carry on untouched.  FkError, changing nothing, for an index outside
+        the batch or a duplicate."""
+        if rows is None:
+            for layers in self._layers:
+                for L in layers:
+                    if L.hist is not None:
+                        L.hist.zero_()
+            self._lengths = [0] * self.batch_size
+            return
+        idx = ops.stream_rows(rows, self.batch_size, "TokenizerStream.reset")
+        if not idx:
+            return
+        dev_idx = torch.tensor(idx, dtype=torch.long).to(self.device)
         for layers in self._layers:
             for L in layers:
                 if L.hist is not None:
-                    L.hist.zero_()
-        self._length = 0
+                    L.hist.index_fill_(1, dev_idx, 0)          # both buffers of the rows
+        for r in idx:
+            self._lengths[r] = 0
 
     def _run(self, layers, x):
         inputs = []
@@ -498,5 +517,5 @@ class TokenizerStream:
             if self.reconstruct:
                 out = out + (self._run(self._layers[1], out[1]),)
         self._cur ^= 1
-        self._length += T
+        self._lengths = [n + T for n in self._lengths]
         return out

@@ -160,6 +160,15 @@ int fk_rope(void* x, long long bs, long long ts, int B, int S, int H, int head_d
  * batch/token strides in elements.  qmin..kmax: per-64-token-tile label ranges from fk_attn_label_ranges.
  * lse: [B,H,Sq] fp32 (log2 domain), nullable in inference. */
 int fk_attn_label_ranges(const int* ids, int B, int S, int* tmin, int* tmax, void* stream);
+/* Positions of one streaming step whose trials sit at different positions (brainformer.EncoderStream after a per-row reset):
+ * trial b holds len_in[b] tokens (int32 [B]) and appends n_new at positions p = len_in[b] + i, i < n_new.  One launch
+ * writes qid [B, n_new] = p / tokens_per_label (the block-causal label of p) with its per-64-token tile ranges qmin / qmax
+ * [B, ceil(n_new / 64)] (as fk_attn_label_ranges), pos [B, n_new] = p (RoPE positions), rows int64 [B, n_new] =
+ * b * cap + p (flat rows of a [B, cap, ...] cache) and len_out[b] = len_in[b] + n_new (len_out a buffer other than len_in).
+ * The caller keeps len_in[b] + n_new <= cap.  B in [1, 65535], n_new in [1, cap], tokens_per_label >= 1; anything else is
+ * rejected before the launch. */
+int fk_stream_positions(const int* len_in, int* len_out, int B, int n_new, int tokens_per_label, int cap, int* qid,
+                        int* qmin, int* qmax, int* pos, long long* rows, void* stream);
 int fk_attn_forward(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq, int Sk,
                     int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs,
                     long long v_ts, long long o_bs, long long o_ts, const int* qid, const int* kid, const int* qmin,
@@ -238,7 +247,10 @@ int fk_attn_forward_tc(const void* q, const void* k, const void* v, void* out, f
  * fill max_ctas CTAs, <= 0: all SMs).  n_chunks == 1 runs the unsplit kernel (part_o / part_ml unused).  Otherwise each item
  * writes unnormalised partials, part_o fp32 [B, H, n_chunks, Sq, head_dim] and part_ml fp32 [B, H, n_chunks, Sq, 2] (running
  * maximum and sum, log2 domain), and a second launch merges them in chunk order (bit-reproducible).  out bf16; lse
- * [B, H, Sq] (log2 domain) nullable; a query that sees no key gives a zero row.  counters: as fk_attn_forward_tc. */
+ * [B, H, Sq] (log2 domain) nullable; a query that sees no key gives a zero row.  counters: as fk_attn_forward_tc.
+ * Every k / v row below Sk must hold finite values, also rows no query sees: a tile that is only partly visible multiplies
+ * P = 0 by every V row of the tile, and 0 * NaN or 0 * inf would reach the output.  (A cache of trials at different
+ * lengths therefore starts zeroed; rows left by an earlier session are finite.) */
 int fk_attn_kv_chunks(int B, int H, int Sq, int Sk, int max_ctas);
 int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq, int Sk,
                           int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs,
@@ -317,12 +329,17 @@ int fk_input_normalize(const float* volt, const float* spk, const long long* off
  * [rope_len, head_dim / 2, 2] fp32 (cos, sin); q row t is rotated by position rope_q0 + t, k row j by rope_k0 + j
  * (apply_rope, brainformer.py:70-91) and dq / dk are rotated back.  The key axis is split into
  * fk_small_attn_chunks(S) chunks of 256: part_o fp32 [B, H, chunks, Tq, head_dim], part_ml fp32 [B, H, chunks, Tq, 2],
- * part_dq like part_o; partials are merged in chunk order (deterministic).  lse [B, H, Tq] in the log2 domain. */
+ * part_dq like part_o; partials are merged in chunk order (deterministic).  lse [B, H, Tq] in the log2 domain.
+ * k_len (forward only, nullable): int32 [B] per-trial key counts (a key / value cache whose trials hold different numbers
+ * of tokens): key j of trial b takes part iff j < min(S, k_len[b]); a chunk past that writes the empty partial (m = -inf,
+ * l = 0, O = 0), which the merge passes over exactly, and a trial with no key gets a zero row (lse = +inf).  Keys past
+ * k_len[b] are never read.  NULL: every trial has S keys. */
 int fk_small_attn_chunks(int S);
 int fk_small_attn_forward(const void* q, long long q_bs, long long q_ts, const void* k, long long k_bs, long long k_ts,
                           const void* v, long long v_bs, long long v_ts, void* out, long long o_bs, long long o_ts,
                           float* lse, int B, int H, int Tq, int S, int head_dim, float scale, const float* rope_table,
-                          int rope_len, int rope_q0, int rope_k0, float* part_o, float* part_ml, void* stream);
+                          int rope_len, int rope_q0, int rope_k0, float* part_o, float* part_ml, const int* k_len,
+                          void* stream);
 int fk_small_attn_backward(const void* q, long long q_bs, long long q_ts, const void* k, long long k_bs, long long k_ts,
                            const void* v, long long v_bs, long long v_ts, const void* out, long long o_bs, long long o_ts,
                            const void* dout, long long do_bs, long long do_ts, const float* lse, void* dq, void* dk,
