@@ -425,9 +425,13 @@ class EncoderStream:
     rounding.
 
     Each batch row is a session of its own: `reset(rows)` restarts only the given rows, and from then on the rows sit at
-    different positions (`lengths`).  A step still advances every row by the same whole patches; each row continues at its
-    own position, and its outputs depend on its own session only.  Until the first per-row reset (and again after
-    `reset()`) every row is at one position and a step runs the lockstep path."""
+    different positions (`lengths`).  A step advances every row by the same whole patches, or, with `counts`, each row by
+    its own count (0 included: a session with no new data waits); each row continues at its own position, and its outputs
+    depend on its own session only.  Until the first per-row reset or step with differing counts (and again after
+    `reset()`) every row is at one position and a step runs the lockstep path.
+
+    The caches hold one scratch row past the last row's window: the k | v rows of the slots past a row's count go there,
+    so no filler ever enters a window."""
 
     def __init__(self, encoder: Encoder, batch_size: int, out_dtype=torch.float32):
         cfg = encoder.config
@@ -443,9 +447,11 @@ class EncoderStream:
         self.n_heads = cfg.n_heads
         self.inner = cfg.n_heads * cfg.head_dim
         dev = encoder.device
-        # zeroed: a row's partly visible key tile multiplies P = 0 by the V rows past its length (fk_attn_forward_kv_tc)
-        self.caches = [torch.zeros(batch_size, encoder.block_size, 2 * self.inner, device=dev, dtype=BF16)
-                       for _ in encoder.transformer.h]
+        # zeroed: a row's partly visible key tile multiplies P = 0 by the V rows past its length (fk_attn_forward_kv_tc).
+        # Flat [B * block_size + 1, 2 * inner]: the last row takes the k | v rows of slots past a row's count.
+        self._flat = [torch.zeros(batch_size * encoder.block_size + 1, 2 * self.inner, device=dev, dtype=BF16)
+                      for _ in encoder.transformer.h]
+        self.caches = [f[:-1].view(batch_size, encoder.block_size, 2 * self.inner) for f in self._flat]
         self._lengths = [0] * batch_size
         # per-row sessions: device lengths in two buffers (a step reads one and writes the other, the roles swap once the
         # step is enqueued) and the key labels of the whole window, shared by every row and built on first use
@@ -474,13 +480,18 @@ class EncoderStream:
         idx = ops.stream_rows(rows, self.batch_size, "EncoderStream.reset")
         if not idx:
             return
-        cur = self._len_dev[self._cur]
-        if not self._ragged:
-            cur.fill_(self._lengths[0])               # the lockstep path keeps the lengths on the host only
-            self._ragged = True
+        cur = self._to_ragged()
         cur.index_fill_(0, torch.tensor(idx, dtype=torch.long).to(cur.device), 0)
         for r in idx:
             self._lengths[r] = 0
+
+    def _to_ragged(self):
+        """the current device lengths, filled from the host on leaving the lockstep path (which keeps them on the host only)"""
+        cur = self._len_dev[self._cur]
+        if not self._ragged:
+            cur.fill_(self._lengths[0])
+            self._ragged = True
+        return cur
 
     def _key_labels(self):
         """block-causal labels of every cache position, [B, block_size], with their tile ranges (built once)."""
@@ -491,16 +502,21 @@ class EncoderStream:
         return self._keys
 
     @torch.no_grad()
-    def step(self, x: torch.Tensor) -> torch.Tensor:
+    def step(self, x: torch.Tensor, counts=None) -> torch.Tensor:
         """x [B, n * patch_size, n_electrodes] (n >= 1 whole patches) -> final-LayerNorm outputs of the n * n_electrodes
-        new tokens, [B, n * n_electrodes, dim] in `out_dtype`.  Raises FkError, leaving the state as it was, on a partial
-        patch, a batch or electrode count that does not match, or a step that takes any row past the window (block_size
-        tokens)."""
-        return self._step(x)[0]
+        new tokens, [B, n * n_electrodes, dim] in `out_dtype`.
 
-    def _step(self, x):
-        """step(x) and, for rows at different positions, the flat cache rows b * block_size + position that the new tokens
-        took (int64 [B * n_new]; None on the lockstep path)."""
+        counts: optional host sequence of B ints, the whole patches of x that are new data for each row (0 ... n).  Row b
+        advances by counts[b] patches; the rest of its bins are ignored whatever they hold (NaN included), and its token
+        slots past counts[b] * n_electrodes are zero.  None, or every count n, is the plain step.
+
+        Raises FkError, leaving the state as it was, on a partial patch, a batch or electrode count that does not match, bad
+        counts (number, range), or a step that takes any row past the window (block_size tokens)."""
+        return self._step(x, counts)[0]
+
+    def _step(self, x, counts=None):
+        """step(x, counts) and, for rows at different positions, the flat cache rows b * block_size + position that the new
+        tokens took, B * block_size for slots past a row's count (int64 [B * n_new]; None on the lockstep path)."""
         enc = self.encoder
         E, p = enc.n_electrodes, enc.patch_size
         if x.dim() != 3 or x.shape[0] != self.batch_size or x.shape[2] != E:
@@ -509,12 +525,21 @@ class EncoderStream:
         if T < p or T % p != 0:
             raise ops.FkError(f"EncoderStream.step: {T} bins is not a positive multiple of patch_size {p}")
         n_new = (T // p) * E
-        over = [b for b, n in enumerate(self._lengths) if n + n_new > enc.block_size]
+        if counts is not None:
+            counts = ops.stream_counts(counts, B, T // p, 1, "EncoderStream.step")
+            if all(c == T // p for c in counts):
+                counts = None                          # every row takes the whole step: the plain step
+        adv = [n_new] * B if counts is None else [c * E for c in counts]
+        over = [b for b, n in enumerate(self._lengths) if n + adv[b] > enc.block_size]
         if over:
-            raise ops.FkError(f"EncoderStream.step: {n_new} new tokens take rows {over} (at {[self._lengths[b] for b in over]} "
-                              f"tokens) past the window of {enc.block_size}")
+            raise ops.FkError(f"EncoderStream.step: {[adv[b] for b in over]} new tokens take rows {over} (at "
+                              f"{[self._lengths[b] for b in over]} tokens) past the window of {enc.block_size}")
         if not x.is_cuda:
             raise ops.FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
+        cnt = None
+        if counts is not None:
+            self._to_ragged()
+            cnt = torch.tensor(adv, dtype=torch.int32).to(x.device)     # the one host-to-device copy of the step
         w_emb = enc.transformer.emb
         if GEMM_IMPL == "own" and gemm.patch_embed_supported(T, E, p, w_emb.weight.shape[0]):
             h_delta = gemm.patch_embed(x.detach(), w_emb.weight, w_emb.bias)
@@ -537,8 +562,9 @@ class EncoderStream:
             # rows' lengths; cached positions at or past a row's length belong to later time patches and are masked
             # (whole tiles of them are skipped by the tile ranges).
             keys = self._key_labels()
+            # With counts, the slots past a row's count see no key and write their k | v to the scratch row.
             qid, qmin, qmax, pos, rows = ops.stream_positions(self._len_dev[self._cur], self._len_dev[self._cur ^ 1], n_new, E,
-                                                              enc.block_size)
+                                                              enc.block_size, cnt)
             mask = LabelMask.from_ranges(qid, keys.qid, qmin, qmax, keys.qmin, keys.qmax)
             rope = RopeSpec(enc.rope_table(), pos, 0)
             Sk = enc.block_size
@@ -559,7 +585,7 @@ class EncoderStream:
             if rows is None:
                 cache[:, L:Sk].copy_(qkv[..., inner:])
             else:
-                cache.view(-1, 2 * inner).index_copy_(0, rows, qkv[..., inner:].reshape(-1, 2 * inner))
+                self._flat[i].index_copy_(0, rows, qkv[..., inner:].reshape(-1, 2 * inner))
             res = ops.attention_kv(qkv[..., :inner], cache[:, :Sk, :inner], cache[:, :Sk, inner:], H, mask)
             a = _linear_bf16(res, at.project.weight)
             h, y = ops.add_layer_norm(h, a, blk_.ln_2.weight, blk_.ln_2.bias, blk_.ln_2.eps)
@@ -567,9 +593,11 @@ class EncoderStream:
             nxt = blocks[i + 1].ln_1 if i + 1 < len(blocks) else enc.transformer.ln_f
             h, y = ops.add_layer_norm(h, m, nxt.weight, nxt.bias, nxt.eps,
                                       BF16 if i + 1 < len(blocks) else self.out_dtype)
+        if cnt is not None:
+            y.masked_fill_((qid == ops.NO_LABEL)[..., None], 0)      # token slots past each row's count
         if self._ragged:
             self._cur ^= 1
-        self._lengths = [n + n_new for n in self._lengths]
+        self._lengths = [n + a for n, a in zip(self._lengths, adv)]
         return y, rows
 
 
@@ -712,8 +740,9 @@ class BrainFormerStream:
     """Streaming state of a `BrainFormer`: an `EncoderStream` plus, per CrossBlock, a bf16 cache of the k | v projection
     of the context tokens [B, block_size, 2 * inner].  The encoder is block-causal, so the context tokens never change
     once produced: a step projects only the new ones, then runs the perceiver over the whole cache in place.  Batch rows
-    are sessions of their own as in `EncoderStream`: after `reset(rows)` the perceiver of each row reads that row's own
-    context tokens only."""
+    are sessions of their own as in `EncoderStream`: after `reset(rows)`, or in a step with per-row `counts`, the perceiver
+    of each row reads that row's own context tokens only.  Like the encoder's caches, each context cache holds one scratch
+    row past the last row's window for the slots past a row's count."""
 
     def __init__(self, model: BrainFormer, batch_size: int):
         cfg = model.config
@@ -723,7 +752,8 @@ class BrainFormerStream:
         self.encoder_stream = model.encoder.stream(batch_size, out_dtype=BF16)
         inner = cfg.n_heads * cfg.head_dim
         block = model.encoder.block_size
-        self.kv = [torch.zeros(batch_size, block, 2 * inner, device=model.device, dtype=BF16) for _ in model.perceiver.h]
+        self._flat = [torch.zeros(batch_size * block + 1, 2 * inner, device=model.device, dtype=BF16) for _ in model.perceiver.h]
+        self.kv = [f[:-1].view(batch_size, block, 2 * inner) for f in self._flat]
 
     @property
     def lengths(self) -> list:
@@ -740,26 +770,28 @@ class BrainFormerStream:
         self.encoder_stream.reset(rows)
 
     @torch.no_grad()
-    def step(self, x: torch.Tensor) -> torch.Tensor:
-        """x [B, n * patch_size, n_electrodes] -> pred [B, n_output_tokens, output_dim] fp32 (errors as EncoderStream.step)."""
+    def step(self, x: torch.Tensor, counts=None) -> torch.Tensor:
+        """x [B, n * patch_size, n_electrodes] -> pred [B, n_output_tokens, output_dim] fp32 over every row's context so far
+        (errors as EncoderStream.step).  counts: optional per-row whole patches of new data, as in `EncoderStream.step`; a
+        row with count 0 gets its prediction again, and a row with no context yet the perceiver over an empty context."""
         m = self.model
         es = self.encoder_stream
         L0 = es.lengths[0]
-        context, rows = es._step(x)                                # [B, n_new, dim] bf16
+        context, rows = es._step(x, counts)                        # [B, n_new, dim] bf16
         L = max(es.lengths)
         k_len = None if rows is None else es._len_dev[es._cur]     # the rows' lengths after this step
-        for cb, kv in zip(m.perceiver.h, self.kv):
+        for cb, kv, flat in zip(m.perceiver.h, self.kv, self._flat):
             ca = cb.cross_attn
             proj = _linear_bf16(context, torch.cat([ca.kw.weight, ca.vw.weight], dim=0))
             if rows is None:
                 kv[:, L0:L].copy_(proj)
             else:
-                kv.view(-1, kv.shape[-1]).index_copy_(0, rows, proj.reshape(-1, kv.shape[-1]))
+                flat.index_copy_(0, rows, proj.reshape(-1, kv.shape[-1]))
         h = m.learnable_queries.expand(x.shape[0], m.n_output_tokens, -1)
         for cb, kv in zip(m.perceiver.h, self.kv):
             ca = cb.cross_attn
             q = _linear_bf16(cb.ln_1(h), ca.qw.weight)
-            res = ops.small_attention_kv_cached(q, kv[:, :L], ca.n_heads, k_len=k_len)
+            res = ops.small_attention_kv_cached(q, kv[:, :max(L, 1)], ca.n_heads, k_len=k_len)   # k_len 0: a zero row
             h = h + _linear_bf16(res, ca.project.weight)
             h = h + cb.mlp(cb.ln_2(h))
             h = cb.sa_block(h, attn_mask=m.self_attn_mask, rope=m.rope_cache)

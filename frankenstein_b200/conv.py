@@ -184,14 +184,19 @@ def _row_strides(x3: torch.Tensor):
     return (x3.stride(0), x3.stride(1)) if x3.shape[0] > 1 else (x3.shape[1] * x3.stride(1), x3.stride(1))
 
 
-def causal_conv1d_step(x: torch.Tensor, r, elu: bool, hist_in, hist_out, w2: torch.Tensor, bias, taps: int, stride: int = 1):
+def causal_conv1d_step(x: torch.Tensor, r, elu: bool, hist_in, hist_out, w2: torch.Tensor, bias, taps: int, stride: int = 1,
+                       counts=None):
     """One step of a streamed causal convolution (inference only): x [B, n, Cin] new rows (fp32 or bf16, row-strided), r
     (None or bf16 [B, n, Cin]) a residual added to x, `elu` the activation applied to x + r, hist_in / hist_out bf16
     [B, taps - 1, Cin] the last input rows of the previous step / of this one (None when taps == 1), w2 [Cout, taps * Cin]
     bf16 (`_w_taps_major`, or `_w_transpose_pairs` for the transposed convolution as 2 taps), bias fp32 or None.
     Returns (y bf16 [B, n / stride, Cout], the bf16 input rows act(x + r) [B, n, Cin] as a view of the GEMM operand).
 
-    The GEMM rows are those of `_CausalConvFn.forward`, with the history in place of the causal zero padding."""
+    The GEMM rows are those of `_CausalConvFn.forward`, with the history in place of the causal zero padding.
+
+    counts: optional device int32 [B], the new rows of each trial (0 ... n, multiples of the stride): rows past a trial's
+    count are zeros in the GEMM input, so the outputs past counts[b] / stride are finite whatever x holds there, and the
+    history advances by counts[b] rows only."""
     B, n, Cin = x.shape
     h, s = taps - 1, stride
     if n % s != 0:
@@ -202,8 +207,9 @@ def causal_conv1d_step(x: torch.Tensor, r, elu: bool, hist_in, hist_out, w2: tor
     total = B * rpt + taps
     buf = torch.empty(total, Cin, device=x.device, dtype=BF16)
     rs = (0, 0) if r is None else _row_strides(r)
-    check(lib().fk_conv_stream_rows(ptr(x), 0 if x.dtype == torch.float32 else 1, *_row_strides(x), ptr(r), *rs,
-                                    ptr(hist_in), ptr(hist_out), B, n, h, Cin, int(elu), ptr(buf), rpt, total, stream()),
+    check(lib().fk_conv_stream_rows_counts(ptr(x), 0 if x.dtype == torch.float32 else 1, *_row_strides(x), ptr(r), *rs,
+                                           ptr(hist_in), ptr(hist_out), ptr(counts), B, n, h, Cin, int(elu), ptr(buf), rpt, total,
+                                           stream()),
           "fk_conv_stream_rows")
     M = B * rpt // s
     y = gemm.gemm_nt(_rows(buf, M, taps, s), w2, bias, name="conv_stream")

@@ -25,6 +25,8 @@
 // Backward = three kernels: delta = rowsum(dO * O); dK/dV (one CTA per key tile, loops over query
 // tiles, transposed products so nothing is transposed through memory and no atomics are used); dQ
 // (one CTA per query tile, loops over key tiles).
+#include <climits>
+
 #include "common.cuh"
 
 namespace fk {
@@ -574,27 +576,35 @@ attn_label_range_kernel(const int* __restrict__ ids, int B, int S, int* __restri
 // ------------------------------------------------------------------------------------------------
 // Positions of a streaming step whose trials sit at different positions (fk_stream_positions): thread (i, b) handles new
 // token i of trial b at position p = len_in[b] + i.  qid is nondecreasing in i, so a 64-token tile's range is the labels of
-// its first and last token.
+// its first and last token.  With per-trial counts (cnt non-null) only the first c = cnt[b] slots are new tokens; a slot
+// at or past c gets the query label INT_MIN, which no key label (>= 0) satisfies, a RoPE position inside the table and
+// the scratch cache row B * cap, outside every trial's window.  The new slots are a prefix of the trial's slots, so a tile
+// holding a padded slot has qmin = INT_MIN and qmax = the label of its last new slot (INT_MIN if it has none).
 // ------------------------------------------------------------------------------------------------
+constexpr int kNoLabel = INT_MIN;
+
 __global__ void __launch_bounds__(256)
-stream_positions_kernel(const int* __restrict__ len_in, int* __restrict__ len_out, int n_new, int per_label, int cap,
-                        int* __restrict__ qid, int* __restrict__ qmin, int* __restrict__ qmax, int* __restrict__ pos,
-                        long long* __restrict__ rows) {
+stream_positions_kernel(const int* __restrict__ len_in, const int* __restrict__ cnt, int* __restrict__ len_out, int n_new,
+                        int per_label, int cap, int* __restrict__ qid, int* __restrict__ qmin, int* __restrict__ qmax,
+                        int* __restrict__ pos, long long* __restrict__ rows) {
   const int b = blockIdx.y;
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n_new) return;
   const int L = len_in[b];
+  const int c = cnt == nullptr ? n_new : min(max(cnt[b], 0), n_new);
   const int p = L + i;
   const long long o = static_cast<long long>(b) * n_new + i;
-  qid[o] = p / per_label;
-  pos[o] = p;
-  rows[o] = static_cast<long long>(b) * cap + p;
+  const bool live = i < c;
+  qid[o] = live ? p / per_label : kNoLabel;
+  pos[o] = min(p, cap - 1);
+  rows[o] = static_cast<long long>(live ? b : gridDim.y) * cap + (live ? p : 0);
   if ((i & 63) == 0) {
     const int t = b * ((n_new + 63) >> 6) + (i >> 6);
-    qmin[t] = p / per_label;
-    qmax[t] = (L + min(i + 63, n_new - 1)) / per_label;
+    const int last = min(i + 63, n_new - 1);
+    qmin[t] = last < c ? p / per_label : kNoLabel;
+    qmax[t] = live ? (L + min(last, c - 1)) / per_label : kNoLabel;
   }
-  if (i == 0) len_out[b] = L + n_new;
+  if (i == 0) len_out[b] = L + c;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -655,18 +665,25 @@ FK_API int fk_attn_label_ranges(const int* ids, int B, int S, int* tmin, int* tm
   return FK_OK;
 }
 
-FK_API int fk_stream_positions(const int* len_in, int* len_out, int B, int n_new, int tokens_per_label, int cap, int* qid,
-                               int* qmin, int* qmax, int* pos, long long* rows, void* stream_) {
+FK_API int fk_stream_positions_counts(const int* len_in, const int* counts, int* len_out, int B, int n_new,
+                                      int tokens_per_label, int cap, int* qid, int* qmin, int* qmax, int* pos, long long* rows,
+                                      void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  FK_REQUIRE(len_in && len_out && len_in != len_out && qid && qmin && qmax && pos && rows,
-             "fk_stream_positions: a buffer is missing, or len_out aliases len_in");
+  FK_REQUIRE(len_in && len_out && len_in != len_out && counts != len_out && qid && qmin && qmax && pos && rows,
+             "fk_stream_positions: a buffer is missing, or len_out aliases len_in or counts");
   FK_REQUIRE(B > 0 && B <= 65535 && n_new > 0 && n_new <= cap && tokens_per_label > 0,
              "fk_stream_positions: bad sizes (B in [1, 65535], n_new in [1, cap], tokens_per_label >= 1)");
-  stream_positions_kernel<<<dim3((n_new + 255) / 256, B), 256, 0, stream>>>(len_in, len_out, n_new, tokens_per_label, cap, qid,
-                                                                             qmin, qmax, pos, rows);
+  stream_positions_kernel<<<dim3((n_new + 255) / 256, B), 256, 0, stream>>>(len_in, counts, len_out, n_new, tokens_per_label,
+                                                                             cap, qid, qmin, qmax, pos, rows);
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;
+}
+
+FK_API int fk_stream_positions(const int* len_in, int* len_out, int B, int n_new, int tokens_per_label, int cap, int* qid,
+                               int* qmin, int* qmax, int* pos, long long* rows, void* stream_) {
+  return fk_stream_positions_counts(len_in, nullptr, len_out, B, n_new, tokens_per_label, cap, qid, qmin, qmax, pos, rows,
+                                    stream_);
 }
 
 FK_API int fk_attn_forward(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq, int Sk,

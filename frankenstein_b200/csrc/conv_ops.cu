@@ -9,7 +9,8 @@
 //   stream_rows_kernel      the GEMM input rows of one STREAMED causal convolution (SoundStream.stream): per trial the h
 //                           history rows of the previous step, then act(x + r) for the n new rows (the ELU between layers
 //                           and the ResidualUnit's `x + layers(x)`, rounded as the offline bf16 ops round), then zeros;
-//                           also writes the next step's history (the last h rows of [history | new rows])
+//                           also writes the next step's history (the last h rows of [history | new rows]); with
+//                           per-trial counts of new rows, rows past a trial's count are zeros and never read from x
 //
 // All HBM-bound: 16-byte accesses, persistent grids of 148 * k CTAs.
 #include "common.cuh"
@@ -83,12 +84,14 @@ __device__ __forceinline__ uint4 stream_new_row(const void* x, int x_f32, long l
   return make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
 }
 
-// one thread = 8 channels of one row; items [0, total_rows * C8) are rows of out, the next B * h * C8 rows of hist_out
+// one thread = 8 channels of one row; items [0, total_rows * C8) are rows of out, the next B * h * C8 rows of hist_out.
+// cnt (nullable): trial b's new rows are its first cnt[b] rows of x; the rest of x is never read, its GEMM rows are zeros
+// and the history advances by cnt[b] rows only (cnt[b] = 0 carries it over unchanged).
 __global__ void __launch_bounds__(256)
 stream_rows_kernel(const void* __restrict__ x, int x_f32, long long x_sb, long long x_st, const __nv_bfloat16* __restrict__ r,
                    long long r_sb, long long r_st, const __nv_bfloat16* __restrict__ hist_in, __nv_bfloat16* __restrict__ hist_out,
-                   long long B, long long n, int h, int C8, int elu, long long rpt, long long total_rows,
-                   __nv_bfloat16* __restrict__ out) {
+                   const int* __restrict__ cnt, long long B, long long n, int h, int C8, int elu, long long rpt,
+                   long long total_rows, __nv_bfloat16* __restrict__ out) {
   const long long n_out = total_rows * C8, n_all = n_out + B * h * C8;
   const long long C = C8 * 8ll;
   for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < n_all;
@@ -101,16 +104,18 @@ stream_rows_kernel(const void* __restrict__ x, int x_f32, long long x_sb, long l
       t = row - b * rpt;
       dst = out + row * C;
     } else {
-      row = (i - n_out) / C8;                  // hist_out row (b, j) = row b * h + j takes row n + j of [history | new rows]
+      row = (i - n_out) / C8;                  // hist_out row (b, j) takes row n_b + j of [history | new rows]
       b = row / h;
-      t = n + (row - b * h);
+      t = row - b * h;
       dst = hist_out + row * C;
     }
+    const long long nb = (cnt != nullptr && b < B) ? min(max(static_cast<long long>(cnt[b]), 0ll), n) : n;
+    if (i >= n_out) t += nb;
     const int c = static_cast<int>(i % C8) * 8;
     uint4 v = make_uint4(0u, 0u, 0u, 0u);
     if (b < B && t < h)
       v = *reinterpret_cast<const uint4*>(hist_in + (b * h + t) * C + c);
-    else if (b < B && t < h + n)
+    else if (b < B && t < h + nb)
       v = stream_new_row(x, x_f32, x_sb, x_st, r, r_sb, r_st, elu, b, t - h, c);
     *reinterpret_cast<uint4*>(dst + c) = v;
   }
@@ -181,9 +186,10 @@ FK_API int fk_pad_rows(const void* x, int x_dtype, long long B, long long T, int
   return FK_OK;
 }
 
-FK_API int fk_conv_stream_rows(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r, long long r_sb,
-                               long long r_st, const void* hist_in, void* hist_out, long long B, long long n, int h, int C,
-                               int act, void* out, long long rows_per_trial, long long total_rows, void* stream_) {
+FK_API int fk_conv_stream_rows_counts(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r,
+                                      long long r_sb, long long r_st, const void* hist_in, void* hist_out, const int* counts,
+                                      long long B, long long n, int h, int C, int act, void* out, long long rows_per_trial,
+                                      long long total_rows, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   FK_REQUIRE(x && out && B > 0 && n > 0 && h >= 0 && C > 0 && C % 8 == 0, "fk_conv_stream_rows: bad argument (n >= 1, C % 8 == 0)");
   FK_REQUIRE(x_dtype == 0 || x_dtype == 1, "fk_conv_stream_rows: x must be f32 (0) or bf16 (1)");
@@ -201,10 +207,18 @@ FK_API int fk_conv_stream_rows(const void* x, int x_dtype, long long x_sb, long 
   if (blocks > cap) blocks = cap;
   stream_rows_kernel<<<static_cast<unsigned>(blocks), 256, 0, stream>>>(
       x, x_dtype == 0, x_sb, x_st, static_cast<const __nv_bfloat16*>(r), r_sb, r_st, static_cast<const __nv_bfloat16*>(hist_in),
-      static_cast<__nv_bfloat16*>(hist_out), B, n, h, C / 8, act, rows_per_trial, total_rows, static_cast<__nv_bfloat16*>(out));
+      static_cast<__nv_bfloat16*>(hist_out), counts, B, n, h, C / 8, act, rows_per_trial, total_rows,
+      static_cast<__nv_bfloat16*>(out));
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;
+}
+
+FK_API int fk_conv_stream_rows(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r, long long r_sb,
+                               long long r_st, const void* hist_in, void* hist_out, long long B, long long n, int h, int C,
+                               int act, void* out, long long rows_per_trial, long long total_rows, void* stream_) {
+  return fk_conv_stream_rows_counts(x, x_dtype, x_sb, x_st, r, r_sb, r_st, hist_in, hist_out, nullptr, B, n, h, C, act, out,
+                                    rows_per_trial, total_rows, stream_);
 }
 
 FK_API int fk_colsum_grid(void) { return fk_sm_count() * 4; }

@@ -279,6 +279,10 @@ class LabelMask:
         return (self.kid[:, None, None, :] <= self.qid[:, None, :, None])
 
 
+# query label of a streamed slot past its row's count (fk_stream_positions_counts): no key label (>= 0) satisfies it
+NO_LABEL = -2 ** 31
+
+
 def stream_rows(rows, batch_size: int, what: str) -> list:
     """Row indices of a per-row stream reset as a list of ints: FkError for an index outside [0, batch_size) or a duplicate."""
     try:
@@ -301,13 +305,21 @@ def stream_length(lengths, what: str) -> int:
 
 
 @on_tensor_device
-def stream_positions(len_in: torch.Tensor, len_out: torch.Tensor, n_new: int, tokens_per_label: int, cap: int):
+def stream_positions(len_in: torch.Tensor, len_out: torch.Tensor, n_new: int, tokens_per_label: int, cap: int,
+                     counts: Optional[torch.Tensor] = None):
     """One launch for the per-row bookkeeping of a streaming step whose rows sit at different positions: row b holds
     len_in[b] tokens (device int32 [B]) and appends n_new at positions p = len_in[b] + i.  Returns (qid [B, n_new] =
     p // tokens_per_label, qmin, qmax [B, ceil(n_new / 64)] its tile ranges, pos [B, n_new] = p, rows int64 [B * n_new] =
-    b * cap + p) and writes len_out = len_in + n_new."""
-    require_cuda(len_in, len_out)
+    b * cap + p) and writes len_out = len_in + n_new.
+
+    counts: optional device int32 [B], the new tokens of each row (0 ... n_new): slots at or past counts[b] get the label
+    INT_MIN, which sees no key, a RoPE position inside the table and the scratch row B * cap of a cache with B * cap + 1
+    rows; len_out = len_in + counts."""
+    require_cuda(len_in, len_out, counts)
     B = len_in.shape[0]
+    if counts is not None and (counts.dtype != torch.int32 or counts.shape != (B,) or not counts.is_contiguous()):
+        raise FkError(f"stream_positions: counts must be a contiguous int32 [{B}] tensor, got {counts.dtype} "
+                      f"{tuple(counts.shape)}")
     dev = len_in.device
     qid = torch.empty(B, n_new, device=dev, dtype=torch.int32)
     nt = (n_new + 63) // 64
@@ -315,9 +327,27 @@ def stream_positions(len_in: torch.Tensor, len_out: torch.Tensor, n_new: int, to
     qmax = torch.empty(B, nt, device=dev, dtype=torch.int32)
     pos = torch.empty(B, n_new, device=dev, dtype=torch.int32)
     rows = torch.empty(B * n_new, device=dev, dtype=torch.int64)
-    check(lib().fk_stream_positions(ptr(len_in), ptr(len_out), B, n_new, tokens_per_label, cap, ptr(qid), ptr(qmin),
-                                    ptr(qmax), ptr(pos), ptr(rows), stream()), "fk_stream_positions")
+    check(lib().fk_stream_positions_counts(ptr(len_in), ptr(counts), ptr(len_out), B, n_new, tokens_per_label, cap, ptr(qid),
+                                           ptr(qmin), ptr(qmax), ptr(pos), ptr(rows), stream()), "fk_stream_positions")
     return qid, qmin, qmax, pos, rows
+
+
+def stream_counts(counts, batch_size: int, limit: int, unit: int, what: str) -> list:
+    """Per-row counts of new data of a streaming step as a list of ints: FkError for a sequence that is not one int per
+    row, or a count outside [0, limit] or not a multiple of `unit`; the message names the rows."""
+    try:
+        c = [operator.index(v) for v in counts]
+    except TypeError:
+        raise FkError(f"{what}: counts must be a sequence of {batch_size} ints, got {counts!r}") from None
+    if len(c) != batch_size:
+        raise FkError(f"{what}: {len(c)} counts for a batch of {batch_size} rows")
+    bad = [b for b, v in enumerate(c) if not 0 <= v <= limit]
+    if bad:
+        raise FkError(f"{what}: counts {[c[b] for b in bad]} of rows {bad} are outside [0, {limit}]")
+    bad = [b for b, v in enumerate(c) if v % unit]
+    if bad:
+        raise FkError(f"{what}: counts {[c[b] for b in bad]} of rows {bad} are not multiples of {unit}")
+    return c
 
 
 class RopeSpec:

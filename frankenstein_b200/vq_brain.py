@@ -411,7 +411,11 @@ class TokenizerStream:
     """Streaming state of a `SoundStream` (from `SoundStream.stream`): per convolution of the encoder (and, with
     `reconstruct`, of the decoder) the last taps - 1 input rows in bf16, two buffers each -- a step reads one and writes
     the other, and the roles swap only once the whole step has been enqueued, so a rejected step leaves the state as it
-    was.  Weights and codebook are a snapshot taken at creation."""
+    was.  Weights and codebook are a snapshot taken at creation.
+
+    With per-row `counts` each row advances by its own number of bins.  The counts reach the device once per step, as a
+    table of the count at each rate of the stacks (bins, half, quarter = tokens); each convolution reads the row of its
+    input rate, so a row's rows past its count never reach a GEMM and its histories advance by its own rows only."""
 
     def __init__(self, model: SoundStream, batch_size: int, reconstruct: bool = False):
         if batch_size < 1:
@@ -470,27 +474,39 @@ class TokenizerStream:
         for r in idx:
             self._lengths[r] = 0
 
-    def _run(self, layers, x):
+    def _run(self, layers, x, cnt=None, level=0):
+        """cnt: None or device int32 [3, B], row k the rows' counts at 1 / 2^k of the bin rate; level: the rate of x."""
         inputs = []
         cur = self._cur
         for L in layers:
             e = L.e
             r = None if e.res is None else inputs[e.res]
             h_in, h_out = (None, None) if L.hist is None else (L.hist[cur], L.hist[cur ^ 1])
-            y, rows = conv.causal_conv1d_step(x, r, e.elu, h_in, h_out, L.w2, L.bias, e.taps, e.stride)
+            y, rows = conv.causal_conv1d_step(x, r, e.elu, h_in, h_out, L.w2, L.bias, e.taps, e.stride,
+                                              None if cnt is None else cnt[level])
             if e.transposed:
                 y = y.reshape(y.shape[0], 2 * y.shape[1], y.shape[2] // 2)
+                level -= 1
+            elif e.stride == 2:
+                level += 1
             inputs.append(rows)
             x = y
         return x
 
     @torch.no_grad()
-    def step(self, x: torch.Tensor):
+    def step(self, x: torch.Tensor, counts=None):
         """x [B, 4n, n_electrodes] (fp32 or bf16, n >= 1) -> (indices [B, n] int64, quantized [B, n, D] fp32), plus, with
         `reconstruct`, the decoder output o [B, 4n, n_electrodes] (bf16) of the new bins.  The quantizer runs with eval
-        semantics whatever the model's mode (no k-means, no EMA update).  Raises FkError, leaving the state as it was, on
-        a bin count that is not a positive multiple of 4, a batch or channel count that does not match the stream, a CPU
-        tensor or a dtype other than fp32 / bf16."""
+        semantics whatever the model's mode (no k-means, no EMA update).
+
+        counts: optional host sequence of B ints, the bins of x that are new data for each row (0 ... 4n, multiples of 4).
+        Row b advances by counts[b] bins; the rest of its bins are ignored whatever they hold (NaN included).  Past a row's
+        count its indices are -1, its quantized vectors zero and its decoder bins zero; a count of 0 leaves the row's
+        histories bit for bit as they were.  None, or every count 4n, is the plain step.
+
+        Raises FkError, leaving the state as it was, on a bin count that is not a positive multiple of 4, a batch or channel
+        count that does not match the stream, bad counts (number, range, multiples of 4), a CPU tensor or a dtype other
+        than fp32 / bf16."""
         B, E = self.batch_size, self.n_electrodes
         if not isinstance(x, torch.Tensor) or x.dim() != 3 or x.shape[0] != B or x.shape[2] != E:
             raise FkError(f"TokenizerStream.step: expected [{B}, 4n, {E}], got "
@@ -504,18 +520,34 @@ class TokenizerStream:
             raise FkError(f"TokenizerStream.step: the stream lives on {self.device}, x on {x.device}")
         if x.dtype not in (torch.float32, torch.bfloat16):
             raise FkError(f"TokenizerStream.step: x must be fp32 or bf16, got {x.dtype}")
+        if counts is not None:
+            counts = ops.stream_counts(counts, B, T, 4, "TokenizerStream.step")
+            if all(c == T for c in counts):
+                counts = None                          # every row takes the whole step: the plain step
         if x.stride(2) != 1 or x.stride(0) % 8 or x.stride(1) % 8 or x.data_ptr() % 16:
             x = x.contiguous()
         n = T // 4
         with torch.cuda.device(self.device):
-            e = self._run(self._layers[0], x.detach())
+            cnt = None
+            if counts is not None:
+                # one host-to-device copy: the counts at the bin, half and token rates of the stacks
+                cnt = torch.tensor([counts, [c // 2 for c in counts], [c // 4 for c in counts]],
+                                   dtype=torch.int32).to(self.device)
+            e = self._run(self._layers[0], x.detach(), cnt, 0)
             D = e.shape[2]
             xn, xb, _ = prepare_input(e.reshape(B * n, D).contiguous(), self.use_cosine)
             cand_val, cand_idx = search(xb, self._cb, self._c2pad, self._embed.shape[0], self.use_cosine)
             indices, quantized, _ = finish(xn, self._embed, cand_val, cand_idx, self.use_cosine, False, 0.0)
             out = (indices.view(B, n), quantized.view(B, n, D))
+            if cnt is not None:
+                past = torch.arange(n, device=self.device)[None] >= cnt[2][:, None]       # token slots past the counts
+                out[0].masked_fill_(past, -1)
+                out[1].masked_fill_(past[..., None], 0)
             if self.reconstruct:
-                out = out + (self._run(self._layers[1], out[1]),)
+                o = self._run(self._layers[1], out[1], cnt, 2)
+                if cnt is not None:
+                    o.masked_fill_((torch.arange(T, device=self.device)[None] >= cnt[0][:, None])[..., None], 0)
+                out = out + (o,)
         self._cur ^= 1
-        self._lengths = [n + T for n in self._lengths]
+        self._lengths = [m + a for m, a in zip(self._lengths, [T] * B if counts is None else counts)]
         return out

@@ -138,6 +138,15 @@ int fk_pad_rows(const void* x, int x_dtype, long long B, long long T, int C, lon
 int fk_conv_stream_rows(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r, long long r_sb,
                         long long r_st, const void* hist_in, void* hist_out, long long B, long long n, int h, int C,
                         int act, void* out, long long rows_per_trial, long long total_rows, void* stream);
+/* fk_conv_stream_rows with per-trial counts of new rows (a step in which the trials received different amounts of data):
+ * counts (nullable) int32 [B] at this convolution's input rate; trial b's new rows are the first c = counts[b] rows of x
+ * (clamped to [0, n]).  Rows h + c ... of its GEMM input are zeros, x[b] past c and r[b] past c are never read, and
+ * hist_out[b] = the last h rows of [hist_in[b] | the c new rows], so c = 0 copies hist_in[b] bit for bit.  NULL: every
+ * trial has n new rows, which is fk_conv_stream_rows. */
+int fk_conv_stream_rows_counts(const void* x, int x_dtype, long long x_sb, long long x_st, const void* r, long long r_sb,
+                               long long r_st, const void* hist_in, void* hist_out, const int* counts, long long B,
+                               long long n, int h, int C, int act, void* out, long long rows_per_trial, long long total_rows,
+                               void* stream);
 /* column sums of a bf16 [M, N] matrix (row stride ld): part [fk_colsum_grid(), N] fp32 per-CTA partials in a fixed order;
  * reduce them with fk_norm_reduce_partials(part, NULL, fk_colsum_grid(), N, out, NULL).  Bias gradient of nn.Linear /
  * nn.Conv1d (sum of dY over tokens). */
@@ -169,6 +178,14 @@ int fk_attn_label_ranges(const int* ids, int B, int S, int* tmin, int* tmax, voi
  * rejected before the launch. */
 int fk_stream_positions(const int* len_in, int* len_out, int B, int n_new, int tokens_per_label, int cap, int* qid,
                         int* qmin, int* qmax, int* pos, long long* rows, void* stream);
+/* fk_stream_positions with per-trial counts of new tokens (trials that received different amounts of data in one step):
+ * counts (nullable) int32 [B], clamped to [0, n_new].  Slot i < counts[b] is written as above.  A slot at or past it gets
+ * qid = INT_MIN (no key label >= 0 satisfies it: the query sees no key, and its tile ranges skip every key tile),
+ * pos = min(p, cap - 1) (inside the RoPE table) and rows = B * cap, a scratch row past every trial's window (the caller's
+ * cache holds B * cap + 1 rows); len_out[b] = len_in[b] + counts[b], and the caller keeps that <= cap.  NULL: every
+ * trial has n_new new tokens, which is fk_stream_positions. */
+int fk_stream_positions_counts(const int* len_in, const int* counts, int* len_out, int B, int n_new, int tokens_per_label,
+                               int cap, int* qid, int* qmin, int* qmax, int* pos, long long* rows, void* stream);
 int fk_attn_forward(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq, int Sk,
                     int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs,
                     long long v_ts, long long o_bs, long long o_ts, const int* qid, const int* kid, const int* qmin,
