@@ -42,6 +42,7 @@ except Exception:  # pragma: no cover - simple_parsing is not installed in the b
         pass
 
 BF16 = torch.bfloat16
+_INT32_MAX = 2 ** 31 - 1
 
 
 @dataclass
@@ -76,9 +77,14 @@ class Config(_ConfigBase):
     rope_theta: int = 10_000
 
 
+def rope_inv_freq(dim: int, theta: float) -> torch.Tensor:
+    """fp32 [dim//2] theta^(-2j/dim), the RoPE frequencies of build_complex_rope_cache."""
+    return 1.0 / (theta ** (torch.arange(0, dim, 2).float() / dim))
+
+
 def build_complex_rope_cache(dim: int, seq_len: int, theta: float) -> torch.Tensor:
     """[seq_len, dim//2] complex64 unit phasors exp(i * t * theta^(-2j/dim))  (models/brainformer.py:56-68)."""
-    inv_freq = 1.0 / (theta ** (torch.arange(0, dim, 2).float() / dim))
+    inv_freq = rope_inv_freq(dim, theta)
     angles = torch.outer(torch.arange(seq_len), inv_freq).float()
     return torch.polar(torch.ones_like(angles), angles)
 
@@ -411,11 +417,16 @@ class Encoder(nn.Module):
         _, y = run_blocks(self.transformer.h, emb, mask, rope, self.transformer.ln_f, out_dtype, h_delta=h_delta)
         return y
 
-    def stream(self, batch_size: int, out_dtype=torch.float32) -> "EncoderStream":
+    def stream(self, batch_size: int, out_dtype=torch.float32, sliding: bool = False) -> "EncoderStream":
         """Online inference: feed the window patch by patch with `EncoderStream.step(x)` and get the outputs of the new
         tokens only.  The mask is block-causal per time patch, so earlier tokens' outputs never change; each layer keeps the
-        rotated keys and values of the tokens seen so far in a bf16 cache of `block_size` tokens."""
-        return EncoderStream(self, batch_size, out_dtype)
+        rotated keys and values of the tokens seen so far in a bf16 cache of `block_size` tokens.
+
+        sliding=True: a stream with no end.  A token at every layer attends to the tokens of its own time patch and of the
+        W - 1 patches before it (W = window_size // patch_size, the model's window), so within the first window this is the
+        model exactly and past it every query sees the relative distances the model was trained on.  Each layer keeps a
+        ring cache of 2 W patches instead of the window."""
+        return EncoderStream(self, batch_size, out_dtype, sliding)
 
 
 class EncoderStream:
@@ -431,9 +442,15 @@ class EncoderStream:
     `reset()`) every row is at one position and a step runs the lockstep path.
 
     The caches hold one scratch row past the last row's window: the k | v rows of the slots past a row's count go there,
-    so no filler ever enters a window."""
+    so no filler ever enters a window.
 
-    def __init__(self, encoder: Encoder, batch_size: int, out_dtype=torch.float32):
+    Sliding (`Encoder.stream(..., sliding=True)`): no length limit.  Each layer's cache is a ring of 2 W patches per row
+    (W patches in the band of the newest query plus up to W new ones), token p in slot p mod 2 W E, and the attention
+    takes a label band of W patches (ops.LabelMask band) over the whole ring.  The ring slots' key labels (p // E, INT_MAX
+    for a slot no session of the row has written) and the RoPE rows of the new positions, computed in fp64, come from one
+    launch per step (fk_stream_ring_positions).  Every step takes the per-row path; a step gives a row at most W patches."""
+
+    def __init__(self, encoder: Encoder, batch_size: int, out_dtype=torch.float32, sliding: bool = False):
         cfg = encoder.config
         if batch_size < 1:
             raise ops.FkError("EncoderStream: batch_size must be positive")
@@ -444,21 +461,33 @@ class EncoderStream:
         self.encoder = encoder
         self.batch_size = batch_size
         self.out_dtype = out_dtype
+        self.sliding = bool(sliding)
         self.n_heads = cfg.n_heads
         self.inner = cfg.n_heads * cfg.head_dim
+        self.window = encoder.n_patches_per_channel                       # W patches: the band of a sliding stream
+        self.cap = 2 * encoder.block_size if self.sliding else encoder.block_size   # cache tokens per row
         dev = encoder.device
         # zeroed: a row's partly visible key tile multiplies P = 0 by the V rows past its length (fk_attn_forward_kv_tc).
-        # Flat [B * block_size + 1, 2 * inner]: the last row takes the k | v rows of slots past a row's count.
-        self._flat = [torch.zeros(batch_size * encoder.block_size + 1, 2 * self.inner, device=dev, dtype=BF16)
+        # Flat [B * cap + 1, 2 * inner]: the last row takes the k | v rows of slots past a row's count.
+        self._flat = [torch.zeros(batch_size * self.cap + 1, 2 * self.inner, device=dev, dtype=BF16)
                       for _ in encoder.transformer.h]
-        self.caches = [f[:-1].view(batch_size, encoder.block_size, 2 * self.inner) for f in self._flat]
+        self.caches = [f[:-1].view(batch_size, self.cap, 2 * self.inner) for f in self._flat]
         self._lengths = [0] * batch_size
         # per-row sessions: device lengths in two buffers (a step reads one and writes the other, the roles swap once the
         # step is enqueued) and the key labels of the whole window, shared by every row and built on first use
-        self._ragged = False
-        self._len_dev = torch.zeros(2, batch_size, device=dev, dtype=torch.int32)
+        self._ragged = self.sliding
+        self._len_dev = torch.zeros(2, batch_size, device=dev, dtype=torch.int64 if self.sliding else torch.int32)
         self._cur = 0
         self._keys = None
+        if self.sliding:
+            # ring key labels [B, cap] with their 64-slot tile ranges, INT_MAX (seen by no query) until a session writes
+            # the slot; the ring kernel keeps them current
+            nt = (self.cap + 63) // 64
+            kid = torch.full((batch_size, self.cap), _INT32_MAX, device=dev, dtype=torch.int32)
+            kmin = torch.full((batch_size, nt), _INT32_MAX, device=dev, dtype=torch.int32)
+            self._keys = LabelMask.from_ranges(None, kid, None, None, kmin, kmin.clone())
+            self._inv_freq = rope_inv_freq(cfg.head_dim, cfg.rope_theta).to(dev)
+            self._rope_pos = {}
 
     @property
     def lengths(self) -> list:
@@ -475,13 +504,23 @@ class EncoderStream:
         the batch or a duplicate."""
         if rows is None:
             self._lengths = [0] * self.batch_size
-            self._ragged = False
+            self._ragged = self.sliding
+            if self.sliding:
+                self._len_dev[self._cur].zero_()
+                for t in (self._keys.kid, self._keys.kmin, self._keys.kmax):
+                    t.fill_(_INT32_MAX)
             return
         idx = ops.stream_rows(rows, self.batch_size, "EncoderStream.reset")
         if not idx:
             return
         cur = self._to_ragged()
-        cur.index_fill_(0, torch.tensor(idx, dtype=torch.long).to(cur.device), 0)
+        sel = torch.tensor(idx, dtype=torch.long).to(cur.device)
+        cur.index_fill_(0, sel, 0)
+        if self.sliding:
+            # the ring slots of the rows' earlier sessions: a restarted session must not see them once its own patch
+            # index passes their labels
+            for t in (self._keys.kid, self._keys.kmin, self._keys.kmax):
+                t.index_fill_(0, sel, _INT32_MAX)
         for r in idx:
             self._lengths[r] = 0
 
@@ -511,7 +550,8 @@ class EncoderStream:
         slots past counts[b] * n_electrodes are zero.  None, or every count n, is the plain step.
 
         Raises FkError, leaving the state as it was, on a partial patch, a batch or electrode count that does not match, bad
-        counts (number, range), or a step that takes any row past the window (block_size tokens)."""
+        counts (number, range), or a step that takes any row past the window (block_size tokens).  A sliding stream has no
+        window limit; it raises instead for a step that gives a row more than W patches or takes its patch index past int32."""
         return self._step(x, counts)[0]
 
     def _step(self, x, counts=None):
@@ -530,6 +570,8 @@ class EncoderStream:
             if all(c == T // p for c in counts):
                 counts = None                          # every row takes the whole step: the plain step
         adv = [n_new] * B if counts is None else [c * E for c in counts]
+        if self.sliding:
+            return self._step_sliding(x, counts, adv)
         over = [b for b, n in enumerate(self._lengths) if n + adv[b] > enc.block_size]
         if over:
             raise ops.FkError(f"EncoderStream.step: {[adv[b] for b in over]} new tokens take rows {over} (at "
@@ -597,6 +639,65 @@ class EncoderStream:
             y.masked_fill_((qid == ops.NO_LABEL)[..., None], 0)      # token slots past each row's count
         if self._ragged:
             self._cur ^= 1
+        self._lengths = [n + a for n, a in zip(self._lengths, adv)]
+        return y, rows
+
+    def _step_sliding(self, x, counts, adv):
+        """_step of a sliding stream: the ring bookkeeping in one launch, each layer's new k | v rows into its ring, and the
+        banded attention over the whole ring (a fixed key axis, so a row's bits depend on its own session only)."""
+        enc = self.encoder
+        E, p, W = enc.n_electrodes, enc.patch_size, self.window
+        B, T, _ = x.shape
+        n_new = (T // p) * E
+        over = [b for b in range(B) if adv[b] > W * E]
+        if over:
+            raise ops.FkError(f"EncoderStream.step: rows {over} get {[adv[b] // E for b in over]} patches in one step; a "
+                              f"sliding stream takes at most W = {W} per row and step")
+        over = [b for b in range(B) if adv[b] and (self._lengths[b] + adv[b] - 1) // E > _INT32_MAX]
+        if over:
+            raise ops.FkError(f"EncoderStream.step: rows {over} (at {[self._lengths[b] for b in over]} tokens) would take "
+                              "their patch index past int32; reset them")
+        if not x.is_cuda:
+            raise ops.FkError("frankenstein_b200 modules run on a B200 only (no CPU fallback)")
+        cnt = None if counts is None else torch.tensor(adv, dtype=torch.int32).to(x.device)   # the step's host-to-device copy
+        w_emb = enc.transformer.emb
+        if GEMM_IMPL == "own" and gemm.patch_embed_supported(T, E, p, w_emb.weight.shape[0]):
+            h_delta = gemm.patch_embed(x.detach(), w_emb.weight, w_emb.bias)
+        else:
+            h_delta = enc.embed(enc.to_patches(x))
+        emb = enc.space_embedding.float().repeat(1, T // p, 1)
+        keys = self._keys
+        qid, qmin, qmax, rows, table = ops.stream_ring_positions(self._len_dev[self._cur], self._len_dev[self._cur ^ 1], n_new,
+                                                                 E, self.cap, keys, self._inv_freq, cnt)
+        mask = LabelMask.from_ranges(qid, keys.kid, qmin, qmax, keys.kmin, keys.kmax, band=W)
+        if n_new not in self._rope_pos:
+            self._rope_pos[n_new] = torch.arange(B * n_new, device=x.device, dtype=torch.int32).view(B, n_new)
+        rope = RopeSpec(table, self._rope_pos[n_new], 0)               # row b * n_new + i of this step's table
+        blocks = enc.transformer.h
+        H, inner = self.n_heads, self.inner
+        l0 = blocks[0].ln_1
+        h, y = ops.add_layer_norm(emb, h_delta, l0.weight, l0.bias, l0.eps)
+        for i, blk_ in enumerate(blocks):
+            at = blk_.attn
+            if GEMM_IMPL == "own" and gemm.qkv_supported(at.qw.weight.shape[1], inner):
+                qkv = gemm.qkv_rope(y, at.qw.weight, at.kw.weight, at.vw.weight, rope, H)
+            else:
+                qkv = _linear_bf16(y, torch.cat([at.qw.weight, at.kw.weight, at.vw.weight], dim=0)).contiguous()
+                q4 = qkv.view(B, n_new, 3, H, -1)
+                ops._rope_inplace(q4[:, :, 0], rope, False)
+                ops._rope_inplace(q4[:, :, 1], rope, False)
+            cache = self.caches[i]
+            self._flat[i].index_copy_(0, rows, qkv[..., inner:].reshape(-1, 2 * inner))
+            res = ops.attention_kv(qkv[..., :inner], cache[..., :inner], cache[..., inner:], H, mask)
+            a = _linear_bf16(res, at.project.weight)
+            h, y = ops.add_layer_norm(h, a, blk_.ln_2.weight, blk_.ln_2.bias, blk_.ln_2.eps)
+            m = blk_.mlp(y)
+            nxt = blocks[i + 1].ln_1 if i + 1 < len(blocks) else enc.transformer.ln_f
+            h, y = ops.add_layer_norm(h, m, nxt.weight, nxt.bias, nxt.eps,
+                                      BF16 if i + 1 < len(blocks) else self.out_dtype)
+        if cnt is not None:
+            y.masked_fill_((qid == ops.NO_LABEL)[..., None], 0)      # token slots past each row's count
+        self._cur ^= 1
         self._lengths = [n + a for n, a in zip(self._lengths, adv)]
         return y, rows
 
@@ -730,10 +831,11 @@ class BrainFormer(nn.Module):
         x = torch.from_numpy(myo)[None].to(self.device).to(self.dtype)
         return self.forward(x, targets=None)[1][0].detach().cpu().numpy().T
 
-    def stream(self, batch_size: int) -> "BrainFormerStream":
+    def stream(self, batch_size: int, sliding: bool = False) -> "BrainFormerStream":
         """Online decoding: `BrainFormerStream.step(x)` takes the next whole patches of the window and returns `pred` as
-        `forward` would for every bin fed so far."""
-        return BrainFormerStream(self, batch_size)
+        `forward` would for every bin fed so far.  sliding=True: a stream with no end (see `Encoder.stream`); `pred` is the
+        perceiver over the context tokens of the last W patches."""
+        return BrainFormerStream(self, batch_size, sliding)
 
 
 class BrainFormerStream:
@@ -742,14 +844,19 @@ class BrainFormerStream:
     once produced: a step projects only the new ones, then runs the perceiver over the whole cache in place.  Batch rows
     are sessions of their own as in `EncoderStream`: after `reset(rows)`, or in a step with per-row `counts`, the perceiver
     of each row reads that row's own context tokens only.  Like the encoder's caches, each context cache holds one scratch
-    row past the last row's window for the slots past a row's count."""
+    row past the last row's window for the slots past a row's count.
 
-    def __init__(self, model: BrainFormer, batch_size: int):
+    Sliding (`BrainFormer.stream(..., sliding=True)`): each context cache is a ring of exactly W patches (block_size
+    tokens) per row, token p in slot p mod block_size, so the valid slots are a prefix until the ring wraps and all of it
+    afterwards.  Cross-attention has no mask and no RoPE, so slot order does not matter: the perceiver reads the first
+    min(length, block_size) slots of each row, the context tokens of its last W patches."""
+
+    def __init__(self, model: BrainFormer, batch_size: int, sliding: bool = False):
         cfg = model.config
         if not ops.small_attention_supported(model.n_output_tokens, cfg.head_dim):
             raise ops.FkError("BrainFormerStream: the cross-attention kernel serves <= 64 queries at head_dim 16 / 32 / 64")
         self.model = model
-        self.encoder_stream = model.encoder.stream(batch_size, out_dtype=BF16)
+        self.encoder_stream = model.encoder.stream(batch_size, out_dtype=BF16, sliding=sliding)
         inner = cfg.n_heads * cfg.head_dim
         block = model.encoder.block_size
         self._flat = [torch.zeros(batch_size * block + 1, 2 * inner, device=model.device, dtype=BF16) for _ in model.perceiver.h]
@@ -780,6 +887,12 @@ class BrainFormerStream:
         context, rows = es._step(x, counts)                        # [B, n_new, dim] bf16
         L = max(es.lengths)
         k_len = None if rows is None else es._len_dev[es._cur]     # the rows' lengths after this step
+        if es.sliding:
+            # ring row b * C + p mod C of the encoder ring row b * 2C + p mod 2C (the scratch row B * 2C -> B * C)
+            C = m.encoder.block_size
+            rows = rows // es.cap * C + rows % C
+            k_len = k_len.clamp(max=C).to(torch.int32)
+            L = C
         for cb, kv, flat in zip(m.perceiver.h, self.kv, self._flat):
             ca = cb.cross_attn
             proj = _linear_bf16(context, torch.cat([ca.kw.weight, ca.vw.weight], dim=0))

@@ -608,6 +608,72 @@ stream_positions_kernel(const int* __restrict__ len_in, const int* __restrict__ 
 }
 
 // ------------------------------------------------------------------------------------------------
+// Positions of a sliding streaming step over ring caches of `cap` tokens (fk_stream_ring_positions): one CTA per trial b.
+// New slot i < c = cnt[b] holds the token at the absolute position p = len_in[b] + i (64-bit, unbounded): query label
+// p / per_label, cache row b * cap + p mod cap, and the same label as key label of that ring slot.  Slots at or past c get
+// kNoLabel, the scratch row B * cap and the RoPE row of position 0.  Once the labels are written, the key tile ranges of
+// every 64-slot tile the step wrote are recomputed from the ring.  The RoPE (cos, sin) rows are formed in fp64, from the
+// model's fp32 inverse frequencies, and rounded: an fp32 angle p * w loses accuracy past a few thousand tokens.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+stream_ring_positions_kernel(const long long* __restrict__ len_in, const int* __restrict__ cnt, long long* __restrict__ len_out,
+                             int n_new, int per_label, int cap, int* __restrict__ qid, int* __restrict__ qmin,
+                             int* __restrict__ qmax, long long* __restrict__ rows, int* __restrict__ kid,
+                             int* __restrict__ kmin, int* __restrict__ kmax, const float* __restrict__ inv_freq, int half,
+                             float2* __restrict__ rope) {
+  const int b = blockIdx.x;
+  const long long L = len_in[b];
+  const int c = cnt == nullptr ? n_new : min(max(cnt[b], 0), n_new);
+  const int s0 = static_cast<int>(L % cap);
+  for (int i = threadIdx.x; i < n_new; i += blockDim.x) {
+    const long long p = L + i;
+    const long long o = static_cast<long long>(b) * n_new + i;
+    const bool live = i < c;
+    const int slot = static_cast<int>(p % cap);
+    const int label = static_cast<int>(p / per_label);
+    qid[o] = live ? label : kNoLabel;
+    rows[o] = live ? static_cast<long long>(b) * cap + slot : static_cast<long long>(gridDim.x) * cap;
+    if (live) kid[static_cast<long long>(b) * cap + slot] = label;
+    if ((i & 63) == 0) {
+      const int t = b * ((n_new + 63) >> 6) + (i >> 6);
+      const int last = min(i + 63, n_new - 1);
+      qmin[t] = last < c ? label : kNoLabel;
+      qmax[t] = live ? static_cast<int>((L + min(last, c - 1)) / per_label) : kNoLabel;
+    }
+  }
+  for (int e = threadIdx.x; e < n_new * half; e += blockDim.x) {
+    const int i = e / half, j = e - i * half;
+    const double ang = static_cast<double>(i < c ? L + i : 0) * static_cast<double>(inv_freq[j]);
+    double sn, cs;
+    sincos(ang, &sn, &cs);
+    rope[(static_cast<long long>(b) * n_new + i) * half + j] = make_float2(static_cast<float>(cs), static_cast<float>(sn));
+  }
+  __syncthreads();                                     // the ring's new key labels are visible to the whole CTA
+  // a tile [a, a + 64) holds a written slot iff it holds s0 or (a - s0) mod cap < c: the c slots from s0 on, mod cap
+  const int ntk = (cap + 63) >> 6, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  for (int t = warp; t < ntk && c > 0; t += blockDim.x >> 5) {
+    const int a = t * 64;
+    if (!((s0 >= a && s0 < a + 64) || (a - s0 + cap) % cap < c)) continue;
+    const int* ring = kid + static_cast<long long>(b) * cap;
+    int lo = INT_MAX, hi = INT_MIN;
+    for (int x = a + lane; x < min(a + 64, cap); x += 32) {
+      lo = min(lo, ring[x]);
+      hi = max(hi, ring[x]);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      lo = min(lo, __shfl_xor_sync(0xffffffffu, lo, o));
+      hi = max(hi, __shfl_xor_sync(0xffffffffu, hi, o));
+    }
+    if (lane == 0) {
+      kmin[b * ntk + t] = lo;
+      kmax[b * ntk + t] = hi;
+    }
+  }
+  if (threadIdx.x == 0) len_out[b] = L + c;
+}
+
+// ------------------------------------------------------------------------------------------------
 // RoPE (brainformer.py:70-91): adjacent pairs rotated by the cached complex exponentials, fp32 math,
 // in place on bf16 [B, S, H, HD] (HD = 16, 32 or 64) with arbitrary token / batch strides.  inverse = conjugate (backward).
 // table: [P, HD / 2] float2 (cos, sin); position of token (b, s) = pos ? pos[b*S+s] : s + pos_offset.
@@ -675,6 +741,21 @@ FK_API int fk_stream_positions_counts(const int* len_in, const int* counts, int*
              "fk_stream_positions: bad sizes (B in [1, 65535], n_new in [1, cap], tokens_per_label >= 1)");
   stream_positions_kernel<<<dim3((n_new + 255) / 256, B), 256, 0, stream>>>(len_in, counts, len_out, n_new, tokens_per_label,
                                                                              cap, qid, qmin, qmax, pos, rows);
+  FK_CHECK_LAUNCH();
+  fk_count_launch();
+  return FK_OK;
+}
+
+FK_API int fk_stream_ring_positions(const long long* len_in, const int* counts, long long* len_out, int B, int n_new,
+                                    int tokens_per_label, int cap, int* qid, int* qmin, int* qmax, long long* rows, int* kid,
+                                    int* kmin, int* kmax, const float* inv_freq, int half, float* rope, void* stream_) {
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  FK_REQUIRE(len_in && len_out && len_in != len_out && qid && qmin && qmax && rows && kid && kmin && kmax && inv_freq && rope,
+             "fk_stream_ring_positions: a buffer is missing, or len_out aliases len_in");
+  FK_REQUIRE(B > 0 && B <= 65535 && n_new > 0 && n_new <= cap && tokens_per_label > 0 && half > 0,
+             "fk_stream_ring_positions: bad sizes (B in [1, 65535], n_new in [1, cap], tokens_per_label >= 1, half >= 1)");
+  stream_ring_positions_kernel<<<B, 256, 0, stream>>>(len_in, counts, len_out, n_new, tokens_per_label, cap, qid, qmin, qmax,
+                                                      rows, kid, kmin, kmax, inv_freq, half, reinterpret_cast<float2*>(rope));
   FK_CHECK_LAUNCH();
   fk_count_launch();
   return FK_OK;

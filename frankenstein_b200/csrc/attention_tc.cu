@@ -1031,10 +1031,15 @@ struct FwdParams {
 // partial O (relative to its reference m) to part_o [B][H][n_chunks][Sq][HD] and (m, l) to part_ml [B][H][n_chunks][Sq][2]
 // (log2 domain; m = -inf, l = 0 for a row that saw no key of the chunk); attn_kv_combine_kernel merges them.  A separate
 // struct keeps the parameter block of the unsplit kernels as it was.
+//
+// band (split kernels only, fk_attn_forward_kv_band_tc): key j is visible to query i iff kid <= qid and qid - kid < band,
+// the difference taken in 64 bits (every int32 is a valid label).  kNoBand exceeds every such difference: no band.
+constexpr long long kNoBand = 1ll << 32;
 struct FwdKvParams : FwdParams {
   float* part_o;
   float* part_ml;
   int n_chunks, chunk_tiles;
+  long long band;
 };
 template <bool kPart>
 using FwdArgs = std::conditional_t<kPart, FwdKvParams, FwdParams>;
@@ -1148,10 +1153,17 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
           kmn = min(p.kmin[b_ * nk64 + i0], p.kmin[b_ * nk64 + i1]);
           kmx = max(p.kmax[b_ * nk64 + i0], p.kmax[b_ * nk64 + i1]);
           vis = kmn <= cta_hi;
+          // banded: skipped as well when every key lies band or more labels below every row
+          if constexpr (kPart) vis = vis && static_cast<long long>(min(wq_lo[0], wq_lo[1])) - kmx < p.band;
         }
         const bool tail = t * kFwdTileK + kFwdTileK > p.Sk;
         if ((masked && kmx > wq_lo[0]) || tail) flags |= 0x4000;
         if ((masked && kmx > wq_lo[1]) || tail) flags |= 0x8000;
+        if constexpr (kPart) {
+          // banded: fully visible to a warpgroup only if no row of it lies band or more labels above a key
+          if (masked && static_cast<long long>(wq_hi[0]) - kmn >= p.band) flags |= 0x4000;
+          if (masked && static_cast<long long>(wq_hi[1]) - kmn >= p.band) flags |= 0x8000;
+        }
       }
       const unsigned m = __ballot_sync(0xffffffffu, vis);
       if (vis) list[cnt + __popc(m & ((1u << lane) - 1u))] = static_cast<uint16_t>(t | flags);
@@ -1304,6 +1316,9 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
     const int row = q0 + g * 128 + r;
     const bool row_ok = row < p.Sq;
     const int my_id = masked ? (row_ok ? p.qid[static_cast<long long>(b) * p.Sq + row] : -0x7fffffff) : 0;
+    // banded: the lowest visible key label, my_id - band + 1 clamped to INT_MIN (qid - kid < band <=> kid >= my_lo)
+    [[maybe_unused]] int my_lo = INT_MIN;
+    if constexpr (kPart) my_lo = static_cast<int>(max(static_cast<long long>(my_id) - p.band + 1, static_cast<long long>(INT_MIN)));
     int* ids_base = reinterpret_cast<int*>(smem + Smem::ids) + g * 256;
     const uint32_t lane_base = static_cast<uint32_t>(q4 * 32) << 16;
     const uint32_t s_addr = tmem_base + lane_base + g * 128;
@@ -1339,9 +1354,17 @@ attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap tm_q, const __grid_consta
       uint32_t sv[2][32];
       auto mask_chunk = [&](uint32_t (&v)[32], int c) {
         if (need_mask) {
+          if constexpr (kPart) {
 #pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if (s_id[c * 32 + i] > my_id) v[i] = 0xff800000u;
+            for (int i = 0; i < 32; ++i) {
+              const int kid = s_id[c * 32 + i];
+              if (kid > my_id || kid < my_lo) v[i] = 0xff800000u;
+            }
+          } else {
+#pragma unroll
+            for (int i = 0; i < 32; ++i)
+              if (s_id[c * 32 + i] > my_id) v[i] = 0xff800000u;
+          }
           if (n_valid < kFwdTileK) {
 #pragma unroll
             for (int i = 0; i < 32; ++i)
@@ -2231,11 +2254,11 @@ FK_API int fk_attn_aug(const void* o, const void* d_o, const float* lse, float* 
 }
 
 // The forward at head_dim 16, 32 or 64 on `grid` persistent CTAs: tensor maps of q / k / v with the swizzle of the head
-// width, then that width's instantiation; the key-split one when p.n_chunks > 1 (the unsplit kernels take the parameter
-// block without the chunk fields).
+// width, then that width's instantiation; the key-split one when `split` (the unsplit kernels take the parameter block
+// without the chunk and band fields).
 static int attn_fwd_launch(int head_dim, const void* q, const void* k, const void* v, long long q_bs, long long q_ts,
                            long long k_bs, long long k_ts, long long v_bs, long long v_ts, const FwdKvParams& p,
-                           unsigned grid, cudaStream_t stream) {
+                           bool split, unsigned grid, cudaStream_t stream) {
   static bool attr_set_dev[FK_MAX_DEVICES];
   bool& attr_set = attr_set_dev[fk_device_ordinal()];
   if (!attr_set) {
@@ -2258,7 +2281,7 @@ static int attn_fwd_launch(int head_dim, const void* q, const void* k, const voi
   rc |= make_map(&mV, v, p.B, p.Sk, p.H, v_bs, v_ts, kFwdTileK);
   if (rc != 0) { fk_set_last_error("cuTensorMapEncodeTiled failed", __FILE__, __LINE__); return FK_ERR_DRIVER; }
   const FwdParams& p1 = p;
-  if (p.n_chunks > 1) {
+  if (split) {
     if (head_dim == 64) attn_fwd_tc_kernel<64, true><<<grid, kFwdThreads, FwdSmem<64>::total, stream>>>(mQ, mK, mV, p);
     else if (head_dim == 16) attn_fwd_tc_kernel<16, true><<<grid, kFwdThreads, FwdSmem<16>::total, stream>>>(mQ, mK, mV, p);
     else attn_fwd_tc_kernel<32, true><<<grid, kFwdThreads, FwdSmem<32>::total, stream>>>(mQ, mK, mV, p);
@@ -2295,7 +2318,7 @@ FK_API int fk_attn_forward_tc(const void* q, const void* k, const void* v, void*
   const long long n_items = static_cast<long long>((S + 255) / 256) * H * B;
   FK_REQUIRE(n_items < (1ll << 31), "fk_attn_forward_tc: too many work items");
   const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
-  const int rc = attn_fwd_launch(head_dim, q, k, v, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, p, grid, stream);
+  const int rc = attn_fwd_launch(head_dim, q, k, v, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, p, false, grid, stream);
   if (rc != FK_OK) return rc;
   fk_count_launch();
   return FK_OK;
@@ -2313,18 +2336,23 @@ FK_API int fk_attn_kv_chunks(int B, int H, int Sq, int Sk, int max_ctas) {
   return (n_k_tiles + per - 1) / per;
 }
 
-FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq,
-                                 int Sk, int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts,
-                                 long long v_bs, long long v_ts, long long o_bs, long long o_ts, const int* qid,
-                                 const int* kid, const int* qmin, const int* qmax, const int* kmin, const int* kmax,
-                                 float scale, float* part_o, float* part_ml, int n_chunks, unsigned int* counters,
-                                 void* stream_) {
+// fk_attn_forward_kv_tc with a label band.  A band below kNoBand runs the split kernel even with one chunk (merged by the
+// combine kernel), so the unsplit kernels, which the training forward shares, never see a band.
+FK_API int fk_attn_forward_kv_band_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H,
+                                      int Sq, int Sk, int head_dim, long long q_bs, long long q_ts, long long k_bs,
+                                      long long k_ts, long long v_bs, long long v_ts, long long o_bs, long long o_ts,
+                                      const int* qid, const int* kid, const int* qmin, const int* qmax, const int* kmin,
+                                      const int* kmax, float scale, float* part_o, float* part_ml, int n_chunks,
+                                      long long band, unsigned int* counters, void* stream_) {
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  FK_REQUIRE(band >= 1, "fk_attn_forward_kv_band_tc: band must be >= 1");
   FK_REQUIRE(head_dim == 16 || head_dim == 32 || head_dim == 64, "fk_attn_forward_kv_tc: head_dim must be 16, 32 or 64");
   FK_REQUIRE(counters != nullptr, "fk_attn_forward_kv_tc: counters (2 zero-initialised uint32, one pair per launch in flight) is null");
   FK_REQUIRE(q && k && v && out && B > 0 && H > 0 && Sq > 0 && Sk > 0, "fk_attn_forward_kv_tc: bad argument");
   FK_REQUIRE((qid == nullptr) == (kid == nullptr), "fk_attn_forward_kv_tc: qid and kid go together");
   FK_REQUIRE(qid == nullptr || (qmin && qmax && kmin && kmax), "fk_attn_forward_kv_tc: label ranges missing");
+  const bool banded = band < kNoBand;
+  FK_REQUIRE(!banded || qid != nullptr, "fk_attn_forward_kv_band_tc: a band needs labels");
   FK_REQUIRE((Sk + kFwdTileK - 1) / kFwdTileK <= kMaxTiles && Sk < (1 << 20) && Sq < (1 << 20),
              "fk_attn_forward_kv_tc: sequence too long");
   FK_REQUIRE(q_bs % 8 == 0 && q_ts % 8 == 0 && k_bs % 8 == 0 && k_ts % 8 == 0 && v_bs % 8 == 0 && v_ts % 8 == 0 &&
@@ -2332,7 +2360,9 @@ FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, vo
              o_ts >= H * head_dim, "fk_attn_forward_kv_tc: strides must cover a token's heads and keep 16-byte alignment");
   const int n_k_tiles = (Sk + kFwdTileK - 1) / kFwdTileK;
   FK_REQUIRE(n_chunks >= 1 && n_chunks <= n_k_tiles, "fk_attn_forward_kv_tc: n_chunks must be in [1, key tiles of 128]");
-  FK_REQUIRE(n_chunks == 1 || (part_o && part_ml), "fk_attn_forward_kv_tc: part_o / part_ml are needed with more than one chunk");
+  const bool split = n_chunks > 1 || banded;
+  FK_REQUIRE(!split || (part_o && part_ml),
+             "fk_attn_forward_kv_tc: part_o / part_ml are needed with more than one chunk or with a band");
   const long long n_units = static_cast<long long>((Sq + 255) / 256) * n_chunks;
   FK_REQUIRE(n_units * H * B < (1ll << 31), "fk_attn_forward_kv_tc: too many work items");
   FwdKvParams p = {};
@@ -2341,12 +2371,13 @@ FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, vo
   p.B = B; p.H = H; p.Sq = Sq; p.Sk = Sk; p.scale_log2 = scale * 1.4426950408889634f;
   p.items = counters;
   p.part_o = part_o; p.part_ml = part_ml; p.n_chunks = n_chunks; p.chunk_tiles = (n_k_tiles + n_chunks - 1) / n_chunks;
+  p.band = banded ? band : kNoBand;
   const long long n_items = n_units * H * B;
   const unsigned grid = static_cast<unsigned>(n_items < bwd_sm_count() ? n_items : bwd_sm_count());
-  const int rc = attn_fwd_launch(head_dim, q, k, v, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, p, grid, stream);
+  const int rc = attn_fwd_launch(head_dim, q, k, v, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, p, split, grid, stream);
   if (rc != FK_OK) return rc;
-  if (n_chunks == 1) {
-    // one chunk: the unsplit kernels write O / l and lse themselves
+  if (!split) {
+    // one chunk and no band: the unsplit kernels write O / l and lse themselves
     fk_count_launch();
     return FK_OK;
   }
@@ -2358,4 +2389,15 @@ FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, vo
   FK_CHECK_LAUNCH();
   fk_count_launch(2);
   return FK_OK;
+}
+
+FK_API int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq,
+                                 int Sk, int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts,
+                                 long long v_bs, long long v_ts, long long o_bs, long long o_ts, const int* qid,
+                                 const int* kid, const int* qmin, const int* qmax, const int* kmin, const int* kmax,
+                                 float scale, float* part_o, float* part_ml, int n_chunks, unsigned int* counters,
+                                 void* stream_) {
+  return fk_attn_forward_kv_band_tc(q, k, v, out, lse, B, H, Sq, Sk, head_dim, q_bs, q_ts, k_bs, k_ts, v_bs, v_ts, o_bs, o_ts,
+                                    qid, kid, qmin, qmax, kmin, kmax, scale, part_o, part_ml, n_chunks, kNoBand, counters,
+                                    stream_);
 }

@@ -221,10 +221,14 @@ def swiglu(h13):
 # mask labels and RoPE description
 # ------------------------------------------------------------------------------------------------
 class LabelMask:
-    """key j visible to query i  <=>  kid[b, j] <= qid[b, i].  Holds the per-tile label ranges, computed once
-    and shared by every layer of a forward pass."""
+    """key j visible to query i  <=>  kid[b, j] <= qid[b, i] (and, with a band, qid[b, i] - kid[b, j] < band).  Holds the
+    per-tile label ranges, computed once and shared by every layer of a forward pass.
 
-    def __init__(self, qid: torch.Tensor, kid: Optional[torch.Tensor] = None):
+    band: optional int >= 1, a sliding window over labels (a query sees the keys of its own label and of the band - 1 labels
+    before it).  Only `attention_kv` takes a banded mask; None is no band."""
+
+    def __init__(self, qid: torch.Tensor, kid: Optional[torch.Tensor] = None, band: Optional[int] = None):
+        self.band = _check_band(band)
         require_cuda(qid)
         self.qid = qid.to(torch.int32).contiguous()
         self.kid = self.qid if kid is None else kid.to(torch.int32).contiguous()
@@ -246,10 +250,11 @@ class LabelMask:
         return lo, hi
 
     @staticmethod
-    def from_ranges(qid, kid, qmin, qmax, kmin, kmax) -> "LabelMask":
+    def from_ranges(qid, kid, qmin, qmax, kmin, kmax, band: Optional[int] = None) -> "LabelMask":
         """labels whose per-tile ranges are already known (fk_stream_positions writes them with the labels)."""
         m = LabelMask.__new__(LabelMask)
         m.qid, m.kid, m.qmin, m.qmax, m.kmin, m.kmax, m._pairs = qid, kid, qmin, qmax, kmin, kmax, None
+        m.band = _check_band(band)
         return m
 
     @staticmethod
@@ -276,7 +281,27 @@ class LabelMask:
 
     def dense(self) -> torch.Tensor:
         """[B, 1, Sq, Sk] bool, True = attend (only for tests / the library-SDPA compatibility path)."""
-        return (self.kid[:, None, None, :] <= self.qid[:, None, :, None])
+        vis = self.kid[:, None, None, :] <= self.qid[:, None, :, None]
+        if self.band is not None:
+            vis &= (self.qid.long()[:, None, :, None] - self.kid.long()[:, None, None, :]) < self.band
+        return vis
+
+
+def _check_band(band) -> Optional[int]:
+    if band is None:
+        return None
+    try:
+        band = operator.index(band)
+    except TypeError:
+        raise FkError(f"LabelMask: band must be an int >= 1 or None, got {band!r}") from None
+    if band < 1:
+        raise FkError(f"LabelMask: band must be >= 1, got {band}")
+    return band
+
+
+def _no_band(mask, what: str) -> None:
+    if mask is not None and mask.band is not None:
+        raise FkError(f"{what}: a banded LabelMask is taken by attention_kv only (no training or backward path has a band)")
 
 
 # query label of a streamed slot past its row's count (fk_stream_positions_counts): no key label (>= 0) satisfies it
@@ -330,6 +355,37 @@ def stream_positions(len_in: torch.Tensor, len_out: torch.Tensor, n_new: int, to
     check(lib().fk_stream_positions_counts(ptr(len_in), ptr(counts), ptr(len_out), B, n_new, tokens_per_label, cap, ptr(qid),
                                            ptr(qmin), ptr(qmax), ptr(pos), ptr(rows), stream()), "fk_stream_positions")
     return qid, qmin, qmax, pos, rows
+
+
+@on_tensor_device
+def stream_ring_positions(len_in: torch.Tensor, len_out: torch.Tensor, n_new: int, tokens_per_label: int, cap: int,
+                          keys: LabelMask, inv_freq: torch.Tensor, counts: Optional[torch.Tensor] = None):
+    """One launch for the per-row bookkeeping of a sliding streaming step over ring caches of `cap` tokens per row: row b
+    holds len_in[b] tokens (device int64 [B], unbounded) and appends its new slots i < counts[b] (all n_new without counts)
+    at positions p = len_in[b] + i.  Returns (qid [B, n_new] = p // tokens_per_label (NO_LABEL past a count), qmin, qmax its
+    tile ranges, rows int64 [B * n_new] = b * cap + p mod cap (B * cap past a count), rope fp32 [B * n_new, hd/2, 2] the
+    (cos, sin) of p * inv_freq computed in fp64), writes the key label p // tokens_per_label into ring slot p mod cap of
+    keys.kid [B, cap] with the tile ranges keys.kmin / kmax of the tiles it wrote, and len_out = len_in + counts."""
+    require_cuda(len_in, len_out, counts, inv_freq)
+    B = len_in.shape[0]
+    for t, shape, dt in ((len_in, (B,), torch.int64), (len_out, (B,), torch.int64), (counts, (B,), torch.int32),
+                         (keys.kid, (B, cap), torch.int32)):
+        if t is not None and (t.dtype != dt or t.shape != shape or not t.is_contiguous()):
+            raise FkError(f"stream_ring_positions: expected a contiguous {dt} {shape} tensor, got {t.dtype} {tuple(t.shape)}")
+    if inv_freq.dtype != torch.float32 or inv_freq.dim() != 1 or not inv_freq.is_contiguous():
+        raise FkError("stream_ring_positions: inv_freq must be a contiguous fp32 vector")
+    half = inv_freq.shape[0]
+    dev = len_in.device
+    qid = torch.empty(B, n_new, device=dev, dtype=torch.int32)
+    nt = (n_new + 63) // 64
+    qmin = torch.empty(B, nt, device=dev, dtype=torch.int32)
+    qmax = torch.empty(B, nt, device=dev, dtype=torch.int32)
+    rows = torch.empty(B * n_new, device=dev, dtype=torch.int64)
+    rope = torch.empty(B * n_new, half, 2, device=dev, dtype=torch.float32)
+    check(lib().fk_stream_ring_positions(ptr(len_in), ptr(counts), ptr(len_out), B, n_new, tokens_per_label, cap, ptr(qid),
+                                         ptr(qmin), ptr(qmax), ptr(rows), ptr(keys.kid), ptr(keys.kmin), ptr(keys.kmax),
+                                         ptr(inv_freq), half, ptr(rope), stream()), "fk_stream_ring_positions")
+    return qid, qmin, qmax, rows, rope
 
 
 def stream_counts(counts, batch_size: int, limit: int, unit: int, what: str) -> list:
@@ -390,6 +446,7 @@ class _AttnQKVFn(torch.autograd.Function):
         projection's epilogue already did it (rope_applied: the backward still rotates dq / dk back)."""
         require_cuda(qkv)
         require_device()
+        _no_band(mask, "attention_qkv")        # (so its backward never sees a band either)
         if qkv.dtype != torch.bfloat16 or not qkv.is_contiguous():
             raise FkError("attention expects a contiguous bf16 QKV buffer")
         B, S, W = qkv.shape
@@ -545,8 +602,9 @@ def attention_kv(q, k, v, n_heads: int, mask: Optional[LabelMask] = None, scale:
     """Inference-only softmax(q k^T * scale + mask) v with queries and keys of different lengths (a streaming step's new
     tokens against a key / value cache): q [B, Sq, H*hd], k / v [B, Sk, H*hd] bf16 views with any 16-byte aligned batch and
     token strides (read in place, never copied) -> [B, Sq, H*hd] bf16.  head_dim 16, 32 or 64.  mask: LabelMask(qid [B, Sq],
-    kid [B, Sk]), key j visible to query i iff kid[b, j] <= qid[b, i]; a query that sees no key gives a zero row.
-    The key axis is split into chunks whose partial results are merged in chunk order (bit-reproducible)."""
+    kid [B, Sk]), key j visible to query i iff kid[b, j] <= qid[b, i] (and qid[b, i] - kid[b, j] < mask.band with a band);
+    a query that sees no key gives a zero row.  The key axis is split into chunks whose partial results are merged in chunk
+    order (bit-reproducible); a banded mask always takes that split path (fk_attn_forward_kv_band_tc)."""
     require_cuda(q, k, v)
     require_device()
     if torch.is_grad_enabled() and (q.requires_grad or k.requires_grad or v.requires_grad):
@@ -566,20 +624,26 @@ def attention_kv(q, k, v, n_heads: int, mask: Optional[LabelMask] = None, scale:
     q4, k4, v4 = _head_view(q, H, hd, "q"), _head_view(k, H, hd, "k"), _head_view(v, H, hd, "v")
     dev = q.device
     nch = lib().fk_attn_kv_chunks(B, H, Sq, Sk, 0)
+    band = None if mask is None else mask.band
     out = torch.empty(B, Sq, W, device=dev, dtype=torch.bfloat16)
     part_o = part_ml = None
-    if nch > 1:
+    if nch > 1 or band is not None:
         part_o = torch.empty(B, H, nch, Sq, hd, device=dev, dtype=torch.float32)
         part_ml = torch.empty(B, H, nch, Sq, 2, device=dev, dtype=torch.float32)
     m = mask
     margs = (ptr(m.qid) if m else 0, ptr(m.kid) if m else 0, ptr(m.qmin) if m else 0, ptr(m.qmax) if m else 0,
              ptr(m.kmin) if m else 0, ptr(m.kmax) if m else 0)
     scale = float(hd ** -0.5 if scale is None else scale)
+    strides = (q4.stride(0), q4.stride(1), k4.stride(0), k4.stride(1), v4.stride(0), v4.stride(1), out.stride(0), out.stride(1))
     with timed("attn_fwd_kv", 4.0 * B * H * Sq * Sk * hd):
-        check(lib().fk_attn_forward_kv_tc(ptr(q4), ptr(k4), ptr(v4), ptr(out), None, B, H, Sq, Sk, hd,
-                                          q4.stride(0), q4.stride(1), k4.stride(0), k4.stride(1), v4.stride(0), v4.stride(1),
-                                          out.stride(0), out.stride(1), *margs, scale, ptr(part_o), ptr(part_ml), nch,
-                                          counters(_lib.CTR_ATTN_FWD), stream()), "fk_attn_forward_kv_tc")
+        if band is None:
+            check(lib().fk_attn_forward_kv_tc(ptr(q4), ptr(k4), ptr(v4), ptr(out), None, B, H, Sq, Sk, hd, *strides, *margs,
+                                              scale, ptr(part_o), ptr(part_ml), nch, counters(_lib.CTR_ATTN_FWD), stream()),
+                  "fk_attn_forward_kv_tc")
+        else:
+            check(lib().fk_attn_forward_kv_band_tc(ptr(q4), ptr(k4), ptr(v4), ptr(out), None, B, H, Sq, Sk, hd, *strides,
+                                                   *margs, scale, ptr(part_o), ptr(part_ml), nch, band,
+                                                   counters(_lib.CTR_ATTN_FWD), stream()), "fk_attn_forward_kv_band_tc")
     return out
 
 

@@ -186,6 +186,19 @@ int fk_stream_positions(const int* len_in, int* len_out, int B, int n_new, int t
  * trial has n_new new tokens, which is fk_stream_positions. */
 int fk_stream_positions_counts(const int* len_in, const int* counts, int* len_out, int B, int n_new, int tokens_per_label,
                                int cap, int* qid, int* qmin, int* qmax, int* pos, long long* rows, void* stream);
+/* fk_stream_positions_counts for ring caches of cap tokens per trial (a sliding stream with no end): trial b holds len_in[b]
+ * tokens (int64 [B], unbounded) and its new slot i < c = counts[b] (nullable, clamped to [0, n_new]; NULL: n_new) is the
+ * token at p = len_in[b] + i.  One launch writes qid [B, n_new] = p / tokens_per_label with its per-64-token tile ranges
+ * qmin / qmax, rows int64 [B, n_new] = b * cap + p mod cap, the key label kid[b][p mod cap] = p / tokens_per_label of the
+ * ring kid int32 [B, cap], the key tile ranges kmin / kmax [B, ceil(cap / 64)] of every 64-slot tile it wrote (recomputed
+ * from the ring), the RoPE rows rope fp32 [B * n_new, half, 2] = (cos, sin)(p * inv_freq[j]) computed in fp64 and rounded
+ * (inv_freq fp32 [half]) and len_out[b] = len_in[b] + c.  A slot at or past c gets qid = INT_MIN (sees no key), the scratch
+ * row B * cap (the caller's cache holds B * cap + 1 rows) and the RoPE row of position 0.  The caller keeps
+ * p / tokens_per_label inside int32 and cap large enough that no slot a query still sees is overwritten.  B in [1, 65535],
+ * n_new in [1, cap], tokens_per_label >= 1, half >= 1; anything else is rejected before the launch. */
+int fk_stream_ring_positions(const long long* len_in, const int* counts, long long* len_out, int B, int n_new,
+                             int tokens_per_label, int cap, int* qid, int* qmin, int* qmax, long long* rows, int* kid,
+                             int* kmin, int* kmax, const float* inv_freq, int half, float* rope, void* stream);
 int fk_attn_forward(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq, int Sk,
                     int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts, long long v_bs,
                     long long v_ts, long long o_bs, long long o_ts, const int* qid, const int* kid, const int* qmin,
@@ -274,6 +287,18 @@ int fk_attn_forward_kv_tc(const void* q, const void* k, const void* v, void* out
                           long long v_ts, long long o_bs, long long o_ts, const int* qid, const int* kid, const int* qmin,
                           const int* qmax, const int* kmin, const int* kmax, float scale, float* part_o, float* part_ml,
                           int n_chunks, unsigned int* counters, void* stream);
+/* fk_attn_forward_kv_tc with a label band (a sliding window over labels): key j is visible to query i iff
+ * kid[b][j] <= qid[b][i] and qid[b][i] - kid[b][j] < band, the difference taken in 64 bits, so INT32_MIN and INT32_MAX stay
+ * valid labels.  band >= 1; a band of 2^32 or more lets every difference of two int32 labels through and is no band, which
+ * is fk_attn_forward_kv_tc bit for bit.  A narrower band needs labels and runs the split kernel even at n_chunks == 1, so
+ * part_o / part_ml are then required at every chunk count; the unsplit kernels never see a band.  band < 1 is rejected
+ * before anything is launched (counters untouched). */
+int fk_attn_forward_kv_band_tc(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int Sq,
+                               int Sk, int head_dim, long long q_bs, long long q_ts, long long k_bs, long long k_ts,
+                               long long v_bs, long long v_ts, long long o_bs, long long o_ts, const int* qid,
+                               const int* kid, const int* qmin, const int* qmax, const int* kmin, const int* kmax,
+                               float scale, float* part_o, float* part_ml, int n_chunks, long long band,
+                               unsigned int* counters, void* stream);
 
 /* Fused residual add + norm on the fp32 residual stream: x_out = x + delta (bf16), y = norm(x_out)
  * (the pair `x = x + branch(...)`; `ln(x)` of models/brainformer.py:243-244).  Backward: dx = norm_backward(g_y) + g_res
